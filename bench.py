@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — OH grid-cell predictions/sec of the B200 path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--grid 360]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--grid 360] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over the whole C<grid> x 72-level slab: the dense feature
 matrix X[N x 27] (resident in HBM) -> tree-ensemble prediction -> 10**x * OHscale -> OH_ML, i.e.
@@ -23,11 +23,15 @@ restatement, OpenMP over all host cores) on a bounded sample of the same workloa
 from __future__ import annotations
 
 import argparse
+import atexit
+import functools
 import json
 import os
+import shutil
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -40,19 +44,31 @@ KM = 72
 NFEAT = 27
 ALGO_BYTES_PER_CELL = NFEAT * 4 + 4  # SURVEY.md 8(d): 27 float32 in + 1 float32 out
 BOOSTER = dict(n_trees=100, max_depth=18)  # "Depth18_eta1_100Trees", OH_GridCompMod.F90:224
+DUMP_CELLS = 1 << 22  # --dump-outputs keeps at most this many cells (16 MB of float32)
 
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
 
 
+@functools.lru_cache(maxsize=None)
 def booster_path():
-    """Seeded prod-like booster (100 trees, depth <= 18, 27 features); grown once and cached."""
+    """Seeded prod-like booster (100 trees, depth <= 18, 27 features); grown once and cached under build/.  A
+    read-only checkout without it gets one grown into a temporary directory for this process."""
     from quickchem_b200 import synth, xgbmodel
 
     d = os.path.join(ROOT, "build")
-    os.makedirs(d, exist_ok=True)
-    p = os.path.join(d, f"oh_booster_{BOOSTER['n_trees']}x{BOOSTER['max_depth']}.model")
+    name = f"oh_booster_{BOOSTER['n_trees']}x{BOOSTER['max_depth']}.model"
+    if os.path.exists(os.path.join(d, name)):
+        return os.path.join(d, name)
+    try:
+        os.makedirs(d, exist_ok=True)
+    except OSError:
+        pass
+    if not os.access(d, os.W_OK):
+        d = tempfile.mkdtemp(prefix="qcoh_bench_")
+        atexit.register(shutil.rmtree, d, True)
+    p = os.path.join(d, name)
     if not os.path.exists(p):
         t0 = time.time()
         f = synth.prod_like_booster(**BOOSTER)
@@ -184,6 +200,30 @@ def workload_config(grid, world):
             "cache": "inputs (>= 0.75 GB per GPU) exceed the 126 MB L2; forest stays L2-resident by design"}  # fmt: skip
 
 
+def dump_outputs(out_dir, grid, col0, ncol, oh, rank, world, dist):
+    """--dump-outputs: this rank's OH values `oh` (the last timed step's result, rows k * ncol + local column) at a
+    fixed set of global cells, gathered on rank 0 into DIR/oh.npy in global cell order (k * 6 grid^2 + column), so
+    that two builds run with the same arguments can be compared value for value at any number of GPUs."""
+    ncol_g = 6 * grid * grid
+    n = ncol_g * KM
+    cells = np.arange(n) if n <= DUMP_CELLS else np.unique(np.random.default_rng(0).integers(0, n, DUMP_CELLS))
+    k, col = np.divmod(cells, ncol_g)
+    mine = (col >= col0) & (col < col0 + ncol)
+    part = (np.nonzero(mine)[0], oh[k[mine] * ncol + col[mine] - col0])
+    parts = [part]
+    if dist:
+        parts = [None] * world
+        dist.all_gather_object(parts, part)
+    if rank != 0:
+        return
+    sample = np.full(cells.size, np.nan, np.float32)
+    for pos, v in parts:
+        sample[pos] = v
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "oh.npy"), sample)
+    log(f"[bench] wrote {sample.size} of {n} OH values to {os.path.join(out_dir, 'oh.npy')}")
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -196,7 +236,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--param", action="append", default=[], help="name=value forwarded to qcoh_set_param")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the OH values of the last timed step to DIR/oh.npy (float32; every cell of a grid of "
+                         f"at most {DUMP_CELLS} cells, else a fixed seeded sample of about that many)")  # fmt: skip
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "qcoh":
+        ap.error("--dump-outputs writes the outputs of the qcoh path")
     args.warmup = max(args.warmup, 3) if args.impl == "qcoh" else args.warmup
 
     if args.impl == "reference":
@@ -314,9 +361,12 @@ def main():
 
     # ---- the result itself: a checksum of the OH bits that must not depend on the number of ranks (the fields are
     # a function of the global column only), and the raw margins for the bit-level parity check below
-    oh_bits = d_pred.get().view(np.uint32)
+    oh_host = d_pred.get()
+    oh_bits = oh_host.view(np.uint32)
     local_ck = [int(np.bitwise_xor.reduce(oh_bits)), int(oh_bits.sum(dtype=np.uint64)), int(oh_bits.size)]
-    del oh_bits
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, args.grid, col0, ncol, oh_host, rank, world, dist)
+    del oh_bits, oh_host
     all_ck = [local_ck]
     if dist:
         all_ck = [None] * world

@@ -2,9 +2,12 @@
 oracle/qc_oracle.h).  Builds the library with oracle/Makefile on first use if it is missing."""
 from __future__ import annotations
 
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -84,8 +87,9 @@ def build_flags() -> str:
 
 
 def build(force=False):
-    """Compile the C restatement (-O3 -march=native).  The built library travels to the GPU box with the repo
-    snapshot; it is rebuilt there if that box's CPU is not the one it was built for."""
+    """Compile the C restatement (-O3 -march=native) next to its source, and rebuild it if the host's CPU is not
+    the one it was built for (oracle/.cpu_stamp).  In a read-only checkout a library that has to be (re)built is
+    built into a temporary directory for this process instead."""
     so = os.path.join(_HERE, "libqc_oracle.so")
     src = os.path.join(_HERE, "qc_oracle.c")
     stamp = os.path.join(_HERE, ".cpu_stamp")
@@ -97,9 +101,15 @@ def build(force=False):
     stale = not os.path.exists(so) or any(os.path.exists(f) and os.path.getmtime(f) > os.path.getmtime(so)
                                           for f in (src, os.path.join(_HERE, "Makefile")))  # fmt: skip
     if force or stale or built_for != cpu:
-        subprocess.check_call(["make", "-C", _HERE, "-B", "libqc_oracle.so"], stdout=subprocess.DEVNULL)
-        with open(stamp, "w") as f:
-            f.write(cpu)
+        writable = os.access(_HERE, os.W_OK) and (not os.path.exists(so) or os.access(so, os.W_OK))
+        if not writable:
+            tmp = tempfile.mkdtemp(prefix="qc_oracle_")
+            atexit.register(shutil.rmtree, tmp, True)
+            so = os.path.join(tmp, "libqc_oracle.so")
+        subprocess.check_call(["make", "-C", _HERE, "-B", "OUT=" + so], stdout=subprocess.DEVNULL)
+        if writable:
+            with open(stamp, "w") as f:
+                f.write(cpu)
     return so
 
 
