@@ -136,6 +136,21 @@ module qcoh_fortran_api
        import :: c_int
      end function
 
+     ! libxgboost 1.6.0's JSON-configured predict; config = '{"type": 2, "training": false, "iteration_begin": 0, '//
+     ! '"iteration_end": 0, "strict_shape": false}'//c_null_char gives per-feature contributions (type 3: approximate).
+     ! out_shape / out_result point at booster-owned buffers (c_f_pointer them; valid until the next predict / free):
+     ! contributions are row-major [nrow][num_feature + 1], the last column the bias, i.e. shape (num_feature + 1, nrow)
+     ! in Fortran order.
+     integer(c_int) function XGBoosterPredictFromDMatrix(handle, dmat, config, out_shape, out_dim, out_result) &
+          bind(C, name="XGBoosterPredictFromDMatrix")
+       import :: c_int, c_ptr, c_char, c_int64_t
+       type(c_ptr), value :: handle, dmat
+       character(len=1, kind=c_char), dimension(*) :: config
+       type(c_ptr) :: out_shape      ! const bst_ulong**
+       integer(c_int64_t) :: out_dim ! bst_ulong*
+       type(c_ptr) :: out_result     ! const float**
+     end function
+
      function XGBGetLastError_c() bind(C, name="XGBGetLastError") result(msg)
        import :: c_ptr
        type(c_ptr) :: msg

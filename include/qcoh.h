@@ -64,6 +64,17 @@ int XGDMatrixCreateFromFile(const char *fname, int silent, DMatrixHandle *out);
 int XGBoosterPredict(BoosterHandle handle, DMatrixHandle dmat, int option_mask, unsigned ntree_limit,
                      int training, bst_ulong *out_len, const float **out_result);
 
+/* libxgboost 1.6.0's JSON-configured predict (not bound by xgb_fortran_api; fortran/qcoh_fortran_api.F90 binds
+ * it).  config: {"type", "training", "iteration_begin", "iteration_end", "strict_shape"}, all required.  type 0 value,
+ * 1 margin, 6 leaf index (the kernels of XGBoosterPredict), 2 exact per-feature contributions (TreeSHAP), 3
+ * approximate contributions (Saabas); 4 / 5 (interactions) fail.  iteration_end = 0: all trees; iteration_begin
+ * must be 0.  Shapes: value / margin (nrow), leaf (nrow, ntree), contributions (nrow, num_feature + 1) — the last
+ * column is the bias; strict_shape: (nrow, 1), (nrow, ntree, 1, 1), (nrow, 1, num_feature + 1).  *out_shape and
+ * *out_result are booster-owned (pinned), valid until the next predict / free on that booster.  Contributions
+ * need the node covers (sum_hess > 0 everywhere) and fail on a booster without them. */
+int XGBoosterPredictFromDMatrix(BoosterHandle handle, DMatrixHandle dmat, const char *config,
+                                const bst_ulong **out_shape, bst_ulong *out_dim, const float **out_result);
+
 /* xgb_fortran_api.F90:75-83; call site OH_GridCompMod.F90:256.  The reference passes a DMatrix
  * handle *by value* as `dmats` with len = 0; dmats is never dereferenced when len == 0. */
 int XGBoosterCreate(const DMatrixHandle dmats[], bst_ulong len, BoosterHandle *out);
@@ -138,6 +149,16 @@ int qcoh_booster_get_duo(BoosterHandle handle, const uint32_t **rec, const uint3
                          int64_t *num_slots);
 int qcoh_booster_get_duo_info(BoosterHandle handle, int *blk_shift, int *has_default_bits);
 
+/* Contribution tables (DESIGN.md "Contributions"), for inspection/tests; built on first use.  bins[num_bins][32][4]:
+ * every root-to-leaf path as a group of consecutive lanes of one 32-lane bin, a bias lane {0, ~0, 0xFF | 1 << 8 |
+ * start << 16 | len << 24, leaf value bits} then one lane per distinct feature of the path {lo_key, hi_key,
+ * feat | missing_goes_here << 8 | start << 16 | len << 24, zero fraction bits}: a present value with order-preserving
+ * key k follows the path iff lo_key <= k < hi_key.  tree_bin[num_trees + 1]: tree t owns bins [tree_bin[t],
+ * tree_bin[t+1]).  node_mean[num_nodes]: libxgboost's node mean values by flat node index.  Fails when the booster
+ * has no covers. */
+int qcoh_booster_get_shap_paths(BoosterHandle handle, const uint32_t **bins, const int64_t **tree_bin,
+                                const float **node_mean, int64_t *num_bins);
+
 /* ---- device-resident predict -------------------------------------------------------- */
 /* A DMatrix whose storage is allocated in HBM and filled by the caller (device pointer
  * returned by qcoh_dmatrix_device_ptr) or by qcoh_dmatrix_upload.  Call qcoh_dmatrix_seal
@@ -161,13 +182,19 @@ typedef struct {
  * epi may be NULL.  Asynchronous on the library stream; qcoh_device_synchronize() to wait. */
 int qcoh_booster_predict_device(BoosterHandle handle, DMatrixHandle dmat, int option_mask,
                                 unsigned ntree_limit, const qcoh_epilogue *epi, float *out_dev);
+/* Per-feature contributions into a DEVICE buffer of nrow * (num_feature + 1) floats, row-major, last column the
+ * bias (XGBoosterPredictFromDMatrix type 2, or type 3 when approximate != 0; ntree_limit 0 = all trees).
+ * Asynchronous on the library stream; qcoh_device_synchronize() to wait. */
+int qcoh_booster_predict_contribs_device(BoosterHandle handle, DMatrixHandle dmat, int approximate,
+                                         unsigned ntree_limit, float *out_dev);
 /* Kernel variant selection for experiments / profiling (0 = default).  See DESIGN.md. */
 int qcoh_set_param(const char *name, const char *value);
 /* How many kernels the library has launched since load (for bench.py's gpu_launches). */
 uint64_t qcoh_launch_count(void);
 /* Which kernel family served a prediction — what the parity tests assert.  Families: "duo" (two-level records),
  * "nodes8" (8-byte depth-ordered nodes), each with the suffixes "_missing" (matrix with missing entries) and
- * "_leaf" (option_mask = 2), e.g. "duo_missing_leaf"; "soa_duo" / "soa_nodes8" (fused Run1); "seal_tiles".
+ * "_leaf" (option_mask = 2), e.g. "duo_missing_leaf"; "soa_duo" / "soa_nodes8" (fused Run1); "seal_tiles";
+ * "shap" (exact contributions) with its slice reduction "shap_reduce", and "shap_approx" (approximate contributions).
  * qcoh_kernel_launches counts launches of one family since load; qcoh_last_predict_kernel names the family of the
  * last XGBoosterPredict-side launch ("" before the first). */
 uint64_t qcoh_kernel_launches(const char *family);

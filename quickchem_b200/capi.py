@@ -63,12 +63,12 @@ class Run1Out(C.Structure):
 # every symbol include/qcoh.h declares (tests check the library exports all of them)
 XGB_SYMBOLS = ("XGBoosterLoadModel", "XGBoosterSaveModel", "XGDMatrixSaveBinary", "XGDMatrixFree",
                "XGDMatrixCreateFromFile", "XGBoosterPredict", "XGBoosterCreate", "XGDMatrixCreateFromMat",
-               "XGDMatrixNumRow", "XGDMatrixNumCol", "XGBoosterFree", "XGBGetLastError")  # fmt: skip
+               "XGDMatrixNumRow", "XGDMatrixNumCol", "XGBoosterFree", "XGBGetLastError", "XGBoosterPredictFromDMatrix")  # fmt: skip
 QCOH_SYMBOLS = ("qcoh_version", "qcoh_device_count", "qcoh_set_device", "qcoh_host_alloc", "qcoh_host_free",
                 "qcoh_device_alloc", "qcoh_device_free", "qcoh_memcpy_h2d", "qcoh_memcpy_d2h",
                 "qcoh_device_synchronize", "qcoh_timer_start", "qcoh_timer_stop", "qcoh_flush_l2",
                 "qcoh_booster_parse", "qcoh_booster_get_info", "qcoh_booster_get_flat", "qcoh_booster_get_duo",
-                "qcoh_booster_get_duo_info",
+                "qcoh_booster_get_duo_info", "qcoh_booster_get_shap_paths", "qcoh_booster_predict_contribs_device",
                 "qcoh_dmatrix_create_device", "qcoh_dmatrix_device_ptr", "qcoh_dmatrix_upload", "qcoh_dmatrix_seal",
                 "qcoh_booster_predict_device", "qcoh_set_param", "qcoh_launch_count", "qcoh_kernel_launches",
                 "qcoh_last_predict_kernel", "qcoh_dmatrix_tiles_ptr", "qcoh_oh_invalidate_sza", "qcoh_oh_create",
@@ -129,6 +129,11 @@ def lib():
         L.qcoh_dmatrix_upload.argtypes = [vp, vp, u64, u64]
         L.qcoh_dmatrix_seal.argtypes = [vp]
         L.qcoh_booster_predict_device.argtypes = [vp, vp, C.c_int, C.c_uint, C.POINTER(Epilogue), vp]
+        L.XGBoosterPredictFromDMatrix.argtypes = [vp, vp, C.c_char_p, C.POINTER(C.POINTER(u64)), C.POINTER(u64),
+                                                  C.POINTER(f32p)]  # fmt: skip
+        L.qcoh_booster_predict_contribs_device.argtypes = [vp, vp, C.c_int, C.c_uint, vp]
+        L.qcoh_booster_get_shap_paths.argtypes = [vp, C.POINTER(C.POINTER(C.c_uint32)), C.POINTER(C.POINTER(C.c_int64)),
+                                                  C.POINTER(C.POINTER(C.c_float)), C.POINTER(C.c_int64)]  # fmt: skip
         L.qcoh_set_param.argtypes = [C.c_char_p, C.c_char_p]
         L.qcoh_oh_create.argtypes = [vp, C.POINTER(OhConfig), C.POINTER(vp)]
         L.qcoh_oh_run1.argtypes = [vp, C.POINTER(Run1In), C.POINTER(Run1Out)]
@@ -408,6 +413,42 @@ class Booster:
     def predict_device(self, dmat: DMatrix, out: DeviceArray, option_mask=0, ntree_limit=0, exp10=False, scale=1.0):
         epi = Epilogue(int(exp10), float(scale))
         check(lib().qcoh_booster_predict_device(self.handle, dmat.handle, option_mask, ntree_limit, C.byref(epi), out.ptr))
+
+    def predict_from_dmatrix(self, dmat: DMatrix, config) -> np.ndarray:
+        """XGBoosterPredictFromDMatrix(handle, dmat, config, shape, dim, result): `config` is a dict or a JSON string
+        (type, training, iteration_begin, iteration_end, strict_shape).  Returns a copy shaped as the library says."""
+        import json
+
+        cfg = config if isinstance(config, str) else json.dumps(config)
+        shp, dim, p = C.POINTER(u64)(), u64(), f32p()
+        check(lib().XGBoosterPredictFromDMatrix(self.handle, None if dmat is None else dmat.handle, cfg.encode(), C.byref(shp), C.byref(dim), C.byref(p)))
+        shape = tuple(int(shp[i]) for i in range(dim.value))
+        n = int(np.prod(shape)) if shape else 0
+        out = np.ctypeslib.as_array(p, (n,)).copy() if n else np.zeros(0, np.float32)
+        return out.reshape(shape)
+
+    def predict_contribs(self, dmat: DMatrix, approximate=False, ntree_limit=0) -> np.ndarray:
+        """[nrow, num_feature + 1] per-feature contributions, last column the bias: exact TreeSHAP, or Saabas when
+        `approximate` (XGBoosterPredictFromDMatrix type 2 / 3, iteration_end = ntree_limit)."""
+        cfg = {"type": 3 if approximate else 2, "training": False, "iteration_begin": 0,
+               "iteration_end": int(ntree_limit), "strict_shape": False}  # fmt: skip
+        return self.predict_from_dmatrix(dmat, cfg)
+
+    def predict_contribs_device(self, dmat: DMatrix, out: DeviceArray, approximate=False, ntree_limit=0):
+        """qcoh_booster_predict_contribs_device: the same into a device buffer of nrow * (num_feature + 1) floats,
+        asynchronous on the library stream."""
+        check(lib().qcoh_booster_predict_contribs_device(self.handle, dmat.handle, int(approximate), ntree_limit, out.ptr))
+
+    def shap_paths(self):
+        """(bins[nbins,32,4] uint32, tree_bin[T+1] int64, node_mean[num_nodes] float32) copies of the contribution
+        tables (host only; raises when the booster has no covers)."""
+        pb, pt, pm, nb = C.POINTER(C.c_uint32)(), C.POINTER(C.c_int64)(), C.POINTER(C.c_float)(), C.c_int64()
+        check(lib().qcoh_booster_get_shap_paths(self.handle, C.byref(pb), C.byref(pt), C.byref(pm), C.byref(nb)))
+        i = self.info()
+        bins = np.ctypeslib.as_array(pb, (nb.value * 128,)).reshape(nb.value, 32, 4).copy() if nb.value else np.zeros((0, 32, 4), np.uint32)
+        tree_bin = np.ctypeslib.as_array(pt, (i.num_trees + 1,)).copy()
+        mean = np.ctypeslib.as_array(pm, (i.num_nodes,)).copy() if i.num_nodes else np.zeros(0, np.float32)
+        return bins, tree_bin, mean
 
     @classmethod
     def cached(cls, model_file):

@@ -212,6 +212,49 @@ static void predict_into(Booster *b, DMatrix *d, int option_mask, unsigned ntree
   launch_predict_chunked(b, a, true, g.stream);
 }
 
+const ShapForest &shap_tables(Booster *b) {
+  if (!b->loaded) throw Error("Booster has no model: call XGBoosterLoadModel first");
+  if (!b->shap.ok) b->shap = build_shap(b->host, b->flat);
+  return b->shap;
+}
+
+// Per-feature contributions into a device buffer [nrow][num_feature + 1], asynchronous on the library stream.  The
+// path bins and node means go to HBM at the first call (not at load: prediction alone never needs them).
+static void contribs_into(Booster *b, DMatrix *d, bool approximate, unsigned ntree_limit, float *out_dev) {
+  const ShapForest &s = shap_tables(b);
+  upload(b);
+  if (!d->sealed) seal(d);
+  const uint32_t nf = b->host.num_feature;
+  if (d->ncol > nf)
+    throw Error("Check failed: Number of columns does not match number of features in booster. Columns: " +
+                std::to_string(d->ncol) + " Features: " + std::to_string(nf));
+  if (!b->shap_uploaded) {
+    const size_t nb = (size_t)s.num_bins(), nn = s.mean.size();
+    CU(cudaMemcpy(b->d_shap_bins.need(nb * 32), s.bins.data(), nb * 32 * sizeof(uint4), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(b->d_shap_mean.need(nn), s.mean.data(), nn * sizeof(float), cudaMemcpyHostToDevice));
+    b->shap_uploaded = true;
+  }
+  const int nt = (int)trees_used(b, ntree_limit);
+  ContribArgs a;
+  a.ncol = (int32_t)d->ncol, a.nfeat = (int32_t)nf;
+  a.bias = shap_bias(s, b->host, b->flat, nt);
+  if (approximate) {
+    a.Xt = d->Xt.p, a.nrow = d->nrow, a.out = out_dev;
+    CU(launch_shap_approx(b->dev, b->d_shap_mean.p, nt, a, g.stream));
+    return;
+  }
+  const int64_t nb = s.tree_bin[(size_t)nt];
+  const int ns = (int)std::min<int64_t>(kShapSlices, nb);
+  double *part = b->d_shap_part.need((size_t)ns * (size_t)std::min<uint64_t>(kShapChunkRows, d->nrow) * nf);
+  for (uint64_t r0 = 0; r0 < d->nrow; r0 += kShapChunkRows) {
+    ContribArgs c = a;
+    c.Xt = d->Xt.p + tile_offset_words(r0, d->ncol), c.nrow = std::min<uint64_t>(kShapChunkRows, d->nrow - r0);
+    c.out = out_dev + r0 * (nf + 1);
+    CU(launch_shap(b->d_shap_bins.p, nb, ns, c, part, g.stream));
+    CU(launch_shap_reduce(part, ns, c, g.stream));
+  }
+}
+
 static cudaEvent_t chunk_event(size_t i) {
   while (g.chunk_events.size() <= i) {
     cudaEvent_t e;
@@ -505,6 +548,7 @@ int qcoh_booster_parse(BoosterHandle handle, const char *fname) {
   FlatForest ff = flatten(hf);
   DuoForest df = build_duo(ff, hf.num_feature);
   b->host = std::move(hf), b->flat = std::move(ff), b->duo = std::move(df);
+  b->shap = ShapForest(), b->shap_uploaded = false;
   b->loaded = true, b->uploaded = false;
   b->version = ++g_version_counter;
   API_END
@@ -610,6 +654,60 @@ int XGBoosterPredict(BoosterHandle handle, DMatrixHandle dmat, int option_mask, 
   CU(cudaMemcpyAsync(hv, dv, n * sizeof(float), cudaMemcpyDeviceToHost, g.stream));
   CU(cudaStreamSynchronize(g.stream));
   *out_len = n;
+  *out_result = hv;
+  API_END
+}
+
+// libxgboost 1.6.0's JSON-configured predict (src/c_api/c_api.cc).  Types 0 / 1 / 6 run the kernels of
+// XGBoosterPredict (option_mask 0 / 1 / 2); 2 and 3 are the per-feature contributions.
+int XGBoosterPredictFromDMatrix(BoosterHandle handle, DMatrixHandle dmat, const char *config, const bst_ulong **out_shape,
+                                bst_ulong *out_dim, const float **out_result) {
+  API_BEGIN
+  Booster *b = B(handle);
+  if (!out_shape || !out_dim || !out_result) throw Error("XGBoosterPredictFromDMatrix: NULL output argument");
+  if (!b->loaded) throw Error("Booster has no model: call XGBoosterLoadModel first");
+  const PredictConfig c = parse_predict_config(config);
+  const std::string ty = std::to_string(c.type);
+  if (c.type == 4 || c.type == 5)
+    throw Error("XGBoosterPredictFromDMatrix: type " + ty + " (SHAP interaction values) is not supported; 2 and 3 give per-feature contributions");
+  const bool contribs = c.type == 2 || c.type == 3;
+  if (!contribs && c.type != 0 && c.type != 1 && c.type != 6)
+    throw Error("XGBoosterPredictFromDMatrix: unknown prediction type " + ty + " (0 value, 1 margin, 2 / 3 contributions, 6 leaf)");
+  if (c.iteration_begin < 0 || c.iteration_end < 0) throw Error("XGBoosterPredictFromDMatrix: negative iteration range");
+  if (contribs && c.iteration_begin != 0)
+    throw Error("XGBoosterPredictFromDMatrix: contributions support only iteration_begin = 0 (predict from iteration 0 to "
+                "iteration_end; slice the model instead)");
+  if (c.iteration_begin != 0)
+    throw Error("XGBoosterPredictFromDMatrix: iteration_begin = " + std::to_string(c.iteration_begin) + " is not supported (only 0)");
+  if (contribs) (void)shap_tables(b);  // a booster without covers fails here, before any device work
+  ensure_device();
+  DMatrix *d = D(dmat);
+  const unsigned limit = (unsigned)std::min<int64_t>(c.iteration_end, (int64_t)UINT32_MAX);
+  const bst_ulong nrow = d->nrow, nt = trees_used(b, limit), nf = b->host.num_feature;
+  std::vector<bst_ulong> shape;
+  size_t n;
+  if (contribs) {
+    n = (size_t)nrow * (nf + 1);
+    shape = c.strict_shape ? std::vector<bst_ulong>{nrow, 1, nf + 1} : std::vector<bst_ulong>{nrow, nf + 1};
+  } else if (c.type == 6) {
+    n = (size_t)nrow * nt;
+    shape = c.strict_shape ? std::vector<bst_ulong>{nrow, nt, 1, 1} : std::vector<bst_ulong>{nrow, nt};
+  } else {
+    n = (size_t)nrow;
+    shape = c.strict_shape ? std::vector<bst_ulong>{nrow, 1} : std::vector<bst_ulong>{nrow};
+  }
+  g_last_booster = b;
+  float *dv = b->d_result.need(n);
+  float *hv = b->h_result.need(n);
+  if (contribs)
+    contribs_into(b, d, c.type == 3, limit, dv);
+  else
+    predict_into(b, d, c.type == 6 ? 2 : c.type, limit, nullptr, dv);
+  CU(cudaMemcpyAsync(hv, dv, n * sizeof(float), cudaMemcpyDeviceToHost, g.stream));
+  CU(cudaStreamSynchronize(g.stream));
+  b->h_shape = std::move(shape);
+  *out_shape = b->h_shape.data();
+  *out_dim = (bst_ulong)b->h_shape.size();
   *out_result = hv;
   API_END
 }
@@ -954,6 +1052,24 @@ int qcoh_booster_predict_device(BoosterHandle handle, DMatrixHandle dmat, int op
                                 const qcoh_epilogue *epi, float *out_dev) {
   API_BEGIN
   predict_into(B(handle), D(dmat), option_mask, ntree_limit, epi, out_dev);
+  API_END
+}
+
+int qcoh_booster_predict_contribs_device(BoosterHandle handle, DMatrixHandle dmat, int approximate, unsigned ntree_limit,
+                                         float *out_dev) {
+  API_BEGIN
+  contribs_into(B(handle), D(dmat), approximate != 0, ntree_limit, out_dev);
+  API_END
+}
+
+int qcoh_booster_get_shap_paths(BoosterHandle handle, const uint32_t **bins, const int64_t **tree_bin, const float **node_mean,
+                                int64_t *num_bins) {
+  API_BEGIN
+  const ShapForest &s = shap_tables(B(handle));
+  if (bins) *bins = s.bins.data();
+  if (tree_bin) *tree_bin = s.tree_bin.data();
+  if (node_mean) *node_mean = s.mean.data();
+  if (num_bins) *num_bins = s.num_bins();
   API_END
 }
 

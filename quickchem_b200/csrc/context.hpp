@@ -223,6 +223,13 @@ struct Booster {
   DevBuf<int32_t> d_depth, d_orig;
   DevBuf<float> d_result;
   PinBuf<float> h_result;
+  std::vector<bst_ulong> h_shape;  // XGBoosterPredictFromDMatrix's out_shape
+  // contributions (forest.hpp ShapForest): built on the host and uploaded at the first contributions call
+  ShapForest shap;
+  bool shap_uploaded = false;
+  DevBuf<uint4> d_shap_bins;
+  DevBuf<float> d_shap_mean;
+  DevBuf<double> d_shap_part;  // float64 partial sums of the bin slices, [kShapSlices][kShapChunkRows][nfeat]
   Booster() = default;
   Booster(const Booster &) = delete;
   Booster &operator=(const Booster &) = delete;
@@ -278,5 +285,7 @@ void upload(Booster *b);
 void sync_const_top(Booster *b, bool allow_duo, int tree0 = 0, int ntree = -1);
 // one prediction = one launch per range of kConstTreesMax trees (capi_xgb.cpp)
 void launch_predict_chunked(Booster *b, PredictArgs a, bool allow_duo, cudaStream_t s);
+// the booster's ShapForest, built on first use (host only; throws when the booster has no covers)
+const ShapForest &shap_tables(Booster *b);
 
 }  // namespace qcoh

@@ -8,6 +8,7 @@
 //   JSON / UBJSON: doc/model.schema; UBJSON is draft-12, big-endian, typed arrays
 #include "forest.hpp"
 
+#include <algorithm>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -870,6 +871,155 @@ DuoForest build_duo(const FlatForest &f, uint32_t num_feature) {
   if (build_duo_with(f, num_feature, 15, wide)) return wide;
   wide.rec.clear(), wide.tree_slot.clear(), wide.top_xy.clear();
   return wide;
+}
+
+// ---- contributions: node means and root-to-leaf paths ---------------------------------------------------
+namespace {
+// libxgboost 1.6.0 FillNodeMeanValue (src/predictor/cpu_predictor.cc), float32 in its order
+float fill_mean(const HostTree &t, int32_t n, std::vector<float> &mean) {
+  float r;
+  if (t.cleft[n] == -1) {
+    r = t.info[n];
+  } else {
+    r = fill_mean(t, t.cleft[n], mean) * t.sum_hess[t.cleft[n]];
+    r += fill_mean(t, t.cright[n], mean) * t.sum_hess[t.cright[n]];
+    r /= t.sum_hess[n];
+  }
+  mean[n] = r;
+  return r;
+}
+
+struct PathElem {
+  uint32_t feat, lo, hi, miss;
+  double zero;
+};
+
+uint32_t threshold_key(float thr) { return 0u - neg_threshold_key(thr); }
+
+void collect_paths(const HostTree &t, int32_t n, std::vector<PathElem> &path,
+                   std::vector<std::pair<std::vector<PathElem>, float>> &out) {
+  if (t.cleft[n] == -1) {
+    out.emplace_back(path, t.info[n]);
+    return;
+  }
+  const uint32_t f = t.sindex[n] & 0x7FFFFFFFu;
+  const bool dl = (t.sindex[n] >> 31) != 0;
+  const uint32_t k = threshold_key(t.info[n]);
+  for (int side = 0; side < 2; ++side) {
+    const int32_t c = side ? t.cright[n] : t.cleft[n];
+    std::vector<PathElem> p(path);
+    size_t i = 0;
+    while (i < p.size() && p[i].feat != f) ++i;
+    if (i == p.size()) p.push_back({f, 0u, 0xFFFFFFFFu, 1u, 1.0});
+    if (side) p[i].lo = std::max(p[i].lo, k);
+    else p[i].hi = std::min(p[i].hi, k);
+    p[i].miss &= (dl == (side == 0)) ? 1u : 0u;
+    p[i].zero *= (double)t.sum_hess[c] / (double)t.sum_hess[n];
+    collect_paths(t, c, p, out);
+  }
+}
+}  // namespace
+
+ShapForest build_shap(const HostForest &h, const FlatForest &f) {
+  ShapForest s;
+  s.mean.assign((size_t)f.num_nodes(), 0.f);
+  s.tree_bin.push_back(0);
+  for (size_t ti = 0; ti < h.trees.size(); ++ti) {
+    const HostTree &t = h.trees[ti];
+    for (int32_t n = 0; n < t.num_nodes(); ++n)
+      if (!std::isfinite(t.sum_hess[n]) || !(t.sum_hess[n] > 0.f))
+        fail("contributions need the node covers (sum_hess), but tree " + std::to_string(ti) + " node " + std::to_string(n) +
+             " has cover " + std::to_string(t.sum_hess[n]) +
+             ": this booster cannot be explained (a JSON model without sum_hessian, or trees converted without covers)");
+    std::vector<float> m((size_t)t.num_nodes());
+    fill_mean(t, 0, m);
+    const uint32_t n0 = f.tree_offset[ti];
+    for (uint32_t i = n0; i < f.tree_offset[ti + 1]; ++i) s.mean[i] = m[(size_t)f.orig_id[i]];
+    std::vector<std::pair<std::vector<PathElem>, float>> paths;
+    std::vector<PathElem> root;
+    collect_paths(t, 0, root, paths);
+    // first-fit decreasing into 32-lane bins; lengths include the bias element (<= kMaxFeatures + 1 = 32)
+    std::vector<size_t> order(paths.size());
+    for (size_t i = 0; i < order.size(); ++i) order[i] = i;
+    std::stable_sort(order.begin(), order.end(), [&](size_t a, size_t b) { return paths[a].first.size() > paths[b].first.size(); });
+    std::vector<int> fill;                      // lanes used per bin of this tree
+    std::vector<std::vector<size_t>> members;   // paths per bin, in placement order
+    std::map<int, std::vector<size_t>> by_free;  // free lanes -> bins with that many free lanes (ascending index)
+    for (size_t pi : order) {
+      const int len = (int)paths[pi].first.size() + 1;
+      size_t bin = fill.size();
+      int have = -1;
+      for (auto it = by_free.lower_bound(len); it != by_free.end(); ++it)
+        if (!it->second.empty() && it->second.front() < bin) bin = it->second.front(), have = it->first;
+      if (have < 0) {
+        fill.push_back(0), members.emplace_back();
+      } else {
+        auto &v = by_free[have];
+        v.erase(v.begin());
+      }
+      fill[bin] += len;
+      members[bin].push_back(pi);
+      auto &v = by_free[32 - fill[bin]];
+      v.insert(std::lower_bound(v.begin(), v.end(), bin), bin);
+      s.max_path_len = std::max(s.max_path_len, len);
+      s.num_paths += 1, s.num_elements += len;
+    }
+    for (size_t b = 0; b < members.size(); ++b) {
+      uint32_t w[32][4];
+      for (uint32_t l = 0; l < 32; ++l) w[l][0] = 0u, w[l][1] = 0xFFFFFFFFu, w[l][2] = kShapNoFeature | (l << 16), w[l][3] = 0u;
+      uint32_t lane = 0;
+      for (size_t pi : members[b]) {
+        const auto &p = paths[pi];
+        const uint32_t g0 = lane, len = (uint32_t)p.first.size() + 1;
+        const uint32_t grp = (g0 << 16) | (len << 24);
+        float v = p.second;
+        w[lane][2] = kShapNoFeature | (1u << 8) | grp;
+        memcpy(&w[lane][3], &v, 4);
+        ++lane;
+        for (const PathElem &e : p.first) {
+          const float z = (float)e.zero;
+          w[lane][0] = e.lo, w[lane][1] = e.hi, w[lane][2] = e.feat | (e.miss << 8) | grp;
+          memcpy(&w[lane][3], &z, 4);
+          ++lane;
+        }
+      }
+      s.bins.insert(s.bins.end(), &w[0][0], &w[0][0] + 128);
+    }
+    s.tree_bin.push_back(s.num_bins());
+  }
+  s.ok = true;
+  return s;
+}
+
+float shap_bias(const ShapForest &s, const HostForest &h, const FlatForest &f, int ntree) {
+  float b = 0.f;
+  for (int t = 0; t < ntree; ++t) b += 0.f + s.mean[f.tree_offset[t]];
+  return b + h.base_score;
+}
+
+PredictConfig parse_predict_config(const char *json) {
+  if (!json) fail("XGBoosterPredictFromDMatrix: config is NULL");
+  const size_t len = strlen(json);
+  JV root;
+  try {
+    JsonReader r{json, json + len};
+    root = r.value();
+  } catch (const std::exception &e) {
+    fail(std::string("XGBoosterPredictFromDMatrix: config is not valid JSON (") + e.what() + ")");
+  }
+  if (root.kind != JV::Obj) fail("XGBoosterPredictFromDMatrix: config must be a JSON object");
+  auto need = [&](const char *key) -> const JV & {
+    const JV *v = root.find(key);
+    if (!v) fail(std::string("XGBoosterPredictFromDMatrix: config is missing the key '") + key + "'");
+    return *v;
+  };
+  PredictConfig c;
+  c.type = (int)need("type").as_int();
+  c.training = need("training").as_int() != 0;
+  c.iteration_begin = need("iteration_begin").as_int();
+  c.iteration_end = need("iteration_end").as_int();
+  c.strict_shape = need("strict_shape").as_int() != 0;
+  return c;
 }
 
 }  // namespace qcoh

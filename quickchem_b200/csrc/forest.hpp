@@ -94,6 +94,39 @@ struct DuoForest {
 };
 DuoForest build_duo(const struct FlatForest &f, uint32_t num_feature);
 
+// Per-feature contributions (DESIGN.md "Contributions"), built at the first contributions call.
+//   mean: FillNodeMeanValue of libxgboost 1.6.0 in float32, by flat (depth-ordered) node index
+//   bins: every root-to-leaf path of every tree as one lane group of a 32-lane bin, 4 words per lane:
+//     {lo_key, hi_key, feat | missing_goes_here << 8 | group_start << 16 | group_len << 24, float bits}
+//   Lane group_start is the path's bias element (feat 0xFF; its float is the leaf value); the others hold one
+//   feature each — repeated splits on a path merged: key bounds intersected, zero fractions (cover(child) /
+//   cover(parent)) multiplied, missing flags ANDed; their float is the zero fraction.  A present value with key k
+//   follows the path iff lo_key <= k < hi_key, a missing one iff the flag is set.  Unused lanes: feat 0xFF, len 0.
+//   Paths never straddle a bin, and a tree's bins are contiguous: bins [tree_bin[t], tree_bin[t + 1]).
+constexpr uint32_t kShapNoFeature = 0xFF;
+struct ShapForest {
+  bool ok = false;
+  std::vector<float> mean;
+  std::vector<uint32_t> bins;      // [num_bins][32][4]
+  std::vector<int64_t> tree_bin;   // [ntree + 1]
+  int32_t max_path_len = 0;        // elements of the longest path, bias included
+  int64_t num_paths = 0, num_elements = 0;
+  int64_t num_bins() const { return (int64_t)(bins.size() / 128); }
+};
+// Throws unless every node of every tree has a finite, positive cover (sum_hess).
+ShapForest build_shap(const struct HostForest &h, const struct FlatForest &f);
+// The bias column of a contributions row: ((0 + mean_0(root)) + mean_1(root) + ...) + base_score in float32.
+float shap_bias(const ShapForest &s, const struct HostForest &h, const struct FlatForest &f, int ntree);
+
+// The config of XGBoosterPredictFromDMatrix (libxgboost 1.6.0 keys); throws naming a missing key.
+struct PredictConfig {
+  int type = 0;
+  bool training = false;
+  int64_t iteration_begin = 0, iteration_end = 0;
+  bool strict_shape = false;
+};
+PredictConfig parse_predict_config(const char *json);
+
 // Throws std::runtime_error with libxgboost-style messages on malformed / unsupported input.
 HostForest load_model_file(const std::string &path);
 HostForest load_model_buffer(const unsigned char *buf, size_t len);

@@ -850,6 +850,212 @@ cudaError_t launch_predict(const DeviceForest &f, const PredictArgs &a, const Tu
 }
 
 // =====================================================================================
+// K6 — per-feature contributions (libxgboost 1.6.0 cpu_predictor PredictContribution)
+// =====================================================================================
+// Exact: path-dependent TreeSHAP in the path-parallel form of GPUTreeShap (Mitchell, Frank, Holmes 2022).  A
+// path's elements sit on consecutive lanes of a 32-lane bin (forest.hpp ShapForest); for one row a lane evaluates
+// its element's one fraction (one key range test, or the missing flag), the lanes of a path run ExtendPath with
+// shuffles, then every lane unwinds its own element (UnwoundPathSum) and adds w * (one - zero) * leaf to its
+// feature.  float64 throughout; a row's sum over the bins of one slice is a float64 in shared memory.
+//   grid = (tiles, slices): a CTA takes one 256-row key tile (TMA, like the predict kernels) and one slice of the
+//   bins; each warp owns 32 tile positions and walks the slice's bins in order, row by row.  Paths of one bin add
+//   into a row's accumulator group by group, so the float64 sums have a fixed order.
+constexpr unsigned kFull = 0xffffffffu;
+
+__device__ __forceinline__ int shap_region_words(int nf) {
+  const int ast = nf | 1;
+  return max(2 * kTileRows * ast, kTileRows * (nf + 2));
+}
+
+__global__ void __launch_bounds__(kTileRows, 2) shap_paths_kernel(const uint4 *__restrict__ bins, int64_t nbins, int nslices,
+                                                                  ContribArgs a, double *__restrict__ part) {
+  extern __shared__ __align__(128) uint32_t smem[];
+  __shared__ __align__(8) unsigned long long bars[1];
+  __shared__ double s_inv[34];  // 1 / k
+  const int nf = a.nfeat, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int ast = nf | 1, kst = nf | 1;  // odd row strides: the lanes of a warp read / add distinct features of one row
+  double *acc = reinterpret_cast<double *>(smem);    // [256][ast] by tile position; the TMA buffer aliases its start
+  uint32_t *keys = smem + shap_region_words(nf);     // [256][kst] keys by tile position
+  uint32_t *order = keys + kTileRows * kst;          // [256] the tile's row order
+  PredictArgs pa;
+  pa.Xt = a.Xt, pa.nrow = a.nrow, pa.ncol = a.ncol;
+  TilePipe<1> pipe;
+  pipe.begin(smem, bars, pa, nf, true, tid);
+  if (tid < 34) s_inv[tid] = tid ? 1.0 / (double)tid : 0.0;
+  (void)pipe.acquire(tid);
+  order[tid] = smem[tid];
+  for (int c = 0; c < nf; ++c) keys[tid * kst + c] = smem[(1 + c) * kStride + tid];
+  __syncthreads();
+  for (int i = tid; i < kTileRows * ast; i += kTileRows) acc[i] = 0.0;
+  __syncthreads();
+  const uint64_t tile = blockIdx.x;
+  const int64_t b0 = nbins * (int64_t)blockIdx.y / nslices, b1 = nbins * (int64_t)(blockIdx.y + 1) / nslices;
+  for (int64_t b = b0; b < b1; ++b) {
+    const uint4 e = __ldg(bins + b * 32 + lane);
+    const uint32_t feat = e.z & 0xFFu, g0 = (e.z >> 16) & 31u, len = e.z >> 24;
+    const int j = lane - (int)g0, D = (int)len - 1;  // my place in my path, and the path's unique depth
+    const bool elem = feat != kShapNoFeature && j >= 1;
+    const bool miss_here = (e.z >> 8) & 1u;
+    const float zf = __uint_as_float(e.w);
+    const double z = elem ? (double)zf : 1.0;
+    const double v = (double)__shfl_sync(kFull, zf, (int)g0);  // leaf value, from the path's bias lane
+    const int maxlen = (int)__reduce_max_sync(kFull, len);
+    const double invz = 1.0 / z, d1 = (double)(D + 1), inv_d1 = s_inv[D + 1 > 0 ? D + 1 : 0];
+    const unsigned starts = __ballot_sync(kFull, len > 0 && j == 0);
+    const int ngroups = __popc(starts), my_group = __popc(starts & ((1u << g0) - 1u));
+    for (int r = warp * 32; r < warp * 32 + 32; ++r) {
+      const uint32_t orig = order[r] & 0xFFu;
+      if (tile * kTileRows + orig >= a.nrow) continue;  // warp-uniform
+      bool one = true;
+      if (elem) {
+        const uint32_t k = keys[r * kst + feat];
+        one = k == kKeyMissing ? miss_here : (e.x <= k && k < e.y);
+      }
+      const float zo = one ? zf : -zf;  // (one, zero) of my element in one word: zero fractions are > 0
+      // ExtendPath, element by element: pw[j] <- zero_i * pw[j] * (i - j) / (i + 1) + one_i * pw[j - 1] * j / (i + 1)
+      double pw = j == 0 ? 1.0 : 0.0;
+      for (int i = 1; i < maxlen; ++i) {
+        const float zi = __shfl_sync(kFull, zo, (int)(g0 + i) & 31);
+        const double left = __shfl_up_sync(kFull, pw, 1);
+        if (i <= D) {
+          const double inv = s_inv[i + 1];
+          pw = (double)fabsf(zi) * pw * (double)max(i - j, 0) * inv + (zi > 0.f ? left : 0.0) * (double)j * inv;
+        }
+      }
+      // UnwoundPathSum of my element
+      double next = __shfl_sync(kFull, pw, (int)(g0 + (D > 0 ? D : 0)) & 31), total = 0.0;
+      for (int i = maxlen - 2; i >= 0; --i) {
+        const double pwi = __shfl_sync(kFull, pw, (int)(g0 + min(i, D > 0 ? D : 0)) & 31);
+        if (i < D) {
+          if (one) {
+            const double tmp = next * d1 * s_inv[i + 1];
+            total += tmp;
+            next = pwi - tmp * z * (double)(D - i) * inv_d1;
+          } else {
+            total += pwi * invz * d1 * s_inv[D - i];
+          }
+        }
+      }
+      const double c = total * ((one ? 1.0 : 0.0) - z) * v;
+      double *arow = acc + r * ast;
+      for (int g = 0; g < ngroups; ++g) {  // paths of the bin in order: a feature may recur across paths
+        if (elem && my_group == g) arow[feat] += c;
+        __syncwarp();
+      }
+    }
+  }
+  __syncthreads();
+  for (int i = tid; i < kTileRows * nf; i += kTileRows) {
+    const int p = i / nf, f = i - p * nf;
+    const uint64_t row = tile * kTileRows + (order[p] & 0xFFu);
+    if (row < a.nrow) part[((uint64_t)blockIdx.y * a.nrow + row) * (uint64_t)nf + f] = acc[p * ast + f];
+  }
+}
+
+__global__ void __launch_bounds__(256) shap_reduce_kernel(const double *__restrict__ part, int nslices, ContribArgs a) {
+  const int nf = a.nfeat;
+  const uint64_t n = a.nrow * (uint64_t)(nf + 1), stride = (uint64_t)gridDim.x * blockDim.x;
+  for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+    const uint64_t row = i / (uint64_t)(nf + 1);
+    const int f = (int)(i - row * (uint64_t)(nf + 1));
+    float v = a.bias;
+    if (f < nf) {
+      double s = 0.0;
+      for (int k = 0; k < nslices; ++k) s += part[((uint64_t)k * a.nrow + row) * (uint64_t)nf + f];
+      v = (float)s;
+    }
+    a.out[i] = v;
+  }
+}
+
+cudaError_t launch_shap(const uint4 *bins, int64_t nbins, int nslices, const ContribArgs &a, double *part, cudaStream_t s) {
+  if (a.nrow == 0 || nbins <= 0 || nslices <= 0) return cudaSuccess;
+  if (a.nrow > kShapChunkRows || a.ncol > a.nfeat || a.nfeat > (int)kMaxFeatures) return cudaErrorInvalidValue;
+  const int nf = a.nfeat, kst = nf | 1, ast = nf | 1;
+  const size_t smem = 4 * ((size_t)std::max(2 * kTileRows * ast, kTileRows * (nf + 2)) + (size_t)kTileRows * kst + kTileRows);
+  cudaError_t e = cudaFuncSetAttribute(shap_paths_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  shap_paths_kernel<<<dim3((unsigned)tile_count(a.nrow), (unsigned)nslices), kTileRows, smem, s>>>(bins, nbins, nslices, a, part);
+  g_last_predict = count_family("shap", false, false);
+  return QC_LAUNCHED();
+}
+
+cudaError_t launch_shap_reduce(const double *part, int nslices, const ContribArgs &a, cudaStream_t s) {
+  if (a.nrow == 0) return cudaSuccess;
+  const uint64_t n = a.nrow * (uint64_t)(a.nfeat + 1);
+  const int blocks = (int)std::min<uint64_t>((n + 255) / 256, (uint64_t)sm_count() * 16);
+  shap_reduce_kernel<<<blocks, 256, 0, s>>>(part, nslices, a);
+  count_family("shap_reduce", false, false);
+  return QC_LAUNCHED();
+}
+
+// Approximate (Saabas): one thread per row walks each tree on the 8-byte nodes and adds mean(next) - mean(node) to
+// the split feature — float32, in libxgboost's order: a per-tree vector (tp, only the features the path touched,
+// tracked in a bit mask) is added into the row's accumulator after every tree.  Both are feature-major [f][row]
+// in shared memory: thread t always hits bank t % 32, like skey.
+__global__ void __launch_bounds__(kBlock, 2) shap_approx_kernel(DeviceForest f, const float *__restrict__ mean, int ntree, ContribArgs a) {
+  extern __shared__ __align__(128) uint32_t skey[];
+  __shared__ __align__(8) unsigned long long bars[1];
+  const int tid = threadIdx.x, nf = a.nfeat;
+  float *acc = reinterpret_cast<float *>(skey + (nf + 2) * kStride);  // [nf][256]
+  float *tp = acc + nf * kStride;                                     // [nf][256]
+  PredictArgs pa;
+  pa.Xt = a.Xt, pa.nrow = a.nrow, pa.ncol = a.ncol;
+  TilePipe<1> pipe;
+  pipe.begin(skey, bars, pa, nf, true, tid);
+  for (int c = 0; c < nf; ++c) acc[c * kStride + tid] = 0.f;
+  const uint32_t buf = pipe.acquire(tid);
+  const uint32_t my = buf + 4u * (uint32_t)(kStride + tid);
+  const uint64_t row = pipe.tile * kTileRows + (lds_u32(buf + 4u * (uint32_t)tid) & 0xFFu);
+  if (row >= a.nrow) return;
+  for (int t = 0; t < ntree; ++t) {
+    uint32_t idx = __ldg(f.tree_offset + t);
+    uint2 nd = __ldg(f.nodes + idx);
+    float node_value = __ldg(mean + idx);
+    uint32_t mask = 0u, last = 0u, rel = nd.y & kMetaRelMask;
+    while (rel != 0u) {
+      const uint32_t ft = nd.y >> kMetaFeatShift;
+      const uint32_t kv = lds_u32(my + ft * 1024u);
+      if (kv == kKeyMissing)
+        idx += rel + ((nd.y & kMetaDefaultLeftBit) ? 0u : 1u);
+      else
+        idx = step_index(idx, rel, nd.x, kv);
+      const float nv = __ldg(mean + idx);
+      float *p = tp + ft * kStride + tid;
+      *p = __fadd_rn((mask >> ft) & 1u ? *p : 0.f, __fsub_rn(nv, node_value));
+      mask |= 1u << ft, last = ft, node_value = nv;
+      nd = __ldg(f.nodes + idx);
+      rel = nd.y & kMetaRelMask;
+    }
+    if (mask) {
+      float *p = tp + last * kStride + tid;
+      *p = __fadd_rn(*p, __fsub_rn(__uint_as_float(nd.x), node_value));  // leaf - mean(leaf): libxgboost adds it too
+      while (mask) {
+        const int c = __ffs(mask) - 1;
+        mask &= mask - 1u;
+        acc[c * kStride + tid] = __fadd_rn(acc[c * kStride + tid], tp[c * kStride + tid]);
+      }
+    }
+  }
+  float *o = a.out + row * (uint64_t)(nf + 1);
+  for (int c = 0; c < nf; ++c) o[c] = acc[c * kStride + tid];
+  o[nf] = a.bias;
+}
+
+cudaError_t launch_shap_approx(const DeviceForest &f, const float *mean, int ntree, const ContribArgs &a, cudaStream_t s) {
+  if (a.nrow == 0) return cudaSuccess;
+  if (a.ncol > a.nfeat || a.nfeat != f.nfeat || a.nfeat > (int)kMaxFeatures) return cudaErrorInvalidValue;
+  const uint64_t ntile = tile_count(a.nrow);
+  if (ntile > 0x7fffffffull) return cudaErrorInvalidConfiguration;
+  const size_t smem = (size_t)kStride * 4 * (size_t)(a.nfeat + 2 + 2 * a.nfeat);
+  cudaError_t e = cudaFuncSetAttribute(shap_approx_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  shap_approx_kernel<<<(unsigned)ntile, kBlock, smem, s>>>(f, mean, ntree, a);
+  g_last_predict = count_family("shap_approx", false, false);
+  return QC_LAUNCHED();
+}
+
+// =====================================================================================
 // K1 — Run1 feature assembly
 // =====================================================================================
 // oh_state: PL_MOD, NDWET (OH_GridCompMod.F90:1247-1257) and the level-slab count (:275-298).

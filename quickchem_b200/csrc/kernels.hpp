@@ -106,6 +106,25 @@ cudaError_t launch_seal_tiles(const float *X, uint64_t nrow, int ncol, float mis
 
 cudaError_t launch_predict(const DeviceForest &f, const PredictArgs &a, const Tunables &t, cudaStream_t s);
 
+// Per-feature contributions (forest.hpp ShapForest).  out: [nrow][nfeat + 1] floats, column nfeat = `bias`.
+//   exact (TreeSHAP on the path bins): launch_shap writes float64 partial sums of bin slice s to
+//   part[s][nrow][nfeat]; launch_shap_reduce adds the slices in slice order and rounds once.  The slicing depends
+//   only on the number of bins, so every row gets the same sums in the same order whatever the launch shape.
+//   approximate (Saabas): launch_shap_approx walks the 8-byte nodes with the node means, float32 in libxgboost's order.
+constexpr int kShapSlices = 16;             // bin slices of one call (a 4096-row call is 16 tiles x 16 slices = 256 CTAs)
+constexpr uint64_t kShapChunkRows = 32768;  // rows per exact launch: part[] holds kShapSlices x 32768 x nfeat doubles
+struct ContribArgs {
+  const uint32_t *Xt = nullptr;  // key tiles of rows [0, nrow) (nrow <= kShapChunkRows for launch_shap)
+  uint64_t nrow = 0;
+  int32_t ncol = 0;
+  int32_t nfeat = 0;
+  float bias = 0.f;
+  float *out = nullptr;
+};
+cudaError_t launch_shap(const uint4 *bins, int64_t nbins, int nslices, const ContribArgs &a, double *part, cudaStream_t s);
+cudaError_t launch_shap_reduce(const double *part, int nslices, const ContribArgs &a, cudaStream_t s);
+cudaError_t launch_shap_approx(const DeviceForest &f, const float *mean, int ntree, const ContribArgs &a, cudaStream_t s);
+
 // Fused Run1 predict: features come straight from the SoA fields (27 sources in feature order)
 struct SoaArgs {
   const float *src3[27];     // [km][ncol] source of feature f, or nullptr if it is a 2-D field
