@@ -187,7 +187,13 @@ int qcoh_booster_predict_device(BoosterHandle handle, DMatrixHandle dmat, int op
  * Asynchronous on the library stream; qcoh_device_synchronize() to wait. */
 int qcoh_booster_predict_contribs_device(BoosterHandle handle, DMatrixHandle dmat, int approximate,
                                          unsigned ntree_limit, float *out_dev);
-/* Kernel variant selection for experiments / profiling (0 = default).  See DESIGN.md. */
+/* Library settings of the calling thread; values are integers.  Any other name fails with "unknown parameter".
+ *   duo         0: predict on the 8-byte nodes only.  Any other value (default -1): on the two-level records
+ *               whenever the booster's records and the matrix allow it.
+ *   speculate   1 (default): XGDMatrixCreateFromMat also predicts with the last-loaded booster, pipelined with
+ *               the copy; 0: it does not.
+ *   chunk_rows  rows per copy chunk of XGDMatrixCreateFromMat, rounded up to a multiple of 256 (at most 2^19 from
+ *               pageable memory); <= 0 restores the default 2^21. */
 int qcoh_set_param(const char *name, const char *value);
 /* How many kernels the library has launched since load (for bench.py's gpu_launches). */
 uint64_t qcoh_launch_count(void);

@@ -15,7 +15,7 @@ import os
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("QCOH_LIB") or os.path.join(_HERE, "libqcoh.so")  # QCOH_LIB: the experiment build
+LIB_PATH = os.environ.get("QCOH_LIB") or os.path.join(_HERE, "libqcoh.so")  # QCOH_LIB: load another build, e.g. to compare two side by side
 
 f32p = C.POINTER(C.c_float)
 u64 = C.c_uint64

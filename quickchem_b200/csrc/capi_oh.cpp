@@ -319,7 +319,7 @@ int qcoh_oh_run1(qcoh_oh_handle h, const qcoh_run1_in *in, qcoh_run1_out *out) {
       a.out = r.OH_ML + (size_t)(k1 - 1) * nc;
       a.pred = out->pred ? o->pred.need(npred) : nullptr;
       a.flags = r.ctl + 2;
-      CU(launch_predict_soa(o->booster->dev, a, g.tun, g.stream));
+      CU(launch_predict_soa(o->booster->dev, a, g.stream));
       if (out->pred) deliver(out->pred, a.pred, npred);
       check_inf_after = true;
     } else if (npred) {

@@ -100,15 +100,9 @@ void upload(Booster *b) {
 // (walk_group_duo).  The owner tag below is therefore per device = per thread; everything else a launch needs
 // travels in the booster's DeviceForest.  allow_duo = false forces the 8-byte-node layout.
 static thread_local uint64_t g_const_top_owner = 0;
-static thread_local int g_const_top_levels = 0;  // kConstDuo = two-level layout
+static thread_local bool g_const_top_duo = false;  // the layout the table holds: two-level tops or 8-byte-node tops
 static thread_local int g_const_tree0 = 0, g_const_ntree = 0;
-constexpr int kConstDuo = -1;
-bool duo_wanted(const Booster *b) {
-  if (b->dev.recs == nullptr || b->dev.tex == 0 || g.tun.duo == 0) return false;
-  if (g.tun.duo > 0) return true;
-  // default: on, unless an experiment knob of the 8-byte-node kernel is set
-  return kDuoDefault && g.tun.variant == 0 && g.tun.park != 0 && g.tun.top_levels < 0 && g.tun.ilp == 0 && g.tun.minb == 0;
-}
+bool duo_wanted(const Booster *b) { return b->dev.recs != nullptr && b->dev.tex != 0 && g.duo != 0; }
 void sync_const_top(Booster *b, bool allow_duo, int tree0, int ntree) {
   b->dev.const_top_levels = 0, b->dev.duo_ready = 0, b->dev.const_tree0 = 0, b->dev.const_ntree = 0;
   if (ntree < 0) ntree = std::min(b->dev.ntree - tree0, kConstTreesMax);
@@ -119,36 +113,34 @@ void sync_const_top(Booster *b, bool allow_duo, int tree0, int ntree) {
   int w0 = tree0 - tree0 % kConstTreesMax;
   if (tree0 + ntree > w0 + kConstTreesMax) w0 = tree0;
   const int hold = std::min(b->dev.ntree - w0, kConstTreesMax);
-  auto holds = [&](int layout) {
-    return g_const_top_owner == b->version && g_const_top_levels == layout && g_const_tree0 <= tree0 &&
+  auto holds = [&](bool duo) {
+    return g_const_top_owner == b->version && g_const_top_duo == duo && g_const_tree0 <= tree0 &&
            tree0 + ntree <= g_const_tree0 + g_const_ntree;
   };
   if (allow_duo && duo_wanted(b)) {
-    if (!holds(kConstDuo)) {
+    if (!holds(true)) {
       g_const_top_owner = 0;
       if (upload_const_duo(b->duo.top_xy.data() + (size_t)w0 * (2u << kDuoTop), b->duo.tree_slot.data() + w0, hold, g.stream) ==
           cudaSuccess) {
-        g_const_top_owner = b->version, g_const_top_levels = kConstDuo, g_const_tree0 = w0, g_const_ntree = hold;
+        g_const_top_owner = b->version, g_const_top_duo = true, g_const_tree0 = w0, g_const_ntree = hold;
       } else {
         (void)cudaGetLastError();
       }
     }
-    if (holds(kConstDuo)) {
+    if (holds(true)) {
       b->dev.duo_ready = 1, b->dev.const_tree0 = g_const_tree0, b->dev.const_ntree = g_const_ntree;
       return;
     }
   }
-  const int want = g.tun.top_levels < 0 ? 4 : g.tun.top_levels;
-  if (want <= 0) return;
-  if (!holds(want)) {
+  if (!holds(false)) {
     g_const_top_owner = 0;
-    if (upload_const_top(b->dev_nodes_host.data(), b->flat.tree_offset.data() + w0, hold, want, g.stream) != cudaSuccess) {
+    if (upload_const_top(b->dev_nodes_host.data(), b->flat.tree_offset.data() + w0, hold, g.stream) != cudaSuccess) {
       (void)cudaGetLastError();
       return;  // does not fit: the kernel runs without the table
     }
-    g_const_top_owner = b->version, g_const_top_levels = want, g_const_tree0 = w0, g_const_ntree = hold;
+    g_const_top_owner = b->version, g_const_top_duo = false, g_const_tree0 = w0, g_const_ntree = hold;
   }
-  b->dev.const_top_levels = want, b->dev.const_tree0 = g_const_tree0, b->dev.const_ntree = g_const_ntree;
+  b->dev.const_top_levels = kDuoTop, b->dev.const_tree0 = g_const_tree0, b->dev.const_ntree = g_const_ntree;
 }
 
 // One prediction = one launch per range of kRangeTrees trees (kernels.hpp; the tables hold kConstTreesMax and are
@@ -165,14 +157,13 @@ void launch_predict_chunked(Booster *b, PredictArgs a, bool allow_duo, cudaStrea
     }
     return;
   }
-  const int range = g.tun.range_trees > 0 ? std::min(g.tun.range_trees, kConstTreesMax) : kRangeTrees;
-  for (int t0 = 0; t0 < t_end; t0 += range) {
-    const int n = std::min(range, t_end - t0);
+  for (int t0 = 0; t0 < t_end; t0 += kRangeTrees) {
+    const int n = std::min(kRangeTrees, t_end - t0);
     sync_const_top(b, allow_duo, t0, n);
     PredictArgs c = a;
     c.tree_begin = t0, c.tree_end = t0 + n;
     c.first = t0 == 0, c.last = t0 + n == t_end;
-    CU(launch_predict(b->dev, c, g.tun, s));
+    CU(launch_predict(b->dev, c, s));
   }
 }
 
@@ -939,16 +930,7 @@ int qcoh_set_param(const char *name, const char *value) {
   if (!name || !value) throw Error("qcoh_set_param: NULL argument");
   const int v = atoi(value);
   std::string n(name);
-  if (n == "variant") g.tun.variant = v;
-  else if (n == "ilp") g.tun.ilp = v;
-  else if (n == "block") g.tun.block = v;
-  else if (n == "top_levels") g.tun.top_levels = v;
-  else if (n == "park") g.tun.park = v;
-  else if (n == "minb") g.tun.minb = v;
-  else if (n == "duo") g.tun.duo = v;
-  else if (n == "duo_mask") g.tun.duo_mask = v;
-  else if (n == "persist") g.tun.persist = v;
-  else if (n == "range_trees") g.tun.range_trees = v;
+  if (n == "duo") g.duo = v;
   else if (n == "speculate") g.speculate = v;
   else if (n == "chunk_rows") g.chunk_rows = v > 0 ? ((uint64_t)v + 255) / 256 * 256 : (1ull << 21);
   else throw Error("qcoh_set_param: unknown parameter '" + n + "'");

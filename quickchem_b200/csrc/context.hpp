@@ -73,11 +73,11 @@ struct Ctx {
   cudaStream_t d2h_stream = nullptr;   // D2H of result chunks
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   std::vector<cudaEvent_t> chunk_events;
+  int duo = -1;                        // two-level records when the booster qualifies; 0 = 8-byte nodes only
   int speculate = 1;                   // pipeline prediction into XGDMatrixCreateFromMat
   uint64_t chunk_rows = 1ull << 21;
   void *flush = nullptr;
   size_t flush_bytes = 0;
-  Tunables tun;
 };
 inline thread_local Ctx g;
 

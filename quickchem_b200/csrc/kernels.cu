@@ -6,8 +6,7 @@
 //   K2b predict_tiles_kernel  tree-ensemble traversal on two-level 16-byte records (one gather per two tree
 //                             levels), replaces libxgboost's CPUPredictor behind XGBoosterPredict (reference call
 //                             site :356) with the export transform 10**x * OHscale (:369,:1569) fused as epilogue;
-//                             sums / leaf indices, clean matrices / missing entries; tiles arrive by TMA, optionally
-//                             in a persistent double-buffered loop (shallow forests: the HBM-bound regime)
+//                             sums / leaf indices, clean matrices / missing entries; tiles arrive by TMA
 //   K2  predict_tiles_nodes8_kernel   the same on the 8-byte depth-ordered nodes (boosters the records do not hold)
 //       predict_soa_kernel    K2 / K2b with the tile assembled straight from the Run1 SoA fields
 //   K1  oh_state / oh_sums / oh_pack    Run1 feature assembly (:1240-1257, :1441-1488, :303-345)
@@ -127,9 +126,9 @@ constexpr int kConstTopNodes = kConstTreesMax << kDuoTop;  // 61 440 B of the 64
 __constant__ uint2 c_top[kConstTopNodes];
 __constant__ uint32_t c_duo_base[kConstTreesMax];
 
-cudaError_t upload_const_top(const uint32_t *dev_nodes_xy, const uint32_t *tree_offset, int ntree, int levels, cudaStream_t s) {
-  const int stride = 1 << levels;
-  if (levels <= 0 || (int64_t)ntree * stride > kConstTopNodes) return cudaErrorInvalidValue;
+cudaError_t upload_const_top(const uint32_t *dev_nodes_xy, const uint32_t *tree_offset, int ntree, cudaStream_t s) {
+  constexpr int stride = 1 << kDuoTop;
+  if (ntree > kConstTreesMax) return cudaErrorInvalidValue;
   std::vector<uint2> host((size_t)ntree * stride);
   for (int t = 0; t < ntree; ++t) {
     const uint32_t n0 = tree_offset[t], n1 = tree_offset[t + 1];
@@ -176,65 +175,52 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
       : "memory");
 }
 
-// The tile loop shared by the predict kernels.  A CTA walks tiles blockIdx.x, + gridDim.x, ...: with a grid of
-// one CTA per tile that is the classic launch (the resident CTAs of an SM overlap each other's loads); with a
-// persistent grid and NBUF = 2 the next tile's bulk copy (TMA, cp.async.bulk completing on an mbarrier —
-// SASS UBLKCP + SYNCS) is in flight while this one is walked.  A tile is ncol KB of keys in its final
-// layout: no LSU instruction, no register, no arithmetic between HBM and the walk.  One thread issues the
-// copy and polls the mbarrier, the CTA then passes a barrier (256 threads polling one word showed up as
-// shared-memory bank-conflict wavefronts on the LSU data pipe, profiles/README.md v4).
-template <int NBUF>
+// The tile loop shared by the predict kernels.  A CTA walks tiles blockIdx.x, + gridDim.x, ...; the grid is one
+// CTA per tile, and the resident CTAs of an SM overlap each other's loads.  A tile arrives with one bulk copy (TMA,
+// cp.async.bulk completing on an mbarrier — SASS UBLKCP + SYNCS) of ncol KB of keys in their final layout: no LSU
+// instruction, no register, no arithmetic between HBM and the walk.  One thread issues the copy and polls the
+// mbarrier, the CTA then passes a barrier (256 threads polling one word showed up as shared-memory bank-conflict
+// wavefronts on the LSU data pipe, profiles/README.md v4).
 struct TilePipe {
-  uint32_t smem0, bar0, buf_bytes, tile_bytes, src_skip, dst_skip;
+  uint32_t smem0, bar0, tile_bytes, src_skip, dst_skip;
   const uint32_t *Xt;
   uint64_t ntile, tile, tile_stride;
   uint32_t it;
-  __device__ __forceinline__ void issue(uint64_t t, int b) const {
-    mbar_expect_tx(bar0 + 8u * b, tile_bytes);
-    if (tile_bytes) bulk_g2s(smem0 + buf_bytes * b + dst_skip, Xt + t * tile_stride + src_skip, tile_bytes, bar0 + 8u * b);
+  __device__ __forceinline__ void issue(uint64_t t) const {
+    mbar_expect_tx(bar0, tile_bytes);
+    if (tile_bytes) bulk_g2s(smem0 + dst_skip, Xt + t * tile_stride + src_skip, tile_bytes, bar0);
   }
-  // A buffer is [row order | nfeat feature slots | key-0 slot], 1 KB each.  Slots the matrix does not have are
+  // The buffer is [row order | nfeat feature slots | key-0 slot], 1 KB each.  Slots the matrix does not have are
   // missing (xgboost FVec::Fill leaves them flagged); the last slot is the key-0 slot leaves point at.  Both are
-  // written once per buffer: the bulk copies only touch the order slot (with_order) and slots 0..ncol-1.
-  __device__ __forceinline__ void begin(uint32_t *smem, unsigned long long *bars, const PredictArgs &a, int nfeat, bool with_order, int tid) {
-    smem0 = (uint32_t)__cvta_generic_to_shared(smem), bar0 = (uint32_t)__cvta_generic_to_shared(bars);
-    buf_bytes = (uint32_t)(nfeat + 2) * kStride * 4u;
+  // written once: the bulk copies only touch the order slot (with_order) and slots 0..ncol-1.
+  __device__ __forceinline__ void begin(uint32_t *smem, unsigned long long *bar, const PredictArgs &a, int nfeat, bool with_order, int tid) {
+    smem0 = (uint32_t)__cvta_generic_to_shared(smem), bar0 = (uint32_t)__cvta_generic_to_shared(bar);
     tile_stride = (uint64_t)(a.ncol + 1) * kStride;
     tile_bytes = (uint32_t)(a.ncol + (with_order ? 1 : 0)) * kStride * 4u;
     src_skip = with_order ? 0u : (uint32_t)kStride, dst_skip = with_order ? 0u : (uint32_t)kStride * 4u;
     Xt = a.Xt, ntile = (a.nrow + kTileRows - 1) / kTileRows, tile = blockIdx.x, it = 0;
-#pragma unroll
-    for (int b = 0; b < NBUF; ++b) {
-      uint32_t *k = smem + (size_t)b * (nfeat + 2) * kStride + kStride;
-      for (int c = a.ncol; c < nfeat; ++c) k[c * kStride + tid] = kKeyMissing;
-      k[nfeat * kStride + tid] = 0u;
-    }
+    uint32_t *k = smem + kStride;
+    for (int c = a.ncol; c < nfeat; ++c) k[c * kStride + tid] = kKeyMissing;
+    k[nfeat * kStride + tid] = 0u;
     if (tid == 0) {
-#pragma unroll
-      for (int b = 0; b < NBUF; ++b) mbar_init(bar0 + 8u * b, 1);
+      mbar_init(bar0, 1);
       mbar_init_fence();
     }
     __syncthreads();
-    if (tid == 0 && tile < ntile) issue(tile, 0);
+    if (tid == 0 && tile < ntile) issue(tile);
   }
   __device__ __forceinline__ bool more() const { return tile < ntile; }
-  // returns the shared address of this iteration's buffer (its row-order slot; the feature slots follow 1 KB later)
+  // returns the shared address of the buffer (its row-order slot; the feature slots follow 1 KB later)
   __device__ __forceinline__ uint32_t acquire(int tid) {
-    const int cur = NBUF == 2 ? (int)(it & 1u) : 0;
-    if (tid == 0) {
-      if (NBUF == 2 && tile + gridDim.x < ntile) issue(tile + gridDim.x, cur ^ 1);
-      mbar_wait(bar0 + 8u * cur, (it / NBUF) & 1u);
-    }
+    if (tid == 0) mbar_wait(bar0, it & 1u);
     __syncthreads();
-    return smem0 + buf_bytes * cur;
+    return smem0;
   }
   __device__ __forceinline__ void release(int tid) {
-    // every thread is done with this buffer before it is refilled
-    if (NBUF == 2) {
-      if (tile + gridDim.x < ntile) __syncthreads();
-    } else if (tile + gridDim.x < ntile) {
+    // every thread is done with the buffer before it is refilled
+    if (tile + gridDim.x < ntile) {
       __syncthreads();
-      if (tid == 0) issue(tile + gridDim.x, 0);
+      if (tid == 0) issue(tile + gridDim.x);
     }
     tile += gridDim.x, ++it;
   }
@@ -324,7 +310,7 @@ cudaError_t launch_seal_tiles(const float *X, uint64_t nrow, int ncol, float mis
 // TEXMODE is a bit mask over the ILP trees in flight: tree j fetches its nodes through the texture pipe
 // (tex1Dfetch on the same buffer) if bit j is set, through the LSU (LDG) otherwise.  ctree0: the first tree
 // the constant table holds.
-template <int ILP, bool HAS_MISSING, bool PARK, int TEXMODE = 0, int CTOP = 0>
+template <int ILP, bool HAS_MISSING, int TEXMODE = 0, int CTOP = 0>
 __device__ __forceinline__ void walk_group(const uint2 *__restrict__ nodes, cudaTextureObject_t tex, const uint32_t *__restrict__ toff,
                                            const int32_t *__restrict__ tdepth, int t, int ctree0, uint32_t my_saddr,
                                            uint32_t (&idx)[ILP], uint32_t (&xbits)[ILP]) {
@@ -341,7 +327,7 @@ __device__ __forceinline__ void walk_group(const uint2 *__restrict__ nodes, cuda
     rel[j] = 1u;
   }
   // depth + 1 fetches per tree: the last one reads the leaf itself, whose x word is the leaf value.
-  // PARK: a lane that has reached its leaf (rel == 0) stops fetching — it would otherwise re-read its
+  // A lane that has reached its leaf (rel == 0) parks: it stops fetching — it would otherwise re-read its
   // own leaf line at every remaining level, and at the deep levels those are up to 32 different
   // lines per warp request; the L1TEX data pipe is the bound of this kernel (DESIGN.md).  The
   // fetch is predicated, so nd[j] keeps the leaf node and no per-level copy of the value is needed.
@@ -377,11 +363,11 @@ __device__ __forceinline__ void walk_group(const uint2 *__restrict__ nodes, cuda
         if (d <= depth) {
 #pragma unroll
           for (int j = 0; j < ILP; ++j) {
-            if (!PARK || rel[j] != 0u) {
+            if (rel[j] != 0u) {
               nd[j] = c_top[cbase[j] + idx[j]];
               visit(j);
             }
-            if (PARK) asm volatile("" : "+r"(rel[j]));
+            asm volatile("" : "+r"(rel[j]));
           }
         }
       }
@@ -396,37 +382,37 @@ __device__ __forceinline__ void walk_group(const uint2 *__restrict__ nodes, cuda
   for (int d = CTOP; d < depth; ++d) {
 #pragma unroll
     for (int j = 0; j < ILP; ++j) {
-      if (!PARK || rel[j] != 0u) {
+      if (rel[j] != 0u) {
         fetch(j);
         visit(j);
       }
       // keep "still walking" in the rel register only (one ISETP per level instead of predicate shuffling)
-      if (PARK) asm volatile("" : "+r"(rel[j]));
+      asm volatile("" : "+r"(rel[j]));
     }
   }
   // level `depth` holds only leaves: the last fetch reads the leaf a lane stands on — its value is all that is needed
   if (depth >= CTOP) {
 #pragma unroll
     for (int j = 0; j < ILP; ++j)
-      if (!PARK || rel[j] != 0u) fetch(j);
+      if (rel[j] != 0u) fetch(j);
   }
 #pragma unroll
   for (int j = 0; j < ILP; ++j) xbits[j] = nd[j].x;
 }
 
 // all trees [t0, t1) on the 8-byte nodes, in tree order; emit(t, value bits, node index)
-template <int ILP, bool HAS_MISSING, bool PARK, int TEXMODE, int CTOP, class Emit>
+template <int ILP, bool HAS_MISSING, int TEXMODE, int CTOP, class Emit>
 __device__ __forceinline__ void forest_walk(const DeviceForest &f, uint32_t my, int t0, int t1, Emit &&emit) {
   int t = t0;
   for (; t + ILP <= t1; t += ILP) {
     uint32_t idx[ILP], xb[ILP];
-    walk_group<ILP, HAS_MISSING, PARK, TEXMODE, CTOP>(f.nodes, f.tex, f.tree_offset, f.tree_depth, t, f.const_tree0, my, idx, xb);
+    walk_group<ILP, HAS_MISSING, TEXMODE, CTOP>(f.nodes, f.tex, f.tree_offset, f.tree_depth, t, f.const_tree0, my, idx, xb);
 #pragma unroll
     for (int j = 0; j < ILP; ++j) emit(t + j, xb[j], idx[j]);
   }
   for (; t < t1; ++t) {
     uint32_t idx[1], xb[1];
-    walk_group<1, HAS_MISSING, PARK, 0, 0>(f.nodes, f.tex, f.tree_offset, f.tree_depth, t, 0, my, idx, xb);
+    walk_group<1, HAS_MISSING, 0, 0>(f.nodes, f.tex, f.tree_offset, f.tree_depth, t, 0, my, idx, xb);
     emit(t, xb[0], idx[0]);
   }
 }
@@ -613,12 +599,12 @@ __device__ __forceinline__ uint64_t tile_row(uint32_t buf, uint64_t tile, int ti
   return tile * kTileRows + orig;
 }
 
-template <int ILP, int MINB, int TEXMODE, bool HAS_MISSING, bool PRED_LEAF, int NBUF>
+template <int ILP, int MINB, int TEXMODE, bool HAS_MISSING, bool PRED_LEAF>
 __global__ void __launch_bounds__(kBlock, MINB) predict_tiles_kernel(DeviceForest f, PredictArgs a) {
   extern __shared__ __align__(128) uint32_t skey[];
-  __shared__ __align__(8) unsigned long long bars[NBUF];
+  __shared__ __align__(8) unsigned long long bars[1];
   const int tid = threadIdx.x;
-  TilePipe<NBUF> pipe;
+  TilePipe pipe;
   pipe.begin(skey, bars, a, f.nfeat, HAS_MISSING, tid);
   while (pipe.more()) {
     const uint32_t buf = pipe.acquire(tid);
@@ -635,12 +621,12 @@ __global__ void __launch_bounds__(kBlock, MINB) predict_tiles_kernel(DeviceFores
   }
 }
 
-template <int ILP, bool HAS_MISSING, bool PRED_LEAF, bool PARK, int MINB, int TEXMODE, int CTOP>
+template <int ILP, bool HAS_MISSING, bool PRED_LEAF, int MINB, int TEXMODE, int CTOP>
 __global__ void __launch_bounds__(kBlock, MINB) predict_tiles_nodes8_kernel(DeviceForest f, PredictArgs a) {
   extern __shared__ __align__(128) uint32_t skey[];
   __shared__ __align__(8) unsigned long long bars[1];
   const int tid = threadIdx.x;
-  TilePipe<1> pipe;
+  TilePipe pipe;
   pipe.begin(skey, bars, a, f.nfeat, HAS_MISSING, tid);
   while (pipe.more()) {
     const uint32_t buf = pipe.acquire(tid);
@@ -650,9 +636,9 @@ __global__ void __launch_bounds__(kBlock, MINB) predict_tiles_nodes8_kernel(Devi
     row_result<PRED_LEAF>(f, a, row, row < a.nrow, [&](auto &&emit) {
       auto leaf = [&](int t, uint32_t xb, uint32_t idx) { emit(t, xb, PRED_LEAF ? (uint32_t)__ldg(f.orig_id + idx) : 0u); };
       if (HAS_MISSING && hm)
-        forest_walk<ILP, true, PARK, TEXMODE, CTOP>(f, my, a.tree_begin, a.tree_end, leaf);
+        forest_walk<ILP, true, TEXMODE, CTOP>(f, my, a.tree_begin, a.tree_end, leaf);
       else
-        forest_walk<ILP, false, PARK, TEXMODE, CTOP>(f, my, a.tree_begin, a.tree_end, leaf);
+        forest_walk<ILP, false, TEXMODE, CTOP>(f, my, a.tree_begin, a.tree_end, leaf);
     });
     pipe.release(tid);
   }
@@ -710,21 +696,21 @@ __global__ void __launch_bounds__(kBlock, DUO ? kDuoMinBlocks : 6) predict_soa_k
     else
       forest_walk_duo<kDuoIlp, kDuoTexMask, false>(f, my, 0, a.ntree_used, add);
   } else if (tile_missing) {
-    forest_walk<4, true, true, TEXMODE, CTOP>(f, my, 0, a.ntree_used, add);
+    forest_walk<4, true, TEXMODE, CTOP>(f, my, 0, a.ntree_used, add);
   } else {
-    forest_walk<4, false, true, TEXMODE, CTOP>(f, my, 0, a.ntree_used, add);
+    forest_walk<4, false, TEXMODE, CTOP>(f, my, 0, a.ntree_used, add);
   }
   if (a.pred) a.pred[m] = acc;
   a.out[m] = export_transform(acc, a.exp10, a.scale);
 }
 
-cudaError_t launch_predict_soa(const DeviceForest &f, const SoaArgs &a, const Tunables &t, cudaStream_t s) {
+cudaError_t launch_predict_soa(const DeviceForest &f, const SoaArgs &a, cudaStream_t s) {
   if (a.nrow == 0) return cudaSuccess;
   if (f.nfeat != 27) return cudaErrorInvalidValue;
   const size_t smem = (size_t)kStride * 28 * sizeof(float);
   const uint64_t nblk = (a.nrow + kBlock - 1) / kBlock;
   if (nblk > 0x7fffffffull) return cudaErrorInvalidConfiguration;
-  const bool tex = f.tex != 0 && t.variant >= 0;
+  const bool tex = f.tex != 0;
   const bool duo = f.duo_ready && f.const_tree0 == 0 && f.const_ntree >= a.ntree_used;
   auto k = !tex ? predict_soa_kernel<0, 0> : (f.const_top_levels == 4 ? predict_soa_kernel<0xA, 4> : predict_soa_kernel<0xA, 0>);
   if (duo) k = predict_soa_kernel<0xA, 0, true>;
@@ -746,12 +732,11 @@ static int sm_count() {
   return g_sm_count;
 }
 
+// one CTA per tile
 template <class K>
-static cudaError_t launch_tiles(K k, const DeviceForest &f, const PredictArgs &a, int nbuf, int persistent_ctas_per_sm, cudaStream_t s) {
-  const size_t smem = (size_t)nbuf * kStride * (size_t)(f.nfeat + 2) * sizeof(uint32_t);
-  const uint64_t ntile = tile_count(a.nrow);
-  uint64_t grid = ntile;
-  if (persistent_ctas_per_sm > 0) grid = std::min<uint64_t>(ntile, (uint64_t)sm_count() * persistent_ctas_per_sm);
+static cudaError_t launch_tiles(K k, const DeviceForest &f, const PredictArgs &a, cudaStream_t s) {
+  const size_t smem = (size_t)kStride * (size_t)(f.nfeat + 2) * sizeof(uint32_t);
+  const uint64_t grid = tile_count(a.nrow);
   if (grid > 0x7fffffffull) return cudaErrorInvalidConfiguration;
   cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
@@ -759,31 +744,26 @@ static cudaError_t launch_tiles(K k, const DeviceForest &f, const PredictArgs &a
   return QC_LAUNCHED();
 }
 
-// two-level records, default shape; HM / PL chosen at run time
-template <int ILP, int MINB, int TEXMODE, int NBUF>
-static cudaError_t launch_duo(const DeviceForest &f, const PredictArgs &a, int persistent, cudaStream_t s) {
+// two-level records; HM / PL chosen at run time
+template <int ILP, int MINB, int TEXMODE>
+static cudaError_t launch_duo(const DeviceForest &f, const PredictArgs &a, cudaStream_t s) {
   const bool hm = a.has_missing != 0, pl = a.pred_leaf != 0;
-  if (hm && pl) return launch_tiles(predict_tiles_kernel<ILP, MINB, TEXMODE, true, true, NBUF>, f, a, NBUF, persistent, s);
-  if (hm) return launch_tiles(predict_tiles_kernel<ILP, MINB, TEXMODE, true, false, NBUF>, f, a, NBUF, persistent, s);
-  if (pl) return launch_tiles(predict_tiles_kernel<ILP, MINB, TEXMODE, false, true, NBUF>, f, a, NBUF, persistent, s);
-  return launch_tiles(predict_tiles_kernel<ILP, MINB, TEXMODE, false, false, NBUF>, f, a, NBUF, persistent, s);
+  if (hm && pl) return launch_tiles(predict_tiles_kernel<ILP, MINB, TEXMODE, true, true>, f, a, s);
+  if (hm) return launch_tiles(predict_tiles_kernel<ILP, MINB, TEXMODE, true, false>, f, a, s);
+  if (pl) return launch_tiles(predict_tiles_kernel<ILP, MINB, TEXMODE, false, true>, f, a, s);
+  return launch_tiles(predict_tiles_kernel<ILP, MINB, TEXMODE, false, false>, f, a, s);
 }
 
-template <int ILP, bool PARK, int MINB, int TEXMODE, int CTOP>
+template <int ILP, int MINB, int TEXMODE, int CTOP>
 static cudaError_t launch_nodes8(const DeviceForest &f, const PredictArgs &a, cudaStream_t s) {
   const bool hm = a.has_missing != 0, pl = a.pred_leaf != 0;
-  if (hm && pl) return launch_tiles(predict_tiles_nodes8_kernel<ILP, true, true, PARK, MINB, TEXMODE, CTOP>, f, a, 1, 0, s);
-  if (hm) return launch_tiles(predict_tiles_nodes8_kernel<ILP, true, false, PARK, MINB, TEXMODE, CTOP>, f, a, 1, 0, s);
-  if (pl) return launch_tiles(predict_tiles_nodes8_kernel<ILP, false, true, PARK, MINB, TEXMODE, CTOP>, f, a, 1, 0, s);
-  return launch_tiles(predict_tiles_nodes8_kernel<ILP, false, false, PARK, MINB, TEXMODE, CTOP>, f, a, 1, 0, s);
+  if (hm && pl) return launch_tiles(predict_tiles_nodes8_kernel<ILP, true, true, MINB, TEXMODE, CTOP>, f, a, s);
+  if (hm) return launch_tiles(predict_tiles_nodes8_kernel<ILP, true, false, MINB, TEXMODE, CTOP>, f, a, s);
+  if (pl) return launch_tiles(predict_tiles_nodes8_kernel<ILP, false, true, MINB, TEXMODE, CTOP>, f, a, s);
+  return launch_tiles(predict_tiles_nodes8_kernel<ILP, false, false, MINB, TEXMODE, CTOP>, f, a, s);
 }
 
-// Persistent double-buffered variant (TMA prefetch of the next tile while this one is walked), for the HBM-bound
-// end of the booster sweep.  Two 28 KB buffers per CTA: three CTAs per SM (four would need 64 bytes more than the SM's 228 KB once the 1 KB
-// the system reserves per CTA is counted).
-constexpr int kPersistCtasPerSm = 3;
-
-cudaError_t launch_predict(const DeviceForest &f, const PredictArgs &a, const Tunables &t, cudaStream_t s) {
+cudaError_t launch_predict(const DeviceForest &f, const PredictArgs &a, cudaStream_t s) {
   if (a.nrow == 0 || a.tree_end <= a.tree_begin) return cudaSuccess;
   if (a.ncol > f.nfeat || f.nfeat > (int)kMaxFeatures) return cudaErrorInvalidValue;
   const bool hm = a.has_missing != 0, pl = a.pred_leaf != 0;
@@ -791,62 +771,18 @@ cudaError_t launch_predict(const DeviceForest &f, const PredictArgs &a, const Tu
   // ---- two-level records (the constant tables hold these trees' tops: capi_xgb.cpp sync_const_top)
   if (f.duo_ready && in_table && (!hm || f.duo_has_dl)) {
     g_last_predict = count_family("duo", hm, pl);
-    // measured (profiles/README.md): with two 28 KB buffers only three CTAs fit an SM, and the lost residency costs
-    // more than the prefetch wins — the persistent loop is opt-in (qcoh_set_param persist=1), not the default
-    const bool persist = t.persist > 0;
-#ifdef QC_EXPERIMENTS
-    // experiment grid (qcoh_set_param duo=1 + ilp / minb / duo_mask): trees in flight x resident CTAs x which
-    // of the trees gather through the texture pipe; measurements in profiles/README.md
-#define QC_DUO(I, M, MASK) \
-  if (t.ilp == I && t.minb == M && t.duo_mask == MASK) return launch_duo<I, M, MASK, 1>(f, a, 0, s);
-    QC_DUO(4, 6, 0xA) QC_DUO(4, 6, 0xE) QC_DUO(4, 6, 0xF) QC_DUO(3, 6, 0x6) QC_DUO(3, 6, 0x2) QC_DUO(6, 5, 0x2A) QC_DUO(8, 4, 0xEE)
-    // shallow forests (the HBM-bound end): more resident CTAs, fewer trees in flight, LSU-only gathers
-    QC_DUO(4, 6, 0x100) QC_DUO(3, 6, 0x100) QC_DUO(2, 6, 0x100) QC_DUO(2, 6, 0x2) QC_DUO(6, 5, 0x100) QC_DUO(6, 5, 0x14)
-    QC_DUO(6, 5, 0x3F) QC_DUO(4, 7, 0x100) QC_DUO(4, 7, 0xA) QC_DUO(3, 7, 0x100) QC_DUO(3, 7, 0x2) QC_DUO(2, 7, 0x100) QC_DUO(5, 6, 0x100) QC_DUO(5, 6, 0xA)
-#undef QC_DUO
-#endif
-    if (persist) return launch_duo<kDuoIlp, kPersistCtasPerSm, kDuoTexMask, 2>(f, a, kPersistCtasPerSm, s);
-    if (f.duo_shallow && t.ilp == 0) return launch_duo<4, 6, 0xA, 1>(f, a, 0, s);  // kernels.hpp kShallowRecBytesPerTree
-    return launch_duo<kDuoIlp, kDuoMinBlocks, kDuoTexMask, 1>(f, a, 0, s);
+    if (f.duo_shallow) return launch_duo<4, 6, 0xA>(f, a, s);  // kernels.hpp kShallowRecBytesPerTree
+    return launch_duo<kDuoIlp, kDuoMinBlocks, kDuoTexMask>(f, a, s);
   }
   // ---- 8-byte depth-ordered nodes: 4 trees in flight per thread; levels 0..3 of every tree from constant
   // memory when the table holds them; below that, trees 1 and 3 of each group fetch their nodes through the
   // texture pipe and trees 0 and 2 through the LSU (mask 0xA).  Measurements: profiles/README.md.
   g_last_predict = count_family("nodes8", hm, pl);
   constexpr int kTex = 0xA;
-  const bool tex = f.tex != 0 && t.variant >= 0;
   const int ctop = in_table ? f.const_top_levels : 0;  // 0 if the table does not hold these trees
-#ifdef QC_EXPERIMENTS
-  if (!hm && !pl) {
-    if (t.park == 0) return launch_nodes8<4, false, 6, 0, 0>(f, a, s);
-    if (t.variant > 0 && f.tex) {
-#define QC_TEX(V, I, MASK) \
-  if (t.variant == V) return ctop == 4 ? launch_nodes8<I, true, 6, MASK, 4>(f, a, s) : launch_nodes8<I, true, 6, MASK, 0>(f, a, s);
-      QC_TEX(1, 4, 0xF) QC_TEX(2, 4, 0xA) QC_TEX(3, 4, 0x8) QC_TEX(4, 4, 0xE)
-      QC_TEX(5, 3, 0x4) QC_TEX(6, 3, 0x6) QC_TEX(7, 6, 0x2A) QC_TEX(8, 6, 0x24) QC_TEX(9, 8, 0xAA)
-      QC_TEX(10, 2, 0x2) QC_TEX(11, 5, 0x0A) QC_TEX(12, 5, 0x15)
-#undef QC_TEX
-    }
-    if (t.ilp > 0 || t.minb > 0) {  // LSU-only builds
-      const int ilp = t.ilp > 0 ? t.ilp : 3, minb = t.minb > 0 ? t.minb : 6;
-#define QC_CASE(I, M) \
-  if (ilp == I && minb == M) return launch_nodes8<I, true, M, 0, 0>(f, a, s);
-      QC_CASE(1, 6) QC_CASE(2, 6) QC_CASE(3, 6) QC_CASE(4, 6) QC_CASE(6, 6)
-      QC_CASE(2, 5) QC_CASE(3, 5) QC_CASE(4, 5) QC_CASE(6, 5)
-      QC_CASE(2, 4) QC_CASE(3, 4) QC_CASE(4, 4) QC_CASE(6, 4) QC_CASE(8, 4)
-      QC_CASE(4, 3) QC_CASE(6, 3) QC_CASE(8, 3)
-#undef QC_CASE
-    }
-    if (tex && (ctop == 3 || ctop == 5 || ctop == 6)) {
-      if (ctop == 3) return launch_nodes8<4, true, 6, kTex, 3>(f, a, s);
-      if (ctop == 5) return launch_nodes8<4, true, 6, kTex, 5>(f, a, s);
-      return launch_nodes8<4, true, 6, kTex, 6>(f, a, s);
-    }
-  }
-#endif
-  if (!tex) return launch_nodes8<4, true, 6, 0, 0>(f, a, s);
-  if (ctop == 4) return launch_nodes8<4, true, 6, kTex, 4>(f, a, s);
-  return launch_nodes8<4, true, 6, kTex, 0>(f, a, s);
+  if (f.tex == 0) return launch_nodes8<4, 6, 0, 0>(f, a, s);
+  if (ctop == 4) return launch_nodes8<4, 6, kTex, 4>(f, a, s);
+  return launch_nodes8<4, 6, kTex, 0>(f, a, s);
 }
 
 // =====================================================================================
@@ -879,7 +815,7 @@ __global__ void __launch_bounds__(kTileRows, 2) shap_paths_kernel(const uint4 *_
   uint32_t *order = keys + kTileRows * kst;          // [256] the tile's row order
   PredictArgs pa;
   pa.Xt = a.Xt, pa.nrow = a.nrow, pa.ncol = a.ncol;
-  TilePipe<1> pipe;
+  TilePipe pipe;
   pipe.begin(smem, bars, pa, nf, true, tid);
   if (tid < 34) s_inv[tid] = tid ? 1.0 / (double)tid : 0.0;
   (void)pipe.acquire(tid);
@@ -1001,7 +937,7 @@ __global__ void __launch_bounds__(kBlock, 2) shap_approx_kernel(DeviceForest f, 
   float *tp = acc + nf * kStride;                                     // [nf][256]
   PredictArgs pa;
   pa.Xt = a.Xt, pa.nrow = a.nrow, pa.ncol = a.ncol;
-  TilePipe<1> pipe;
+  TilePipe pipe;
   pipe.begin(skey, bars, pa, nf, true, tid);
   for (int c = 0; c < nf; ++c) acc[c * kStride + tid] = 0.f;
   const uint32_t buf = pipe.acquire(tid);

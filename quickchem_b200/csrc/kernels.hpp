@@ -73,29 +73,14 @@ struct PredictArgs {
   float *out = nullptr;      // device: [nrow] or [nrow][out_stride]
 };
 
-struct Tunables {
-  int variant = 0;   // 0 = default
-  int ilp = 0;       // trees walked concurrently per thread (0 = default)
-  int block = 0;     // threads per CTA (0 = default)
-  int top_levels = -1;  // tree levels served from constant memory: -1 = default (4), 0 = none
-  int park = -1;     // -1 = default (on)
-  int minb = 0;      // min resident CTAs per SM the kernel is compiled for (register budget)
-  int duo = -1;      // two-level records: -1 = default, 0 = off, 1 = on
-  int duo_mask = 0;  // (experiment) texture-pipe tree mask of the two-level kernel, 0 = default
-  int persist = -1;  // persistent double-buffered tile loop: 1 = on (default off, see kernels.cu)
-  int range_trees = 0;  // trees per launch (<= kConstTreesMax): 0 = default
-};
-
-constexpr bool kDuoDefault = true;  // two-level records by default when the booster qualifies
-
 uint64_t launch_count();
 // launches per kernel family since load, and the family that served the last predict launch
 // ("duo", "duo_missing", "duo_leaf", "duo_missing_leaf", "nodes8", "nodes8_missing", "nodes8_leaf", ...)
 uint64_t kernel_launches(const char *family);
 const char *last_predict_kernel();
 
-// (experiment) copy levels 0..levels-1 of every tree into the kernel's __constant__ table
-cudaError_t upload_const_top(const uint32_t *dev_nodes_xy, const uint32_t *tree_offset, int ntree, int levels, cudaStream_t s);
+// 8-byte-node layout: levels 0..kDuoTop-1 of every tree into the tree-top table
+cudaError_t upload_const_top(const uint32_t *dev_nodes_xy, const uint32_t *tree_offset, int ntree, cudaStream_t s);
 // two-level layout: DuoForest::top_xy into the tree-top table and DuoForest::tree_slot into its base table
 cudaError_t upload_const_duo(const uint32_t *top_xy, const uint32_t *tree_slot, int ntree, cudaStream_t s);
 
@@ -104,7 +89,7 @@ cudaError_t upload_const_duo(const uint32_t *top_xy, const uint32_t *tree_slot, 
 // X and Xt cover `nrow` rows starting at a tile boundary.
 cudaError_t launch_seal_tiles(const float *X, uint64_t nrow, int ncol, float missing, uint32_t *Xt, int *flags, cudaStream_t s);
 
-cudaError_t launch_predict(const DeviceForest &f, const PredictArgs &a, const Tunables &t, cudaStream_t s);
+cudaError_t launch_predict(const DeviceForest &f, const PredictArgs &a, cudaStream_t s);
 
 // Per-feature contributions (forest.hpp ShapForest).  out: [nrow][nfeat + 1] floats, column nfeat = `bias`.
 //   exact (TreeSHAP on the path bins): launch_shap writes float64 partial sums of bin slice s to
@@ -141,7 +126,7 @@ struct SoaArgs {
   float *pred = nullptr;     // optional raw booster output
   int *flags = nullptr;      // |= 2 on +-inf input
 };
-cudaError_t launch_predict_soa(const DeviceForest &f, const SoaArgs &a, const Tunables &t, cudaStream_t s);
+cudaError_t launch_predict_soa(const DeviceForest &f, const SoaArgs &a, cudaStream_t s);
 
 // ---- fused Run1 pieces (OH_GridCompMod.F90:1232-1599) ---------------------------------
 struct Run1Dev {

@@ -164,30 +164,23 @@ def test_seal_builds_key_tiles(capi):
         d.free()
 
 
-def test_persistent_prefetch_loop_matches(capi, oracle, tmp_path, small_forest, small_model_path):
-    """Shallow forests run the persistent double-buffered tile loop (TMA prefetch); same bits as one CTA per tile,
-    over sizes where a CTA walks 1, 2 and many tiles, with a ragged last tile, with and without missing entries."""
-    x_all = synth.quick_features(synth.raw_fields(24))  # 248 832 rows = 972 tiles > 148 x 3 CTAs
+def test_tile_loop_over_sizes_and_ragged_tiles(capi, oracle, tmp_path, small_forest, small_model_path):
+    """The tile loop of the two-level kernel gives the oracle's sums and leaf ids over sizes from one tile to 972
+    tiles, with a ragged last tile, with and without missing entries."""
+    x_all = synth.quick_features(synth.raw_fields(24))  # 248 832 rows = 972 tiles
     om = oracle.Model(small_model_path)
     b = capi.Booster(small_model_path)
     rng = np.random.default_rng(2)
-    try:
-        for nrow in (255, 256 * 148 * 3 + 17, x_all.shape[0]):
-            for special in (False, True):
-                x = x_all[:nrow]
-                if special:
-                    x = inject_specials(x, small_forest, rng)
-                ref = om.predict(x)
-                ref_leaf = om.predict(x, option_mask=2)
-                for persist in (1, 0):
-                    capi.set_param("persist", persist)
-                    d = capi.DMatrix(x)
-                    assert np.array_equal(b.predict(d).view(np.uint32), ref.view(np.uint32)), (nrow, special, persist)
-                    assert capi.last_predict_kernel() == ("duo_missing" if special else "duo")
-                    assert np.array_equal(b.predict(d, option_mask=2), ref_leaf), (nrow, special, persist)
-                    d.free()
-    finally:
-        capi.set_param("persist", -1)
+    for nrow in (255, 256 * 148 * 3 + 17, x_all.shape[0]):
+        for special in (False, True):
+            x = x_all[:nrow]
+            if special:
+                x = inject_specials(x, small_forest, rng)
+            d = capi.DMatrix(x)
+            assert np.array_equal(b.predict(d).view(np.uint32), om.predict(x).view(np.uint32)), (nrow, special)
+            assert capi.last_predict_kernel() == ("duo_missing" if special else "duo")
+            assert np.array_equal(b.predict(d, option_mask=2), om.predict(x, option_mask=2)), (nrow, special)
+            d.free()
 
 
 def test_more_than_480_trees_stay_on_the_fast_path(capi, oracle, tmp_path):

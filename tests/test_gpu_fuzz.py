@@ -102,7 +102,7 @@ def _neighbours(thr):
 
 
 @pytest.mark.parametrize("duo", [1, 0], ids=["duo", "nodes8"])
-def test_rows_with_missing_entries_in_any_number(capi, oracle, tmp_path, duo):
+def test_any_number_of_rows_with_missing_entries(capi, oracle, tmp_path, duo):
     """The seal kernel orders each tile's rows (clean first) so that only warps holding rows with missing entries
     take the default-direction walk: any number of such rows per tile — none, one, a warp's worth +-1, all — in the
     first, a middle and the ragged last tile must give the oracle's leaf ids and sums, on both layouts."""
@@ -130,10 +130,6 @@ def test_rows_with_missing_entries_in_any_number(capi, oracle, tmp_path, duo):
             fam = ("duo" if duo else "nodes8") + ("_missing" if nmiss else "")
             assert capi.last_predict_kernel() == fam
             assert np.array_equal(b.predict(d, option_mask=2), om.predict(x, option_mask=2)), nmiss
-            for persist in (1,) if duo else ():
-                capi.set_param("persist", persist)
-                assert np.array_equal(b.predict(d, ntree_limit=7).view(np.uint32), om.predict(x, ntree_limit=7).view(np.uint32))
-                capi.set_param("persist", -1)
+            assert np.array_equal(b.predict(d, ntree_limit=7).view(np.uint32), om.predict(x, ntree_limit=7).view(np.uint32)), nmiss
     finally:
         capi.set_param("duo", -1)
-        capi.set_param("persist", -1)

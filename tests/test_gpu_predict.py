@@ -197,59 +197,31 @@ def test_device_resident_predict_and_epilogue(capi, oracle, small_model_path, sm
     assert rel.max() <= REL_TOL_OH
 
 
-def test_kernel_variants_agree(capi, oracle, small_model_path, small_forest):
-    """Every tunable build of the predict kernel (trees in flight, residency target, parked lanes on/off)
-    gives the same bits; the clean matrix exercises the no-missing specialisation."""
-    x = synth.quick_features(synth.raw_fields(8))
-    ref = oracle.Model(small_model_path).predict(x)
-    b = capi.Booster(small_model_path)
-    d = capi.DMatrix(x)
-    try:
-        for park in (0, 1):
-            capi.set_param("park", park)
-            for ilp in (1, 2, 3, 4, 6, 8):
-                for minb in (3, 4, 5, 6):
-                    capi.set_param("ilp", ilp)
-                    capi.set_param("minb", minb)
-                    assert np.array_equal(b.predict(d).view(np.uint32), ref.view(np.uint32)), (park, ilp, minb)
-        capi.set_param("ilp", 0)
-        capi.set_param("minb", 0)
-        capi.set_param("park", -1)
-        for top in (0, 3, 4, 5, 6, -1):  # tree levels served from constant memory
-            capi.set_param("top_levels", top)
-            for variant in (-1, 0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12):  # LSU / texture-pipe mixes
-                capi.set_param("variant", variant)
-                assert np.array_equal(b.predict(d).view(np.uint32), ref.view(np.uint32)), (top, variant)
-        capi.set_param("variant", 0)
-        capi.set_param("top_levels", -1)
-        # two-level records: default shape and the experiment grid (an unknown combination runs the default)
-        capi.set_param("duo", 1)
-        for ilp, minb, mask in ((0, 0, 0), (4, 6, 0xA), (4, 6, 0xE), (4, 6, 0xF), (3, 6, 0x6), (3, 6, 0x2), (6, 5, 0x2A),
-                                (8, 4, 0xEE), (5, 5, 0x1)):  # fmt: skip
-            capi.set_param("ilp", ilp)
-            capi.set_param("minb", minb)
-            capi.set_param("duo_mask", mask)
-            assert np.array_equal(b.predict(d).view(np.uint32), ref.view(np.uint32)), ("duo", ilp, minb, mask)
-            for nt in (1, 5, 7, 11):  # group remainders: 6-wide, 3-wide, single
-                assert np.array_equal(b.predict(d, ntree_limit=nt).view(np.uint32),
-                                      oracle.Model(small_model_path).predict(x, ntree_limit=nt).view(np.uint32)), (ilp, nt)
-        capi.set_param("ilp", 0)
-        capi.set_param("minb", 0)
-        capi.set_param("duo_mask", 0)
-        capi.set_param("duo", -1)
-        xm = inject_specials(x, small_forest, np.random.default_rng(5))  # the has-missing build with the table
-        refm = oracle.Model(small_model_path).predict(xm)
-        for top in (0, 4):
-            capi.set_param("top_levels", top)
-            assert np.array_equal(b.predict(capi.DMatrix(xm)).view(np.uint32), refm.view(np.uint32)), top
-    finally:
-        capi.set_param("ilp", 0)
-        capi.set_param("minb", 0)
-        capi.set_param("park", -1)
-        capi.set_param("variant", 0)
-        capi.set_param("top_levels", -1)
-        capi.set_param("duo_mask", 0)
-        capi.set_param("duo", -1)
+def test_launch_shapes_agree(capi, oracle, tmp_path, small_model_path, small_forest, duo_mode):
+    """Every launch shape of the predict kernels gives the oracle's bits, on both layouts of the duo_mode fixture.
+    The two-level records run in the shallow shape on the small forest and in the default 6-wide shape on a forest
+    whose records average more than 4 KB per tree; the 8-byte nodes run with the constant-memory table.
+    ntree_limit 1, 5, 7 and 11 end the walks in the narrower groups (6-wide, 3-wide, single tree), and a matrix
+    with missing entries takes the default-direction walk.  The 8-byte nodes without the table and the LSU-only
+    fetch are covered by test_wide_tree_records_without_default_bits (nodes8_missing) and by the single-tree tail
+    of every group walk."""
+    deep = synth.random_forest_structure(13, 11, seed=6, p_leaf=0.12)
+    deep_path = str(tmp_path / "deep.model")
+    xgbmodel.write_legacy_binary(deep, deep_path)
+    family = "duo" if duo_mode else "nodes8"
+    rng = np.random.default_rng(5)
+    for path, forest, x in ((small_model_path, small_forest, synth.quick_features(synth.raw_fields(8))),
+                            (deep_path, deep, rng.normal(0, 1, (20000, 27)).astype(np.float32))):  # fmt: skip
+        b, om = capi.Booster(path), oracle.Model(path)
+        if forest is deep:
+            assert b.duo()[0].nbytes >= 4096 * deep.num_trees  # not a shallow forest: the default launch shape
+        d = capi.DMatrix(x)
+        for nt in (0, 1, 5, 7, 11):
+            assert np.array_equal(b.predict(d, ntree_limit=nt).view(np.uint32), om.predict(x, ntree_limit=nt).view(np.uint32)), (path, nt)
+            assert capi.last_predict_kernel() == family
+        xm = inject_specials(x, forest, rng)
+        assert np.array_equal(b.predict(capi.DMatrix(xm)).view(np.uint32), om.predict(xm).view(np.uint32)), path
+        assert capi.last_predict_kernel() == family + "_missing"
 
 
 def test_pipelined_create_matches_plain_path(capi, oracle, tmp_path, small_model_path, small_forest):

@@ -29,10 +29,4 @@ for m in ("100x6", "100x10", "30x6"):
                 continue
             print(json.dumps(dict(model=m, duo=val, ntree_limit=lim, ms=round(t(b, lim), 4), kernel=capi.last_predict_kernel())), flush=True)
     capi.set_param("duo", -1)
-    if os.environ.get("QCOH_LIB"):
-        for shp in ("6:5:0x100", "4:6:0x100", "4:6:0xF", "6:5:0x3F"):
-            ilp, minb, mask = (int(v, 0) for v in shp.split(":"))
-            capi.set_param("duo", 1); capi.set_param("ilp", ilp); capi.set_param("minb", minb); capi.set_param("duo_mask", mask)
-            print(json.dumps(dict(model=m, shape=shp, ms=round(t(b), 4), kernel=capi.last_predict_kernel())), flush=True)
-        capi.set_param("duo", -1); capi.set_param("ilp", 0); capi.set_param("minb", 0); capi.set_param("duo_mask", 0)
     b.free()

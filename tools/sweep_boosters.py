@@ -10,7 +10,7 @@
     default-direction test, against the clean matrix;
 (c) one model day of 24 hourly steps with compute_once_per_day (1 boost step + 23 steps that reuse the persistent
     OH_ML), fields resident in HBM.
-    python tools/sweep_boosters.py [--grid 180] [--grow-only] [--part a,b,c] [--persist -1]"""
+    python tools/sweep_boosters.py [--grid 180] [--grow-only] [--part a,b,c]"""
 import argparse
 import json
 import os
@@ -30,7 +30,6 @@ ap.add_argument("--grow-only", action="store_true")
 ap.add_argument("--trees", default="10,30,100,500,1000")
 ap.add_argument("--depths", default="6,10,14,18")
 ap.add_argument("--part", default="a,b,d,c")
-ap.add_argument("--persist", default="-1", help="comma list of qcoh_set_param persist values to time (sweep a)")
 ap.add_argument("--iters", type=int, default=10)
 a = ap.parse_args()
 os.makedirs(os.path.join(ROOT, "build"), exist_ok=True)
@@ -141,11 +140,8 @@ if "a" in parts:
         p = model_file(t, d)
         b = capi.Booster(p)
         dX, hx = matrix(b)
-        for persist in a.persist.split(","):
-            capi.set_param("persist", persist)
-            ms = time_predict(b, dX)
-            row(b, dX, hx, ms, sweep="trees x depth", persist=int(persist), grown=t in GROWN)
-        capi.set_param("persist", -1)
+        ms = time_predict(b, dX)
+        row(b, dX, hx, ms, sweep="trees x depth", grown=t in GROWN)
         b.free()
         if t not in GROWN:
             os.remove(p)
