@@ -301,9 +301,9 @@ int qcoh_oh_run1(qcoh_oh_handle h, const qcoh_run1_in *in, qcoh_run1_out *out) {
     CU(launch_oh_sums(r, g.stream));
     B(o->booster);  // the handle holds a reference (XGBoosterFree refuses while it does); checked all the same
     upload(o->booster);
-    sync_const_top(o->booster, true);  // tiles walk the two-level records when the booster qualifies
     CU(cudaMemsetAsync(r.OH_ML, 0, n3 * 4, g.stream));  // self%OH_ML = 0.0 (:1559)
-    const bool too_many_trees = o->booster->dev.ntree > kRangeTrees;  // ranged launches need the matrix form
+    const int ntree = o->booster->dev.ntree;
+    const bool too_many_trees = ntree > kRangeTrees;  // ranged launches need the matrix form
     if (npred && !out->X && !too_many_trees) {
       // fused: pack (:303-345) + create (:347) + predict (:356) + 10**x (:369) * OHscale (:1569) in one
       // kernel reading the SoA fields; the [N x 27] matrix is never formed
@@ -315,11 +315,11 @@ int qcoh_oh_run1(qcoh_oh_handle h, const qcoh_run1_in *in, qcoh_run1_out *out) {
       s2[0] = r.lat_deg, s2[21] = r.so3, s2[22] = r.ALBUV, s2[26] = r.SZA;
       for (int f = 0; f < 27; ++f) a.src3[f] = s3[f], a.src2[f] = s2[f];
       a.ple = r.PLE_BST, a.ncol = nc, a.e0 = (uint64_t)(k1 - 1) * nc, a.nrow = npred, a.missing = c.missing;
-      a.ntree_used = o->booster->dev.ntree, a.exp10 = 1, a.scale = c.ohscale;
+      a.ntree_used = ntree, a.exp10 = 1, a.scale = c.ohscale;
       a.out = r.OH_ML + (size_t)(k1 - 1) * nc;
       a.pred = out->pred ? o->pred.need(npred) : nullptr;
       a.flags = r.ctl + 2;
-      CU(launch_predict_soa(o->booster->dev, a, g.stream));
+      CU(launch_predict_soa(o->booster->dev, hold(o->booster, 0, ntree), a, g.stream));
       if (out->pred) deliver(out->pred, a.pred, npred);
       check_inf_after = true;
     } else if (npred) {
@@ -335,13 +335,13 @@ int qcoh_oh_run1(qcoh_oh_handle h, const qcoh_run1_in *in, qcoh_run1_out *out) {
       CU(launch_seal_tiles(X, npred, 27, c.missing, Xt, r.ctl + 3, g.stream));
       PredictArgs a;
       a.Xt = Xt, a.nrow = npred, a.ncol = 27, a.has_missing = flags & 1, a.pred_leaf = 0;
-      a.tree_begin = 0, a.tree_end = o->booster->dev.ntree, a.out_stride = a.tree_end;
+      a.tree_begin = 0, a.tree_end = ntree, a.out_stride = a.tree_end;
       a.exp10 = 1, a.scale = c.ohscale;
       a.out = r.OH_ML + (size_t)(k1 - 1) * nc;
-      launch_predict_chunked(o->booster, a, true, g.stream);
+      launch_predict_chunked(o->booster, a, g.stream);
       if (out->pred) {
         a.exp10 = 0, a.scale = 1.f, a.out = o->pred.need(npred);
-        launch_predict_chunked(o->booster, a, true, g.stream);
+        launch_predict_chunked(o->booster, a, g.stream);
         deliver(out->pred, a.out, npred);
       }
       if (out->X) deliver(out->X, X, npred * 27);

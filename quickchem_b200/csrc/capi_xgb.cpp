@@ -15,6 +15,23 @@
 using namespace qcoh;
 
 namespace qcoh {
+// n elements of device memory p as a 1-D linear texture
+template <class T>
+static cudaTextureObject_t linear_texture(T *p, size_t n) {
+  cudaResourceDesc rd;
+  memset(&rd, 0, sizeof rd);
+  rd.resType = cudaResourceTypeLinear;
+  rd.res.linear.devPtr = p;
+  rd.res.linear.desc = cudaCreateChannelDesc<T>();
+  rd.res.linear.sizeInBytes = n * sizeof(T);
+  cudaTextureDesc td;
+  memset(&td, 0, sizeof td);
+  td.readMode = cudaReadModeElementType;
+  cudaTextureObject_t t = 0;
+  CU(cudaCreateTextureObject(&t, &rd, &td, nullptr));
+  return t;
+}
+
 void upload(Booster *b) {
   if (b->uploaded) return;
   if (!b->loaded) throw Error("Booster has no model: call XGBoosterLoadModel first");
@@ -47,44 +64,19 @@ void upload(Booster *b) {
     CU(cudaMemcpy(b->d_depth.need(dd.size()), dd.data(), dd.size() * 4, cudaMemcpyHostToDevice));
   }
   CU(cudaMemcpy(b->d_orig.need(nn), f.orig_id.data(), nn * 4, cudaMemcpyHostToDevice));
+  if (b->dev.tex) cudaDestroyTextureObject(b->dev.tex);
+  if (b->dev.tex4) cudaDestroyTextureObject(b->dev.tex4);
+  b->dev = DeviceForest();
   b->dev.nodes = b->d_nodes.p, b->dev.tree_offset = b->d_off.p, b->dev.tree_depth = b->d_depth.p, b->dev.orig_id = b->d_orig.p;
   b->dev.ntree = (int32_t)b->host.trees.size();
   b->dev.nfeat = (int32_t)b->host.num_feature;
-  b->dev.max_depth = f.max_depth;
-  b->dev.num_nodes = f.num_nodes();
   b->dev.base_score = b->host.base_score;
-  b->dev.sum_depth = 0;
-  for (int32_t d : f.tree_depth) b->dev.sum_depth += d;
-  if (b->dev.tex) cudaDestroyTextureObject(b->dev.tex);
-  b->dev.tex = 0;
-  if (nn > 0 && nn < ((size_t)1 << 27)) {
-    cudaResourceDesc rd;
-    memset(&rd, 0, sizeof rd);
-    rd.resType = cudaResourceTypeLinear;
-    rd.res.linear.devPtr = b->d_nodes.p;
-    rd.res.linear.desc = cudaCreateChannelDesc<uint2>();
-    rd.res.linear.sizeInBytes = nn * 8;
-    cudaTextureDesc td;
-    memset(&td, 0, sizeof td);
-    td.readMode = cudaReadModeElementType;
-    CU(cudaCreateTextureObject(&b->dev.tex, &rd, &td, nullptr));
-  }
+  if (nn > 0 && nn < ((size_t)1 << 27)) b->dev.tex = linear_texture(b->d_nodes.p, nn);
   // two-level records, when every tree qualifies
-  if (b->dev.tex4) cudaDestroyTextureObject(b->dev.tex4);
-  b->dev.tex4 = 0, b->dev.recs = nullptr, b->dev.duo_ready = 0, b->dev.duo_has_dl = 0, b->dev.duo_blk_mul = 0, b->dev.duo_shallow = 0;
   if (b->duo.ok && b->duo.num_slots() > 0 && b->duo.num_slots() < ((int64_t)1 << 27)) {
     const size_t ns = (size_t)b->duo.num_slots();
     CU(cudaMemcpy(b->d_recs.need(ns), b->duo.rec.data(), ns * 16, cudaMemcpyHostToDevice));
-    cudaResourceDesc rd;
-    memset(&rd, 0, sizeof rd);
-    rd.resType = cudaResourceTypeLinear;
-    rd.res.linear.devPtr = b->d_recs.p;
-    rd.res.linear.desc = cudaCreateChannelDesc<uint4>();
-    rd.res.linear.sizeInBytes = ns * 16;
-    cudaTextureDesc td;
-    memset(&td, 0, sizeof td);
-    td.readMode = cudaReadModeElementType;
-    CU(cudaCreateTextureObject(&b->dev.tex4, &rd, &td, nullptr));
+    b->dev.tex4 = linear_texture(b->d_recs.p, ns);
     b->dev.recs = b->d_recs.p;
     b->dev.duo_has_dl = b->duo.has_default_bits ? 1 : 0;
     b->dev.duo_shallow = (int64_t)ns * 16 < kShallowRecBytesPerTree * std::max<int64_t>(1, b->dev.ntree) ? 1 : 0;
@@ -94,59 +86,47 @@ void upload(Booster *b) {
 }
 
 // The constant-memory tables of tree tops exist once per device (one __constant__ bank per loaded module and
-// device), and a device is driven by exactly one host thread (context.hpp): they hold one range of
-// <= kConstTreesMax trees of one booster at a time, in one of two layouts — the first levels
+// device), and a device is driven by exactly one host thread (context.hpp), so what they hold is tracked per
+// thread: one window of <= kConstTreesMax trees of one booster version, in one of two layouts — the first levels
 // of the depth-ordered nodes (walk_group), or the complete heap-ordered tops of the two-level records
-// (walk_group_duo).  The owner tag below is therefore per device = per thread; everything else a launch needs
-// travels in the booster's DeviceForest.  allow_duo = false forces the 8-byte-node layout.
-static thread_local uint64_t g_const_top_owner = 0;
-static thread_local bool g_const_top_duo = false;  // the layout the table holds: two-level tops or 8-byte-node tops
-static thread_local int g_const_tree0 = 0, g_const_ntree = 0;
-bool duo_wanted(const Booster *b) { return b->dev.recs != nullptr && b->dev.tex != 0 && g.duo != 0; }
-void sync_const_top(Booster *b, bool allow_duo, int tree0, int ntree) {
-  b->dev.const_top_levels = 0, b->dev.duo_ready = 0, b->dev.const_tree0 = 0, b->dev.const_ntree = 0;
-  if (ntree < 0) ntree = std::min(b->dev.ntree - tree0, kConstTreesMax);
-  if (ntree <= 0 || ntree > kConstTreesMax || tree0 + ntree > b->dev.ntree) return;
+// (walk_group_duo) when the booster has records and a node texture and `duo` is not 0.
+static thread_local struct {
+  uint64_t owner = 0;  // Booster::version of the trees the window holds, 0 = none
+  ConstWindow w;
+} g_const;
+
+ConstWindow hold(Booster *b, int tree0, int ntree) {
+  if (ntree <= 0 || ntree > kConstTreesMax || tree0 + ntree > b->dev.ntree) return {};
   // The table holds a window of up to kConstTreesMax trees: the aligned window around the request when the request
   // fits in it (so that ranges of one forest and calls with different ntree_limit share an upload), else one that
   // starts at the request.
   int w0 = tree0 - tree0 % kConstTreesMax;
   if (tree0 + ntree > w0 + kConstTreesMax) w0 = tree0;
-  const int hold = std::min(b->dev.ntree - w0, kConstTreesMax);
-  auto holds = [&](bool duo) {
-    return g_const_top_owner == b->version && g_const_top_duo == duo && g_const_tree0 <= tree0 &&
-           tree0 + ntree <= g_const_tree0 + g_const_ntree;
-  };
-  if (allow_duo && duo_wanted(b)) {
-    if (!holds(true)) {
-      g_const_top_owner = 0;
-      if (upload_const_duo(b->duo.top_xy.data() + (size_t)w0 * (2u << kDuoTop), b->duo.tree_slot.data() + w0, hold, g.stream) ==
-          cudaSuccess) {
-        g_const_top_owner = b->version, g_const_top_duo = true, g_const_tree0 = w0, g_const_ntree = hold;
-      } else {
-        (void)cudaGetLastError();
-      }
-    }
-    if (holds(true)) {
-      b->dev.duo_ready = 1, b->dev.const_tree0 = g_const_tree0, b->dev.const_ntree = g_const_ntree;
-      return;
-    }
-  }
-  if (!holds(false)) {
-    g_const_top_owner = 0;
-    if (upload_const_top(b->dev_nodes_host.data(), b->flat.tree_offset.data() + w0, hold, g.stream) != cudaSuccess) {
+  const int n = std::min(b->dev.ntree - w0, kConstTreesMax);
+  auto held = [&](TopLayout l) { return g_const.owner == b->version && g_const.w.holds(l, tree0, tree0 + ntree); };
+  // stream-ordered re-fill; a failed upload leaves the table unowned and the launch runs without it
+  auto fill = [&](TopLayout l) {
+    g_const.owner = 0;
+    const cudaError_t e = l == TopLayout::kRecordTops
+                              ? upload_const_duo(b->duo.top_xy.data() + (size_t)w0 * (2u << kDuoTop), b->duo.tree_slot.data() + w0, n, g.stream)
+                              : upload_const_top(b->dev_nodes_host.data(), b->flat.tree_offset.data() + w0, n, g.stream);
+    if (e != cudaSuccess) {
       (void)cudaGetLastError();
-      return;  // does not fit: the kernel runs without the table
+      return false;
     }
-    g_const_top_owner = b->version, g_const_top_duo = false, g_const_tree0 = w0, g_const_ntree = hold;
-  }
-  b->dev.const_top_levels = kDuoTop, b->dev.const_tree0 = g_const_tree0, b->dev.const_ntree = g_const_ntree;
+    g_const.owner = b->version, g_const.w = ConstWindow{l, w0, n};
+    return true;
+  };
+  const bool records = b->dev.recs != nullptr && b->dev.tex != 0 && g.duo != 0;
+  if (records && (held(TopLayout::kRecordTops) || fill(TopLayout::kRecordTops))) return g_const.w;
+  if (held(TopLayout::kNodeTops) || fill(TopLayout::kNodeTops)) return g_const.w;
+  return {};
 }
 
 // One prediction = one launch per range of kRangeTrees trees (kernels.hpp; the tables hold kConstTreesMax and are
-// re-filled, stream-ordered, when a range leaves them) and the float32 partial sum travels through `out`, so the sum order — tree 0, 1, 2, ... — and
-// with it every bit of the result is the same as in a single launch.
-void launch_predict_chunked(Booster *b, PredictArgs a, bool allow_duo, cudaStream_t s) {
+// re-filled, stream-ordered, when a range leaves them) and the float32 partial sum travels through `out`, so the sum
+// order — tree 0, 1, 2, ... — and with it every bit of the result is the same as in a single launch.
+void launch_predict_chunked(Booster *b, PredictArgs a, cudaStream_t s) {
   const int t_end = a.tree_end;
   if (a.nrow == 0) return;
   if (t_end <= 0) {  // a booster without trees predicts its base score
@@ -159,11 +139,11 @@ void launch_predict_chunked(Booster *b, PredictArgs a, bool allow_duo, cudaStrea
   }
   for (int t0 = 0; t0 < t_end; t0 += kRangeTrees) {
     const int n = std::min(kRangeTrees, t_end - t0);
-    sync_const_top(b, allow_duo, t0, n);
+    const ConstWindow w = hold(b, t0, n);
     PredictArgs c = a;
     c.tree_begin = t0, c.tree_end = t0 + n;
     c.first = t0 == 0, c.last = t0 + n == t_end;
-    CU(launch_predict(b->dev, c, s));
+    CU(launch_predict(b->dev, w, c, s));
   }
 }
 
@@ -200,7 +180,7 @@ static void predict_into(Booster *b, DMatrix *d, int option_mask, unsigned ntree
   a.exp10 = epi ? epi->exp10 : 0;
   a.scale = epi ? epi->scale : 1.f;
   a.out = out_dev;
-  launch_predict_chunked(b, a, true, g.stream);
+  launch_predict_chunked(b, a, g.stream);
 }
 
 const ShapForest &shap_tables(Booster *b) {
@@ -462,7 +442,7 @@ static void create_pipelined(DMatrix *d, const float *data, Booster *b) {
     a.has_missing = ((hfl[c] & 1) || ncol < b->host.num_feature) ? 1 : 0;
     a.tree_begin = 0, a.tree_end = (int32_t)b->host.trees.size(), a.out_stride = a.tree_end;
     a.out = sdev + r0;
-    launch_predict_chunked(b, a, true, g.stream);
+    launch_predict_chunked(b, a, g.stream);
     CU(cudaEventRecord(chunk_event(2 * c + 1), g.stream));
     CU(cudaStreamWaitEvent(g.d2h_stream, chunk_event(2 * c + 1), 0));
     CU(cudaMemcpyAsync(shost + r0, sdev + r0, nr * sizeof(float), cudaMemcpyDeviceToHost, g.d2h_stream));

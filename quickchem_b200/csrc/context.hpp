@@ -60,8 +60,8 @@ struct NvtxRange {
 
 // ---- device context ---------------------------------------------------------------
 // Thread model (SURVEY.md 8e: "one process per GPU" and "one process, one host thread per device" are both
-// supported): ALL mutable library state — the device context below, the buffer pools, the constant-table owner
-// tag, the live-handle set, the model cache, the mirror's SAVE'd booster, the NCCL communicator — is
+// supported): ALL mutable library state — the device context below, the buffer pools, the constant-table
+// window, the live-handle set, the model cache, the mirror's SAVE'd booster, the NCCL communicator — is
 // thread_local.  A host thread is one "rank": it binds to one GPU (qcoh_set_device / $LOCAL_RANK) and owns the
 // handles it creates; a handle is not valid in another thread.  One thread per device: the constant-memory tables
 // are per device, so a second thread binding to a device that already has an owner is refused.
@@ -281,10 +281,11 @@ inline DMatrix *D(DMatrixHandle h) {
 
 // capi_xgb.cpp
 void upload(Booster *b);
-// make the constant-memory tables of tree tops hold trees [tree0, tree0 + ntree) of this booster (see capi_xgb.cpp)
-void sync_const_top(Booster *b, bool allow_duo, int tree0 = 0, int ntree = -1);
-// one prediction = one launch per range of kConstTreesMax trees (capi_xgb.cpp)
-void launch_predict_chunked(Booster *b, PredictArgs a, bool allow_duo, cudaStream_t s);
+// make the constant-memory tables of tree tops hold trees [tree0, tree0 + ntree) of this booster, uploading them if
+// they do not yet, and return what the tables hold (see capi_xgb.cpp)
+ConstWindow hold(Booster *b, int tree0, int ntree);
+// one prediction = one launch per range of kRangeTrees trees (capi_xgb.cpp)
+void launch_predict_chunked(Booster *b, PredictArgs a, cudaStream_t s);
 // the booster's ShapForest, built on first use (host only; throws when the booster has no covers)
 const ShapForest &shap_tables(Booster *b);
 

@@ -41,12 +41,12 @@ struct HostForest {
 //   y: meta = feat << 26 | default_left << 23 | rel   (rel = left-child index - own index; the top byte is
 //      feat * 4, so one byte-permute turns it into the byte offset feat * 1024 of the kernel's feature tile)
 // A leaf has rel = 0 and feat = num_feature: the predict kernel keeps one extra per-row
-// slot holding -inf at that feature index, so `!(v < x)` is false and the walk self-loops
-// without a leaf test.
+// slot holding key 0 at that feature index, so the compare never says "right" and the walk
+// self-loops without a leaf test.
 constexpr uint32_t kMetaFeatShift = 26;
 constexpr uint32_t kMetaDefaultLeftBit = 1u << 23;
 constexpr uint32_t kMetaRelMask = (1u << 23) - 1;
-constexpr uint32_t kMaxFeatures = 31;  // the predict kernel stages a row through 32 registers
+constexpr uint32_t kMaxFeatures = 31;  // the 5-bit feature fields of the two-level records also hold the leaf slot num_feature
 
 struct FlatForest {
   std::vector<uint32_t> nodes_xy;     // 2 words per node

@@ -3,12 +3,14 @@
 //   K3  seal_tiles_kernel     the missing / inf scan of XGDMatrixCreateFromMat (OH_GridCompMod.F90:347) fused with
 //                             the conversion of the row-major float matrix into the DMatrix's device form:
 //                             feature-major tiles of order-preserving integer keys
-//   K2b predict_tiles_kernel  tree-ensemble traversal on two-level 16-byte records (one gather per two tree
-//                             levels), replaces libxgboost's CPUPredictor behind XGBoosterPredict (reference call
-//                             site :356) with the export transform 10**x * OHscale (:369,:1569) fused as epilogue;
-//                             sums / leaf indices, clean matrices / missing entries; tiles arrive by TMA
-//   K2  predict_tiles_nodes8_kernel   the same on the 8-byte depth-ordered nodes (boosters the records do not hold)
-//       predict_soa_kernel    K2 / K2b with the tile assembled straight from the Run1 SoA fields
+//   K2  predict_tiles_kernel  tree-ensemble traversal, replaces libxgboost's CPUPredictor behind XGBoosterPredict
+//                             (reference call site :356) with the export transform 10**x * OHscale (:369,:1569) fused
+//                             as epilogue; sums / leaf indices, clean matrices / missing entries; tiles arrive by TMA.
+//                             Its walk policy picks the node layout and the launch shape: DuoWalk on the two-level
+//                             16-byte records (one gather per two tree levels), NodesWalk on the 8-byte depth-ordered
+//                             nodes (boosters the records do not hold)
+//       predict_soa_kernel    K2 with the tile assembled straight from the Run1 SoA fields
+//   K6  shap_paths / shap_reduce / shap_approx   per-feature contributions (exact TreeSHAP, approximate Saabas)
 //   K1  oh_state / oh_sums / oh_pack    Run1 feature assembly (:1240-1257, :1441-1488, :303-345)
 //   K5  oh_finalize           troposphere mask + unit conversion (:1579-1595)
 //   K4  oh_diag               build-defined mass-weighted mean OH / CH4 lifetime partial sums
@@ -32,29 +34,22 @@ uint64_t launch_count() { return g_launches; }
 
 #define QC_LAUNCHED() (++g_launches, cudaGetLastError())
 
-// launches per kernel family: what the parity tests assert ("this launch was served by the two-level kernel")
+// launches per kernel family: what the parity tests assert ("this launch was served by the two-level kernel").  The
+// predict families are ordered base, _missing, _leaf, _missing_leaf: base + has_missing + 2 * pred_leaf.
 namespace {
-struct FamilyCount {
-  char name[32];
-  uint64_t n;
-};
-thread_local FamilyCount g_family[24];
-thread_local int g_nfamily = 0;
+enum Family { kDuo, kNodes8 = kDuo + 4, kSoaDuo = kNodes8 + 4, kSoaNodes8, kSealTiles, kShap, kShapReduce, kShapApprox, kFamilies };
+const char *const kFamilyName[kFamilies] = {"duo", "duo_missing", "duo_leaf", "duo_missing_leaf", "nodes8", "nodes8_missing",
+                                            "nodes8_leaf", "nodes8_missing_leaf", "soa_duo", "soa_nodes8", "seal_tiles",
+                                            "shap", "shap_reduce", "shap_approx"};
+thread_local uint64_t g_family[kFamilies];
 thread_local const char *g_last_predict = "";
-const char *count_family(const char *base, bool hm, bool pl) {
-  char name[32];
-  snprintf(name, sizeof name, "%s%s%s", base, hm ? "_missing" : "", pl ? "_leaf" : "");
-  for (int i = 0; i < g_nfamily; ++i)
-    if (!strcmp(g_family[i].name, name)) return ++g_family[i].n, g_family[i].name;
-  if (g_nfamily == 24) return "";
-  strcpy(g_family[g_nfamily].name, name);
-  g_family[g_nfamily].n = 1;
-  return g_family[g_nfamily++].name;
-}
+void count_family(int f) { ++g_family[f]; }
+// the predict and contribution launches also record the family that served the last of them
+void count_predict(int f) { ++g_family[f], g_last_predict = kFamilyName[f]; }
 }  // namespace
 uint64_t kernel_launches(const char *family) {
-  for (int i = 0; i < g_nfamily; ++i)
-    if (!strcmp(g_family[i].name, family)) return g_family[i].n;
+  for (int i = 0; i < kFamilies; ++i)
+    if (!strcmp(kFamilyName[i], family)) return g_family[i];
   return 0;
 }
 const char *last_predict_kernel() { return g_last_predict; }
@@ -300,12 +295,12 @@ cudaError_t launch_seal_tiles(const float *X, uint64_t nrow, int ncol, float mis
   if (e != cudaSuccess) return e;
   // xgboost src/data/data.cc: `!std::isinf(missing) && std::isinf(value)` invalidates the input
   seal_tiles_kernel<<<(unsigned)ntile, kTileRows, smem, s>>>(X, nrow, ncol, missing, std::isinf(missing) ? 0 : 1, Xt, flags);
-  count_family("seal_tiles", false, false);
+  count_family(kSealTiles);
   return QC_LAUNCHED();
 }
 
 // =====================================================================================
-// K2 — walk on the 8-byte depth-ordered nodes
+// Walk on the 8-byte depth-ordered nodes
 // =====================================================================================
 // TEXMODE is a bit mask over the ILP trees in flight: tree j fetches its nodes through the texture pipe
 // (tex1Dfetch on the same buffer) if bit j is set, through the LSU (LDG) otherwise.  ctree0: the first tree
@@ -402,11 +397,11 @@ __device__ __forceinline__ void walk_group(const uint2 *__restrict__ nodes, cuda
 
 // all trees [t0, t1) on the 8-byte nodes, in tree order; emit(t, value bits, node index)
 template <int ILP, bool HAS_MISSING, int TEXMODE, int CTOP, class Emit>
-__device__ __forceinline__ void forest_walk(const DeviceForest &f, uint32_t my, int t0, int t1, Emit &&emit) {
+__device__ __forceinline__ void forest_walk(const DeviceForest &f, uint32_t my, int ctree0, int t0, int t1, Emit &&emit) {
   int t = t0;
   for (; t + ILP <= t1; t += ILP) {
     uint32_t idx[ILP], xb[ILP];
-    walk_group<ILP, HAS_MISSING, TEXMODE, CTOP>(f.nodes, f.tex, f.tree_offset, f.tree_depth, t, f.const_tree0, my, idx, xb);
+    walk_group<ILP, HAS_MISSING, TEXMODE, CTOP>(f.nodes, f.tex, f.tree_offset, f.tree_depth, t, ctree0, my, idx, xb);
 #pragma unroll
     for (int j = 0; j < ILP; ++j) emit(t + j, xb[j], idx[j]);
   }
@@ -418,19 +413,15 @@ __device__ __forceinline__ void forest_walk(const DeviceForest &f, uint32_t my, 
 }
 
 // =====================================================================================
-// K2b — walk on the two-level records (forest.hpp DuoForest)
+// Walk on the two-level records (forest.hpp DuoForest)
 // =====================================================================================
 // Levels 0..3 come from constant memory as complete heap-ordered tops (entry i, children 2i and 2i + 1: no
 // branch, no predicate); from level 4 on one 16-byte record {root, left, right thresholds; features; block
 // pointer} decides two levels, and the four possible successors are contiguous.  Against the 8-byte nodes
 // this halves the dependent gathers of a walk and takes ~40 % of the distinct lines per warp request off the
 // L1TEX data pipes (tools/replay_two_level_records.py).
-// Default shape (B200, profiles/README.md "two-level records"): 6 trees in flight, 4 of them gathering through
-// the texture pipe, 5 resident CTAs per SM — LSU and TEX data pipes, ALU and issue slots all end up at
-// 76-86 % busy.
 // HAS_MISSING: a missing entry (key 0xFFFFFFFF) takes the node's default child (bits 17..15 of w3 / bit 0 of a
 // top entry's y word); the records carry those bits when DeviceForest::duo_has_dl.
-constexpr int kDuoIlp = 6, kDuoTexMask = 0x36, kDuoMinBlocks = 5;
 template <int ILP, int TEXMODE, bool HAS_MISSING>
 __device__ __forceinline__ void walk_group_duo(const uint4 *__restrict__ recs, cudaTextureObject_t tex4,
                                                const int32_t *__restrict__ tdepth, uint32_t blk_mul, int t, int ctree0, uint32_t my_saddr,
@@ -535,11 +526,11 @@ __device__ __forceinline__ void walk_group_duo(const uint4 *__restrict__ recs, c
 // the texture pipe), then one by one — always in tree order (float32 sum order is part of parity).
 // emit(t, leaf value bits, XGBoost node id of the leaf)
 template <int ILP, int TEXMODE, bool HAS_MISSING, class Emit>
-__device__ __forceinline__ void forest_walk_duo(const DeviceForest &f, uint32_t my, int t0, int t1, Emit &&emit) {
+__device__ __forceinline__ void forest_walk_duo(const DeviceForest &f, uint32_t my, int ctree0, int t0, int t1, Emit &&emit) {
   int t = t0;
   for (; t + ILP <= t1; t += ILP) {
     uint32_t xb[ILP], id[ILP];
-    walk_group_duo<ILP, TEXMODE, HAS_MISSING>(f.recs, f.tex4, f.tree_depth, f.duo_blk_mul, t, f.const_tree0, my, xb, id);
+    walk_group_duo<ILP, TEXMODE, HAS_MISSING>(f.recs, f.tex4, f.tree_depth, f.duo_blk_mul, t, ctree0, my, xb, id);
 #pragma unroll
     for (int j = 0; j < ILP; ++j) emit(t + j, xb[j], id[j]);
   }
@@ -547,17 +538,55 @@ __device__ __forceinline__ void forest_walk_duo(const DeviceForest &f, uint32_t 
   if (H >= 2) {
     for (; t + H <= t1; t += H) {
       uint32_t xb[H > 0 ? H : 1], id[H > 0 ? H : 1];
-      walk_group_duo<(H > 0 ? H : 1), ((1 << H) - 2), HAS_MISSING>(f.recs, f.tex4, f.tree_depth, f.duo_blk_mul, t, f.const_tree0, my, xb, id);
+      walk_group_duo<(H > 0 ? H : 1), ((1 << H) - 2), HAS_MISSING>(f.recs, f.tex4, f.tree_depth, f.duo_blk_mul, t, ctree0, my, xb, id);
 #pragma unroll
       for (int j = 0; j < H; ++j) emit(t + j, xb[j], id[j]);
     }
   }
   for (; t < t1; ++t) {
     uint32_t xb[1], id[1];
-    walk_group_duo<1, 0, HAS_MISSING>(f.recs, f.tex4, f.tree_depth, f.duo_blk_mul, t, f.const_tree0, my, xb, id);
+    walk_group_duo<1, 0, HAS_MISSING>(f.recs, f.tex4, f.tree_depth, f.duo_blk_mul, t, ctree0, my, xb, id);
     emit(t, xb[0], id[0]);
   }
 }
+
+// ---- walk policies: which walk a launch runs, and its launch shape ------------------------------------------
+// run<HAS_MISSING, PRED_LEAF>(f, my, ctree0, t0, t1, emit) walks trees [t0, t1) of one row in tree order and calls
+// emit(t, leaf value bits, XGBoost node id of the leaf); the node id is looked up only when PRED_LEAF.
+// walks_missing(f): whether a row with missing entries may take this walk.
+template <int ILP, int TEXMASK, int MINB>
+struct DuoWalk {
+  static constexpr int kMinBlocks = MINB, kFamily = kDuo;
+  __device__ static bool walks_missing(const DeviceForest &f) { return f.duo_has_dl != 0; }
+  template <bool HAS_MISSING, bool PRED_LEAF, class Emit>
+  __device__ __forceinline__ static void run(const DeviceForest &f, uint32_t my, int ctree0, int t0, int t1, Emit &&emit) {
+    forest_walk_duo<ILP, TEXMASK, HAS_MISSING>(f, my, ctree0, t0, t1, emit);
+  }
+};
+template <int ILP, int TEXMASK, int CTOP, int MINB>
+struct NodesWalk {
+  static constexpr int kMinBlocks = MINB, kFamily = kNodes8;
+  __device__ static bool walks_missing(const DeviceForest &) { return true; }
+  template <bool HAS_MISSING, bool PRED_LEAF, class Emit>
+  __device__ __forceinline__ static void run(const DeviceForest &f, uint32_t my, int ctree0, int t0, int t1, Emit &&emit) {
+    forest_walk<ILP, HAS_MISSING, TEXMASK, CTOP>(f, my, ctree0, t0, t1, [&](int t, uint32_t xb, uint32_t idx) {
+      emit(t, xb, PRED_LEAF ? (uint32_t)__ldg(f.orig_id + idx) : 0u);
+    });
+  }
+};
+
+// The launch shapes (B200; measurements in profiles/README.md):
+//   two-level records, default ("two-level records"): 6 trees in flight, 4 of them (mask 0x36) gathering through the
+//     texture pipe, 5 resident CTAs per SM — LSU and TEX data pipes, ALU and issue slots all end up at 76-86 % busy
+//   two-level records, shallow (kernels.hpp kShallowRecBytesPerTree): 4 trees in flight, 6 resident CTAs
+//   8-byte nodes: 4 trees in flight, 6 resident CTAs; levels 0..3 of every tree from constant memory when the table
+//     holds them; below that trees 1 and 3 of each group fetch their nodes through the texture pipe and trees 0 and 2
+//     through the LSU (mask 0xA), or all through the LSU when the booster has no node texture
+using RecordsWalk = DuoWalk<6, 0x36, 5>;
+using RecordsShallowWalk = DuoWalk<4, 0xA, 6>;
+using NodesTableWalk = NodesWalk<4, 0xA, kDuoTop, 6>;
+using NodesTexWalk = NodesWalk<4, 0xA, 0, 6>;
+using NodesLsuWalk = NodesWalk<4, 0, 0, 6>;
 
 __device__ __forceinline__ float export_transform(float acc, int exp10_on, float scale) {
   if (!exp10_on) return acc;
@@ -599,8 +628,8 @@ __device__ __forceinline__ uint64_t tile_row(uint32_t buf, uint64_t tile, int ti
   return tile * kTileRows + orig;
 }
 
-template <int ILP, int MINB, int TEXMODE, bool HAS_MISSING, bool PRED_LEAF>
-__global__ void __launch_bounds__(kBlock, MINB) predict_tiles_kernel(DeviceForest f, PredictArgs a) {
+template <class Walk, bool HAS_MISSING, bool PRED_LEAF>
+__global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_tiles_kernel(DeviceForest f, PredictArgs a) {
   extern __shared__ __align__(128) uint32_t skey[];
   __shared__ __align__(8) unsigned long long bars[1];
   const int tid = threadIdx.x;
@@ -613,32 +642,9 @@ __global__ void __launch_bounds__(kBlock, MINB) predict_tiles_kernel(DeviceFores
     const uint64_t row = tile_row<HAS_MISSING>(buf, pipe.tile, tid, a.ncol < f.nfeat, hm);
     row_result<PRED_LEAF>(f, a, row, row < a.nrow, [&](auto &&emit) {
       if (HAS_MISSING && hm)
-        forest_walk_duo<ILP, TEXMODE, true>(f, my, a.tree_begin, a.tree_end, emit);
+        Walk::template run<true, PRED_LEAF>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
       else
-        forest_walk_duo<ILP, TEXMODE, false>(f, my, a.tree_begin, a.tree_end, emit);
-    });
-    pipe.release(tid);
-  }
-}
-
-template <int ILP, bool HAS_MISSING, bool PRED_LEAF, int MINB, int TEXMODE, int CTOP>
-__global__ void __launch_bounds__(kBlock, MINB) predict_tiles_nodes8_kernel(DeviceForest f, PredictArgs a) {
-  extern __shared__ __align__(128) uint32_t skey[];
-  __shared__ __align__(8) unsigned long long bars[1];
-  const int tid = threadIdx.x;
-  TilePipe pipe;
-  pipe.begin(skey, bars, a, f.nfeat, HAS_MISSING, tid);
-  while (pipe.more()) {
-    const uint32_t buf = pipe.acquire(tid);
-    const uint32_t my = buf + 4u * (uint32_t)(kStride + tid);
-    bool hm;
-    const uint64_t row = tile_row<HAS_MISSING>(buf, pipe.tile, tid, a.ncol < f.nfeat, hm);
-    row_result<PRED_LEAF>(f, a, row, row < a.nrow, [&](auto &&emit) {
-      auto leaf = [&](int t, uint32_t xb, uint32_t idx) { emit(t, xb, PRED_LEAF ? (uint32_t)__ldg(f.orig_id + idx) : 0u); };
-      if (HAS_MISSING && hm)
-        forest_walk<ILP, true, TEXMODE, CTOP>(f, my, a.tree_begin, a.tree_end, leaf);
-      else
-        forest_walk<ILP, false, TEXMODE, CTOP>(f, my, a.tree_begin, a.tree_end, leaf);
+        Walk::template run<false, PRED_LEAF>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
     });
     pipe.release(tid);
   }
@@ -650,10 +656,10 @@ __global__ void __launch_bounds__(kBlock, MINB) predict_tiles_nodes8_kernel(Devi
 // field, so every load is coalesced and lands directly in the transposed tile — the [N x 27] matrix is
 // never formed, and no transposition is needed.  Whether a tile holds missing entries is decided per
 // tile (block-wide OR) and selects the walk specialisation at run time; +-inf raises the error flag.
-// DUO: the constant table holds the heap-ordered tops of the two-level records; a tile with missing entries
-// walks them too when they carry the default bits, else the 8-byte nodes without a table (CTOP must be 0).
-template <int TEXMODE, int CTOP, bool DUO = false>
-__global__ void __launch_bounds__(kBlock, DUO ? kDuoMinBlocks : 6) predict_soa_kernel(DeviceForest f, SoaArgs a) {
+// Walk serves the tiles, and the tiles with missing entries too when it walks_missing(); MissingWalk serves those
+// otherwise (the two-level records without the default bits).
+template <class Walk, class MissingWalk>
+__global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_soa_kernel(DeviceForest f, SoaArgs a) {
   extern __shared__ __align__(128) uint32_t skey[];
   const int tid = threadIdx.x;
   constexpr int B = kBlock;
@@ -690,34 +696,47 @@ __global__ void __launch_bounds__(kBlock, DUO ? kDuoMinBlocks : 6) predict_soa_k
   const uint32_t my = (uint32_t)__cvta_generic_to_shared(skey + tid);
   float acc = f.base_score;
   auto add = [&](int, uint32_t xb, uint32_t) { acc = __fadd_rn(acc, __uint_as_float(xb)); };
-  if (DUO && (!tile_missing || f.duo_has_dl)) {
+  if (!tile_missing || Walk::walks_missing(f)) {
     if (tile_missing)
-      forest_walk_duo<kDuoIlp, kDuoTexMask, true>(f, my, 0, a.ntree_used, add);
+      Walk::template run<true, false>(f, my, a.ctree0, 0, a.ntree_used, add);
     else
-      forest_walk_duo<kDuoIlp, kDuoTexMask, false>(f, my, 0, a.ntree_used, add);
-  } else if (tile_missing) {
-    forest_walk<4, true, TEXMODE, CTOP>(f, my, 0, a.ntree_used, add);
+      Walk::template run<false, false>(f, my, a.ctree0, 0, a.ntree_used, add);
   } else {
-    forest_walk<4, false, TEXMODE, CTOP>(f, my, 0, a.ntree_used, add);
+    MissingWalk::template run<true, false>(f, my, a.ctree0, 0, a.ntree_used, add);
   }
   if (a.pred) a.pred[m] = acc;
   a.out[m] = export_transform(acc, a.exp10, a.scale);
 }
 
-cudaError_t launch_predict_soa(const DeviceForest &f, const SoaArgs &a, cudaStream_t s) {
-  if (a.nrow == 0) return cudaSuccess;
+// The layout rule of the predict launches: the two-level records when the window holds the record tops of trees
+// [t0, t1) and the rows have no missing entries or the records carry the default bits; otherwise the 8-byte nodes,
+// with the table when the window holds their node tops, and through the LSU alone when there is no node texture.
+enum class Layout { kRecords, kNodesTable, kNodesTex, kNodesLsu };
+static Layout layout(const DeviceForest &f, const ConstWindow &w, int t0, int t1, bool has_missing) {
+  if (w.holds(TopLayout::kRecordTops, t0, t1) && (!has_missing || f.duo_has_dl)) return Layout::kRecords;
+  if (f.tex == 0) return Layout::kNodesLsu;
+  return w.holds(TopLayout::kNodeTops, t0, t1) ? Layout::kNodesTable : Layout::kNodesTex;
+}
+
+cudaError_t launch_predict_soa(const DeviceForest &f, const ConstWindow &w, const SoaArgs &args, cudaStream_t s) {
+  if (args.nrow == 0) return cudaSuccess;
   if (f.nfeat != 27) return cudaErrorInvalidValue;
   const size_t smem = (size_t)kStride * 28 * sizeof(float);
-  const uint64_t nblk = (a.nrow + kBlock - 1) / kBlock;
+  const uint64_t nblk = (args.nrow + kBlock - 1) / kBlock;
   if (nblk > 0x7fffffffull) return cudaErrorInvalidConfiguration;
-  const bool tex = f.tex != 0;
-  const bool duo = f.duo_ready && f.const_tree0 == 0 && f.const_ntree >= a.ntree_used;
-  auto k = !tex ? predict_soa_kernel<0, 0> : (f.const_top_levels == 4 ? predict_soa_kernel<0xA, 4> : predict_soa_kernel<0xA, 0>);
-  if (duo) k = predict_soa_kernel<0xA, 0, true>;
+  SoaArgs a = args;
+  a.ctree0 = w.tree0;
+  // whether a tile has missing entries is known only in the kernel: the layout is that of clean rows, and the
+  // kernel sends a tile with missing entries the records cannot walk to the 8-byte nodes without the table
+  const Layout l = layout(f, w, 0, a.ntree_used, false);
+  auto k = predict_soa_kernel<RecordsWalk, NodesTexWalk>;
+  if (l == Layout::kNodesTable) k = predict_soa_kernel<NodesTableWalk, NodesTableWalk>;
+  if (l == Layout::kNodesTex) k = predict_soa_kernel<NodesTexWalk, NodesTexWalk>;
+  if (l == Layout::kNodesLsu) k = predict_soa_kernel<NodesLsuWalk, NodesLsuWalk>;
   cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   k<<<dim3((unsigned)nblk), kBlock, smem, s>>>(f, a);
-  count_family(duo ? "soa_duo" : "soa_nodes8", false, false);
+  count_family(l == Layout::kRecords ? kSoaDuo : kSoaNodes8);
   return QC_LAUNCHED();
 }
 
@@ -744,45 +763,29 @@ static cudaError_t launch_tiles(K k, const DeviceForest &f, const PredictArgs &a
   return QC_LAUNCHED();
 }
 
-// two-level records; HM / PL chosen at run time
-template <int ILP, int MINB, int TEXMODE>
-static cudaError_t launch_duo(const DeviceForest &f, const PredictArgs &a, cudaStream_t s) {
+// HM / PL chosen at run time
+template <class Walk>
+static cudaError_t launch_walk(const DeviceForest &f, const PredictArgs &a, cudaStream_t s) {
   const bool hm = a.has_missing != 0, pl = a.pred_leaf != 0;
-  if (hm && pl) return launch_tiles(predict_tiles_kernel<ILP, MINB, TEXMODE, true, true>, f, a, s);
-  if (hm) return launch_tiles(predict_tiles_kernel<ILP, MINB, TEXMODE, true, false>, f, a, s);
-  if (pl) return launch_tiles(predict_tiles_kernel<ILP, MINB, TEXMODE, false, true>, f, a, s);
-  return launch_tiles(predict_tiles_kernel<ILP, MINB, TEXMODE, false, false>, f, a, s);
+  count_predict(Walk::kFamily + hm + 2 * pl);
+  if (hm && pl) return launch_tiles(predict_tiles_kernel<Walk, true, true>, f, a, s);
+  if (hm) return launch_tiles(predict_tiles_kernel<Walk, true, false>, f, a, s);
+  if (pl) return launch_tiles(predict_tiles_kernel<Walk, false, true>, f, a, s);
+  return launch_tiles(predict_tiles_kernel<Walk, false, false>, f, a, s);
 }
 
-template <int ILP, int MINB, int TEXMODE, int CTOP>
-static cudaError_t launch_nodes8(const DeviceForest &f, const PredictArgs &a, cudaStream_t s) {
-  const bool hm = a.has_missing != 0, pl = a.pred_leaf != 0;
-  if (hm && pl) return launch_tiles(predict_tiles_nodes8_kernel<ILP, true, true, MINB, TEXMODE, CTOP>, f, a, s);
-  if (hm) return launch_tiles(predict_tiles_nodes8_kernel<ILP, true, false, MINB, TEXMODE, CTOP>, f, a, s);
-  if (pl) return launch_tiles(predict_tiles_nodes8_kernel<ILP, false, true, MINB, TEXMODE, CTOP>, f, a, s);
-  return launch_tiles(predict_tiles_nodes8_kernel<ILP, false, false, MINB, TEXMODE, CTOP>, f, a, s);
-}
-
-cudaError_t launch_predict(const DeviceForest &f, const PredictArgs &a, cudaStream_t s) {
-  if (a.nrow == 0 || a.tree_end <= a.tree_begin) return cudaSuccess;
-  if (a.ncol > f.nfeat || f.nfeat > (int)kMaxFeatures) return cudaErrorInvalidValue;
-  const bool hm = a.has_missing != 0, pl = a.pred_leaf != 0;
-  const bool in_table = a.tree_begin >= f.const_tree0 && a.tree_end <= f.const_tree0 + f.const_ntree;
-  // ---- two-level records (the constant tables hold these trees' tops: capi_xgb.cpp sync_const_top)
-  if (f.duo_ready && in_table && (!hm || f.duo_has_dl)) {
-    g_last_predict = count_family("duo", hm, pl);
-    if (f.duo_shallow) return launch_duo<4, 6, 0xA>(f, a, s);  // kernels.hpp kShallowRecBytesPerTree
-    return launch_duo<kDuoIlp, kDuoMinBlocks, kDuoTexMask>(f, a, s);
+cudaError_t launch_predict(const DeviceForest &f, const ConstWindow &w, const PredictArgs &args, cudaStream_t s) {
+  if (args.nrow == 0 || args.tree_end <= args.tree_begin) return cudaSuccess;
+  if (args.ncol > f.nfeat || f.nfeat > (int)kMaxFeatures) return cudaErrorInvalidValue;
+  PredictArgs a = args;
+  a.ctree0 = w.tree0;
+  switch (layout(f, w, a.tree_begin, a.tree_end, a.has_missing != 0)) {
+    case Layout::kRecords: return f.duo_shallow ? launch_walk<RecordsShallowWalk>(f, a, s) : launch_walk<RecordsWalk>(f, a, s);
+    case Layout::kNodesTable: return launch_walk<NodesTableWalk>(f, a, s);
+    case Layout::kNodesTex: return launch_walk<NodesTexWalk>(f, a, s);
+    case Layout::kNodesLsu: break;
   }
-  // ---- 8-byte depth-ordered nodes: 4 trees in flight per thread; levels 0..3 of every tree from constant
-  // memory when the table holds them; below that, trees 1 and 3 of each group fetch their nodes through the
-  // texture pipe and trees 0 and 2 through the LSU (mask 0xA).  Measurements: profiles/README.md.
-  g_last_predict = count_family("nodes8", hm, pl);
-  constexpr int kTex = 0xA;
-  const int ctop = in_table ? f.const_top_levels : 0;  // 0 if the table does not hold these trees
-  if (f.tex == 0) return launch_nodes8<4, 6, 0, 0>(f, a, s);
-  if (ctop == 4) return launch_nodes8<4, 6, kTex, 4>(f, a, s);
-  return launch_nodes8<4, 6, kTex, 0>(f, a, s);
+  return launch_walk<NodesLsuWalk>(f, a, s);
 }
 
 // =====================================================================================
@@ -912,7 +915,7 @@ cudaError_t launch_shap(const uint4 *bins, int64_t nbins, int nslices, const Con
   cudaError_t e = cudaFuncSetAttribute(shap_paths_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   shap_paths_kernel<<<dim3((unsigned)tile_count(a.nrow), (unsigned)nslices), kTileRows, smem, s>>>(bins, nbins, nslices, a, part);
-  g_last_predict = count_family("shap", false, false);
+  count_predict(kShap);
   return QC_LAUNCHED();
 }
 
@@ -921,7 +924,7 @@ cudaError_t launch_shap_reduce(const double *part, int nslices, const ContribArg
   const uint64_t n = a.nrow * (uint64_t)(a.nfeat + 1);
   const int blocks = (int)std::min<uint64_t>((n + 255) / 256, (uint64_t)sm_count() * 16);
   shap_reduce_kernel<<<blocks, 256, 0, s>>>(part, nslices, a);
-  count_family("shap_reduce", false, false);
+  count_family(kShapReduce);
   return QC_LAUNCHED();
 }
 
@@ -987,7 +990,7 @@ cudaError_t launch_shap_approx(const DeviceForest &f, const float *mean, int ntr
   cudaError_t e = cudaFuncSetAttribute(shap_approx_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   shap_approx_kernel<<<(unsigned)ntile, kBlock, smem, s>>>(f, mean, ntree, a);
-  g_last_predict = count_family("shap_approx", false, false);
+  count_predict(kShapApprox);
   return QC_LAUNCHED();
 }
 

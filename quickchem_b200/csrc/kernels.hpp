@@ -6,27 +6,31 @@
 
 namespace qcoh {
 
-// Device copy of a FlatForest (forest.hpp).
+// Device copy of a FlatForest (forest.hpp) and of its two-level records, as upload() builds it.
 struct DeviceForest {
   const uint2 *nodes = nullptr;          // {value bits, meta}
   const uint32_t *tree_offset = nullptr; // [ntree + 1]
   const int32_t *tree_depth = nullptr;   // [ntree]
   const int32_t *orig_id = nullptr;      // [num_nodes]
   cudaTextureObject_t tex = 0;           // the same nodes as a 1-D linear uint2 texture (TEX pipe)
-  int const_top_levels = 0;              // levels of every tree currently held in the constant-memory table
   const uint4 *recs = nullptr;           // two-level records (forest.hpp DuoForest), or nullptr
   cudaTextureObject_t tex4 = 0;          // the records as a 1-D linear uint4 texture
-  int duo_ready = 0;                     // the constant-memory tables hold trees [const_tree0, const_tree0 + const_ntree) of this booster's records
   int duo_has_dl = 0;                    // the records carry the default-direction bits (DuoForest::has_default_bits)
   uint32_t duo_blk_mul = 0;              // 1 << (32 - DuoForest::blk_shift): blk = mulhi(w3, duo_blk_mul)
-  int32_t const_tree0 = 0, const_ntree = 0;
   int32_t ntree = 0;
   int32_t nfeat = 0;
-  int32_t max_depth = 0;
-  int64_t num_nodes = 0;
-  int64_t sum_depth = 0;                 // sum over trees of the deepest leaf's depth
   int duo_shallow = 0;                   // records average < kShallowRecBytesPerTree per tree (picks the launch shape)
   float base_score = 0.f;
+};
+
+// What the constant-memory tables of tree tops hold: one window of trees [tree0, tree0 + ntree) of one booster, as
+// the first levels of its 8-byte nodes or as the heap-ordered tops of its two-level records.  The tables exist once
+// per device; capi_xgb.cpp hold() fills them and returns the window, and the launchers take it as an argument.
+enum class TopLayout { kNone, kRecordTops, kNodeTops };
+struct ConstWindow {
+  TopLayout layout = TopLayout::kNone;
+  int32_t tree0 = 0, ntree = 0;
+  bool holds(TopLayout l, int t0, int t1) const { return layout == l && tree0 <= t0 && t1 <= tree0 + ntree; }
 };
 
 // How many trees the constant-memory tables hold at once (4 levels x 16 entries per tree in 61 440 B), and how
@@ -71,6 +75,7 @@ struct PredictArgs {
   int exp10 = 0;             // fused export transform, OH_GridCompMod.F90:369,1569
   float scale = 1.f;
   float *out = nullptr;      // device: [nrow] or [nrow][out_stride]
+  int32_t ctree0 = 0;        // first tree of the constant-table window (set by launch_predict)
 };
 
 uint64_t launch_count();
@@ -89,7 +94,7 @@ cudaError_t upload_const_duo(const uint32_t *top_xy, const uint32_t *tree_slot, 
 // X and Xt cover `nrow` rows starting at a tile boundary.
 cudaError_t launch_seal_tiles(const float *X, uint64_t nrow, int ncol, float missing, uint32_t *Xt, int *flags, cudaStream_t s);
 
-cudaError_t launch_predict(const DeviceForest &f, const PredictArgs &a, cudaStream_t s);
+cudaError_t launch_predict(const DeviceForest &f, const ConstWindow &w, const PredictArgs &a, cudaStream_t s);
 
 // Per-feature contributions (forest.hpp ShapForest).  out: [nrow][nfeat + 1] floats, column nfeat = `bias`.
 //   exact (TreeSHAP on the path bins): launch_shap writes float64 partial sums of bin slice s to
@@ -120,13 +125,14 @@ struct SoaArgs {
   uint64_t nrow = 0;         // ncol * ksub
   float missing = -999.f;
   int32_t ntree_used = 0;
+  int32_t ctree0 = 0;        // first tree of the constant-table window (set by launch_predict_soa)
   int exp10 = 1;
   float scale = 1.f;
   float *out = nullptr;      // OH_ML slab
   float *pred = nullptr;     // optional raw booster output
   int *flags = nullptr;      // |= 2 on +-inf input
 };
-cudaError_t launch_predict_soa(const DeviceForest &f, const SoaArgs &a, cudaStream_t s);
+cudaError_t launch_predict_soa(const DeviceForest &f, const ConstWindow &w, const SoaArgs &a, cudaStream_t s);
 
 // ---- fused Run1 pieces (OH_GridCompMod.F90:1232-1599) ---------------------------------
 struct Run1Dev {

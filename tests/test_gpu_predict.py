@@ -289,9 +289,11 @@ def test_dmatrix_file_roundtrip(capi, tmp_path, small_model_path):
     assert np.array_equal(b.predict(d), b.predict(d2))
 
 
-def test_more_trees_than_the_constant_table_holds(capi, oracle, tmp_path):
-    """The constant-memory table of tree tops holds 7680 nodes (480 trees x 16); a bigger forest must run
-    without it (and without the two-level records, which need the table) and still match."""
+def test_more_trees_than_the_constant_table_holds(capi, oracle, tmp_path, duo_mode):
+    """The constant-memory table of tree tops holds 7680 nodes (480 trees x 16); a bigger forest runs on the
+    two-level records (or, with duo = 0, the 8-byte nodes) in launches of 120 trees, the table re-filled with the
+    next window of 480 trees when a launch leaves it, and still matches, with and without missing entries."""
+    family = "duo" if duo_mode else "nodes8"
     rng = np.random.default_rng(8)
     trees = [xgbmodel.tree_from_nested((int(rng.integers(27)), float(rng.normal()), bool(rng.random() < 0.5),
                                         float(rng.normal()), (int(rng.integers(27)), float(rng.normal()), False, 1.0, -1.0)))
@@ -300,9 +302,11 @@ def test_more_trees_than_the_constant_table_holds(capi, oracle, tmp_path):
     x = rng.normal(0, 1, (3000, 27)).astype(np.float32)
     got, ref = _both(capi, oracle, f, x, tmp_path)
     assert np.array_equal(got.view(np.uint32), ref.view(np.uint32))
+    assert capi.last_predict_kernel() == family
     x[::3, 5] = np.nan
     got, ref = _both(capi, oracle, f, x, tmp_path)
     assert np.array_equal(got.view(np.uint32), ref.view(np.uint32))
+    assert capi.last_predict_kernel() == family + "_missing"
 
 
 def test_dmatrix_from_libsvm_and_csv(capi, oracle, tmp_path, small_model_path):
