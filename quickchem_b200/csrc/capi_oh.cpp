@@ -58,9 +58,8 @@ struct Oh {
   uint32_t magic = kOhMagic;
   Booster *booster = nullptr;
   qcoh_oh_config cfg;
-  // resident copies of host-provided inputs, one slot per input field
-  static constexpr int kNumIn = 13 + 7 + 11 + 5 + 1 + 1;
-  DevBuf<float> in[kNumIn];
+  // resident copies of host-provided inputs: one slot per pointer-sized word of qcoh_run1_in (SLOT)
+  DevBuf<float> in[sizeof(qcoh_run1_in) / sizeof(const float *)];
   DevBuf<float> PL_MOD, NDWET, sums[6], aod, pl_bst, OH_ML, OH, OH_boost, X, pred, sza, lat_deg, so3, loss_ch4, loss_co;
   DevBuf<uint32_t> Xt;
   DevBuf<int> ctl;
@@ -108,7 +107,7 @@ void bind_booster(Oh *o, Booster *b) {
 }
 
 // host pointer -> resident device copy; device pointer -> used in place
-const float *resident(Oh *o, int slot, const float *p, size_t n, const char *name) {
+const float *resident(Oh *o, size_t slot, const float *p, size_t n, const char *name) {
   if (!p) throw Error(std::string("qcoh_oh_run1: input field ") + name + " is NULL");
   if (is_device_ptr(p)) return p;
   float *d = o->in[slot].need(n);
@@ -122,6 +121,11 @@ void deliver(float *user, const float *dev, size_t n) {
 }
 
 }  // namespace
+
+// The resident buffer of input field F is the one at F's position in qcoh_run1_in: the order in which qcoh_oh_run1
+// reads its inputs does not matter, and skipped inputs leave the others where they are.
+#define SLOT(F) (offsetof(qcoh_run1_in, F) / sizeof(const float *))
+#define RESIDENT(F, n) resident(o, SLOT(F), in->F, n, #F)
 
 extern "C" {
 
@@ -222,44 +226,29 @@ int qcoh_oh_run1(qcoh_oh_handle h, const qcoh_run1_in *in, qcoh_run1_out *out) {
   r.eps = c.mapl_epsilon, r.avogad = c.mapl_avogad, r.runiv = c.mapl_runiv, r.r2d = c.mapl_radians_to_degrees;
   r.ohscale = c.ohscale, r.tropp_min = c.tropp_min, r.missing = c.missing;
   r.dynamic_k = c.compute_once_per_day ? 0 : 1;  // :1561
-  int s = 0;
-  r.T_MOD = resident(o, s++, in->T_MOD, n3, "T_MOD");
-  r.Q_MOD = resident(o, s++, in->Q_MOD, n3, "Q_MOD");
-  r.PLE_MOD = resident(o, s++, in->PLE_MOD, ne, "PLE_MOD");
-  r.TROPP = resident(o, s++, in->TROPP, n2, "TROPP");
-  r.OH_CLIM = resident(o, s++, in->OH_CLIM, n3, "OH_CLIM");
+  r.T_MOD = RESIDENT(T_MOD, n3);
+  r.Q_MOD = RESIDENT(Q_MOD, n3);
+  r.PLE_MOD = RESIDENT(PLE_MOD, ne);
+  r.TROPP = RESIDENT(TROPP, n2);
+  r.OH_CLIM = RESIDENT(OH_CLIM, n3);
   const bool boost = in->need_to_call_boost != 0;
   if (!boost && !o->oh_ml_valid) throw Error("qcoh_oh_run1: need_to_call_boost = 0 before any boost call (OH_ML is undefined)");
   const bool want_diag = in->AREA != nullptr;
   if (boost || want_diag) {
-    r.ZLE_BST = resident(o, s++, in->ZLE_BST, ne, "ZLE_BST");
-    r.CH4 = resident(o, s++, in->CH4, n3, "CH4");
-  } else {
-    s += 2;
+    r.ZLE_BST = RESIDENT(ZLE_BST, ne);
+    r.CH4 = RESIDENT(CH4, n3);
   }
+  Run1Features feat{};
   if (boost) {
-    // aliasing (ONLINE_INST hands the same arrays as model state and boost input) is preserved:
-    // identical host pointers are uploaded once
-    auto same = [&](const float *p, const float *q, const float *dq) { return p == q ? dq : nullptr; };
-    const float *d;
-    r.T_BST = (d = same(in->T_BST, in->T_MOD, r.T_MOD)) ? d : resident(o, s, in->T_BST, n3, "T_BST");
-    ++s;
-    r.Q_BST = (d = same(in->Q_BST, in->Q_MOD, r.Q_MOD)) ? d : resident(o, s, in->Q_BST, n3, "Q_BST");
-    ++s;
-    r.PLE_BST = (d = same(in->PLE_BST, in->PLE_MOD, r.PLE_MOD)) ? d : resident(o, s, in->PLE_BST, ne, "PLE_BST");
-    ++s;
-    r.TAUCLW = resident(o, s++, in->TAUCLW, n3, "TAUCLW");
-    r.TAUCLI = resident(o, s++, in->TAUCLI, n3, "TAUCLI");
-    r.FCLD = resident(o, s++, in->FCLD, n3, "FCLD");
-    r.CO = resident(o, s++, in->CO, n3, "CO");
-    for (int i = 0; i < 7; ++i) r.SCA[i] = resident(o, s++, in->SCA[i], n3, "SCACOEF");
-    const float *const gases[11] = {in->NO2, in->O3, in->ISOP, in->ACET, in->C2H6, in->C3H8, in->PRPE, in->ALK4, in->MP, in->H2O2, in->CH2O};
-    const float **dst[11] = {&r.NO2, &r.O3, &r.ISOP, &r.ACET, &r.C2H6, &r.C3H8, &r.PRPE, &r.ALK4, &r.MP, &r.H2O2, &r.CH2O};
-    for (int i = 0; i < 11; ++i) *dst[i] = resident(o, s++, gases[i], n3, "climatological gas");
-    r.GMITO3 = resident(o, s++, in->GMITO3, n2, "GMITO3");
-    r.GMITTO3 = resident(o, s++, in->GMITTO3, n2, "GMITTO3");
-    r.ALBUV = resident(o, s++, in->ALBUV, n2, "ALBUV");
-    r.LATS = resident(o, s++, in->LATS, n2, "LATS");
+    // aliasing (ONLINE_INST hands the same arrays as model state and boost input) is preserved: identical host
+    // pointers are uploaded once (PLE here, T and Q in the feature table)
+    r.PLE_BST = in->PLE_BST == in->PLE_MOD ? r.PLE_MOD : RESIDENT(PLE_BST, ne);
+    r.TAUCLW = RESIDENT(TAUCLW, n3);
+    r.TAUCLI = RESIDENT(TAUCLI, n3);
+    for (int i = 0; i < 7; ++i) r.SCA[i] = resident(o, SLOT(SCA) + i, in->SCA[i], n3, ("SCA[" + std::to_string(i) + "]").c_str());
+    r.GMITO3 = RESIDENT(GMITO3, n2);
+    r.GMITTO3 = RESIDENT(GMITTO3, n2);
+    r.LATS = RESIDENT(LATS, n2);
     if (!in->LONS) throw Error("qcoh_oh_run1: input field LONS is NULL");
     // noon SZA (host libm, cached per day and grid)
     const int jday = julian_day(in->nymd);
@@ -273,30 +262,55 @@ int qcoh_oh_run1(qcoh_oh_handle h, const qcoh_run1_in *in, qcoh_run1_out *out) {
       CU(cudaMemcpyAsync(o->sza.need(n2), hs, n2 * 4, cudaMemcpyHostToDevice, g.stream));
       o->sza_jday = jday, o->sza_lat_key = in->LATS, o->sza_lon_key = in->LONS, o->sza_n = n2, o->sza_hash = probe;
     }
-    r.SZA = o->sza.p;
+    for (int i = 0; i < 6; ++i) r.sums[i] = o->sums[i].need(n3);
+    r.lat_deg = o->lat_deg.need(n2), r.so3 = o->so3.need(n2);
+    // The 27 features of predict_OH_with_XGB, in its order (OH_GridCompMod.F90:303-345): the fused predict and the
+    // matrix pack both read them from this table.
+    feat.src2[0] = r.lat_deg;  // LATS * radToDeg (:1444), written by oh_sums
+    feat.ple = r.PLE_BST;      // feature 1: PL_BST / 100 (:314), computed by run1_feature
+    feat.src3[2] = in->T_BST == in->T_MOD ? r.T_MOD : RESIDENT(T_BST, n3);
+    feat.src3[3] = RESIDENT(NO2, n3);
+    feat.src3[4] = RESIDENT(O3, n3);
+    feat.src3[5] = r.CH4;
+    feat.src3[6] = RESIDENT(CO, n3);
+    feat.src3[7] = RESIDENT(ISOP, n3);
+    feat.src3[8] = RESIDENT(ACET, n3);
+    feat.src3[9] = RESIDENT(C2H6, n3);
+    feat.src3[10] = RESIDENT(C3H8, n3);
+    feat.src3[11] = RESIDENT(PRPE, n3);
+    feat.src3[12] = RESIDENT(ALK4, n3);
+    feat.src3[13] = RESIDENT(MP, n3);
+    feat.src3[14] = RESIDENT(H2O2, n3);
+    for (int i = 0; i < 4; ++i) feat.src3[15 + i] = r.sums[i];  // TAUCLWDN TAUCLIDN TAUCLIUP TAUCLWUP
+    feat.src3[19] = RESIDENT(FCLD, n3);
+    feat.src3[20] = in->Q_BST == in->Q_MOD ? r.Q_MOD : RESIDENT(Q_BST, n3);
+    feat.src2[21] = r.so3;     // GMITO3 - GMITTO3 (:1446), written by oh_sums
+    feat.src2[22] = RESIDENT(ALBUV, n2);
+    feat.src3[23] = r.sums[4];  // AODUP
+    feat.src3[24] = r.sums[5];  // AODDN
+    feat.src3[25] = RESIDENT(CH2O, n3);
+    feat.src2[26] = o->sza.p;  // noon SZA
   }
-  if (want_diag) r.AREA = resident(o, Oh::kNumIn - 1, in->AREA, n2, "AREA");
+  if (want_diag) r.AREA = RESIDENT(AREA, n2);
   r.PL_MOD = o->PL_MOD.need(n3), r.NDWET = o->NDWET.need(n3);
   r.OH_ML = o->OH_ML.p, r.OH = o->OH.need(n3), r.OH_boost = o->OH_boost.need(n3);
   r.LOSS_CH4 = out->LOSS_CH4 ? o->loss_ch4.need(n3) : nullptr;
   r.LOSS_CO = out->LOSS_CO ? o->loss_co.need(n3) : nullptr;
-  r.ctl = o->ctl.need(4);
+  r.ctl = o->ctl.need(3);
   r.diag = o->diag.need(4);
-  CU(cudaMemsetAsync(r.ctl, 0, 4 * sizeof(int), g.stream));
+  CU(cudaMemsetAsync(r.ctl, 0, 3 * sizeof(int), g.stream));
   CU(launch_oh_state(r, g.stream));
   out->k1 = 0;
   bool check_inf_after = false;
   if (boost) {
-    int ctl[4];
+    int ctl[2];
     CU(cudaMemcpyAsync(ctl, r.ctl, sizeof ctl, cudaMemcpyDeviceToHost, g.stream));
     CU(cudaStreamSynchronize(g.stream));
     if (!r.dynamic_k && ctl[1] != 0) throw Error("OH Prediction: Minimum tropopause pressure is not low enough!");  // :288
     const int ksub = ctl[0];
     const int k1 = km - ksub + 1;  // :300
     out->k1 = k1;
-    const uint64_t npred = (uint64_t)nc * ksub;
-    for (int i = 0; i < 6; ++i) r.sums[i] = o->sums[i].need(n3);
-    r.lat_deg = o->lat_deg.need(n2), r.so3 = o->so3.need(n2);
+    const uint64_t npred = (uint64_t)nc * ksub, e0 = (uint64_t)(k1 - 1) * nc;
     r.aod = o->aod.need(n3), r.pl_bst = o->pl_bst.need(n3);
     CU(launch_oh_sums(r, g.stream));
     B(o->booster);  // the handle holds a reference (XGBoosterFree refuses while it does); checked all the same
@@ -308,15 +322,9 @@ int qcoh_oh_run1(qcoh_oh_handle h, const qcoh_run1_in *in, qcoh_run1_out *out) {
       // fused: pack (:303-345) + create (:347) + predict (:356) + 10**x (:369) * OHscale (:1569) in one
       // kernel reading the SoA fields; the [N x 27] matrix is never formed
       SoaArgs a;
-      const float *s3[27] = {nullptr, nullptr, r.T_BST, r.NO2, r.O3, r.CH4, r.CO, r.ISOP, r.ACET, r.C2H6, r.C3H8, r.PRPE,
-                             r.ALK4, r.MP, r.H2O2, r.sums[0], r.sums[1], r.sums[2], r.sums[3], r.FCLD, r.Q_BST, nullptr,
-                             nullptr, r.sums[4], r.sums[5], r.CH2O, nullptr};
-      const float *s2[27] = {nullptr};
-      s2[0] = r.lat_deg, s2[21] = r.so3, s2[22] = r.ALBUV, s2[26] = r.SZA;
-      for (int f = 0; f < 27; ++f) a.src3[f] = s3[f], a.src2[f] = s2[f];
-      a.ple = r.PLE_BST, a.ncol = nc, a.e0 = (uint64_t)(k1 - 1) * nc, a.nrow = npred, a.missing = c.missing;
+      a.feat = feat, a.ncol = nc, a.e0 = e0, a.nrow = npred, a.missing = c.missing;
       a.ntree_used = ntree, a.exp10 = 1, a.scale = c.ohscale;
-      a.out = r.OH_ML + (size_t)(k1 - 1) * nc;
+      a.out = r.OH_ML + e0;
       a.pred = out->pred ? o->pred.need(npred) : nullptr;
       a.flags = r.ctl + 2;
       CU(launch_predict_soa(o->booster->dev, hold(o->booster, 0, ntree), a, g.stream));
@@ -325,19 +333,19 @@ int qcoh_oh_run1(qcoh_oh_handle h, const qcoh_run1_in *in, qcoh_run1_out *out) {
     } else if (npred) {
       // debug / parity path: materialise xx_carr so that it can be handed back (out->X)
       float *X = o->X.need(npred * 27);
-      CU(launch_oh_pack(r, k1, X, g.stream));
+      CU(launch_oh_pack(feat, e0, nc, npred, X, g.stream));
+      // XGDMatrixCreateFromMat (:347): scan + key tiles
+      uint32_t *Xt = o->Xt.need(tile_words(npred, 27));
+      CU(launch_seal_tiles(X, npred, 27, c.missing, Xt, r.ctl + 2, g.stream));
       int flags = 0;
       CU(cudaMemcpyAsync(&flags, r.ctl + 2, sizeof(int), cudaMemcpyDeviceToHost, g.stream));
       CU(cudaStreamSynchronize(g.stream));
       if ((flags & 2) && !std::isinf(c.missing)) throw Error("Check failed: valid: Input data contains `inf` or `nan`");
-      // XGDMatrixCreateFromMat (:347): scan + key tiles
-      uint32_t *Xt = o->Xt.need(tile_words(npred, 27));
-      CU(launch_seal_tiles(X, npred, 27, c.missing, Xt, r.ctl + 3, g.stream));
       PredictArgs a;
       a.Xt = Xt, a.nrow = npred, a.ncol = 27, a.has_missing = flags & 1, a.pred_leaf = 0;
       a.tree_begin = 0, a.tree_end = ntree, a.out_stride = a.tree_end;
       a.exp10 = 1, a.scale = c.ohscale;
-      a.out = r.OH_ML + (size_t)(k1 - 1) * nc;
+      a.out = r.OH_ML + e0;
       launch_predict_chunked(o->booster, a, g.stream);
       if (out->pred) {
         a.exp10 = 0, a.scale = 1.f, a.out = o->pred.need(npred);

@@ -9,7 +9,8 @@
 //                             Its walk policy picks the node layout and the launch shape: DuoWalk on the two-level
 //                             16-byte records (one gather per two tree levels), NodesWalk on the 8-byte depth-ordered
 //                             nodes (boosters the records do not hold)
-//       predict_soa_kernel    K2 with the tile assembled straight from the Run1 SoA fields
+//       predict_soa_kernel    K2 with the tile assembled straight from the Run1 SoA fields (run1_feature, which
+//                             oh_pack reads the features with too)
 //   K6  shap_paths / shap_reduce / shap_approx   per-feature contributions (exact TreeSHAP, approximate Saabas)
 //   K1  oh_state / oh_sums / oh_pack    Run1 feature assembly (:1240-1257, :1441-1488, :303-345)
 //   K5  oh_finalize           troposphere mask + unit conversion (:1579-1595)
@@ -650,6 +651,14 @@ __global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_tiles_kernel
   }
 }
 
+// Feature ft of cell e in column c, as predict_OH_with_XGB packs it (:303-345): what the fused predict puts in its
+// tiles and oh_pack_kernel in the matrix.
+__device__ __forceinline__ float run1_feature(const Run1Features &x, int ft, size_t e, int c, int ncol) {
+  if (ft == 1)  // PL_BST = (PLE(k-1) + PLE(k)) * 0.5 (:1488), / 100.0 as a true divide (:314)
+    return __fdiv_rn(__fmul_rn(__fadd_rn(__ldg(x.ple + e), __ldg(x.ple + e + ncol)), 0.5f), 100.0f);
+  return x.src3[ft] ? __ldg(x.src3[ft] + e) : __ldg(x.src2[ft] + c);
+}
+
 // ---- fused Run1 variant: the tile is assembled straight from the SoA feature fields ------------------
 // (OH_GridCompMod.F90:303-345 pack + :347 create + :356 predict + :369,:1569 transform in one kernel).
 // Row m of the slab is cell e = e0 + m; per feature the CTA's 256 cells are contiguous in the source
@@ -672,11 +681,7 @@ __global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_soa_kernel(D
     const bool chk_inf = !isinf(a.missing);
 #pragma unroll
     for (int ft = 0; ft < 27; ++ft) {
-      float x;
-      if (ft == 1)  // PL_BST = (PLE(k-1) + PLE(k)) * 0.5 (:1488), / 100.0 as a true divide (:314)
-        x = __fdiv_rn(__fmul_rn(__fadd_rn(__ldg(a.ple + e), __ldg(a.ple + e + a.ncol)), 0.5f), 100.0f);
-      else
-        x = a.src3[ft] ? __ldg(a.src3[ft] + e) : __ldg(a.src2[ft] + c);
+      const float x = run1_feature(a.feat, ft, e, c, a.ncol);
       uint32_t k = float_key(x);
       if (x != x || x == a.missing) k = kKeyMissing, flags |= 1;
       if (chk_inf && isinf(x)) flags |= 2;
@@ -1110,55 +1115,18 @@ cudaError_t launch_oh_sums(const Run1Dev &r, cudaStream_t s) {
 // oh_pack: xx_carr(27, N) in the reference's order (OH_GridCompMod.F90:308-345): row m runs
 // over k = k1..km, then column (i fastest).  A CTA packs 256 consecutive rows: per feature the
 // 256 sources are contiguous (coalesced), the [256][27] tile is transposed through shared
-// memory (stride 27 is odd: conflict-free) and written back as one contiguous run.
-__global__ void __launch_bounds__(256) oh_pack_kernel(Run1Dev r, int k1, uint64_t npred, float *__restrict__ X) {
+// memory (stride 27 is odd: conflict-free) and written back as one contiguous run.  The
+// missing / inf scan is seal_tiles', which reads the matrix next.
+__global__ void __launch_bounds__(256) oh_pack_kernel(Run1Features x, uint64_t e0, int ncol, uint64_t npred, float *__restrict__ X) {
   __shared__ float tile[256 * 27];
   const int tid = threadIdx.x;
   const uint64_t m0 = (uint64_t)blockIdx.x * 256;
   const uint64_t m = m0 + tid;
-  int flags = 0;
   if (m < npred) {
-    const size_t e = (size_t)(k1 - 1) * r.ncol + m;
-    const int c = (int)(m % (uint64_t)r.ncol);
-    float *row = tile + tid * 27;
-    row[0] = __fmul_rn(r.LATS[c], r.r2d);  // :1444
-    // PL_BST = (PLE(k-1) + PLE(k)) * 0.5 (:1488), then / 100.0 as a true divide (:314)
-    row[1] = __fdiv_rn(__fmul_rn(__fadd_rn(r.PLE_BST[e], r.PLE_BST[e + r.ncol]), 0.5f), 100.0f);
-    row[2] = r.T_BST[e];
-    row[3] = r.NO2[e];
-    row[4] = r.O3[e];
-    row[5] = r.CH4[e];
-    row[6] = r.CO[e];
-    row[7] = r.ISOP[e];
-    row[8] = r.ACET[e];
-    row[9] = r.C2H6[e];
-    row[10] = r.C3H8[e];
-    row[11] = r.PRPE[e];
-    row[12] = r.ALK4[e];
-    row[13] = r.MP[e];
-    row[14] = r.H2O2[e];
-    row[15] = r.sums[0][e];  // TAUCLWDN
-    row[16] = r.sums[1][e];  // TAUCLIDN
-    row[17] = r.sums[2][e];  // TAUCLIUP
-    row[18] = r.sums[3][e];  // TAUCLWUP
-    row[19] = r.FCLD[e];
-    row[20] = r.Q_BST[e];
-    row[21] = __fadd_rn(r.GMITO3[c], -r.GMITTO3[c]);  // :1446
-    row[22] = r.ALBUV[c];
-    row[23] = r.sums[4][e];  // AODUP
-    row[24] = r.sums[5][e];  // AODDN
-    row[25] = r.CH2O[e];
-    row[26] = r.SZA[c];
-    const bool fin = !isinf(r.missing);
+    const int c = (int)(m % (uint64_t)ncol);
 #pragma unroll
-    for (int f = 0; f < 27; ++f) {
-      const float v = row[f];
-      if (v != v || v == r.missing) flags |= 1;
-      if (fin && isinf(v)) flags |= 2;
-    }
+    for (int ft = 0; ft < 27; ++ft) tile[tid * 27 + ft] = run1_feature(x, ft, e0 + m, c, ncol);
   }
-  flags = __reduce_or_sync(0xffffffffu, flags);
-  if ((tid & 31) == 0 && flags) atomicOr(&r.ctl[2], flags);
   __syncthreads();
   const uint64_t left = npred - m0;
   const int n = (int)(left < 256 ? left : 256) * 27;
@@ -1166,10 +1134,9 @@ __global__ void __launch_bounds__(256) oh_pack_kernel(Run1Dev r, int k1, uint64_
   for (int i = tid; i < n; i += 256) dst[i] = tile[i];
 }
 
-cudaError_t launch_oh_pack(const Run1Dev &r, int k1, float *X, cudaStream_t s) {
-  const uint64_t npred = (uint64_t)r.ncol * (uint64_t)(r.km - k1 + 1);
+cudaError_t launch_oh_pack(const Run1Features &x, uint64_t e0, int32_t ncol, uint64_t npred, float *X, cudaStream_t s) {
   if (npred == 0) return cudaSuccess;
-  oh_pack_kernel<<<(unsigned)((npred + 255) / 256), 256, 0, s>>>(r, k1, npred, X);
+  oh_pack_kernel<<<(unsigned)((npred + 255) / 256), 256, 0, s>>>(x, e0, ncol, npred, X);
   return QC_LAUNCHED();
 }
 

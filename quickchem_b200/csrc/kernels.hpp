@@ -115,11 +115,18 @@ cudaError_t launch_shap(const uint4 *bins, int64_t nbins, int nslices, const Con
 cudaError_t launch_shap_reduce(const double *part, int nslices, const ContribArgs &a, cudaStream_t s);
 cudaError_t launch_shap_approx(const DeviceForest &f, const float *mean, int ntree, const ContribArgs &a, cudaStream_t s);
 
-// Fused Run1 predict: features come straight from the SoA fields (27 sources in feature order)
-struct SoaArgs {
+// Where the 27 Run1 features come from, in feature order (filled by qcoh_oh_run1): feature f of cell e in column c is
+// src3[f][e], or src2[f][c] for a 2-D field; feature 1 is PL_BST / 100, computed from ple.  kernels.cu run1_feature
+// reads it for both the fused predict and the matrix pack.
+struct Run1Features {
   const float *src3[27];     // [km][ncol] source of feature f, or nullptr if it is a 2-D field
   const float *src2[27];     // [ncol] source of a 2-D feature
-  const float *ple = nullptr;  // PLE_BST [km+1][ncol] (feature 1 is computed from it)
+  const float *ple = nullptr;  // PLE_BST [km+1][ncol]
+};
+
+// Fused Run1 predict: the tile of every CTA is assembled straight from the feature sources
+struct SoaArgs {
+  Run1Features feat;
   int32_t ncol = 0;
   uint64_t e0 = 0;           // cell index of slab row 0: (k1 - 1) * ncol
   uint64_t nrow = 0;         // ncol * ksub
@@ -133,6 +140,8 @@ struct SoaArgs {
   int *flags = nullptr;      // |= 2 on +-inf input
 };
 cudaError_t launch_predict_soa(const DeviceForest &f, const ConstWindow &w, const SoaArgs &a, cudaStream_t s);
+// The same features as the row-major [npred][27] matrix xx_carr: row m is cell e0 + m
+cudaError_t launch_oh_pack(const Run1Features &x, uint64_t e0, int32_t ncol, uint64_t npred, float *X, cudaStream_t s);
 
 // ---- fused Run1 pieces (OH_GridCompMod.F90:1232-1599) ---------------------------------
 struct Run1Dev {
@@ -140,15 +149,15 @@ struct Run1Dev {
   float eps = 0, avogad = 0, runiv = 0, r2d = 0;
   float ohscale = 1.f, tropp_min = 4000.f, missing = -999.f;
   int dynamic_k = 0;
+  // Inputs the four kernels read (the 27 features reach the predict and the pack through Run1Features).  The order is
+  // part of the kernels' code: when a kernel reads both pointers of one 16-byte word of its parameters, the compiler
+  // loads them at once, so moving a field changes the SASS of oh_state / oh_sums (tools/compare_sass.py shows it).
   const float *T_MOD, *Q_MOD, *PLE_MOD, *TROPP;
-  const float *T_BST, *Q_BST, *PLE_BST, *ZLE_BST;
-  const float *TAUCLW, *TAUCLI, *FCLD, *CH4, *CO;
+  const float *PLE_BST, *ZLE_BST;
+  const float *TAUCLW, *TAUCLI, *CH4;
   const float *SCA[7];
-  const float *NO2, *O3, *ISOP, *ACET, *C2H6, *C3H8, *PRPE, *ALK4, *MP, *H2O2, *CH2O;
-  const float *GMITO3, *GMITTO3, *ALBUV, *LATS;
-  const float *SZA;      // [ncol] degrees (host-computed with libm, see oh_host.cpp)
   const float *OH_CLIM;
-  const float *AREA;
+  const float *GMITO3, *GMITTO3, *LATS;
   // work / outputs (device)
   float *PL_MOD, *NDWET;             // [km][ncol]
   float *sums[6];                    // wdn idn iup wup aup adn, [km][ncol]
@@ -157,13 +166,14 @@ struct Run1Dev {
   float *OH_ML;                      // persistent [km][ncol]
   float *OH, *OH_boost;              // [km][ncol]
   float *LOSS_CH4, *LOSS_CO;         // optional [km][ncol] 1/s (build-defined, SURVEY.md 8(f)4)
-  int *ctl;                          // [0] ksub (atomicMax) [1] tropp<=tropp_min count [2] matrix flags
-  double *diag;                      // [4]
+  int *ctl;                          // [0] ksub (atomicMax) [1] tropp<=tropp_min count [2] the slab's missing / inf
+                                     // flags (predict_soa or seal_tiles)
+  const float *AREA;                 // [ncol] m2, input of the optional diagnostic
+  double *diag;                      // [4] its partial sums
 };
 
 cudaError_t launch_oh_state(const Run1Dev &r, cudaStream_t s);
 cudaError_t launch_oh_sums(const Run1Dev &r, cudaStream_t s);
-cudaError_t launch_oh_pack(const Run1Dev &r, int k1, float *X, cudaStream_t s);
 cudaError_t launch_oh_finalize(const Run1Dev &r, cudaStream_t s);
 cudaError_t launch_oh_diag(const Run1Dev &r, cudaStream_t s);
 cudaError_t launch_fill(float *p, uint64_t n, float v, cudaStream_t s);
