@@ -151,6 +151,33 @@ module qcoh_fortran_api
        type(c_ptr) :: out_result     ! const float**
      end function
 
+     ! Inplace prediction straight from a REAL(4) array, without a DMatrix (include/qcoh.h).  values is a JSON array
+     ! interface, e.g. for a field XX(nrow, ncol) held feature-major as Fortran does ('//' joins):
+     !   '{"data": [<address>, false], "shape": [nrow, ncol], "strides": [4, <4 * nrow>], "typestr": "<f4", "version": 3}'
+     ! and config '{"type": 0, "missing": -999.0, "iteration_begin": 0, "iteration_end": 0, "strict_shape": false}',
+     ! both ending in c_null_char; m must be c_null_ptr.  FromDense takes a C-contiguous host array ([nrow][ncol] in C
+     ! order, i.e. XX(ncol, nrow) in Fortran) and returns a booster-owned host buffer; FromCudaArray takes device memory
+     ! with any strides (the feature-major layout above) and returns a booster-owned DEVICE buffer.
+     integer(c_int) function XGBoosterPredictFromDense(handle, values, config, m, out_shape, out_dim, out_result) &
+          bind(C, name="XGBoosterPredictFromDense")
+       import :: c_int, c_ptr, c_char, c_int64_t
+       type(c_ptr), value :: handle, m
+       character(len=1, kind=c_char), dimension(*) :: values, config
+       type(c_ptr) :: out_shape      ! const bst_ulong**
+       integer(c_int64_t) :: out_dim ! bst_ulong*
+       type(c_ptr) :: out_result     ! const float**
+     end function
+
+     integer(c_int) function XGBoosterPredictFromCudaArray(handle, values, config, m, out_shape, out_dim, out_result) &
+          bind(C, name="XGBoosterPredictFromCudaArray")
+       import :: c_int, c_ptr, c_char, c_int64_t
+       type(c_ptr), value :: handle, m
+       character(len=1, kind=c_char), dimension(*) :: values, config
+       type(c_ptr) :: out_shape      ! const bst_ulong**
+       integer(c_int64_t) :: out_dim ! bst_ulong*
+       type(c_ptr) :: out_result     ! const float** (device memory)
+     end function
+
      function XGBGetLastError_c() bind(C, name="XGBGetLastError") result(msg)
        import :: c_ptr
        type(c_ptr) :: msg

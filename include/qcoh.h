@@ -75,6 +75,29 @@ int XGBoosterPredict(BoosterHandle handle, DMatrixHandle dmat, int option_mask, 
 int XGBoosterPredictFromDMatrix(BoosterHandle handle, DMatrixHandle dmat, const char *config,
                                 const bst_ulong **out_shape, bst_ulong *out_dim, const float **out_result);
 
+/* libxgboost 1.6.0's inplace predicts (what xgboost's Python Booster.inplace_predict calls; fortran/qcoh_fortran_api.F90
+ * binds them): prediction straight from a dense float32 array, without a DMatrix.  The predict kernel builds its key
+ * tiles from the array in shared memory, so nothing but the result is written to HBM — no copy of the matrix, no key
+ * tiles.  values: a JSON array interface {"data": [address, readonly], "shape": [nrow, ncol], "strides": null |
+ * [row_bytes, col_bytes], "typestr": "<f4", "version": 3}; other types, masks, shapes that are not 2-D, negative strides
+ * or strides that are not a multiple of 4, and a NULL address for a non-empty array fail.  ncol <= the booster's
+ * num_feature; absent columns are missing.  config: {"type", "missing", "iteration_begin", "iteration_end",
+ * "strict_shape"}, all required (other keys are ignored); type 0 value or 1 margin (both the float32 margin, no
+ * transform); entries that are NaN or == missing are missing (NaN is written NaN), +-inf with a finite missing fails
+ * like XGDMatrixCreateFromMat; iteration_begin must be 0, iteration_end = 0: all trees.  m (the proxy DMatrix) must be
+ * NULL.  Shape (nrow), or (nrow, 1) with strict_shape.  Both return when the result is complete; result and shape are
+ * booster-owned, valid until the next predict / free on that booster.
+ *   FromDense: HOST memory (pinned or pageable), C-contiguous; it is copied to HBM in chunks, each predicted as it lands,
+ *   and read completely before the call returns.  A device address (detected) is read like FromCudaArray.  The
+ *   result is a pinned host buffer.
+ *   FromCudaArray: DEVICE memory, any strides (a feature-major [ncol][nrow] array is [4, 4 * nrow]).  An optional
+ *   "stream" entry (CUDA Array Interface v3: 1 legacy default stream, 2 per-thread default stream, else a cudaStream_t;
+ *   0 is invalid) is waited for before the array is read.  The result is a DEVICE buffer. */
+int XGBoosterPredictFromDense(BoosterHandle handle, const char *values, const char *config, DMatrixHandle m,
+                              const bst_ulong **out_shape, bst_ulong *out_dim, const float **out_result);
+int XGBoosterPredictFromCudaArray(BoosterHandle handle, const char *values, const char *config, DMatrixHandle m,
+                                  const bst_ulong **out_shape, bst_ulong *out_dim, const float **out_result);
+
 /* xgb_fortran_api.F90:75-83; call site OH_GridCompMod.F90:256.  The reference passes a DMatrix
  * handle *by value* as `dmats` with len = 0; dmats is never dereferenced when len == 0. */
 int XGBoosterCreate(const DMatrixHandle dmats[], bst_ulong len, BoosterHandle *out);

@@ -63,7 +63,8 @@ class Run1Out(C.Structure):
 # every symbol include/qcoh.h declares (tests check the library exports all of them)
 XGB_SYMBOLS = ("XGBoosterLoadModel", "XGBoosterSaveModel", "XGDMatrixSaveBinary", "XGDMatrixFree",
                "XGDMatrixCreateFromFile", "XGBoosterPredict", "XGBoosterCreate", "XGDMatrixCreateFromMat",
-               "XGDMatrixNumRow", "XGDMatrixNumCol", "XGBoosterFree", "XGBGetLastError", "XGBoosterPredictFromDMatrix")  # fmt: skip
+               "XGDMatrixNumRow", "XGDMatrixNumCol", "XGBoosterFree", "XGBGetLastError", "XGBoosterPredictFromDMatrix",
+               "XGBoosterPredictFromDense", "XGBoosterPredictFromCudaArray")  # fmt: skip
 QCOH_SYMBOLS = ("qcoh_version", "qcoh_device_count", "qcoh_set_device", "qcoh_host_alloc", "qcoh_host_free",
                 "qcoh_device_alloc", "qcoh_device_free", "qcoh_memcpy_h2d", "qcoh_memcpy_d2h",
                 "qcoh_device_synchronize", "qcoh_timer_start", "qcoh_timer_stop", "qcoh_flush_l2",
@@ -131,6 +132,8 @@ def lib():
         L.qcoh_booster_predict_device.argtypes = [vp, vp, C.c_int, C.c_uint, C.POINTER(Epilogue), vp]
         L.XGBoosterPredictFromDMatrix.argtypes = [vp, vp, C.c_char_p, C.POINTER(C.POINTER(u64)), C.POINTER(u64),
                                                   C.POINTER(f32p)]  # fmt: skip
+        for name in ("XGBoosterPredictFromDense", "XGBoosterPredictFromCudaArray"):
+            getattr(L, name).argtypes = [vp, C.c_char_p, C.c_char_p, vp, C.POINTER(C.POINTER(u64)), C.POINTER(u64), C.POINTER(f32p)]
         L.qcoh_booster_predict_contribs_device.argtypes = [vp, vp, C.c_int, C.c_uint, vp]
         L.qcoh_booster_get_shap_paths.argtypes = [vp, C.POINTER(C.POINTER(C.c_uint32)), C.POINTER(C.POINTER(C.c_int64)),
                                                   C.POINTER(C.POINTER(C.c_float)), C.POINTER(C.c_int64)]  # fmt: skip
@@ -426,6 +429,53 @@ class Booster:
         n = int(np.prod(shape)) if shape else 0
         out = np.ctypeslib.as_array(p, (n,)).copy() if n else np.zeros(0, np.float32)
         return out.reshape(shape)
+
+    def inplace_predict(self, data, missing=-999.0, type=0, iteration_end=0, strict_shape=False, *, shape=None,
+                        strides=None, offset=0) -> np.ndarray:
+        """xgboost's Booster.inplace_predict: value (type 0) or margin (1) straight from a dense float32 array, without a
+        DMatrix.  A numpy array goes through XGBoosterPredictFromDense, a DeviceArray or anything with
+        __cuda_array_interface__ (e.g. a torch CUDA tensor) through XGBoosterPredictFromCudaArray.  A DeviceArray takes
+        an explicit `shape` (nrow, ncol), `strides` in bytes (None: C-contiguous) and `offset` in floats.  Returns a copy
+        of the margins, shaped as the library says."""
+        shape_, p, on_device = self.inplace_predict_raw(data, missing, type, iteration_end, strict_shape, shape=shape,
+                                                        strides=strides, offset=offset)  # fmt: skip
+        n = int(np.prod(shape_))
+        out = np.empty(n, np.float32)
+        if n and on_device:
+            check(lib().qcoh_memcpy_d2h(_ptr(out), C.cast(p, vp), out.nbytes))
+        elif n:
+            out[:] = np.ctypeslib.as_array(p, (n,))
+        return out.reshape(shape_)
+
+    def inplace_predict_raw(self, data, missing=-999.0, type=0, iteration_end=0, strict_shape=False, *, shape=None,
+                            strides=None, offset=0, stream=None):
+        """As inplace_predict(), but returns (shape, borrowed result pointer, whether it points at device memory)
+        without copying; `stream` adds a "stream" entry to the interface of a device array."""
+        import json
+
+        if isinstance(data, np.ndarray):
+            if data.dtype != np.float32:
+                raise TypeError("inplace_predict takes float32 arrays")
+            iface, cuda = dict(data.__array_interface__), False
+        elif isinstance(data, DeviceArray):
+            nrow, ncol = shape
+            iface = {"data": [data.ptr.value + 4 * offset if data.ptr.value else 0, False], "shape": [nrow, ncol],
+                     "strides": None if strides is None else list(strides), "typestr": "<f4", "version": 3}  # fmt: skip
+            cuda = True
+        else:
+            iface, cuda = dict(data.__cuda_array_interface__), True
+        iface["data"] = list(iface["data"])
+        iface["shape"] = list(iface["shape"])
+        if iface.get("strides") is not None:
+            iface["strides"] = list(iface["strides"])
+        if stream is not None:
+            iface["stream"] = stream
+        cfg = {"type": int(type), "training": False, "missing": float(missing), "iteration_begin": 0,
+               "iteration_end": int(iteration_end), "strict_shape": bool(strict_shape)}  # fmt: skip
+        shp, dim, p = C.POINTER(u64)(), u64(), f32p()
+        fn = lib().XGBoosterPredictFromCudaArray if cuda else lib().XGBoosterPredictFromDense
+        check(fn(self.handle, json.dumps(iface).encode(), json.dumps(cfg).encode(), None, C.byref(shp), C.byref(dim), C.byref(p)))
+        return tuple(int(shp[i]) for i in range(dim.value)), p, cuda
 
     def predict_contribs(self, dmat: DMatrix, approximate=False, ntree_limit=0) -> np.ndarray:
         """[nrow, num_feature + 1] per-feature contributions, last column the bias: exact TreeSHAP, or Saabas when

@@ -126,7 +126,9 @@ ConstWindow hold(Booster *b, int tree0, int ntree) {
 // One prediction = one launch per range of kRangeTrees trees (kernels.hpp; the tables hold kConstTreesMax and are
 // re-filled, stream-ordered, when a range leaves them) and the float32 partial sum travels through `out`, so the sum
 // order — tree 0, 1, 2, ... — and with it every bit of the result is the same as in a single launch.
-void launch_predict_chunked(Booster *b, PredictArgs a, cudaStream_t s) {
+// launch(window, range args) launches one range: launch_predict on key tiles, launch_predict_dense on a dense array.
+template <class Launch>
+static void predict_ranges(Booster *b, const PredictArgs &a, cudaStream_t s, Launch &&launch) {
   const int t_end = a.tree_end;
   if (a.nrow == 0) return;
   if (t_end <= 0) {  // a booster without trees predicts its base score
@@ -143,8 +145,12 @@ void launch_predict_chunked(Booster *b, PredictArgs a, cudaStream_t s) {
     PredictArgs c = a;
     c.tree_begin = t0, c.tree_end = t0 + n;
     c.first = t0 == 0, c.last = t0 + n == t_end;
-    CU(launch_predict(b->dev, w, c, s));
+    CU(launch(w, c));
   }
+}
+
+void launch_predict_chunked(Booster *b, PredictArgs a, cudaStream_t s) {
+  predict_ranges(b, a, s, [&](const ConstWindow &w, const PredictArgs &c) { return launch_predict(b->dev, w, c, s); });
 }
 
 static void seal(DMatrix *d) {
@@ -379,33 +385,23 @@ static thread_local cudaEvent_t g_stage_free[kStageSlots] = {nullptr, nullptr, n
 // memcpy so that the DMA engine never waits on the driver's own bounce buffer.  The caller's buffer
 // is fully consumed before this returns.
 //   copy_stream : H2D(c) -> seal(c): scan + key tiles -> flag D2H(c)      g.stream : predict(c)      d2h_stream : result D2H(c)
-static void create_pipelined(DMatrix *d, const float *data, Booster *b) {
-  const uint64_t nrow = d->nrow, ncol = d->ncol;
-  const bool pinned = is_pinned_host(data);
-  uint64_t cr = g.chunk_rows;
-  if (!pinned && cr > (1ull << 19)) cr = 1ull << 19;
+static uint64_t chunk_rows(bool pinned) { return pinned ? g.chunk_rows : std::min<uint64_t>(g.chunk_rows, 1ull << 19); }
+
+// The chunked copy of a row-major host matrix into HBM, shared by XGDMatrixCreateFromMat and XGBoosterPredictFromDense:
+// rows [0, nrow) of `data` go to X in chunks of cr rows (a multiple of 256) on g.copy_stream.  Pinned memory goes by
+// direct DMA, every copy queued up front; pageable memory is staged through the ring of pinned slots by the copy pool,
+// which stages chunk c + 1 while this thread queues the CUDA work of chunk c.  landed(c, r0, nr) queues, after H2D(c),
+// the work that reads chunk c; process(c) is the host side of chunk c, called in chunk order (two chunks behind on
+// pageable memory).  Returns when every chunk has been copied: the caller's buffer may go.
+template <class Landed, class Process>
+static void copy_chunks(const float *data, uint64_t nrow, uint64_t ncol, bool pinned, uint64_t cr, float *X, Landed &&landed,
+                        Process &&process) {
   const size_t nchunk = (size_t)((nrow + cr - 1) / cr);
-  float *X = d->X.p;
-  if (g_spare_Xt.cap >= tile_words(nrow, ncol) && g_spare_Xt.p && !d->Xt.p) d->Xt.swap(g_spare_Xt);
-  uint32_t *Xt = d->Xt.need(tile_words(nrow, ncol));
-  const bool spec = b != nullptr;
-  float *sdev = nullptr, *shost = nullptr;
-  if (spec) {
-    upload(b);
-    if (g_spare_spec.cap >= nrow && g_spare_spec.p) d->spec_dev.swap(g_spare_spec);
-    sdev = d->spec_dev.need(nrow);
-    if (g_spare_pin.cap >= nrow && g_spare_pin.p) d->spec_host.swap(g_spare_pin);
-    shost = d->spec_host.need(nrow);
-  }
-  int *fl = g_chunk_flags.need(nchunk);
-  int *hfl = g_h_chunk_flags.need(nchunk);
-  CU(cudaMemsetAsync(fl, 0, nchunk * sizeof(int), g.copy_stream));
   if (!pinned)
     for (int s = 0; s < kStageSlots; ++s)
       if (!g_stage_free[s]) CU(cudaEventCreateWithFlags(&g_stage_free[s], cudaEventDisableTiming));
-  int flags = 0;
   // pageable source: stage_begin(c) starts the workers on chunk c (into ring slot c % 3, once its previous H2D has
-  // drained), stage_end() waits for them; issue(c) queues H2D(c) -> seal(c) -> flag D2H(c)
+  // drained), stage_end() waits for them; issue(c) queues H2D(c) and what reads chunk c
   auto stage_begin = [&](size_t c) {
     const uint64_t r0 = c * cr, nr = std::min(cr, nrow - r0);
     const int s = (int)(c % kStageSlots);
@@ -423,6 +419,53 @@ static void create_pipelined(DMatrix *d, const float *data, Booster *b) {
     } else {
       CU(cudaMemcpyAsync(X + r0 * ncol, data + r0 * ncol, bytes, cudaMemcpyHostToDevice, g.copy_stream));
     }
+    landed(c, r0, nr);
+  };
+  if (pinned) {  // every copy can be queued up front
+    for (size_t c = 0; c < nchunk; ++c) issue(c);
+    for (size_t c = 0; c < nchunk; ++c) process(c);
+  } else {  // the workers stage chunk c + 1 while this thread queues the CUDA work of chunk c and processes chunk c - 2
+    struct PoolGuard {  // an exception between begin() and wait() must not leave the pool locked
+      bool busy = false;
+      ~PoolGuard() {
+        if (busy) CopyPool::get().wait();
+      }
+    } pool;
+    if (nchunk) stage_begin(0), pool.busy = true;
+    for (size_t c = 0; c < nchunk; ++c) {
+      CopyPool::get().wait(), pool.busy = false;
+      if (c + 1 < nchunk) stage_begin(c + 1), pool.busy = true;
+      issue(c);
+      if (c >= 2) process(c - 2);
+    }
+    for (size_t c = nchunk >= 2 ? nchunk - 2 : 0; c < nchunk; ++c) process(c);
+  }
+  CU(cudaStreamSynchronize(g.copy_stream));  // the borrowed host buffer has been read completely
+}
+
+static void create_pipelined(DMatrix *d, const float *data, Booster *b) {
+  const uint64_t nrow = d->nrow, ncol = d->ncol;
+  const bool pinned = is_pinned_host(data);
+  const uint64_t cr = chunk_rows(pinned);
+  const size_t nchunk = (size_t)((nrow + cr - 1) / cr);
+  float *X = d->X.p;
+  if (g_spare_Xt.cap >= tile_words(nrow, ncol) && g_spare_Xt.p && !d->Xt.p) d->Xt.swap(g_spare_Xt);
+  uint32_t *Xt = d->Xt.need(tile_words(nrow, ncol));
+  const bool spec = b != nullptr;
+  float *sdev = nullptr, *shost = nullptr;
+  if (spec) {
+    upload(b);
+    if (g_spare_spec.cap >= nrow && g_spare_spec.p) d->spec_dev.swap(g_spare_spec);
+    sdev = d->spec_dev.need(nrow);
+    if (g_spare_pin.cap >= nrow && g_spare_pin.p) d->spec_host.swap(g_spare_pin);
+    shost = d->spec_host.need(nrow);
+  }
+  int *fl = g_chunk_flags.need(nchunk);
+  int *hfl = g_h_chunk_flags.need(nchunk);
+  CU(cudaMemsetAsync(fl, 0, nchunk * sizeof(int), g.copy_stream));
+  int flags = 0;
+  // H2D(c) -> seal(c): scan + key tiles -> flag D2H(c) on the copy stream
+  auto landed = [&](size_t c, uint64_t r0, uint64_t nr) {
     // chunks start on tile boundaries (chunk_rows is a multiple of 256)
     CU(launch_seal_tiles(X + r0 * ncol, nr, (int)ncol, d->missing, Xt + tile_offset_words(r0, ncol), fl + c, g.copy_stream));
     CU(cudaMemcpyAsync(hfl + c, fl + c, sizeof(int), cudaMemcpyDeviceToHost, g.copy_stream));
@@ -447,29 +490,105 @@ static void create_pipelined(DMatrix *d, const float *data, Booster *b) {
     CU(cudaStreamWaitEvent(g.d2h_stream, chunk_event(2 * c + 1), 0));
     CU(cudaMemcpyAsync(shost + r0, sdev + r0, nr * sizeof(float), cudaMemcpyDeviceToHost, g.d2h_stream));
   };
-  if (pinned) {  // every copy can be queued up front
-    for (size_t c = 0; c < nchunk; ++c) issue(c);
-    for (size_t c = 0; c < nchunk; ++c) process(c);
-  } else {  // the workers stage chunk c + 1 while this thread queues the CUDA work of chunk c and predicts chunk c - 2
-    struct PoolGuard {  // an exception between begin() and wait() must not leave the pool locked
-      bool busy = false;
-      ~PoolGuard() {
-        if (busy) CopyPool::get().wait();
-      }
-    } pool;
-    if (nchunk) stage_begin(0), pool.busy = true;
-    for (size_t c = 0; c < nchunk; ++c) {
-      CopyPool::get().wait(), pool.busy = false;
-      if (c + 1 < nchunk) stage_begin(c + 1), pool.busy = true;
-      issue(c);
-      if (c >= 2) process(c - 2);
-    }
-    for (size_t c = nchunk >= 2 ? nchunk - 2 : 0; c < nchunk; ++c) process(c);
-  }
-  CU(cudaStreamSynchronize(g.copy_stream));  // the borrowed host buffer has been read completely
+  copy_chunks(data, nrow, ncol, pinned, cr, X, landed, process);
   d->hflags = flags;
   d->sealed = true;
   if (spec) d->spec_booster = b, d->spec_version = b->version, d->spec_ready = true;
+}
+
+static thread_local cudaEvent_t g_input_ready = nullptr;
+
+// XGBoosterPredictFromDense / XGBoosterPredictFromCudaArray (libxgboost 1.6.0 Learner::InplacePredict, value and
+// margin): predict_dense_kernel builds the key tiles from the caller's array in shared memory.  A device array is read
+// where it is, with its strides; a host array is copied chunk by chunk (copy_chunks) and each chunk predicted as it
+// lands.  Returns the float32 margins, in the booster's device buffer (on_device) or its pinned host buffer; both stay
+// valid until the next predict or free on that booster.  Every refusal comes before any device work.
+static const float *predict_inplace(const char *caller, bool cuda_array, BoosterHandle handle, const char *values,
+                                    const char *config, DMatrixHandle m, const bst_ulong **out_shape, bst_ulong *out_dim) {
+  const std::string pre = std::string(caller) + ": ";
+  Booster *b = B(handle);
+  if (!out_shape || !out_dim) throw Error(pre + "NULL output argument");
+  if (!b->loaded) throw Error("Booster has no model: call XGBoosterLoadModel first");
+  const ArrayInterface ai = parse_array_interface(values, caller);
+  const PredictConfig c = parse_predict_config(config, caller, true);
+  if (m) throw Error(pre + "the proxy DMatrix must be NULL (inplace prediction takes no base margin)");
+  if (c.type != 0 && c.type != 1)
+    throw Error(pre + "prediction type " + std::to_string(c.type) + " is not supported inplace (0 value, 1 margin)");
+  if (c.iteration_begin < 0 || c.iteration_end < 0) throw Error(pre + "negative iteration range");
+  if (c.iteration_begin != 0) throw Error(pre + "iteration_begin = " + std::to_string(c.iteration_begin) + " is not supported (only 0)");
+  if (ai.ncol > b->host.num_feature)
+    throw Error("Check failed: Number of columns does not match number of features in booster. Columns: " +
+                std::to_string(ai.ncol) + " Features: " + std::to_string(b->host.num_feature));
+  if (ai.ncol > kMaxMatrixCols)
+    throw Error(pre + std::to_string(ai.ncol) + " columns; libqcoh's tile form holds at most " + std::to_string(kMaxMatrixCols));
+  const uint64_t nrow = ai.nrow, ncol = ai.ncol;
+  const bool empty = nrow * ncol == 0;
+  // the pointer query binds the CUDA runtime to this thread's device first; with no device visible every address is host memory
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) == cudaSuccess && ndev > 0) ensure_device();
+  else (void)cudaGetLastError();
+  const float *data = reinterpret_cast<const float *>((uintptr_t)ai.addr);
+  const bool on_device = !empty && is_device_ptr(data);
+  if (cuda_array && !empty && !on_device) throw Error(pre + "the array is in host memory (XGBoosterPredictFromDense takes host arrays)");
+  if (!empty && !on_device && (ai.col_bytes != 4 || ai.row_bytes != (int64_t)(4 * ncol)))
+    throw Error(pre + "a host array must be C-contiguous: strides [" + std::to_string(4 * ncol) + ", 4] or null, got [" +
+                std::to_string(ai.row_bytes) + ", " + std::to_string(ai.col_bytes) + "]");
+  ensure_device();
+  upload(b);
+  const unsigned limit = (unsigned)std::min<int64_t>(c.iteration_end, (int64_t)UINT32_MAX);
+  float *dv = b->d_result.need(nrow);
+  int *fl = g_chunk_flags.need(1);
+  int *hfl = g_h_chunk_flags.need(1);
+  CU(cudaMemsetAsync(fl, 0, sizeof(int), g.stream));
+  PredictArgs a;
+  a.nrow = nrow, a.ncol = (int32_t)ncol;
+  a.tree_begin = 0, a.tree_end = (int32_t)trees_used(b, limit);
+  a.out = dv;
+  DenseArgs da;
+  da.missing = c.missing, da.flags = fl;
+  auto predict = [&](const PredictArgs &pa, const DenseArgs &d) {
+    predict_ranges(b, pa, g.stream, [&](const ConstWindow &w, const PredictArgs &r) { return launch_predict_dense(b->dev, w, r, d, g.stream); });
+  };
+  if (on_device || empty) {
+    if (ai.has_stream) {  // the work queued on the caller's stream before this call has written the array
+      const cudaStream_t cs = ai.stream == 1 ? cudaStreamLegacy : ai.stream == 2 ? cudaStreamPerThread : (cudaStream_t)(uintptr_t)ai.stream;
+      if (!g_input_ready) CU(cudaEventCreateWithFlags(&g_input_ready, cudaEventDisableTiming));
+      CU(cudaEventRecord(g_input_ready, cs));
+      CU(cudaStreamWaitEvent(g.stream, g_input_ready, 0));
+    }
+    da.X = data, da.row_stride = ai.row_bytes / 4, da.col_stride = ai.col_bytes / 4;
+    predict(a, da);
+  } else {
+    // the chunks land in the spare matrix buffer of XGDMatrixFree, which is given back afterwards
+    DevBuf<float> X;
+    if (g_spare_X.cap >= nrow * ncol) X.swap(g_spare_X);
+    X.need(nrow * ncol);
+    const bool pinned = is_pinned_host(data);
+    copy_chunks(data, nrow, ncol, pinned, chunk_rows(pinned), X.p, [&](size_t ci, uint64_t r0, uint64_t nr) {
+      CU(cudaEventRecord(chunk_event(ci), g.copy_stream));
+      CU(cudaStreamWaitEvent(g.stream, chunk_event(ci), 0));
+      PredictArgs pa = a;
+      pa.nrow = nr, pa.out = dv + r0;
+      DenseArgs d = da;
+      d.X = X.p + r0 * ncol, d.row_stride = (int64_t)ncol, d.col_stride = 1;
+      predict(pa, d);
+    }, [](size_t) {});
+    CU(cudaStreamSynchronize(g.stream));  // the chunk buffer is read before it goes back to the pool
+    if (X.cap > g_spare_X.cap) X.swap(g_spare_X);
+  }
+  CU(cudaMemcpyAsync(hfl, fl, sizeof(int), cudaMemcpyDeviceToHost, g.stream));
+  float *out = dv;
+  if (!cuda_array) {
+    out = b->h_result.need(nrow);
+    CU(cudaMemcpyAsync(out, dv, nrow * sizeof(float), cudaMemcpyDeviceToHost, g.stream));
+  }
+  CU(cudaStreamSynchronize(g.stream));
+  // xgboost src/data/data.cc SparsePage::Push: a finite `missing` with inf data is an error (the kernel's flag)
+  if (*hfl & 2) throw Error("Check failed: valid: Input data contains `inf` or `nan`");
+  b->h_shape = c.strict_shape ? std::vector<bst_ulong>{nrow, 1} : std::vector<bst_ulong>{nrow};
+  *out_shape = b->h_shape.data();
+  *out_dim = (bst_ulong)b->h_shape.size();
+  return out;
 }
 
 }  // namespace qcoh
@@ -680,6 +799,23 @@ int XGBoosterPredictFromDMatrix(BoosterHandle handle, DMatrixHandle dmat, const 
   *out_shape = b->h_shape.data();
   *out_dim = (bst_ulong)b->h_shape.size();
   *out_result = hv;
+  API_END
+}
+
+// libxgboost 1.6.0's inplace predicts (src/c_api/c_api.cc), what xgboost's Python Booster.inplace_predict calls
+int XGBoosterPredictFromDense(BoosterHandle handle, const char *values, const char *config, DMatrixHandle m,
+                              const bst_ulong **out_shape, bst_ulong *out_dim, const float **out_result) {
+  API_BEGIN
+  if (!out_result) throw Error("XGBoosterPredictFromDense: NULL output argument");
+  *out_result = predict_inplace("XGBoosterPredictFromDense", false, handle, values, config, m, out_shape, out_dim);
+  API_END
+}
+
+int XGBoosterPredictFromCudaArray(BoosterHandle handle, const char *values, const char *config, DMatrixHandle m,
+                                  const bst_ulong **out_shape, bst_ulong *out_dim, const float **out_result) {
+  API_BEGIN
+  if (!out_result) throw Error("XGBoosterPredictFromCudaArray: NULL output argument");
+  *out_result = predict_inplace("XGBoosterPredictFromCudaArray", true, handle, values, config, m, out_shape, out_dim);
   API_END
 }
 

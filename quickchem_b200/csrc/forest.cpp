@@ -997,29 +997,83 @@ float shap_bias(const ShapForest &s, const HostForest &h, const FlatForest &f, i
   return b + h.base_score;
 }
 
-PredictConfig parse_predict_config(const char *json) {
-  if (!json) fail("XGBoosterPredictFromDMatrix: config is NULL");
-  const size_t len = strlen(json);
+namespace {
+JV parse_json_object(const char *json, const std::string &what) {
+  if (!json) fail(what + " is NULL");
   JV root;
   try {
-    JsonReader r{json, json + len};
+    JsonReader r{json, json + strlen(json)};
     root = r.value();
   } catch (const std::exception &e) {
-    fail(std::string("XGBoosterPredictFromDMatrix: config is not valid JSON (") + e.what() + ")");
+    fail(what + " is not valid JSON (" + e.what() + ")");
   }
-  if (root.kind != JV::Obj) fail("XGBoosterPredictFromDMatrix: config must be a JSON object");
+  if (root.kind != JV::Obj) fail(what + " must be a JSON object");
+  return root;
+}
+}  // namespace
+
+PredictConfig parse_predict_config(const char *json, const char *caller, bool inplace) {
+  const std::string pre = std::string(caller) + ": ";
+  const JV root = parse_json_object(json, pre + "config");
   auto need = [&](const char *key) -> const JV & {
     const JV *v = root.find(key);
-    if (!v) fail(std::string("XGBoosterPredictFromDMatrix: config is missing the key '") + key + "'");
+    if (!v) fail(pre + "config is missing the key '" + key + "'");
     return *v;
   };
   PredictConfig c;
   c.type = (int)need("type").as_int();
-  c.training = need("training").as_int() != 0;
+  if (inplace) {
+    const JV &m = need("missing");
+    if (m.kind != JV::Num) fail(pre + "config: 'missing' must be a number (NaN is written NaN)");
+    c.missing = m.f32;
+  } else {
+    c.training = need("training").as_int() != 0;
+  }
   c.iteration_begin = need("iteration_begin").as_int();
   c.iteration_end = need("iteration_end").as_int();
   c.strict_shape = need("strict_shape").as_int() != 0;
   return c;
+}
+
+ArrayInterface parse_array_interface(const char *json, const char *caller) {
+  const std::string pre = std::string(caller) + ": ";
+  const JV root = parse_json_object(json, pre + "array interface");
+  auto need = [&](const char *key) -> const JV & {
+    const JV *v = root.find(key);
+    if (!v) fail(pre + "array interface is missing the key '" + key + "'");
+    return *v;
+  };
+  const JV &ty = need("typestr");
+  if (ty.kind != JV::Str || ty.str != "<f4")
+    fail(pre + "typestr '" + (ty.kind == JV::Str ? ty.str : std::string("?")) + "': only little-endian float32 ('<f4') is accepted");
+  if (root.find("mask")) fail(pre + "masked arrays are not supported (the array interface has a 'mask' entry)");
+  const JV &shape = need("shape");
+  if (shape.kind != JV::Arr || shape.arr.size() != 2)
+    fail(pre + "the array must be 2-D [nrow, ncol]; its shape has " + std::to_string(shape.kind == JV::Arr ? shape.arr.size() : 0) + " dimensions");
+  ArrayInterface a;
+  const int64_t nr = shape.arr[0].as_int(), nc = shape.arr[1].as_int();
+  if (nr < 0 || nc < 0) fail(pre + "negative shape [" + std::to_string(nr) + ", " + std::to_string(nc) + "]");
+  a.nrow = (uint64_t)nr, a.ncol = (uint64_t)nc;
+  a.row_bytes = 4 * nc;
+  const JV *st = root.find("strides");
+  if (st && st->kind != JV::Null) {
+    if (st->kind != JV::Arr || st->arr.size() != 2) fail(pre + "strides must be null or [row_bytes, col_bytes]");
+    const int64_t rb = st->arr[0].as_int(), cb = st->arr[1].as_int();
+    if (rb < 0 || cb < 0 || rb % 4 || cb % 4)
+      fail(pre + "strides [" + std::to_string(rb) + ", " + std::to_string(cb) + "]: they must be non-negative multiples of 4 bytes");
+    a.row_bytes = rb, a.col_bytes = cb;
+  }
+  const JV &data = need("data");
+  if (data.kind != JV::Arr || data.arr.empty()) fail(pre + "'data' must be [address, readonly]");
+  a.addr = (uint64_t)data.arr[0].as_int();
+  if (a.addr == 0 && a.nrow * a.ncol > 0) fail(pre + "the data address is NULL for a " + std::to_string(nr) + " x " + std::to_string(nc) + " array");
+  const JV *s = root.find("stream");
+  if (s && s->kind != JV::Null) {
+    a.stream = (uint64_t)s->as_int();
+    if (a.stream == 0) fail(pre + "stream 0 is not valid in the CUDA Array Interface (1: legacy default stream, 2: per-thread default stream)");
+    a.has_stream = true;
+  }
+  return a;
 }
 
 }  // namespace qcoh

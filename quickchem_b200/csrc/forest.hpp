@@ -118,14 +118,30 @@ ShapForest build_shap(const struct HostForest &h, const struct FlatForest &f);
 // The bias column of a contributions row: ((0 + mean_0(root)) + mean_1(root) + ...) + base_score in float32.
 float shap_bias(const ShapForest &s, const struct HostForest &h, const struct FlatForest &f, int ntree);
 
-// The config of XGBoosterPredictFromDMatrix (libxgboost 1.6.0 keys); throws naming a missing key.
+// The config of XGBoosterPredictFromDMatrix (libxgboost 1.6.0 keys); throws naming a missing key.  `inplace`: the
+// config of the inplace predicts, which require `missing` instead of `training`; messages start with `caller`.
 struct PredictConfig {
   int type = 0;
   bool training = false;
   int64_t iteration_begin = 0, iteration_end = 0;
   bool strict_shape = false;
+  float missing = 0.f;  // inplace only
 };
-PredictConfig parse_predict_config(const char *json);
+PredictConfig parse_predict_config(const char *json, const char *caller = "XGBoosterPredictFromDMatrix", bool inplace = false);
+
+// A 2-D float32 array interface (numpy __array_interface__ / CUDA Array Interface v3, as JSON) for the inplace
+// predicts: {"data": [address, readonly], "shape": [nrow, ncol], "strides": null | [row_bytes, col_bytes],
+// "typestr": "<f4", "version": 3[, "stream": s]}.  Throws, prefixed with `caller`, on any other type, a mask, a shape
+// that is not 2-D, negative strides or strides that are not a multiple of 4, a NULL address for a non-empty array, and
+// stream 0.
+struct ArrayInterface {
+  uint64_t addr = 0;
+  uint64_t nrow = 0, ncol = 0;
+  int64_t row_bytes = 0, col_bytes = 4;  // C-contiguous when "strides" is null
+  bool has_stream = false;
+  uint64_t stream = 0;                   // CUDA Array Interface: 1 legacy default stream, 2 per-thread default stream
+};
+ArrayInterface parse_array_interface(const char *json, const char *caller);
 
 // Throws std::runtime_error with libxgboost-style messages on malformed / unsupported input.
 HostForest load_model_file(const std::string &path);

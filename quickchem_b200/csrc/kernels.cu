@@ -11,6 +11,7 @@
 //                             nodes (boosters the records do not hold)
 //       predict_soa_kernel    K2 with the tile assembled straight from the Run1 SoA fields (run1_feature, which
 //                             oh_pack reads the features with too)
+//       predict_dense_kernel  K2 with the tile assembled from a caller's strided float array (inplace prediction)
 //   K6  shap_paths / shap_reduce / shap_approx   per-feature contributions (exact TreeSHAP, approximate Saabas)
 //   K1  oh_state / oh_sums / oh_pack    Run1 feature assembly (:1240-1257, :1441-1488, :303-345)
 //   K5  oh_finalize           troposphere mask + unit conversion (:1579-1595)
@@ -38,10 +39,13 @@ uint64_t launch_count() { return g_launches; }
 // launches per kernel family: what the parity tests assert ("this launch was served by the two-level kernel").  The
 // predict families are ordered base, _missing, _leaf, _missing_leaf: base + has_missing + 2 * pred_leaf.
 namespace {
-enum Family { kDuo, kNodes8 = kDuo + 4, kSoaDuo = kNodes8 + 4, kSoaNodes8, kSealTiles, kShap, kShapReduce, kShapApprox, kFamilies };
+enum Family {
+  kDuo, kNodes8 = kDuo + 4, kSoaDuo = kNodes8 + 4, kSoaNodes8, kSealTiles, kShap, kShapReduce, kShapApprox, kDenseDuo, kDenseNodes8,
+  kFamilies
+};
 const char *const kFamilyName[kFamilies] = {"duo", "duo_missing", "duo_leaf", "duo_missing_leaf", "nodes8", "nodes8_missing",
                                             "nodes8_leaf", "nodes8_missing_leaf", "soa_duo", "soa_nodes8", "seal_tiles",
-                                            "shap", "shap_reduce", "shap_approx"};
+                                            "shap", "shap_reduce", "shap_approx", "dense_duo", "dense_nodes8"};
 thread_local uint64_t g_family[kFamilies];
 thread_local const char *g_last_predict = "";
 void count_family(int f) { ++g_family[f]; }
@@ -713,6 +717,80 @@ __global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_soa_kernel(D
   a.out[m] = export_transform(acc, a.exp10, a.scale);
 }
 
+// ---- inplace variant: the tile is assembled straight from a caller's dense float array ------------------------
+// (XGBoosterPredictFromDense / XGBoosterPredictFromCudaArray).  The same tile as predict_tiles_kernel walks — feature
+// slots of 1 KB, absent columns missing, the key-0 slot last — built in shared memory from the strided array, so no
+// copy of the array and no key tiles go to HBM.  Rows keep their order: a warp takes the default-direction walk when
+// one of its 32 rows holds a missing entry, and MissingWalk serves it when Walk cannot walk missing entries.  Ranges
+// of trees are separate launches (the partial sum travels through `out` as in predict_tiles_kernel); each one
+// reassembles the tile.
+template <class Walk, class MissingWalk>
+__global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_dense_kernel(DeviceForest f, PredictArgs a, DenseArgs d) {
+  extern __shared__ __align__(128) uint32_t skey[];
+  const int tid = threadIdx.x, ncol = a.ncol;
+  const uint64_t r0 = (uint64_t)blockIdx.x * kBlock;
+  const uint64_t left = a.nrow - r0;
+  const int nr = left < (uint64_t)kBlock ? (int)left : kBlock;
+  const bool live = tid < nr;
+  const bool chk_inf = !isinf(d.missing);
+  int flags = 0;
+  auto key = [&](float x) {
+    if (chk_inf && isinf(x)) flags |= 2;
+    if (x != x || x == d.missing) {
+      flags |= 1;
+      return kKeyMissing;
+    }
+    return float_key(x);
+  };
+  if (d.col_stride == 1 && d.row_stride == ncol) {
+    // contiguous rows: one flat coalesced copy into a row-major staging area of odd stride (conflict-free per-thread
+    // row reads, as in seal_tiles_kernel) that aliases the key slots; each thread lifts its row through registers
+    float *stage = reinterpret_cast<float *>(skey);
+    const int ld = ncol | 1, n = nr * ncol;
+    const float *__restrict__ src = d.X + r0 * (uint64_t)ncol;
+    if (ld == ncol && (((uintptr_t)src) & 15u) == 0u) {
+      const float4 *s4 = reinterpret_cast<const float4 *>(src);
+      float4 *d4 = reinterpret_cast<float4 *>(stage);
+      for (int i = tid; i < (n >> 2); i += kBlock) d4[i] = __ldg(s4 + i);
+      for (int i = (n & ~3) + tid; i < n; i += kBlock) stage[i] = __ldg(src + i);
+    } else if (ld == ncol) {
+      for (int i = tid; i < n; i += kBlock) stage[i] = __ldg(src + i);
+    } else {
+      for (int i = tid; i < n; i += kBlock) stage[(i / ncol) * ld + (i % ncol)] = __ldg(src + i);
+    }
+    __syncthreads();
+    uint32_t k[kMaxFeatures];
+#pragma unroll
+    for (int c = 0; c < (int)kMaxFeatures; ++c)
+      if (c < ncol) k[c] = live ? key(stage[tid * ld + c]) : 0u;
+    __syncthreads();
+#pragma unroll
+    for (int c = 0; c < (int)kMaxFeatures; ++c)
+      if (c < ncol) skey[c * kStride + tid] = k[c];
+  } else {
+    // any other strides: element by element; a feature-major array is coalesced per feature
+    const float *__restrict__ src = d.X + (r0 + (uint64_t)tid) * d.row_stride;
+    for (int c = 0; c < ncol; ++c) skey[c * kStride + tid] = live ? key(__ldg(src + (int64_t)c * d.col_stride)) : 0u;
+  }
+  for (int c = ncol; c < f.nfeat; ++c) skey[c * kStride + tid] = kKeyMissing;
+  skey[f.nfeat * kStride + tid] = 0u;
+  // __syncthreads_or returns a truth value, not the bitwise OR: one vote for the inf flag
+  if (__syncthreads_or(flags & 2) != 0) {
+    if (tid == 0) atomicOr(d.flags, 2);
+  }
+  const bool hm = __any_sync(0xffffffffu, flags & 1) || ncol < f.nfeat;
+  if (!live) return;
+  const uint32_t my = (uint32_t)__cvta_generic_to_shared(skey + tid);
+  row_result<false>(f, a, r0 + (uint64_t)tid, true, [&](auto &&emit) {
+    if (!hm)
+      Walk::template run<false, false>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
+    else if (Walk::walks_missing(f))
+      Walk::template run<true, false>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
+    else
+      MissingWalk::template run<true, false>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
+  });
+}
+
 // The layout rule of the predict launches: the two-level records when the window holds the record tops of trees
 // [t0, t1) and the rows have no missing entries or the records carry the default bits; otherwise the 8-byte nodes,
 // with the table when the window holds their node tops, and through the LSU alone when there is no node texture.
@@ -742,6 +820,30 @@ cudaError_t launch_predict_soa(const DeviceForest &f, const ConstWindow &w, cons
   if (e != cudaSuccess) return e;
   k<<<dim3((unsigned)nblk), kBlock, smem, s>>>(f, a);
   count_family(l == Layout::kRecords ? kSoaDuo : kSoaNodes8);
+  return QC_LAUNCHED();
+}
+
+cudaError_t launch_predict_dense(const DeviceForest &f, const ConstWindow &w, const PredictArgs &args, const DenseArgs &d, cudaStream_t s) {
+  if (args.nrow == 0 || args.tree_end <= args.tree_begin) return cudaSuccess;
+  if (args.ncol > f.nfeat || f.nfeat > (int)kMaxFeatures || args.pred_leaf) return cudaErrorInvalidValue;
+  // the key slots 0..nfeat; the row-major staging area of the contiguous loader ((ncol | 1) KB) fits in them
+  const size_t smem = (size_t)kStride * (size_t)(f.nfeat + 1) * sizeof(uint32_t);
+  const uint64_t grid = tile_count(args.nrow);
+  if (grid > 0x7fffffffull) return cudaErrorInvalidConfiguration;
+  PredictArgs a = args;
+  a.ctree0 = w.tree0;
+  // as in launch_predict_soa: the layout of clean rows; the kernel sends a warp with missing entries the records cannot
+  // walk to the 8-byte nodes without the table
+  const Layout l = layout(f, w, a.tree_begin, a.tree_end, false);
+  auto k = predict_dense_kernel<RecordsWalk, NodesTexWalk>;
+  if (f.duo_shallow) k = predict_dense_kernel<RecordsShallowWalk, NodesTexWalk>;
+  if (l == Layout::kNodesTable) k = predict_dense_kernel<NodesTableWalk, NodesTableWalk>;
+  if (l == Layout::kNodesTex) k = predict_dense_kernel<NodesTexWalk, NodesTexWalk>;
+  if (l == Layout::kNodesLsu) k = predict_dense_kernel<NodesLsuWalk, NodesLsuWalk>;
+  cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  k<<<dim3((unsigned)grid), kBlock, smem, s>>>(f, a, d);
+  count_predict(l == Layout::kRecords ? kDenseDuo : kDenseNodes8);
   return QC_LAUNCHED();
 }
 

@@ -96,6 +96,18 @@ cudaError_t launch_seal_tiles(const float *X, uint64_t nrow, int ncol, float mis
 
 cudaError_t launch_predict(const DeviceForest &f, const ConstWindow &w, const PredictArgs &a, cudaStream_t s);
 
+// Inplace prediction from a dense float array (XGBoosterPredictFromDense / FromCudaArray): row r, column c of the
+// array is X[r * row_stride + c * col_stride].  The predict kernel builds its key tiles from it in shared memory
+// (value / margin sums only); PredictArgs::Xt and has_missing are not read.
+struct DenseArgs {
+  const float *X = nullptr;  // device
+  int64_t row_stride = 0;    // in floats
+  int64_t col_stride = 1;
+  float missing = -999.f;    // entries that are NaN or == missing are missing
+  int *flags = nullptr;      // |= 2 on +-inf input when `missing` is finite
+};
+cudaError_t launch_predict_dense(const DeviceForest &f, const ConstWindow &w, const PredictArgs &a, const DenseArgs &d, cudaStream_t s);
+
 // Per-feature contributions (forest.hpp ShapForest).  out: [nrow][nfeat + 1] floats, column nfeat = `bias`.
 //   exact (TreeSHAP on the path bins): launch_shap writes float64 partial sums of bin slice s to
 //   part[s][nrow][nfeat]; launch_shap_reduce adds the slices in slice order and rounds once.  The slicing depends
