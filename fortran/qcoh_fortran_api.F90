@@ -178,6 +178,19 @@ module qcoh_fortran_api
        type(c_ptr) :: out_result     ! const float** (device memory)
      end function
 
+     ! SHAP interaction values of a DMatrix into a DEVICE buffer of nrow * (num_feature + 1)**2 floats (out_dev, e.g. from
+     ! qcoh_device_alloc): row-major [nrow][i][j], i the conditioning feature, index num_feature the bias, i.e.
+     ! M(j, i, row) in Fortran order.  approximate /= 0 gives libxgboost's type 5; ntree_limit 0 = all trees (C unsigned:
+     ! pass a non-negative value).  Asynchronous: qcoh_device_synchronize before reading.  Explain a slab of rows at a
+     ! time: each row takes 3136 B of output at 27 features.
+     integer(c_int) function qcoh_booster_predict_interactions_device(handle, dmat, approximate, ntree_limit, out_dev) &
+          bind(C, name="qcoh_booster_predict_interactions_device")
+       import :: c_int, c_ptr
+       type(c_ptr), value :: handle, dmat
+       integer(c_int), value :: approximate, ntree_limit
+       type(c_ptr), value :: out_dev
+     end function
+
      function XGBGetLastError_c() bind(C, name="XGBGetLastError") result(msg)
        import :: c_ptr
        type(c_ptr) :: msg

@@ -210,6 +210,14 @@ int qcoh_booster_predict_device(BoosterHandle handle, DMatrixHandle dmat, int op
  * Asynchronous on the library stream; qcoh_device_synchronize() to wait. */
 int qcoh_booster_predict_contribs_device(BoosterHandle handle, DMatrixHandle dmat, int approximate,
                                          unsigned ntree_limit, float *out_dev);
+/* SHAP interaction values into a DEVICE buffer of nrow * (num_feature + 1)^2 floats, out[row][i][j] row-major, row i
+ * the conditioning feature, index num_feature the bias (libxgboost's pred_interactions, PredictInteractionContributions:
+ * type 4, or type 5 when approximate != 0; ntree_limit 0 = all trees).  Every row of M sums to the row's contribution,
+ * M[F][F] is the contributions' bias, and the bias row and column are otherwise 0.  Exact values take about 57
+ * conditioned TreeSHAP passes per row: explain a slab of rows at a time.  Asynchronous on the library stream;
+ * qcoh_device_synchronize() to wait. */
+int qcoh_booster_predict_interactions_device(BoosterHandle handle, DMatrixHandle dmat, int approximate,
+                                             unsigned ntree_limit, float *out_dev);
 /* Library settings of the calling thread; values are integers.  Any other name fails with "unknown parameter".
  *   duo         0: predict on the 8-byte nodes only.  Any other value (default -1): on the two-level records
  *               whenever the booster's records and the matrix allow it.
@@ -223,7 +231,9 @@ uint64_t qcoh_launch_count(void);
 /* Which kernel family served a prediction — what the parity tests assert.  Families: "duo" (two-level records),
  * "nodes8" (8-byte depth-ordered nodes), each with the suffixes "_missing" (matrix with missing entries) and
  * "_leaf" (option_mask = 2), e.g. "duo_missing_leaf"; "soa_duo" / "soa_nodes8" (fused Run1); "seal_tiles";
- * "shap" (exact contributions) with its slice reduction "shap_reduce", and "shap_approx" (approximate contributions).
+ * "shap" (exact contributions) with its slice reduction "shap_reduce", and "shap_approx" (approximate contributions);
+ * "shap_inter" (exact interaction values, after a "shap" launch for the same rows) with "shap_inter_reduce", and
+ * "shap_inter_expand" (approximate interaction values, after a "shap_approx" launch).
  * qcoh_kernel_launches counts launches of one family since load; qcoh_last_predict_kernel names the family of the
  * last XGBoosterPredict-side launch ("" before the first). */
 uint64_t qcoh_kernel_launches(const char *family);

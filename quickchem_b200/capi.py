@@ -70,6 +70,7 @@ QCOH_SYMBOLS = ("qcoh_version", "qcoh_device_count", "qcoh_set_device", "qcoh_ho
                 "qcoh_device_synchronize", "qcoh_timer_start", "qcoh_timer_stop", "qcoh_flush_l2",
                 "qcoh_booster_parse", "qcoh_booster_get_info", "qcoh_booster_get_flat", "qcoh_booster_get_duo",
                 "qcoh_booster_get_duo_info", "qcoh_booster_get_shap_paths", "qcoh_booster_predict_contribs_device",
+                "qcoh_booster_predict_interactions_device",
                 "qcoh_dmatrix_create_device", "qcoh_dmatrix_device_ptr", "qcoh_dmatrix_upload", "qcoh_dmatrix_seal",
                 "qcoh_booster_predict_device", "qcoh_set_param", "qcoh_launch_count", "qcoh_kernel_launches",
                 "qcoh_last_predict_kernel", "qcoh_dmatrix_tiles_ptr", "qcoh_oh_invalidate_sza", "qcoh_oh_create",
@@ -135,6 +136,7 @@ def lib():
         for name in ("XGBoosterPredictFromDense", "XGBoosterPredictFromCudaArray"):
             getattr(L, name).argtypes = [vp, C.c_char_p, C.c_char_p, vp, C.POINTER(C.POINTER(u64)), C.POINTER(u64), C.POINTER(f32p)]
         L.qcoh_booster_predict_contribs_device.argtypes = [vp, vp, C.c_int, C.c_uint, vp]
+        L.qcoh_booster_predict_interactions_device.argtypes = [vp, vp, C.c_int, C.c_uint, vp]
         L.qcoh_booster_get_shap_paths.argtypes = [vp, C.POINTER(C.POINTER(C.c_uint32)), C.POINTER(C.POINTER(C.c_int64)),
                                                   C.POINTER(C.POINTER(C.c_float)), C.POINTER(C.c_int64)]  # fmt: skip
         L.qcoh_set_param.argtypes = [C.c_char_p, C.c_char_p]
@@ -488,6 +490,26 @@ class Booster:
         """qcoh_booster_predict_contribs_device: the same into a device buffer of nrow * (num_feature + 1) floats,
         asynchronous on the library stream."""
         check(lib().qcoh_booster_predict_contribs_device(self.handle, dmat.handle, int(approximate), ntree_limit, out.ptr))
+
+    def predict_interactions(self, dmat: DMatrix, approximate=False, ntree_limit=0) -> np.ndarray:
+        """[nrow, num_feature + 1, num_feature + 1] SHAP interaction values (libxgboost's pred_interactions, type 4 /
+        5): M[i][j] is the part of feature i's contribution shared with feature j, index num_feature the bias; each row
+        of M sums to the contribution, the whole matrix to the margin."""
+        nc = self.info().num_feature + 1
+        nrow = dmat.num_row
+        out = DeviceArray(nrow * nc * nc)
+        try:
+            self.predict_interactions_device(dmat, out, approximate, ntree_limit)
+            synchronize()
+            return out.get().reshape(nrow, nc, nc)
+        finally:
+            out.free()
+
+    def predict_interactions_device(self, dmat: DMatrix | None, out: DeviceArray | None, approximate=False, ntree_limit=0):
+        """qcoh_booster_predict_interactions_device: the same into a device buffer of nrow * (num_feature + 1)**2
+        floats, asynchronous on the library stream."""
+        check(lib().qcoh_booster_predict_interactions_device(self.handle, None if dmat is None else dmat.handle,
+                                                             int(approximate), ntree_limit, None if out is None else out.ptr))  # fmt: skip
 
     def shap_paths(self):
         """(bins[nbins,32,4] uint32, tree_bin[T+1] int64, node_mean[num_nodes] float32) copies of the contribution

@@ -195,9 +195,9 @@ const ShapForest &shap_tables(Booster *b) {
   return b->shap;
 }
 
-// Per-feature contributions into a device buffer [nrow][num_feature + 1], asynchronous on the library stream.  The
-// path bins and node means go to HBM at the first call (not at load: prediction alone never needs them).
-static void contribs_into(Booster *b, DMatrix *d, bool approximate, unsigned ntree_limit, float *out_dev) {
+// The contribution tables of the booster in HBM, for a sealed matrix of at most num_feature columns.  The path bins
+// and node means go to HBM at the first call (not at load: prediction alone never needs them).
+static const ShapForest &shap_on_device(Booster *b, DMatrix *d) {
   const ShapForest &s = shap_tables(b);
   upload(b);
   if (!d->sealed) seal(d);
@@ -211,6 +211,13 @@ static void contribs_into(Booster *b, DMatrix *d, bool approximate, unsigned ntr
     CU(cudaMemcpy(b->d_shap_mean.need(nn), s.mean.data(), nn * sizeof(float), cudaMemcpyHostToDevice));
     b->shap_uploaded = true;
   }
+  return s;
+}
+
+// Per-feature contributions into a device buffer [nrow][num_feature + 1], asynchronous on the library stream.
+static void contribs_into(Booster *b, DMatrix *d, bool approximate, unsigned ntree_limit, float *out_dev) {
+  const ShapForest &s = shap_on_device(b, d);
+  const uint32_t nf = b->host.num_feature;
   const int nt = (int)trees_used(b, ntree_limit);
   ContribArgs a;
   a.ncol = (int32_t)d->ncol, a.nfeat = (int32_t)nf;
@@ -229,6 +236,48 @@ static void contribs_into(Booster *b, DMatrix *d, bool approximate, unsigned ntr
     c.out = out_dev + r0 * (nf + 1);
     CU(launch_shap(b->d_shap_bins.p, nb, ns, c, part, g.stream));
     CU(launch_shap_reduce(part, ns, c, g.stream));
+  }
+}
+
+// SHAP interaction values into a device buffer [nrow][num_feature + 1][num_feature + 1], asynchronous on the library
+// stream.  Exact: per chunk of kInterChunkRows rows, the contribution slices (phi) and the conditioned paths of every
+// feature, reduced together.  The per-feature bin lists are built and go to HBM at the first interactions call.
+static void interactions_into(Booster *b, DMatrix *d, bool approximate, unsigned ntree_limit, float *out_dev) {
+  const ShapForest &s = shap_on_device(b, d);
+  const uint32_t nf = b->host.num_feature;
+  if (d->nrow && !out_dev) throw Error("qcoh_booster_predict_interactions_device: NULL output buffer");
+  const int nt = (int)trees_used(b, ntree_limit);
+  ContribArgs a;
+  a.ncol = (int32_t)d->ncol, a.nfeat = (int32_t)nf;
+  a.bias = shap_bias(s, b->host, b->flat, nt);
+  if (approximate) {
+    float *phi = b->d_inter_phi.need((size_t)d->nrow * (nf + 1));
+    a.Xt = d->Xt.p, a.nrow = d->nrow, a.out = phi;
+    CU(launch_shap_approx(b->dev, b->d_shap_mean.p, nt, a, g.stream));
+    a.out = out_dev;
+    CU(launch_shap_inter_expand(phi, a, g.stream));
+    return;
+  }
+  if (!b->inter_uploaded) {
+    if (s.feat_off.empty()) build_shap_by_feature(b->shap, nf);
+    CU(cudaMemcpy(b->d_inter_off.need(s.feat_off.size()), s.feat_off.data(), s.feat_off.size() * sizeof(int64_t),
+                  cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(b->d_inter_bins.need(s.feat_bins.size()), s.feat_bins.data(), s.feat_bins.size() * sizeof(uint32_t),
+                  cudaMemcpyHostToDevice));
+    b->inter_uploaded = true;
+  }
+  const int64_t nb = s.tree_bin[(size_t)nt];
+  const int ns = (int)std::min<int64_t>(kShapSlices, nb);
+  const size_t rows = (size_t)std::min<uint64_t>(kInterChunkRows, d->nrow), nc = (size_t)nf + 1;
+  double *shap_part = b->d_shap_part.need((size_t)ns * rows * nf);
+  double *part = b->d_inter_part.need((size_t)nf * kInterSlices * rows * nf);
+  for (uint64_t r0 = 0; r0 < d->nrow; r0 += kInterChunkRows) {
+    ContribArgs c = a;
+    c.Xt = d->Xt.p + tile_offset_words(r0, d->ncol), c.nrow = std::min<uint64_t>(kInterChunkRows, d->nrow - r0);
+    c.out = out_dev + r0 * nc * nc;
+    CU(launch_shap(b->d_shap_bins.p, nb, ns, c, shap_part, g.stream));
+    CU(launch_shap_inter(b->d_shap_bins.p, b->d_inter_off.p, b->d_inter_bins.p, nb, c, part, g.stream));
+    CU(launch_shap_inter_reduce(part, shap_part, ns, c, g.stream));
   }
 }
 
@@ -638,7 +687,7 @@ int qcoh_booster_parse(BoosterHandle handle, const char *fname) {
   FlatForest ff = flatten(hf);
   DuoForest df = build_duo(ff, hf.num_feature);
   b->host = std::move(hf), b->flat = std::move(ff), b->duo = std::move(df);
-  b->shap = ShapForest(), b->shap_uploaded = false;
+  b->shap = ShapForest(), b->shap_uploaded = false, b->inter_uploaded = false;
   b->loaded = true, b->uploaded = false;
   b->version = ++g_version_counter;
   API_END
@@ -759,7 +808,8 @@ int XGBoosterPredictFromDMatrix(BoosterHandle handle, DMatrixHandle dmat, const 
   const PredictConfig c = parse_predict_config(config);
   const std::string ty = std::to_string(c.type);
   if (c.type == 4 || c.type == 5)
-    throw Error("XGBoosterPredictFromDMatrix: type " + ty + " (SHAP interaction values) is not supported; 2 and 3 give per-feature contributions");
+    throw Error("XGBoosterPredictFromDMatrix: type " + ty + " (SHAP interaction values) is not supported; 2 and 3 give per-feature contributions, and "
+                "qcoh_booster_predict_interactions_device computes interaction values");
   const bool contribs = c.type == 2 || c.type == 3;
   if (!contribs && c.type != 0 && c.type != 1 && c.type != 6)
     throw Error("XGBoosterPredictFromDMatrix: unknown prediction type " + ty + " (0 value, 1 margin, 2 / 3 contributions, 6 leaf)");
@@ -1157,6 +1207,16 @@ int qcoh_booster_predict_contribs_device(BoosterHandle handle, DMatrixHandle dma
                                          float *out_dev) {
   API_BEGIN
   contribs_into(B(handle), D(dmat), approximate != 0, ntree_limit, out_dev);
+  API_END
+}
+
+int qcoh_booster_predict_interactions_device(BoosterHandle handle, DMatrixHandle dmat, int approximate, unsigned ntree_limit,
+                                             float *out_dev) {
+  API_BEGIN
+  Booster *b = B(handle);
+  (void)shap_tables(b);  // a booster without covers fails here, before any device work
+  ensure_device();
+  interactions_into(b, D(dmat), approximate != 0, ntree_limit, out_dev);
   API_END
 }
 

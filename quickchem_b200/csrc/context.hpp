@@ -230,6 +230,12 @@ struct Booster {
   DevBuf<uint4> d_shap_bins;
   DevBuf<float> d_shap_mean;
   DevBuf<double> d_shap_part;  // float64 partial sums of the bin slices, [kShapSlices][kShapChunkRows][nfeat]
+  // interactions: the per-feature bin lists (ShapForest::feat_off / feat_bins), uploaded at the first interactions call
+  bool inter_uploaded = false;
+  DevBuf<int64_t> d_inter_off;
+  DevBuf<uint32_t> d_inter_bins;
+  DevBuf<double> d_inter_part;  // [nfeat][kInterSlices][kInterChunkRows][nfeat]
+  DevBuf<float> d_inter_phi;    // approximate: the Saabas contributions [nrow][nfeat + 1] that go on the diagonal
   Booster() = default;
   Booster(const Booster &) = delete;
   Booster &operator=(const Booster &) = delete;

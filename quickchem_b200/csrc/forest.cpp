@@ -991,6 +991,24 @@ ShapForest build_shap(const HostForest &h, const FlatForest &f) {
   return s;
 }
 
+void build_shap_by_feature(ShapForest &s, uint32_t nfeat) {
+  std::vector<std::vector<uint32_t>> lists(nfeat);
+  const int64_t nb = s.num_bins();
+  for (int64_t b = 0; b < nb; ++b) {
+    uint32_t seen = 0u;  // features < kMaxFeatures = 31
+    for (int l = 0; l < 32; ++l) {
+      const uint32_t f = s.bins[(size_t)(b * 32 + l) * 4 + 2] & 0xFFu;
+      if (f < nfeat && !((seen >> f) & 1u)) seen |= 1u << f, lists[f].push_back((uint32_t)b);
+    }
+  }
+  s.feat_off.assign(1, 0);
+  s.feat_bins.clear();
+  for (const auto &v : lists) {
+    s.feat_bins.insert(s.feat_bins.end(), v.begin(), v.end());
+    s.feat_off.push_back((int64_t)s.feat_bins.size());
+  }
+}
+
 float shap_bias(const ShapForest &s, const HostForest &h, const FlatForest &f, int ntree) {
   float b = 0.f;
   for (int t = 0; t < ntree; ++t) b += 0.f + s.mean[f.tree_offset[t]];

@@ -111,10 +111,16 @@ struct ShapForest {
   std::vector<int64_t> tree_bin;   // [ntree + 1]
   int32_t max_path_len = 0;        // elements of the longest path, bias included
   int64_t num_paths = 0, num_elements = 0;
+  // interactions only (build_shap_by_feature, at the first interactions call): the bins holding a path that contains
+  // feature f are feat_bins[feat_off[f] .. feat_off[f + 1]), ascending, so the bins of the first t trees are a prefix
+  std::vector<int64_t> feat_off;
+  std::vector<uint32_t> feat_bins;
   int64_t num_bins() const { return (int64_t)(bins.size() / 128); }
 };
 // Throws unless every node of every tree has a finite, positive cover (sum_hess).
 ShapForest build_shap(const struct HostForest &h, const struct FlatForest &f);
+// Fills s.feat_off / s.feat_bins for features [0, nfeat).
+void build_shap_by_feature(ShapForest &s, uint32_t nfeat);
 // The bias column of a contributions row: ((0 + mean_0(root)) + mean_1(root) + ...) + base_score in float32.
 float shap_bias(const ShapForest &s, const struct HostForest &h, const struct FlatForest &f, int ntree);
 

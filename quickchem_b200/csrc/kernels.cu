@@ -13,6 +13,7 @@
 //                             oh_pack reads the features with too)
 //       predict_dense_kernel  K2 with the tile assembled from a caller's strided float array (inplace prediction)
 //   K6  shap_paths / shap_reduce / shap_approx   per-feature contributions (exact TreeSHAP, approximate Saabas)
+//       shap_inter / shap_inter_reduce / shap_inter_expand   SHAP interaction values (conditioned TreeSHAP)
 //   K1  oh_state / oh_sums / oh_pack    Run1 feature assembly (:1240-1257, :1441-1488, :303-345)
 //   K5  oh_finalize           troposphere mask + unit conversion (:1579-1595)
 //   K4  oh_diag               build-defined mass-weighted mean OH / CH4 lifetime partial sums
@@ -41,11 +42,12 @@ uint64_t launch_count() { return g_launches; }
 namespace {
 enum Family {
   kDuo, kNodes8 = kDuo + 4, kSoaDuo = kNodes8 + 4, kSoaNodes8, kSealTiles, kShap, kShapReduce, kShapApprox, kDenseDuo, kDenseNodes8,
-  kFamilies
+  kShapInter, kShapInterReduce, kShapInterExpand, kFamilies
 };
 const char *const kFamilyName[kFamilies] = {"duo", "duo_missing", "duo_leaf", "duo_missing_leaf", "nodes8", "nodes8_missing",
                                             "nodes8_leaf", "nodes8_missing_leaf", "soa_duo", "soa_nodes8", "seal_tiles",
-                                            "shap", "shap_reduce", "shap_approx", "dense_duo", "dense_nodes8"};
+                                            "shap", "shap_reduce", "shap_approx", "dense_duo", "dense_nodes8",
+                                            "shap_inter", "shap_inter_reduce", "shap_inter_expand"};
 thread_local uint64_t g_family[kFamilies];
 thread_local const char *g_last_predict = "";
 void count_family(int f) { ++g_family[f]; }
@@ -1014,11 +1016,16 @@ __global__ void __launch_bounds__(256) shap_reduce_kernel(const double *__restri
   }
 }
 
+// dynamic shared memory of shap_paths_kernel and shap_inter_kernel: shap_region_words, then keys and row order
+static size_t shap_smem_bytes(int nf) {
+  const int kst = nf | 1, ast = nf | 1;
+  return 4 * ((size_t)std::max(2 * kTileRows * ast, kTileRows * (nf + 2)) + (size_t)kTileRows * kst + kTileRows);
+}
+
 cudaError_t launch_shap(const uint4 *bins, int64_t nbins, int nslices, const ContribArgs &a, double *part, cudaStream_t s) {
   if (a.nrow == 0 || nbins <= 0 || nslices <= 0) return cudaSuccess;
   if (a.nrow > kShapChunkRows || a.ncol > a.nfeat || a.nfeat > (int)kMaxFeatures) return cudaErrorInvalidValue;
-  const int nf = a.nfeat, kst = nf | 1, ast = nf | 1;
-  const size_t smem = 4 * ((size_t)std::max(2 * kTileRows * ast, kTileRows * (nf + 2)) + (size_t)kTileRows * kst + kTileRows);
+  const size_t smem = shap_smem_bytes(a.nfeat);
   cudaError_t e = cudaFuncSetAttribute(shap_paths_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   shap_paths_kernel<<<dim3((unsigned)tile_count(a.nrow), (unsigned)nslices), kTileRows, smem, s>>>(bins, nbins, nslices, a, part);
@@ -1098,6 +1105,196 @@ cudaError_t launch_shap_approx(const DeviceForest &f, const float *mean, int ntr
   if (e != cudaSuccess) return e;
   shap_approx_kernel<<<(unsigned)ntile, kBlock, smem, s>>>(f, mean, ntree, a);
   count_predict(kShapApprox);
+  return QC_LAUNCHED();
+}
+
+// SHAP interaction values (libxgboost 1.6.0 PredictInteractionContributions).  libxgboost runs TreeShap conditioned
+// on feature c: c is never extended into the unique path, and at c's splits the cold branch gets condition fraction
+// 0 (c on) or each branch its cover ratio (c off).  On a path P with leaf v, where c's merged element has the one
+// fraction o_c and the zero fraction z_c, (on - off) / 2 adds to M[c][f_i], for every other element i,
+//     1/2 (o_c - z_c) W_i(P \ c) (o_i - z_i) v
+// with W_i(P \ c) the UnwoundPathSum of i in P extended without c (unique depth D - 1).  shap_inter_kernel is
+// shap_paths_kernel over the bins of c's list, with c's lane left out: the lanes of the path without c are addressed
+// through lane_of(p), so nothing is divided by o_c or z_c.  It accumulates (o_c - z_c) W_i (o_i - z_i) v; the reduce
+// halves the slice sums.  grid = (tiles, kInterSlices, nfeat): blockIdx.z is c.
+__global__ void __launch_bounds__(kTileRows, 2) shap_inter_kernel(const uint4 *__restrict__ bins, const int64_t *__restrict__ feat_off,
+                                                                  const uint32_t *__restrict__ feat_bins, int64_t nbins,
+                                                                  ContribArgs a, double *__restrict__ part) {
+  extern __shared__ __align__(128) uint32_t smem[];
+  __shared__ __align__(8) unsigned long long bars[1];
+  __shared__ double s_inv[34];  // 1 / k
+  __shared__ int64_t s_list[2];  // this CTA's range of c's list
+  const int nf = a.nfeat, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const uint32_t cf = blockIdx.z;
+  const int ast = nf | 1, kst = nf | 1;
+  double *acc = reinterpret_cast<double *>(smem);    // [256][ast] by tile position; the TMA buffer aliases its start
+  uint32_t *keys = smem + shap_region_words(nf);     // [256][kst] keys by tile position
+  uint32_t *order = keys + kTileRows * kst;          // [256] the tile's row order
+  PredictArgs pa;
+  pa.Xt = a.Xt, pa.nrow = a.nrow, pa.ncol = a.ncol;
+  TilePipe pipe;
+  pipe.begin(smem, bars, pa, nf, true, tid);
+  if (tid < 34) s_inv[tid] = tid ? 1.0 / (double)tid : 0.0;
+  if (tid == 0) {  // c's bins among the first nbins are a prefix of its ascending list; this CTA takes one slice of it
+    const int64_t l0 = feat_off[cf];
+    int64_t lo = l0, hi = feat_off[cf + 1];
+    while (lo < hi) {
+      const int64_t m = (lo + hi) >> 1;
+      if ((int64_t)feat_bins[m] < nbins) lo = m + 1;
+      else hi = m;
+    }
+    s_list[0] = l0 + (lo - l0) * (int64_t)blockIdx.y / kInterSlices;
+    s_list[1] = l0 + (lo - l0) * (int64_t)(blockIdx.y + 1) / kInterSlices;
+  }
+  (void)pipe.acquire(tid);
+  order[tid] = smem[tid];
+  for (int c = 0; c < nf; ++c) keys[tid * kst + c] = smem[(1 + c) * kStride + tid];
+  __syncthreads();
+  for (int i = tid; i < kTileRows * ast; i += kTileRows) acc[i] = 0.0;
+  __syncthreads();
+  const uint64_t tile = blockIdx.x;
+  const int64_t q0 = s_list[0], q1 = s_list[1];
+  for (int64_t q = q0; q < q1; ++q) {
+    const uint4 e = __ldg(bins + (int64_t)__ldg(feat_bins + q) * 32 + lane);
+    const uint32_t feat = e.z & 0xFFu, g0 = (e.z >> 16) & 31u, len = e.z >> 24;
+    const int j = lane - (int)g0;  // my place in my path
+    const bool elem = feat != kShapNoFeature && j >= 1, is_c = elem && feat == cf;
+    const bool miss_here = (e.z >> 8) & 1u;
+    const float zf = __uint_as_float(e.w);
+    const double z = elem ? (double)zf : 1.0;
+    const double v = (double)__shfl_sync(kFull, zf, (int)g0);  // leaf value, from the path's bias lane
+    const unsigned c_lanes = __ballot_sync(kFull, is_c) & (unsigned)(((1ull << len) - 1ull) << g0);
+    const bool has_c = c_lanes != 0u;
+    const int pc = has_c ? __ffs(c_lanes) - 1 - (int)g0 : 0;  // c's place in my path
+    const int Dr = has_c && !is_c ? (int)len - 2 : -1;        // unique depth of my path without c; -1: lane idle
+    const int jr = j < pc ? j : j - 1;                         // my place in the path without c
+    const bool adds = elem && Dr >= 0;
+    auto lane_of = [&](int p) { return ((int)g0 + p + (p >= pc ? 1 : 0)) & 31; };  // lane of place p without c
+    const int left = jr >= 1 ? lane_of(jr - 1) : lane, top = lane_of(Dr > 0 ? Dr : 0), c_lane = ((int)g0 + pc) & 31;
+    const int maxlen = (int)__reduce_max_sync(kFull, has_c ? len - 1u : 0u);  // lanes of the longest path without c
+    const double invz = 1.0 / z, d1 = (double)(Dr + 1), inv_d1 = s_inv[Dr + 1 > 0 ? Dr + 1 : 0];
+    const unsigned starts = __ballot_sync(kFull, has_c && j == 0);  // the paths that contain c, in lane order
+    for (int r = warp * 32; r < warp * 32 + 32; ++r) {
+      const uint32_t orig = order[r] & 0xFFu;
+      if (tile * kTileRows + orig >= a.nrow) continue;  // warp-uniform
+      bool one = true;
+      if (elem) {
+        const uint32_t k = keys[r * kst + feat];
+        one = k == kKeyMissing ? miss_here : (e.x <= k && k < e.y);
+      }
+      const float zo = one ? zf : -zf;  // (one, zero) of my element in one word: zero fractions are > 0
+      const float zc = __shfl_sync(kFull, zo, c_lane);
+      // ExtendPath over the elements other than c
+      double pw = jr == 0 ? 1.0 : 0.0;
+      for (int i = 1; i < maxlen; ++i) {
+        const float zi = __shfl_sync(kFull, zo, lane_of(i));
+        const double l = __shfl_sync(kFull, pw, left);
+        if (i <= Dr) {
+          const double inv = s_inv[i + 1];
+          pw = (double)fabsf(zi) * pw * (double)max(i - jr, 0) * inv + (zi > 0.f ? l : 0.0) * (double)jr * inv;
+        }
+      }
+      // UnwoundPathSum of my element in the path without c
+      double next = __shfl_sync(kFull, pw, top), total = 0.0;
+      for (int i = maxlen - 2; i >= 0; --i) {
+        const double pwi = __shfl_sync(kFull, pw, lane_of(min(i, Dr > 0 ? Dr : 0)));
+        if (i < Dr) {
+          if (one) {
+            const double tmp = next * d1 * s_inv[i + 1];
+            total += tmp;
+            next = pwi - tmp * z * (double)(Dr - i) * inv_d1;
+          } else {
+            total += pwi * invz * d1 * s_inv[Dr - i];
+          }
+        }
+      }
+      const double t = total * ((one ? 1.0 : 0.0) - z) * v * ((zc > 0.f ? 1.0 : 0.0) - (double)fabsf(zc));
+      double *arow = acc + r * ast;
+      for (unsigned g = starts; g; g &= g - 1u) {  // paths of the bin in order: a feature may recur across paths
+        if (adds && (int)g0 == __ffs(g) - 1) arow[feat] += t;
+        __syncwarp();
+      }
+    }
+  }
+  __syncthreads();
+  double *out = part + ((uint64_t)cf * kInterSlices + blockIdx.y) * a.nrow * (uint64_t)nf;
+  for (int i = tid; i < kTileRows * nf; i += kTileRows) {
+    const int p = i / nf, f = i - p * nf;
+    const uint64_t row = tile * kTileRows + (order[p] & 0xFFu);
+    if (row < a.nrow) out[row * (uint64_t)nf + f] = acc[p * ast + f];
+  }
+}
+
+// One thread per (row, conditioning feature): a row of M.  Off-diagonal: half the slice sums, added in slice order;
+// diagonal: phi_c (the contribution slices, in slice order) minus the off-diagonal sum of the row, in float64; bias
+// row: 0 and the contributions' bias.  Each output is rounded once.
+__global__ void __launch_bounds__(256) shap_inter_reduce_kernel(const double *__restrict__ part, const double *__restrict__ shap_part,
+                                                                int shap_slices, ContribArgs a) {
+  const int nf = a.nfeat, nc = nf + 1;
+  const uint64_t n = a.nrow * (uint64_t)nc, stride = (uint64_t)gridDim.x * blockDim.x;
+  for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+    const uint64_t row = i / (uint64_t)nc;
+    const int c = (int)(i - row * (uint64_t)nc);
+    float *o = a.out + i * (uint64_t)nc;
+    if (c == nf) {
+      for (int k = 0; k < nf; ++k) o[k] = 0.f;
+      o[nf] = a.bias;
+      continue;
+    }
+    double rs = 0.0;
+    for (int k = 0; k < nf; ++k) {
+      if (k == c) continue;
+      double s = 0.0;
+      for (int sl = 0; sl < kInterSlices; ++sl) s += part[(((uint64_t)c * kInterSlices + sl) * a.nrow + row) * (uint64_t)nf + k];
+      s *= 0.5;
+      o[k] = (float)s;
+      rs += s;
+    }
+    double phi = 0.0;
+    for (int sl = 0; sl < shap_slices; ++sl) phi += shap_part[((uint64_t)sl * a.nrow + row) * (uint64_t)nf + c];
+    o[c] = (float)(phi - rs);
+    o[nf] = 0.f;
+  }
+}
+
+// Approximate: libxgboost's loop with on == off gives +0 off the diagonal and 0 + phi_i on it.
+__global__ void __launch_bounds__(256) shap_inter_expand_kernel(const float *__restrict__ contribs, ContribArgs a) {
+  const uint64_t nc = (uint64_t)a.nfeat + 1, n = a.nrow * nc * nc, stride = (uint64_t)gridDim.x * blockDim.x;
+  for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+    const uint64_t row = i / (nc * nc), rem = i - row * nc * nc, c = rem / nc, k = rem - c * nc;
+    a.out[i] = k == c ? __fadd_rn(0.f, contribs[row * nc + c]) : 0.f;
+  }
+}
+
+cudaError_t launch_shap_inter(const uint4 *bins, const int64_t *feat_off, const uint32_t *feat_bins, int64_t nbins,
+                              const ContribArgs &a, double *part, cudaStream_t s) {
+  if (a.nrow == 0 || a.nfeat == 0) return cudaSuccess;
+  if (a.nrow > kInterChunkRows || a.ncol > a.nfeat || a.nfeat > (int)kMaxFeatures) return cudaErrorInvalidValue;
+  const size_t smem = shap_smem_bytes(a.nfeat);
+  cudaError_t e = cudaFuncSetAttribute(shap_inter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  const dim3 grid((unsigned)tile_count(a.nrow), (unsigned)kInterSlices, (unsigned)a.nfeat);
+  shap_inter_kernel<<<grid, kTileRows, smem, s>>>(bins, feat_off, feat_bins, nbins, a, part);
+  count_predict(kShapInter);
+  return QC_LAUNCHED();
+}
+
+cudaError_t launch_shap_inter_reduce(const double *part, const double *shap_part, int shap_slices, const ContribArgs &a,
+                                     cudaStream_t s) {
+  if (a.nrow == 0) return cudaSuccess;
+  const uint64_t n = a.nrow * (uint64_t)(a.nfeat + 1);
+  const int blocks = (int)std::min<uint64_t>((n + 255) / 256, (uint64_t)sm_count() * 16);
+  shap_inter_reduce_kernel<<<blocks, 256, 0, s>>>(part, shap_part, shap_slices, a);
+  count_family(kShapInterReduce);
+  return QC_LAUNCHED();
+}
+
+cudaError_t launch_shap_inter_expand(const float *contribs, const ContribArgs &a, cudaStream_t s) {
+  if (a.nrow == 0) return cudaSuccess;
+  const uint64_t n = a.nrow * (uint64_t)(a.nfeat + 1) * (uint64_t)(a.nfeat + 1);
+  const int blocks = (int)std::min<uint64_t>((n + 255) / 256, (uint64_t)sm_count() * 16);
+  shap_inter_expand_kernel<<<blocks, 256, 0, s>>>(contribs, a);
+  count_family(kShapInterExpand);
   return QC_LAUNCHED();
 }
 

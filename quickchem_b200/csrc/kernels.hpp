@@ -127,6 +127,23 @@ cudaError_t launch_shap(const uint4 *bins, int64_t nbins, int nslices, const Con
 cudaError_t launch_shap_reduce(const double *part, int nslices, const ContribArgs &a, cudaStream_t s);
 cudaError_t launch_shap_approx(const DeviceForest &f, const float *mean, int ntree, const ContribArgs &a, cudaStream_t s);
 
+// SHAP interaction values (libxgboost 1.6.0 PredictInteractionContributions).  out: [nrow][nfeat + 1][nfeat + 1]
+// floats, row i the conditioning feature, index nfeat the bias.
+//   exact: launch_shap_inter runs, for every conditioning feature c, the paths of c's bins (ShapForest::feat_bins,
+//   the first nbins of the booster only) extended without c's element, and writes float64 partial sums of slice s of
+//   c's list to part[c][s][nrow][nfeat]; launch_shap_inter_reduce adds the slices in slice order, halves them for the
+//   off-diagonal and takes the diagonal as phi_c (the slices of launch_shap in shap_part) minus the row's
+//   off-diagonal sum, rounding each output once.  The slicing of c's list depends only on the list and nbins.
+//   approximate: launch_shap_inter_expand puts the Saabas row contribs[nrow][nfeat + 1] of launch_shap_approx on the
+//   diagonal (0 + phi) and +0 elsewhere, as libxgboost's loop does when on == off.
+constexpr int kInterSlices = 16;
+constexpr uint64_t kInterChunkRows = 4096;  // part[] holds nfeat x 16 x 4096 x nfeat doubles: 382 MB at 27 features
+cudaError_t launch_shap_inter(const uint4 *bins, const int64_t *feat_off, const uint32_t *feat_bins, int64_t nbins,
+                              const ContribArgs &a, double *part, cudaStream_t s);
+cudaError_t launch_shap_inter_reduce(const double *part, const double *shap_part, int shap_slices, const ContribArgs &a,
+                                     cudaStream_t s);
+cudaError_t launch_shap_inter_expand(const float *contribs, const ContribArgs &a, cudaStream_t s);
+
 // Where the 27 Run1 features come from, in feature order (filled by qcoh_oh_run1): feature f of cell e in column c is
 // src3[f][e], or src2[f][c] for a 2-D field; feature 1 is PL_BST / 100, computed from ple.  kernels.cu run1_feature
 // reads it for both the fused predict and the matrix pack.
