@@ -178,6 +178,46 @@ module qcoh_fortran_api
        type(c_ptr) :: out_result     ! const float** (device memory)
      end function
 
+     ! Columnar inplace prediction: values is a JSON LIST of 1-D interfaces, one per feature column in device memory, e.g.
+     ! for 27 level-slab fields F_f(ncells) ('//' joins, one entry per field):
+     !   '[{"data": [<address of F_1>, false], "shape": [ncells], "strides": null, "typestr": "<f4", "version": 3}, ...]'
+     ! Config, checks and result (a booster-owned DEVICE buffer) are those of XGBoosterPredictFromCudaArray.
+     integer(c_int) function XGBoosterPredictFromCudaColumnar(handle, values, config, m, out_shape, out_dim, out_result) &
+          bind(C, name="XGBoosterPredictFromCudaColumnar")
+       import :: c_int, c_ptr, c_char, c_int64_t
+       type(c_ptr), value :: handle, m
+       character(len=1, kind=c_char), dimension(*) :: values, config
+       type(c_ptr) :: out_shape      ! const bst_ulong**
+       integer(c_int64_t) :: out_dim ! bst_ulong*
+       type(c_ptr) :: out_result     ! const float** (device memory)
+     end function
+
+     ! A DMatrix from arrays, without a transpose (include/qcoh.h): data is one array interface as for the inplace calls
+     ! above (FromDense: C-contiguous host memory; FromCudaArrayInterface: device memory with any strides, e.g. XX(nrow, 27)
+     ! as '"shape": [nrow, 27], "strides": [4, <4 * nrow>]') or, for FromCudaColumnar, a list of column interfaces as for
+     ! XGBoosterPredictFromCudaColumnar.  config is '{"missing": -999.0}' (ending in c_null_char).  The DMatrix is sealed
+     ! when the call returns and is the one XGDMatrixCreateFromMat makes from the same values in row-major order; explain
+     ! it with qcoh_booster_predict_contribs_device / qcoh_booster_predict_interactions_device and free it with
+     ! XGDMatrixFree.
+     integer(c_int) function XGDMatrixCreateFromDense(data, config, out) bind(C, name="XGDMatrixCreateFromDense")
+       import :: c_int, c_ptr, c_char
+       character(len=1, kind=c_char), dimension(*) :: data, config
+       type(c_ptr) :: out
+     end function
+
+     integer(c_int) function XGDMatrixCreateFromCudaArrayInterface(data, config, out) &
+          bind(C, name="XGDMatrixCreateFromCudaArrayInterface")
+       import :: c_int, c_ptr, c_char
+       character(len=1, kind=c_char), dimension(*) :: data, config
+       type(c_ptr) :: out
+     end function
+
+     integer(c_int) function XGDMatrixCreateFromCudaColumnar(data, config, out) bind(C, name="XGDMatrixCreateFromCudaColumnar")
+       import :: c_int, c_ptr, c_char
+       character(len=1, kind=c_char), dimension(*) :: data, config
+       type(c_ptr) :: out
+     end function
+
      ! SHAP interaction values of a DMatrix into a DEVICE buffer of nrow * (num_feature + 1)**2 floats (out_dev, e.g. from
      ! qcoh_device_alloc): row-major [nrow][i][j], i the conditioning feature, index num_feature the bias, i.e.
      ! M(j, i, row) in Fortran order.  approximate /= 0 gives libxgboost's type 5; ntree_limit 0 = all trees (C unsigned:

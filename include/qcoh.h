@@ -97,6 +97,17 @@ int XGBoosterPredictFromDense(BoosterHandle handle, const char *values, const ch
                               const bst_ulong **out_shape, bst_ulong *out_dim, const float **out_result);
 int XGBoosterPredictFromCudaArray(BoosterHandle handle, const char *values, const char *config, DMatrixHandle m,
                                   const bst_ulong **out_shape, bst_ulong *out_dim, const float **out_result);
+/* libxgboost 1.6.0 c_api.h (declarations restated; parity with libxgboost's own behaviour is not pinned, as for the
+ * rest of its surface here): the columnar inplace predict, the call behind xgboost's Booster.inplace_predict(cuDF).
+ * values: a JSON LIST of 1-D array interfaces, one per column, each {"data": [address, readonly], "shape": [nrow],
+ * "strides": null | [bytes] (a positive multiple of 4), "typestr": "<f4"[, "stream": s]}; a value that is not a list,
+ * an empty list, a column that is not 1-D, columns of different lengths, more than 192 columns, another type, a mask, a
+ * NULL address for a non-empty column, stream 0 and a column in host memory fail, naming the column.  Each distinct
+ * stream is waited for before the columns are read.  Config, checks, result and shape are those of
+ * XGBoosterPredictFromCudaArray: the result is a DEVICE buffer.  dtypes other than <f4 and cuDF validity masks are not
+ * supported. */
+int XGBoosterPredictFromCudaColumnar(BoosterHandle handle, const char *values, const char *config, DMatrixHandle m,
+                                     const bst_ulong **out_shape, bst_ulong *out_dim, const float **out_result);
 
 /* xgb_fortran_api.F90:75-83; call site OH_GridCompMod.F90:256.  The reference passes a DMatrix
  * handle *by value* as `dmats` with len = 0; dmats is never dereferenced when len == 0. */
@@ -108,6 +119,26 @@ int XGBoosterCreate(const DMatrixHandle dmats[], bst_ulong len, BoosterHandle *o
  * fails like libxgboost.  The matrix is copied to HBM here. */
 int XGDMatrixCreateFromMat(const float *data, bst_ulong nrow, bst_ulong ncol, float missing,
                            DMatrixHandle *out);
+
+/* libxgboost 1.6.0 c_api.h (declarations restated; parity with libxgboost's own behaviour is not pinned): the
+ * array-interface DMatrix constructors, what xgboost's Python DMatrix(numpy / cupy / torch / cuDF) calls.  data: one
+ * 2-D array interface as for XGBoosterPredictFromDense / FromCudaArray (the same refusals, naming the new caller), or
+ * for FromCudaColumnar a list of 1-D column interfaces as for XGBoosterPredictFromCudaColumnar.  config: {"missing":
+ * number, "nthread": int}; missing is required (NaN is written NaN), nthread and other keys are ignored.  Entries that
+ * are NaN or == missing are missing; +-inf with a finite missing fails like XGDMatrixCreateFromMat, and then no handle
+ * is created.  "stream" entries are waited for before the input is read.  Each call returns when the DMatrix is sealed
+ * (the caller may then free or overwrite its arrays), and the DMatrix is the one XGDMatrixCreateFromMat makes from the
+ * same values in row-major order: the same X, key tiles, flags, NumRow / NumCol, and every call on it behaves alike.
+ *   FromDense: HOST memory, C-contiguous (other strides fail); it takes XGDMatrixCreateFromMat's host path, including
+ *   the `speculate` setting.  A device address (detected) is read like FromCudaArrayInterface.
+ *   FromCudaArrayInterface: DEVICE memory, any strides.  A C-contiguous array is copied and sealed as
+ *   XGDMatrixCreateFromMat does; any other layout (e.g. feature-major [ncol][nrow], strides [4, 4 * nrow]) is read in
+ *   place by the seal_columns kernel, without a transpose.
+ *   FromCudaColumnar: DEVICE columns (e.g. the 27 fields of a level slab), each read in place by seal_columns.
+ * dtypes other than <f4, cuDF validity masks and XGDMatrixSliceDMatrix are not supported. */
+int XGDMatrixCreateFromDense(const char *data, const char *config, DMatrixHandle *out);
+int XGDMatrixCreateFromCudaArrayInterface(const char *data, const char *config, DMatrixHandle *out);
+int XGDMatrixCreateFromCudaColumnar(const char *data, const char *config, DMatrixHandle *out);
 
 /* xgb_fortran_api.F90:97-104 and :106-113.  Unused by OH. */
 int XGDMatrixNumRow(DMatrixHandle handle, bst_ulong *out);

@@ -64,7 +64,8 @@ class Run1Out(C.Structure):
 XGB_SYMBOLS = ("XGBoosterLoadModel", "XGBoosterSaveModel", "XGDMatrixSaveBinary", "XGDMatrixFree",
                "XGDMatrixCreateFromFile", "XGBoosterPredict", "XGBoosterCreate", "XGDMatrixCreateFromMat",
                "XGDMatrixNumRow", "XGDMatrixNumCol", "XGBoosterFree", "XGBGetLastError", "XGBoosterPredictFromDMatrix",
-               "XGBoosterPredictFromDense", "XGBoosterPredictFromCudaArray")  # fmt: skip
+               "XGBoosterPredictFromDense", "XGBoosterPredictFromCudaArray", "XGBoosterPredictFromCudaColumnar",
+               "XGDMatrixCreateFromDense", "XGDMatrixCreateFromCudaArrayInterface", "XGDMatrixCreateFromCudaColumnar")  # fmt: skip
 QCOH_SYMBOLS = ("qcoh_version", "qcoh_device_count", "qcoh_set_device", "qcoh_host_alloc", "qcoh_host_free",
                 "qcoh_device_alloc", "qcoh_device_free", "qcoh_memcpy_h2d", "qcoh_memcpy_d2h",
                 "qcoh_device_synchronize", "qcoh_timer_start", "qcoh_timer_stop", "qcoh_flush_l2",
@@ -133,7 +134,9 @@ def lib():
         L.qcoh_booster_predict_device.argtypes = [vp, vp, C.c_int, C.c_uint, C.POINTER(Epilogue), vp]
         L.XGBoosterPredictFromDMatrix.argtypes = [vp, vp, C.c_char_p, C.POINTER(C.POINTER(u64)), C.POINTER(u64),
                                                   C.POINTER(f32p)]  # fmt: skip
-        for name in ("XGBoosterPredictFromDense", "XGBoosterPredictFromCudaArray"):
+        for name in ("XGDMatrixCreateFromDense", "XGDMatrixCreateFromCudaArrayInterface", "XGDMatrixCreateFromCudaColumnar"):
+            getattr(L, name).argtypes = [C.c_char_p, C.c_char_p, C.POINTER(vp)]
+        for name in ("XGBoosterPredictFromDense", "XGBoosterPredictFromCudaArray", "XGBoosterPredictFromCudaColumnar"):
             getattr(L, name).argtypes = [vp, C.c_char_p, C.c_char_p, vp, C.POINTER(C.POINTER(u64)), C.POINTER(u64), C.POINTER(f32p)]
         L.qcoh_booster_predict_contribs_device.argtypes = [vp, vp, C.c_int, C.c_uint, vp]
         L.qcoh_booster_predict_interactions_device.argtypes = [vp, vp, C.c_int, C.c_uint, vp]
@@ -266,6 +269,44 @@ class DeviceArray:
             pass
 
 
+def _array_interface(data, shape=None, strides=None, offset=0):
+    """(interface dict, on device) of a numpy array, a DeviceArray (explicit `shape`, `strides` in bytes or None for
+    C-contiguous, `offset` in floats) or anything with __cuda_array_interface__ (e.g. a torch CUDA tensor or view)."""
+    if isinstance(data, np.ndarray):
+        if data.dtype != np.float32:
+            raise TypeError("float32 arrays only")
+        iface, cuda = dict(data.__array_interface__), False
+    elif isinstance(data, DeviceArray):
+        iface = {"data": [data.ptr.value + 4 * offset if data.ptr.value else 0, False], "shape": list(shape),
+                 "strides": None if strides is None else list(strides), "typestr": "<f4", "version": 3}  # fmt: skip
+        cuda = True
+    else:
+        iface, cuda = dict(data.__cuda_array_interface__), True
+    iface["data"] = list(iface["data"])
+    iface["shape"] = list(iface["shape"])
+    if iface.get("strides") is not None:
+        iface["strides"] = list(iface["strides"])
+    return iface, cuda
+
+
+def _columns_interface(cols, stream=None):
+    """JSON list of the 1-D interfaces of `cols`: objects with __cuda_array_interface__ (e.g. torch CUDA tensors or views)
+    or (DeviceArray, nrow, stride in bytes or None, offset in floats) tuples."""
+    import json
+
+    out = []
+    for c in cols:
+        if isinstance(c, tuple):
+            dev, n, st, off = (tuple(c) + (None, 0))[:4]
+            iface, _ = _array_interface(dev, shape=(n,), strides=None if st is None else (st,), offset=off)
+        else:
+            iface, _ = _array_interface(c)
+        if stream is not None:
+            iface["stream"] = stream
+        out.append(iface)
+    return json.dumps(out)
+
+
 class DMatrix:
     def __init__(self, data: np.ndarray | None = None, missing=-999.0, *, handle=None):
         self.handle = vp()
@@ -281,6 +322,33 @@ class DMatrix:
     def device(cls, nrow, ncol, missing=-999.0):
         h = vp()
         check(lib().qcoh_dmatrix_create_device(nrow, ncol, missing, C.byref(h)))
+        return cls(handle=h)
+
+    @classmethod
+    def from_array(cls, data, missing=float("nan"), *, shape=None, strides=None, offset=0, stream=None):
+        """xgboost's DMatrix(array): a numpy float32 array through XGDMatrixCreateFromDense, a DeviceArray (explicit
+        `shape`, `strides` in bytes, `offset` in floats) or anything with __cuda_array_interface__ (e.g. a torch CUDA
+        tensor or a transposed view of one) through XGDMatrixCreateFromCudaArrayInterface, read in place with its
+        strides.  `stream` adds a "stream" entry to a device array's interface."""
+        import json
+
+        iface, cuda = _array_interface(data, shape, strides, offset)
+        if stream is not None:
+            iface["stream"] = stream
+        fn = lib().XGDMatrixCreateFromCudaArrayInterface if cuda else lib().XGDMatrixCreateFromDense
+        h = vp()
+        check(fn(json.dumps(iface).encode(), json.dumps({"missing": float(missing), "nthread": 0}).encode(), C.byref(h)))
+        return cls(handle=h)
+
+    @classmethod
+    def from_columns(cls, cols, missing=float("nan"), *, stream=None):
+        """xgboost's DMatrix(cuDF): one device column per feature (torch CUDA tensors or views, or (DeviceArray, nrow,
+        stride in bytes, offset in floats) tuples) through XGDMatrixCreateFromCudaColumnar, each read in place."""
+        import json
+
+        h = vp()
+        cfg = json.dumps({"missing": float(missing), "nthread": 0}).encode()
+        check(lib().XGDMatrixCreateFromCudaColumnar(_columns_interface(cols, stream).encode(), cfg, C.byref(h)))
         return cls(handle=h)
 
     @classmethod
@@ -455,21 +523,9 @@ class Booster:
         without copying; `stream` adds a "stream" entry to the interface of a device array."""
         import json
 
-        if isinstance(data, np.ndarray):
-            if data.dtype != np.float32:
-                raise TypeError("inplace_predict takes float32 arrays")
-            iface, cuda = dict(data.__array_interface__), False
-        elif isinstance(data, DeviceArray):
-            nrow, ncol = shape
-            iface = {"data": [data.ptr.value + 4 * offset if data.ptr.value else 0, False], "shape": [nrow, ncol],
-                     "strides": None if strides is None else list(strides), "typestr": "<f4", "version": 3}  # fmt: skip
-            cuda = True
-        else:
-            iface, cuda = dict(data.__cuda_array_interface__), True
-        iface["data"] = list(iface["data"])
-        iface["shape"] = list(iface["shape"])
-        if iface.get("strides") is not None:
-            iface["strides"] = list(iface["strides"])
+        if isinstance(data, np.ndarray) and data.dtype != np.float32:
+            raise TypeError("inplace_predict takes float32 arrays")
+        iface, cuda = _array_interface(data, shape, strides, offset)
         if stream is not None:
             iface["stream"] = stream
         cfg = {"type": int(type), "training": False, "missing": float(missing), "iteration_begin": 0,
@@ -478,6 +534,25 @@ class Booster:
         fn = lib().XGBoosterPredictFromCudaArray if cuda else lib().XGBoosterPredictFromDense
         check(fn(self.handle, json.dumps(iface).encode(), json.dumps(cfg).encode(), None, C.byref(shp), C.byref(dim), C.byref(p)))
         return tuple(int(shp[i]) for i in range(dim.value)), p, cuda
+
+    def inplace_predict_columns(self, cols, missing=-999.0, type=0, iteration_end=0, strict_shape=False, *,
+                                stream=None) -> np.ndarray:  # fmt: skip
+        """xgboost's Booster.inplace_predict(cuDF): value (type 0) or margin (1) straight from one device column per
+        feature (as DMatrix.from_columns takes them) through XGBoosterPredictFromCudaColumnar.  Returns a copy of the
+        margins, shaped as the library says."""
+        import json
+
+        cfg = {"type": int(type), "training": False, "missing": float(missing), "iteration_begin": 0,
+               "iteration_end": int(iteration_end), "strict_shape": bool(strict_shape)}  # fmt: skip
+        shp, dim, p = C.POINTER(u64)(), u64(), f32p()
+        check(lib().XGBoosterPredictFromCudaColumnar(self.handle, _columns_interface(cols, stream).encode(), json.dumps(cfg).encode(),
+                                                     None, C.byref(shp), C.byref(dim), C.byref(p)))  # fmt: skip
+        shape_ = tuple(int(shp[i]) for i in range(dim.value))
+        n = int(np.prod(shape_))
+        out = np.empty(n, np.float32)
+        if n:
+            check(lib().qcoh_memcpy_d2h(_ptr(out), C.cast(p, vp), out.nbytes))
+        return out.reshape(shape_)
 
     def predict_contribs(self, dmat: DMatrix, approximate=False, ntree_limit=0) -> np.ndarray:
         """[nrow, num_feature + 1] per-feature contributions, last column the bias: exact TreeSHAP, or Saabas when

@@ -547,18 +547,58 @@ static void create_pipelined(DMatrix *d, const float *data, Booster *b) {
 
 static thread_local cudaEvent_t g_input_ready = nullptr;
 
-// XGBoosterPredictFromDense / XGBoosterPredictFromCudaArray (libxgboost 1.6.0 Learner::InplacePredict, value and
-// margin): predict_dense_kernel builds the key tiles from the caller's array in shared memory.  A device array is read
-// where it is, with its strides; a host array is copied chunk by chunk (copy_chunks) and each chunk predicted as it
-// lands.  Returns the float32 margins, in the booster's device buffer (on_device) or its pinned host buffer; both stay
-// valid until the next predict or free on that booster.  Every refusal comes before any device work.
-static const float *predict_inplace(const char *caller, bool cuda_array, BoosterHandle handle, const char *values,
+// The work queued on the caller's streams before this call has written the input (CUDA Array Interface "stream": 1 the
+// legacy default stream, 2 the per-thread default stream, else a cudaStream_t): the library stream waits for each.
+static void wait_for_streams(const std::vector<uint64_t> &streams) {
+  for (const uint64_t v : streams) {
+    const cudaStream_t cs = v == 1 ? cudaStreamLegacy : v == 2 ? cudaStreamPerThread : (cudaStream_t)(uintptr_t)v;
+    if (!g_input_ready) CU(cudaEventCreateWithFlags(&g_input_ready, cudaEventDisableTiming));
+    CU(cudaEventRecord(g_input_ready, cs));
+    CU(cudaStreamWaitEvent(g.stream, g_input_ready, 0));
+  }
+}
+
+// Binds the CUDA runtime to this thread's device before a pointer query, when there is a device; with none visible every
+// address is host memory.
+static void bind_for_pointer_query() {
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) == cudaSuccess && ndev > 0) ensure_device();
+  else (void)cudaGetLastError();
+}
+
+// The column table of a columnar interface whose columns are all in device memory: col[c] and stride[c] in floats.
+static void device_columns(const std::string &pre, const ColumnarInterface &ci, std::vector<const float *> &col, std::vector<int64_t> &stride) {
+  bind_for_pointer_query();
+  col.clear(), stride.clear();
+  for (size_t c = 0; c < ci.addr.size(); ++c) {
+    const float *p = reinterpret_cast<const float *>((uintptr_t)ci.addr[c]);
+    if (ci.nrow && !is_device_ptr(p)) throw Error(pre + "column " + std::to_string(c) + " is in host memory (the Cuda calls take device columns)");
+    col.push_back(p), stride.push_back(ci.stride_bytes[c] / 4);
+  }
+}
+
+// XGBoosterPredictFromDense / XGBoosterPredictFromCudaArray / XGBoosterPredictFromCudaColumnar (libxgboost 1.6.0
+// Learner::InplacePredict, value and margin): predict_dense_kernel (predict_columns_kernel for a list of columns) builds
+// the key tiles from the caller's array in shared memory.  A device array is read where it is, with its strides; a host
+// array is copied chunk by chunk (copy_chunks) and each chunk predicted as it lands.  Returns the float32 margins, in
+// the booster's device buffer (on_device) or its pinned host buffer; both stay valid until the next predict or free on
+// that booster.  Every refusal comes before any device work.
+enum class Inplace { kDense, kCudaArray, kCudaColumnar };
+static const float *predict_inplace(const char *caller, Inplace kind, BoosterHandle handle, const char *values,
                                     const char *config, DMatrixHandle m, const bst_ulong **out_shape, bst_ulong *out_dim) {
   const std::string pre = std::string(caller) + ": ";
+  const bool cuda_array = kind != Inplace::kDense, columnar = kind == Inplace::kCudaColumnar;
   Booster *b = B(handle);
   if (!out_shape || !out_dim) throw Error(pre + "NULL output argument");
   if (!b->loaded) throw Error("Booster has no model: call XGBoosterLoadModel first");
-  const ArrayInterface ai = parse_array_interface(values, caller);
+  ArrayInterface ai;
+  ColumnarInterface cl;
+  if (columnar) {
+    cl = parse_columnar_interface(values, caller);
+    ai.nrow = cl.nrow, ai.ncol = cl.addr.size();
+  } else {
+    ai = parse_array_interface(values, caller);
+  }
   const PredictConfig c = parse_predict_config(config, caller, true);
   if (m) throw Error(pre + "the proxy DMatrix must be NULL (inplace prediction takes no base margin)");
   if (c.type != 0 && c.type != 1)
@@ -572,16 +612,21 @@ static const float *predict_inplace(const char *caller, bool cuda_array, Booster
     throw Error(pre + std::to_string(ai.ncol) + " columns; libqcoh's tile form holds at most " + std::to_string(kMaxMatrixCols));
   const uint64_t nrow = ai.nrow, ncol = ai.ncol;
   const bool empty = nrow * ncol == 0;
-  // the pointer query binds the CUDA runtime to this thread's device first; with no device visible every address is host memory
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) == cudaSuccess && ndev > 0) ensure_device();
-  else (void)cudaGetLastError();
+  std::vector<const float *> cols;
+  std::vector<int64_t> strides;
+  bool on_device = false;
   const float *data = reinterpret_cast<const float *>((uintptr_t)ai.addr);
-  const bool on_device = !empty && is_device_ptr(data);
-  if (cuda_array && !empty && !on_device) throw Error(pre + "the array is in host memory (XGBoosterPredictFromDense takes host arrays)");
-  if (!empty && !on_device && (ai.col_bytes != 4 || ai.row_bytes != (int64_t)(4 * ncol)))
-    throw Error(pre + "a host array must be C-contiguous: strides [" + std::to_string(4 * ncol) + ", 4] or null, got [" +
-                std::to_string(ai.row_bytes) + ", " + std::to_string(ai.col_bytes) + "]");
+  if (columnar) {
+    device_columns(pre, cl, cols, strides);
+    on_device = true;
+  } else {
+    bind_for_pointer_query();
+    on_device = !empty && is_device_ptr(data);
+    if (cuda_array && !empty && !on_device) throw Error(pre + "the array is in host memory (XGBoosterPredictFromDense takes host arrays)");
+    if (!empty && !on_device && (ai.col_bytes != 4 || ai.row_bytes != (int64_t)(4 * ncol)))
+      throw Error(pre + "a host array must be C-contiguous: strides [" + std::to_string(4 * ncol) + ", 4] or null, got [" +
+                  std::to_string(ai.row_bytes) + ", " + std::to_string(ai.col_bytes) + "]");
+  }
   ensure_device();
   upload(b);
   const unsigned limit = (unsigned)std::min<int64_t>(c.iteration_end, (int64_t)UINT32_MAX);
@@ -598,13 +643,13 @@ static const float *predict_inplace(const char *caller, bool cuda_array, Booster
   auto predict = [&](const PredictArgs &pa, const DenseArgs &d) {
     predict_ranges(b, pa, g.stream, [&](const ConstWindow &w, const PredictArgs &r) { return launch_predict_dense(b->dev, w, r, d, g.stream); });
   };
-  if (on_device || empty) {
-    if (ai.has_stream) {  // the work queued on the caller's stream before this call has written the array
-      const cudaStream_t cs = ai.stream == 1 ? cudaStreamLegacy : ai.stream == 2 ? cudaStreamPerThread : (cudaStream_t)(uintptr_t)ai.stream;
-      if (!g_input_ready) CU(cudaEventCreateWithFlags(&g_input_ready, cudaEventDisableTiming));
-      CU(cudaEventRecord(g_input_ready, cs));
-      CU(cudaStreamWaitEvent(g.stream, g_input_ready, 0));
-    }
+  if (columnar) {
+    wait_for_streams(cl.streams);
+    predict_ranges(b, a, g.stream, [&](const ConstWindow &w, const PredictArgs &r) {
+      return launch_predict_columns(b->dev, w, r, cols.data(), strides.data(), c.missing, fl, g.stream);
+    });
+  } else if (on_device || empty) {
+    if (ai.has_stream) wait_for_streams({ai.stream});
     da.X = data, da.row_stride = ai.row_bytes / 4, da.col_stride = ai.col_bytes / 4;
     predict(a, da);
   } else {
@@ -638,6 +683,97 @@ static const float *predict_inplace(const char *caller, bool cuda_array, Booster
   *out_shape = b->h_shape.data();
   *out_dim = (bst_ulong)b->h_shape.size();
   return out;
+}
+
+// XGDMatrixFree's pooling: the matrix's buffers become the spares of the next create when they are larger
+static void pool_buffers(DMatrix *d) {
+  if (d->X.cap > g_spare_X.cap) d->X.swap(g_spare_X);
+  if (d->Xt.cap > g_spare_Xt.cap) d->Xt.swap(g_spare_Xt);
+  if (d->spec_host.cap > g_spare_pin.cap) d->spec_host.swap(g_spare_pin);
+  if (d->spec_dev.cap > g_spare_spec.cap) d->spec_dev.swap(g_spare_spec);
+}
+
+// Where the values of a new DMatrix are: C-contiguous host rows, or a column table in device memory, element (r, c) at
+// col[c][r * stride[c]] (strides in floats).  `row_major`: the table is one C-contiguous [nrow][ncol] device array at
+// col[0].
+struct MatrixSource {
+  uint64_t nrow = 0, ncol = 0;
+  const float *host = nullptr;
+  std::vector<const float *> col;
+  std::vector<int64_t> stride;
+  bool row_major = false;
+  std::vector<uint64_t> streams;  // CUDA Array Interface streams the device input was written on
+};
+
+// The DMatrix of XGDMatrixCreateFromDense / FromCudaArrayInterface / FromCudaColumnar, sealed when this returns (the
+// caller may then free or overwrite its arrays).  It is the DMatrix XGDMatrixCreateFromMat makes from the same values in
+// row-major order, bit for bit: host rows take create_pipelined, as there (with the `speculate` setting); a C-contiguous
+// device array is copied and sealed by seal_tiles, as there; any other layout is sealed by seal_columns, which also
+// writes the row-major X.  On failure no handle is created and the buffers go back to the pools.
+static void create_from_columns(const MatrixSource &src, float missing, DMatrixHandle *out) {
+  ensure_device();
+  std::unique_ptr<DMatrix> d(new DMatrix());
+  d->nrow = src.nrow, d->ncol = src.ncol, d->missing = missing;
+  const size_t n = (size_t)src.nrow * src.ncol;
+  if (g_spare_X.cap >= n && g_spare_X.p) d->X.swap(g_spare_X);
+  try {
+    d->X.need(n);
+    if (n && src.host) {
+      Booster *b = g.speculate ? g_last_booster : nullptr;
+      if (b && !(b->loaded && src.ncol <= b->host.num_feature)) b = nullptr;
+      create_pipelined(d.get(), src.host, b);
+    } else if (n == 0 || src.row_major) {
+      if (n) {
+        wait_for_streams(src.streams);
+        CU(cudaMemcpyAsync(d->X.p, src.col[0], n * sizeof(float), cudaMemcpyDeviceToDevice, g.stream));
+        CU(cudaStreamSynchronize(g.stream));
+      }
+      seal(d.get());
+    } else {
+      wait_for_streams(src.streams);
+      if (g_spare_Xt.cap >= tile_words(d->nrow, d->ncol) && g_spare_Xt.p) d->Xt.swap(g_spare_Xt);
+      int *fl = d->flags.need(1);
+      CU(cudaMemsetAsync(fl, 0, sizeof(int), g.stream));
+      CU(launch_seal_columns(src.col.data(), src.stride.data(), d->nrow, (int)d->ncol, missing, d->X.p,
+                             d->Xt.need(tile_words(d->nrow, d->ncol)), fl, g.stream));
+      CU(cudaMemcpyAsync(&d->hflags, fl, sizeof(int), cudaMemcpyDeviceToHost, g.stream));
+      CU(cudaStreamSynchronize(g.stream));
+      d->sealed = true;
+      // xgboost src/data/data.cc SparsePage::Push: a finite `missing` with inf data is an error
+      if (d->hflags & 2) throw Error("Check failed: valid: Input data contains `inf` or `nan`");
+    }
+  } catch (...) {
+    drain();
+    pool_buffers(d.get());
+    throw;
+  }
+  g_live_handles.insert(d.get());
+  *out = d.release();
+}
+
+// The source of XGDMatrixCreateFromDense (cuda = false) / FromCudaArrayInterface (cuda = true): a 2-D array interface,
+// column c at base + c * col_stride with the row stride.  Refusals come before any device work.
+static MatrixSource array_source(const std::string &pre, const ArrayInterface &ai, bool cuda) {
+  if (ai.ncol > kMaxMatrixCols)
+    throw Error(pre + std::to_string(ai.ncol) + " columns; libqcoh's tile form holds at most " + std::to_string(kMaxMatrixCols));
+  MatrixSource src;
+  src.nrow = ai.nrow, src.ncol = ai.ncol;
+  const bool empty = ai.nrow * ai.ncol == 0;
+  const float *data = reinterpret_cast<const float *>((uintptr_t)ai.addr);
+  bind_for_pointer_query();
+  const bool on_device = !empty && is_device_ptr(data);
+  if (cuda && !empty && !on_device) throw Error(pre + "the array is in host memory (XGDMatrixCreateFromDense takes host arrays)");
+  if (!empty && !on_device && (ai.col_bytes != 4 || ai.row_bytes != (int64_t)(4 * ai.ncol)))
+    throw Error(pre + "a host array must be C-contiguous: strides [" + std::to_string(4 * ai.ncol) + ", 4] or null, got [" +
+                std::to_string(ai.row_bytes) + ", " + std::to_string(ai.col_bytes) + "]");
+  if (!empty && !on_device) {
+    src.host = data;
+    return src;
+  }
+  src.row_major = ai.col_bytes == 4 && ai.row_bytes == (int64_t)(4 * ai.ncol);
+  for (uint64_t c = 0; c < ai.ncol; ++c) src.col.push_back(data + c * (uint64_t)(ai.col_bytes / 4)), src.stride.push_back(ai.row_bytes / 4);
+  if (ai.has_stream) src.streams.push_back(ai.stream);
+  return src;
 }
 
 }  // namespace qcoh
@@ -745,10 +881,7 @@ int XGDMatrixFree(DMatrixHandle handle) {
   // them — neither the pipelined create nor an asynchronous qcoh_booster_predict_device on the compute stream.
   if (g.ready) drain();
   d->magic = 0;
-  if (d->X.cap > g_spare_X.cap) d->X.swap(g_spare_X);
-  if (d->Xt.cap > g_spare_Xt.cap) d->Xt.swap(g_spare_Xt);
-  if (d->spec_host.cap > g_spare_pin.cap) d->spec_host.swap(g_spare_pin);
-  if (d->spec_dev.cap > g_spare_spec.cap) d->spec_dev.swap(g_spare_spec);
+  pool_buffers(d);
   g_live_handles.erase(d);
   delete d;
   API_END
@@ -857,7 +990,7 @@ int XGBoosterPredictFromDense(BoosterHandle handle, const char *values, const ch
                               const bst_ulong **out_shape, bst_ulong *out_dim, const float **out_result) {
   API_BEGIN
   if (!out_result) throw Error("XGBoosterPredictFromDense: NULL output argument");
-  *out_result = predict_inplace("XGBoosterPredictFromDense", false, handle, values, config, m, out_shape, out_dim);
+  *out_result = predict_inplace("XGBoosterPredictFromDense", Inplace::kDense, handle, values, config, m, out_shape, out_dim);
   API_END
 }
 
@@ -865,7 +998,51 @@ int XGBoosterPredictFromCudaArray(BoosterHandle handle, const char *values, cons
                                   const bst_ulong **out_shape, bst_ulong *out_dim, const float **out_result) {
   API_BEGIN
   if (!out_result) throw Error("XGBoosterPredictFromCudaArray: NULL output argument");
-  *out_result = predict_inplace("XGBoosterPredictFromCudaArray", true, handle, values, config, m, out_shape, out_dim);
+  *out_result = predict_inplace("XGBoosterPredictFromCudaArray", Inplace::kCudaArray, handle, values, config, m, out_shape, out_dim);
+  API_END
+}
+
+int XGBoosterPredictFromCudaColumnar(BoosterHandle handle, const char *values, const char *config, DMatrixHandle m,
+                                     const bst_ulong **out_shape, bst_ulong *out_dim, const float **out_result) {
+  API_BEGIN
+  if (!out_result) throw Error("XGBoosterPredictFromCudaColumnar: NULL output argument");
+  *out_result = predict_inplace("XGBoosterPredictFromCudaColumnar", Inplace::kCudaColumnar, handle, values, config, m, out_shape, out_dim);
+  API_END
+}
+
+// libxgboost 1.6.0's array-interface DMatrix constructors (src/c_api/c_api.cc), what xgboost's Python DMatrix(cupy /
+// torch / cuDF) calls: `config` is {"missing": number, "nthread": int}.  The result is an ordinary DMatrix
+// (create_from_columns).
+int XGDMatrixCreateFromDense(const char *data, const char *config, DMatrixHandle *out) {
+  API_BEGIN
+  const char *caller = "XGDMatrixCreateFromDense";
+  if (!out) throw Error(std::string(caller) + ": out is NULL");
+  const ArrayInterface ai = parse_array_interface(data, caller);
+  const float missing = parse_dmatrix_config(config, caller);
+  create_from_columns(array_source(std::string(caller) + ": ", ai, false), missing, out);
+  API_END
+}
+
+int XGDMatrixCreateFromCudaArrayInterface(const char *data, const char *config, DMatrixHandle *out) {
+  API_BEGIN
+  const char *caller = "XGDMatrixCreateFromCudaArrayInterface";
+  if (!out) throw Error(std::string(caller) + ": out is NULL");
+  const ArrayInterface ai = parse_array_interface(data, caller);
+  const float missing = parse_dmatrix_config(config, caller);
+  create_from_columns(array_source(std::string(caller) + ": ", ai, true), missing, out);
+  API_END
+}
+
+int XGDMatrixCreateFromCudaColumnar(const char *data, const char *config, DMatrixHandle *out) {
+  API_BEGIN
+  const char *caller = "XGDMatrixCreateFromCudaColumnar";
+  if (!out) throw Error(std::string(caller) + ": out is NULL");
+  const ColumnarInterface ci = parse_columnar_interface(data, caller);
+  const float missing = parse_dmatrix_config(config, caller);
+  MatrixSource src;
+  src.nrow = ci.nrow, src.ncol = ci.addr.size(), src.streams = ci.streams;
+  device_columns(std::string(caller) + ": ", ci, src.col, src.stride);
+  create_from_columns(src, missing, out);
   API_END
 }
 

@@ -7,6 +7,7 @@
 //                  strings / vectors are dmlc-serializer uint64-length-prefixed
 //   JSON / UBJSON: doc/model.schema; UBJSON is draft-12, big-endian, typed arrays
 #include "forest.hpp"
+#include "kernels.hpp"
 
 #include <algorithm>
 #include <cmath>
@@ -1028,6 +1029,16 @@ JV parse_json_object(const char *json, const std::string &what) {
   if (root.kind != JV::Obj) fail(what + " must be a JSON object");
   return root;
 }
+JV parse_json_value(const char *json, const std::string &what) {
+  if (!json) fail(what + " is NULL");
+  try {
+    JsonReader r{json, json + strlen(json)};
+    return r.value();
+  } catch (const std::exception &e) {
+    fail(what + " is not valid JSON (" + e.what() + ")");
+  }
+  return JV();
+}
 }  // namespace
 
 PredictConfig parse_predict_config(const char *json, const char *caller, bool inplace) {
@@ -1092,6 +1103,68 @@ ArrayInterface parse_array_interface(const char *json, const char *caller) {
     a.has_stream = true;
   }
   return a;
+}
+
+float parse_dmatrix_config(const char *json, const char *caller) {
+  const std::string pre = std::string(caller) + ": ";
+  const JV root = parse_json_object(json, pre + "config");
+  const JV *m = root.find("missing");
+  if (!m) fail(pre + "config is missing the key 'missing'");
+  if (m->kind != JV::Num) fail(pre + "config: 'missing' must be a number (NaN is written NaN)");
+  return m->f32;
+}
+
+ColumnarInterface parse_columnar_interface(const char *json, const char *caller) {
+  const std::string pre = std::string(caller) + ": ";
+  const JV root = parse_json_value(json, pre + "columnar interface");
+  if (root.kind != JV::Arr) fail(pre + "the columnar interface must be a JSON list of 1-D array interfaces, one per column");
+  if (root.arr.empty()) fail(pre + "the list of columns is empty");
+  if (root.arr.size() > kMaxMatrixCols)
+    fail(pre + std::to_string(root.arr.size()) + " columns; libqcoh's tile form holds at most " + std::to_string(kMaxMatrixCols));
+  ColumnarInterface ci;
+  for (size_t c = 0; c < root.arr.size(); ++c) {
+    const JV &col = root.arr[c];
+    const std::string at = pre + "column " + std::to_string(c) + ": ";
+    if (col.kind != JV::Obj) fail(at + "must be an array interface (a JSON object)");
+    auto need = [&](const char *key) -> const JV & {
+      const JV *v = col.find(key);
+      if (!v) fail(at + "array interface is missing the key '" + key + "'");
+      return *v;
+    };
+    const JV &ty = need("typestr");
+    if (ty.kind != JV::Str || ty.str != "<f4")
+      fail(at + "typestr '" + (ty.kind == JV::Str ? ty.str : std::string("?")) + "': only little-endian float32 ('<f4') is accepted");
+    if (col.find("mask")) fail(at + "masked arrays are not supported (the array interface has a 'mask' entry)");
+    const JV &shape = need("shape");
+    if (shape.kind != JV::Arr || shape.arr.size() != 1)
+      fail(at + "a column must be 1-D [nrow]; its shape has " + std::to_string(shape.kind == JV::Arr ? shape.arr.size() : 0) + " dimensions");
+    const int64_t nr = shape.arr[0].as_int();
+    if (nr < 0) fail(at + "negative shape [" + std::to_string(nr) + "]");
+    if (c == 0) ci.nrow = (uint64_t)nr;
+    else if ((uint64_t)nr != ci.nrow)
+      fail(at + "the columns differ in length: column " + std::to_string(c) + " has " + std::to_string(nr) + " rows, column 0 has " +
+           std::to_string(ci.nrow));
+    int64_t sb = 4;
+    const JV *st = col.find("strides");
+    if (st && st->kind != JV::Null) {
+      if (st->kind != JV::Arr || st->arr.size() != 1) fail(at + "strides must be null or [bytes]");
+      sb = st->arr[0].as_int();
+      if (sb <= 0 || sb % 4) fail(at + "strides [" + std::to_string(sb) + "]: the stride must be a positive multiple of 4 bytes");
+    }
+    const JV &data = need("data");
+    if (data.kind != JV::Arr || data.arr.empty()) fail(at + "'data' must be [address, readonly]");
+    const uint64_t addr = (uint64_t)data.arr[0].as_int();
+    if (addr == 0 && nr > 0) fail(at + "the data address is NULL for a column of " + std::to_string(nr) + " rows");
+    const JV *s = col.find("stream");
+    if (s && s->kind != JV::Null) {
+      const uint64_t v = (uint64_t)s->as_int();
+      if (v == 0) fail(at + "stream 0 is not valid in the CUDA Array Interface (1: legacy default stream, 2: per-thread default stream)");
+      if (std::find(ci.streams.begin(), ci.streams.end(), v) == ci.streams.end()) ci.streams.push_back(v);
+    }
+    ci.addr.push_back(addr);
+    ci.stride_bytes.push_back(sb);
+  }
+  return ci;
 }
 
 }  // namespace qcoh

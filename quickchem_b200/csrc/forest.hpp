@@ -149,6 +149,22 @@ struct ArrayInterface {
 };
 ArrayInterface parse_array_interface(const char *json, const char *caller);
 
+// A JSON list of 1-D float32 array interfaces, one per column (the columnar DMatrix and inplace predict): each
+// {"data": [address, readonly], "shape": [nrow], "strides": null | [bytes], "typestr": "<f4"[, "stream": s]}.  Throws,
+// prefixed with `caller` and naming the column index, on a value that is not a list, an empty list, more than
+// kMaxMatrixCols (kernels.hpp) columns, another type, a mask, a column that is not 1-D, columns of different lengths, a stride that is
+// not a positive multiple of 4, a NULL address for a non-empty column and stream 0.
+struct ColumnarInterface {
+  uint64_t nrow = 0;
+  std::vector<uint64_t> addr;          // per column
+  std::vector<int64_t> stride_bytes;   // per column; 4 when "strides" is null
+  std::vector<uint64_t> streams;       // the distinct "stream" values of the columns
+};
+ColumnarInterface parse_columnar_interface(const char *json, const char *caller);
+// The config of the array-interface DMatrix constructors: {"missing": number, "nthread": int}; `missing` is required
+// (NaN is written NaN), every other key is ignored.  Returns `missing`.
+float parse_dmatrix_config(const char *json, const char *caller);
+
 // Throws std::runtime_error with libxgboost-style messages on malformed / unsupported input.
 HostForest load_model_file(const std::string &path);
 HostForest load_model_buffer(const unsigned char *buf, size_t len);

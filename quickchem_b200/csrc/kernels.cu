@@ -3,6 +3,8 @@
 //   K3  seal_tiles_kernel     the missing / inf scan of XGDMatrixCreateFromMat (OH_GridCompMod.F90:347) fused with
 //                             the conversion of the row-major float matrix into the DMatrix's device form:
 //                             feature-major tiles of order-preserving integer keys
+//       seal_columns_kernel   the same seal from a column table (a strided 2-D array or a list of device columns), which
+//                             also writes the row-major matrix the DMatrix keeps
 //   K2  predict_tiles_kernel  tree-ensemble traversal, replaces libxgboost's CPUPredictor behind XGBoosterPredict
 //                             (reference call site :356) with the export transform 10**x * OHscale (:369,:1569) fused
 //                             as epilogue; sums / leaf indices, clean matrices / missing entries; tiles arrive by TMA.
@@ -12,6 +14,7 @@
 //       predict_soa_kernel    K2 with the tile assembled straight from the Run1 SoA fields (run1_feature, which
 //                             oh_pack reads the features with too)
 //       predict_dense_kernel  K2 with the tile assembled from a caller's strided float array (inplace prediction)
+//       predict_columns_kernel  the same from a column table (columnar inplace prediction)
 //   K6  shap_paths / shap_reduce / shap_approx   per-feature contributions (exact TreeSHAP, approximate Saabas)
 //       shap_inter / shap_inter_reduce / shap_inter_expand   SHAP interaction values (conditioned TreeSHAP)
 //   K1  oh_state / oh_sums / oh_pack    Run1 feature assembly (:1240-1257, :1441-1488, :303-345)
@@ -42,12 +45,13 @@ uint64_t launch_count() { return g_launches; }
 namespace {
 enum Family {
   kDuo, kNodes8 = kDuo + 4, kSoaDuo = kNodes8 + 4, kSoaNodes8, kSealTiles, kShap, kShapReduce, kShapApprox, kDenseDuo, kDenseNodes8,
-  kShapInter, kShapInterReduce, kShapInterExpand, kFamilies
+  kShapInter, kShapInterReduce, kShapInterExpand, kSealColumns, kColumnsDuo, kColumnsNodes8, kFamilies
 };
 const char *const kFamilyName[kFamilies] = {"duo", "duo_missing", "duo_leaf", "duo_missing_leaf", "nodes8", "nodes8_missing",
                                             "nodes8_leaf", "nodes8_missing_leaf", "soa_duo", "soa_nodes8", "seal_tiles",
                                             "shap", "shap_reduce", "shap_approx", "dense_duo", "dense_nodes8",
-                                            "shap_inter", "shap_inter_reduce", "shap_inter_expand"};
+                                            "shap_inter", "shap_inter_reduce", "shap_inter_expand", "seal_columns",
+                                            "columns_duo", "columns_nodes8"};
 thread_local uint64_t g_family[kFamilies];
 thread_local const char *g_last_predict = "";
 void count_family(int f) { ++g_family[f]; }
@@ -231,29 +235,22 @@ struct TilePipe {
 // =====================================================================================
 // K3 — seal: row-major float matrix -> key tiles, with the missing / inf scan
 // =====================================================================================
-__global__ void __launch_bounds__(kTileRows) seal_tiles_kernel(const float *__restrict__ X, uint64_t nrow, int ncol, float missing,
-                                                               int check_inf, uint32_t *__restrict__ Xt, int *flags) {
-  extern __shared__ __align__(16) float srows[];  // [256][ld] row-major, ld odd: the per-thread row reads are conflict-free
+// The seal of one 256-row tile, shared by seal_tiles_kernel and seal_columns_kernel: load(srows, ld, tid, r0, nr) stages
+// the tile's nr rows from row r0 on in shared memory ([nr][ld] row-major, ld = ncol | 1 odd: the per-thread row reads
+// are conflict-free), then come the missing / inf scan, the stable clean-first row order, the row-order word and the keys.
+// The kernel passes threadIdx.x as `tid` and its own dynamic shared memory as `srows`. Only inside the kernel does the
+// compiler know that tid is below the launch bound, and the module's dynamic shared-memory symbols are placed in the
+// order they first appear; both keep seal_tiles_kernel's code what it was before the seal was shared.
+template <class Load>
+__device__ __forceinline__ void seal_tile(float *srows, int tid, uint64_t nrow, int ncol, float missing, int check_inf,
+                                          uint32_t *__restrict__ Xt, int *flags, Load &&load) {
   __shared__ int warp_clean[kTileRows / 32];
-  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+  const int lane = tid & 31, wid = tid >> 5;
   const int ld = ncol | 1;
   const uint64_t r0 = (uint64_t)blockIdx.x * kTileRows;
   const uint64_t left = nrow - r0;
   const int nr = left < (uint64_t)kTileRows ? (int)left : kTileRows;
-  const float *__restrict__ src = X + r0 * (uint64_t)ncol;
-  const int n = nr * ncol;
-  if (ld == ncol) {  // the tile's rows are one contiguous run of X: flat, coalesced copy
-    if ((((uintptr_t)src) & 15u) == 0u) {
-      const float4 *s4 = reinterpret_cast<const float4 *>(src);
-      float4 *d4 = reinterpret_cast<float4 *>(srows);
-      for (int i = tid; i < (n >> 2); i += kTileRows) d4[i] = __ldg(s4 + i);
-      for (int i = (n & ~3) + tid; i < n; i += kTileRows) srows[i] = __ldg(src + i);
-    } else {
-      for (int i = tid; i < n; i += kTileRows) srows[i] = __ldg(src + i);
-    }
-  } else {
-    for (int i = tid; i < n; i += kTileRows) srows[(i / ncol) * ld + (i % ncol)] = __ldg(src + i);
-  }
+  load(srows, ld, tid, r0, nr);
   __syncthreads();
   // pass 1: does my row hold a missing entry?  (rows past the end of the matrix count as clean; never stored)
   int fl = 0;
@@ -293,6 +290,35 @@ __global__ void __launch_bounds__(kTileRows) seal_tiles_kernel(const float *__re
   if (lane == 0 && fl) atomicOr(flags, fl);
 }
 
+// The loaders of seal_tile are functors with a forced-inline call: a lambda would be inlined only after the seal had been
+// optimised around the call, and seal_tiles_kernel's code would change.
+struct RowMajorLoad {  // rows of a C-contiguous row-major matrix
+  const float *__restrict__ X;
+  int ncol;
+  __device__ __forceinline__ void operator()(float *srows, int ld, int tid, uint64_t r0, int nr) const {
+    const float *__restrict__ src = X + r0 * (uint64_t)ncol;
+    const int n = nr * ncol;
+    if (ld == ncol) {  // the tile's rows are one contiguous run of X: flat, coalesced copy
+      if ((((uintptr_t)src) & 15u) == 0u) {
+        const float4 *s4 = reinterpret_cast<const float4 *>(src);
+        float4 *d4 = reinterpret_cast<float4 *>(srows);
+        for (int i = tid; i < (n >> 2); i += kTileRows) d4[i] = __ldg(s4 + i);
+        for (int i = (n & ~3) + tid; i < n; i += kTileRows) srows[i] = __ldg(src + i);
+      } else {
+        for (int i = tid; i < n; i += kTileRows) srows[i] = __ldg(src + i);
+      }
+    } else {
+      for (int i = tid; i < n; i += kTileRows) srows[(i / ncol) * ld + (i % ncol)] = __ldg(src + i);
+    }
+  }
+};
+
+__global__ void __launch_bounds__(kTileRows) seal_tiles_kernel(const float *__restrict__ X, uint64_t nrow, int ncol, float missing,
+                                                               int check_inf, uint32_t *__restrict__ Xt, int *flags) {
+  extern __shared__ __align__(16) float srows[];  // [256][ld] row-major, ld odd: the per-thread row reads are conflict-free
+  seal_tile(srows, threadIdx.x, nrow, ncol, missing, check_inf, Xt, flags, RowMajorLoad{X, ncol});
+}
+
 cudaError_t launch_seal_tiles(const float *X, uint64_t nrow, int ncol, float missing, uint32_t *Xt, int *flags, cudaStream_t s) {
   if (nrow == 0) return cudaSuccess;
   const uint64_t ntile = tile_count(nrow);
@@ -303,6 +329,63 @@ cudaError_t launch_seal_tiles(const float *X, uint64_t nrow, int ncol, float mis
   // xgboost src/data/data.cc: `!std::isinf(missing) && std::isinf(value)` invalidates the input
   seal_tiles_kernel<<<(unsigned)ntile, kTileRows, smem, s>>>(X, nrow, ncol, missing, std::isinf(missing) ? 0 : 1, Xt, flags);
   count_family(kSealTiles);
+  return QC_LAUNCHED();
+}
+
+// ---- seal from a column table (XGDMatrixCreateFromCudaColumnar / FromCudaArrayInterface with any layout) -----------
+// Element (r, c) is col[c][r * stride[c]].  The table travels in the kernel parameters (kMaxMatrixCols x 16 B).
+template <int N>
+struct ColumnParams {
+  const float *col[N];
+  int64_t stride[N];  // in floats
+};
+
+struct ColumnLoad {  // rows of a column table, column by column: 256 consecutive rows of a unit-stride column are coalesced
+  const ColumnParams<kMaxMatrixCols> &t;
+  int ncol;
+  __device__ __forceinline__ void operator()(float *srows, int ld, int tid, uint64_t r0, int nr) const {
+    if (tid >= nr) return;
+    const int64_t r = (int64_t)(r0 + (uint64_t)tid);
+#pragma unroll 8
+    for (int c = 0; c < ncol; ++c) srows[tid * ld + c] = __ldg(t.col[c] + r * t.stride[c]);
+  }
+};
+
+// seal_tiles_kernel's seal with the column-table loader, plus the row-major X the DMatrix keeps: the staged rows are
+// written flat and coalesced to X, so the result is the matrix XGDMatrixCreateFromMat would have copied.
+__global__ void __launch_bounds__(kTileRows) seal_columns_kernel(const __grid_constant__ ColumnParams<kMaxMatrixCols> t, uint64_t nrow,
+                                                                 int ncol, float missing, int check_inf, float *__restrict__ X,
+                                                                 uint32_t *__restrict__ Xt, int *flags) {
+  extern __shared__ __align__(16) float scols[];  // [256][ld] row-major, ld odd
+  const int tid = threadIdx.x;
+  seal_tile(scols, tid, nrow, ncol, missing, check_inf, Xt, flags, [&](float *srows, int ld, int tid_, uint64_t r0, int nr) {
+    ColumnLoad{t, ncol}(srows, ld, tid_, r0, nr);
+    __syncthreads();
+    // X rows [r0, r0 + nr): element i of the run is row i / ncol, column i % ncol (a multiply-high by 2^32 / ncol
+    // rounded up is exact for i < 2^32 / ncol, far above 256 x 192)
+    float *__restrict__ dst = X + r0 * (uint64_t)ncol;
+    const uint32_t n = (uint32_t)(nr * ncol), mul = (uint32_t)(0xFFFFFFFFu / (uint32_t)ncol) + 1u;
+    for (uint32_t i = (uint32_t)tid_; i < n; i += kTileRows) {
+      const uint32_t row = __umulhi(i, mul);
+      dst[i] = srows[row * (uint32_t)ld + (i - row * (uint32_t)ncol)];
+    }
+  });
+}
+
+cudaError_t launch_seal_columns(const float *const *col, const int64_t *stride, uint64_t nrow, int ncol, float missing, float *X,
+                                uint32_t *Xt, int *flags, cudaStream_t s) {
+  if (nrow == 0) return cudaSuccess;
+  if (ncol <= 0 || ncol > (int)kMaxMatrixCols) return cudaErrorInvalidValue;
+  const uint64_t ntile = tile_count(nrow);
+  if (ntile > 0x7fffffffull) return cudaErrorInvalidConfiguration;
+  ColumnParams<kMaxMatrixCols> t;
+  memset(&t, 0, sizeof t);
+  for (int c = 0; c < ncol; ++c) t.col[c] = col[c], t.stride[c] = stride[c];
+  const size_t smem = (size_t)kTileRows * (size_t)(ncol | 1) * sizeof(float);
+  cudaError_t e = cudaFuncSetAttribute(seal_columns_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  seal_columns_kernel<<<(unsigned)ntile, kTileRows, smem, s>>>(t, nrow, ncol, missing, std::isinf(missing) ? 0 : 1, X, Xt, flags);
+  count_family(kSealColumns);
   return QC_LAUNCHED();
 }
 
@@ -726,6 +809,43 @@ __global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_soa_kernel(D
 // one of its 32 rows holds a missing entry, and MissingWalk serves it when Walk cannot walk missing entries.  Ranges
 // of trees are separate launches (the partial sum travels through `out` as in predict_tiles_kernel); each one
 // reassembles the tile.
+// The key of one entry of an inplace tile: NaN and == missing are missing (flags |= 1), +-inf with a finite `missing`
+// sets flags |= 2
+__device__ __forceinline__ uint32_t inplace_key(float x, float missing, bool chk_inf, int &flags) {
+  if (chk_inf && isinf(x)) flags |= 2;
+  if (x != x || x == missing) {
+    flags |= 1;
+    return kKeyMissing;
+  }
+  return float_key(x);
+}
+
+// The rest of an inplace launch once the loader has put a tile's keys in slots 0..ncol-1, shared by predict_dense_kernel
+// and predict_columns_kernel: absent columns are missing, the key-0 slot goes last, the inf flag is voted, and each live
+// thread walks its row (the default-direction walk when one of the warp's rows holds a missing entry).
+template <class Walk, class MissingWalk>
+__device__ __forceinline__ void walk_inplace_tile(const DeviceForest &f, const PredictArgs &a, uint32_t *skey, int tid, uint64_t r0,
+                                                  bool live, int flags, int *flag_out) {
+  const int ncol = a.ncol;
+  for (int c = ncol; c < f.nfeat; ++c) skey[c * kStride + tid] = kKeyMissing;
+  skey[f.nfeat * kStride + tid] = 0u;
+  // __syncthreads_or returns a truth value, not the bitwise OR: one vote for the inf flag
+  if (__syncthreads_or(flags & 2) != 0) {
+    if (tid == 0) atomicOr(flag_out, 2);
+  }
+  const bool hm = __any_sync(0xffffffffu, flags & 1) || ncol < f.nfeat;
+  if (!live) return;
+  const uint32_t my = (uint32_t)__cvta_generic_to_shared(skey + tid);
+  row_result<false>(f, a, r0 + (uint64_t)tid, true, [&](auto &&emit) {
+    if (!hm)
+      Walk::template run<false, false>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
+    else if (Walk::walks_missing(f))
+      Walk::template run<true, false>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
+    else
+      MissingWalk::template run<true, false>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
+  });
+}
+
 template <class Walk, class MissingWalk>
 __global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_dense_kernel(DeviceForest f, PredictArgs a, DenseArgs d) {
   extern __shared__ __align__(128) uint32_t skey[];
@@ -736,14 +856,7 @@ __global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_dense_kernel
   const bool live = tid < nr;
   const bool chk_inf = !isinf(d.missing);
   int flags = 0;
-  auto key = [&](float x) {
-    if (chk_inf && isinf(x)) flags |= 2;
-    if (x != x || x == d.missing) {
-      flags |= 1;
-      return kKeyMissing;
-    }
-    return float_key(x);
-  };
+  auto key = [&](float x) { return inplace_key(x, d.missing, chk_inf, flags); };
   if (d.col_stride == 1 && d.row_stride == ncol) {
     // contiguous rows: one flat coalesced copy into a row-major staging area of odd stride (conflict-free per-thread
     // row reads, as in seal_tiles_kernel) that aliases the key slots; each thread lifts its row through registers
@@ -774,23 +887,33 @@ __global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_dense_kernel
     const float *__restrict__ src = d.X + (r0 + (uint64_t)tid) * d.row_stride;
     for (int c = 0; c < ncol; ++c) skey[c * kStride + tid] = live ? key(__ldg(src + (int64_t)c * d.col_stride)) : 0u;
   }
-  for (int c = ncol; c < f.nfeat; ++c) skey[c * kStride + tid] = kKeyMissing;
-  skey[f.nfeat * kStride + tid] = 0u;
-  // __syncthreads_or returns a truth value, not the bitwise OR: one vote for the inf flag
-  if (__syncthreads_or(flags & 2) != 0) {
-    if (tid == 0) atomicOr(d.flags, 2);
-  }
-  const bool hm = __any_sync(0xffffffffu, flags & 1) || ncol < f.nfeat;
-  if (!live) return;
-  const uint32_t my = (uint32_t)__cvta_generic_to_shared(skey + tid);
-  row_result<false>(f, a, r0 + (uint64_t)tid, true, [&](auto &&emit) {
-    if (!hm)
-      Walk::template run<false, false>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
-    else if (Walk::walks_missing(f))
-      Walk::template run<true, false>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
-    else
-      MissingWalk::template run<true, false>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
-  });
+  walk_inplace_tile<Walk, MissingWalk>(f, a, skey, tid, r0, live, flags, d.flags);
+}
+
+// ---- columnar inplace variant (XGBoosterPredictFromCudaColumnar): predict_dense_kernel's element-wise loader fed from a
+// column table, element (r, c) at col[c][r * stride[c]]; a column of unit stride is coalesced.  The table (31 x 16 B)
+// travels in the kernel parameters.
+struct ColumnsArgs {
+  ColumnParams<kMaxFeatures> t;
+  float missing;
+  int *flags;  // |= 2 on +-inf input when `missing` is finite
+};
+
+template <class Walk, class MissingWalk>
+__global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_columns_kernel(DeviceForest f, PredictArgs a,
+                                                                                    const __grid_constant__ ColumnsArgs d) {
+  extern __shared__ __align__(128) uint32_t skey[];
+  const int tid = threadIdx.x, ncol = a.ncol;
+  const uint64_t r0 = (uint64_t)blockIdx.x * kBlock;
+  const uint64_t left = a.nrow - r0;
+  const int nr = left < (uint64_t)kBlock ? (int)left : kBlock;
+  const bool live = tid < nr;
+  const bool chk_inf = !isinf(d.missing);
+  int flags = 0;
+  const int64_t r = (int64_t)(r0 + (uint64_t)tid);
+  for (int c = 0; c < ncol; ++c)
+    skey[c * kStride + tid] = live ? inplace_key(__ldg(d.t.col[c] + r * d.t.stride[c]), d.missing, chk_inf, flags) : 0u;
+  walk_inplace_tile<Walk, MissingWalk>(f, a, skey, tid, r0, live, flags, d.flags);
 }
 
 // The layout rule of the predict launches: the two-level records when the window holds the record tops of trees
@@ -846,6 +969,33 @@ cudaError_t launch_predict_dense(const DeviceForest &f, const ConstWindow &w, co
   if (e != cudaSuccess) return e;
   k<<<dim3((unsigned)grid), kBlock, smem, s>>>(f, a, d);
   count_predict(l == Layout::kRecords ? kDenseDuo : kDenseNodes8);
+  return QC_LAUNCHED();
+}
+
+cudaError_t launch_predict_columns(const DeviceForest &f, const ConstWindow &w, const PredictArgs &args, const float *const *col,
+                                  const int64_t *stride, float missing, int *flags, cudaStream_t s) {
+  if (args.nrow == 0 || args.tree_end <= args.tree_begin) return cudaSuccess;
+  if (args.ncol > f.nfeat || f.nfeat > (int)kMaxFeatures || args.pred_leaf) return cudaErrorInvalidValue;
+  const size_t smem = (size_t)kStride * (size_t)(f.nfeat + 1) * sizeof(uint32_t);
+  const uint64_t grid = tile_count(args.nrow);
+  if (grid > 0x7fffffffull) return cudaErrorInvalidConfiguration;
+  PredictArgs a = args;
+  a.ctree0 = w.tree0;
+  ColumnsArgs d;
+  memset(&d, 0, sizeof d);
+  for (int c = 0; c < a.ncol; ++c) d.t.col[c] = col[c], d.t.stride[c] = stride[c];
+  d.missing = missing, d.flags = flags;
+  // the layout rule and the instantiations of launch_predict_dense
+  const Layout l = layout(f, w, a.tree_begin, a.tree_end, false);
+  auto k = predict_columns_kernel<RecordsWalk, NodesTexWalk>;
+  if (f.duo_shallow) k = predict_columns_kernel<RecordsShallowWalk, NodesTexWalk>;
+  if (l == Layout::kNodesTable) k = predict_columns_kernel<NodesTableWalk, NodesTableWalk>;
+  if (l == Layout::kNodesTex) k = predict_columns_kernel<NodesTexWalk, NodesTexWalk>;
+  if (l == Layout::kNodesLsu) k = predict_columns_kernel<NodesLsuWalk, NodesLsuWalk>;
+  cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  k<<<dim3((unsigned)grid), kBlock, smem, s>>>(f, a, d);
+  count_predict(l == Layout::kRecords ? kColumnsDuo : kColumnsNodes8);
   return QC_LAUNCHED();
 }
 

@@ -93,6 +93,10 @@ cudaError_t upload_const_duo(const uint32_t *top_xy, const uint32_t *tree_slot, 
 // entry is +-inf (and `missing` is finite) — what XGDMatrixCreateFromMat checks (xgboost src/data/data.cc).
 // X and Xt cover `nrow` rows starting at a tile boundary.
 cudaError_t launch_seal_tiles(const float *X, uint64_t nrow, int ncol, float missing, uint32_t *Xt, int *flags, cudaStream_t s);
+// The same seal from a column table: element (r, c) of the matrix is col[c][r * stride[c]] (device addresses, strides in
+// floats; host arrays of ncol entries, copied into the kernel parameters).  Also writes the row-major matrix to X.
+cudaError_t launch_seal_columns(const float *const *col, const int64_t *stride, uint64_t nrow, int ncol, float missing, float *X,
+                                uint32_t *Xt, int *flags, cudaStream_t s);
 
 cudaError_t launch_predict(const DeviceForest &f, const ConstWindow &w, const PredictArgs &a, cudaStream_t s);
 
@@ -107,6 +111,10 @@ struct DenseArgs {
   int *flags = nullptr;      // |= 2 on +-inf input when `missing` is finite
 };
 cudaError_t launch_predict_dense(const DeviceForest &f, const ConstWindow &w, const PredictArgs &a, const DenseArgs &d, cudaStream_t s);
+// The same from a column table (XGBoosterPredictFromCudaColumnar): element (r, c) is col[c][r * stride[c]], as for
+// launch_seal_columns; at most kMaxFeatures columns.
+cudaError_t launch_predict_columns(const DeviceForest &f, const ConstWindow &w, const PredictArgs &a, const float *const *col,
+                                   const int64_t *stride, float missing, int *flags, cudaStream_t s);
 
 // Per-feature contributions (forest.hpp ShapForest).  out: [nrow][nfeat + 1] floats, column nfeat = `bias`.
 //   exact (TreeSHAP on the path bins): launch_shap writes float64 partial sums of bin slice s to
