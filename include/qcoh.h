@@ -90,8 +90,8 @@ int XGBoosterPredictFromDMatrix(BoosterHandle handle, DMatrixHandle dmat, const 
  *   FromDense: HOST memory (pinned or pageable), C-contiguous; it is copied to HBM in chunks, each predicted as it lands,
  *   and read completely before the call returns.  A device address (detected) is read like FromCudaArray.  The
  *   result is a pinned host buffer.
- *   FromCudaArray: DEVICE memory, any strides (a feature-major [ncol][nrow] array is [4, 4 * nrow]).  An optional
- *   "stream" entry (CUDA Array Interface v3: 1 legacy default stream, 2 per-thread default stream, else a cudaStream_t;
+ *   FromCudaArray: DEVICE memory, any strides (a feature-major [ncol][nrow] array is [4, 4 * nrow]): a C-contiguous
+ *   array is read as rows, any other layout as the table of its columns.  An optional "stream" entry (CUDA Array Interface v3: 1 legacy default stream, 2 per-thread default stream, else a cudaStream_t;
  *   0 is invalid) is waited for before the array is read.  The result is a DEVICE buffer. */
 int XGBoosterPredictFromDense(BoosterHandle handle, const char *values, const char *config, DMatrixHandle m,
                               const bst_ulong **out_shape, bst_ulong *out_dim, const float **out_result);
@@ -261,7 +261,9 @@ int qcoh_set_param(const char *name, const char *value);
 uint64_t qcoh_launch_count(void);
 /* Which kernel family served a prediction — what the parity tests assert.  Families: "duo" (two-level records),
  * "nodes8" (8-byte depth-ordered nodes), each with the suffixes "_missing" (matrix with missing entries) and
- * "_leaf" (option_mask = 2), e.g. "duo_missing_leaf"; "soa_duo" / "soa_nodes8" (fused Run1); "seal_tiles";
+ * "_leaf" (option_mask = 2), e.g. "duo_missing_leaf"; "soa_duo" / "soa_nodes8" (fused Run1); "dense_duo" /
+ * "dense_nodes8" (inplace prediction from C-contiguous rows) and "columns_duo" / "columns_nodes8" (from a column table:
+ * FromCudaColumnar, or FromCudaArray with any other layout); "seal_tiles" and "seal_columns";
  * "shap" (exact contributions) with its slice reduction "shap_reduce", and "shap_approx" (approximate contributions);
  * "shap_inter" (exact interaction values, after a "shap" launch for the same rows) with "shap_inter_reduce", and
  * "shap_inter_expand" (approximate interaction values, after a "shap_approx" launch).

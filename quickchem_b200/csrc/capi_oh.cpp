@@ -340,7 +340,7 @@ int qcoh_oh_run1(qcoh_oh_handle h, const qcoh_run1_in *in, qcoh_run1_out *out) {
       int flags = 0;
       CU(cudaMemcpyAsync(&flags, r.ctl + 2, sizeof(int), cudaMemcpyDeviceToHost, g.stream));
       CU(cudaStreamSynchronize(g.stream));
-      if ((flags & 2) && !std::isinf(c.missing)) throw Error("Check failed: valid: Input data contains `inf` or `nan`");
+      if ((flags & 2) && !std::isinf(c.missing)) throw inf_error();
       PredictArgs a;
       a.Xt = Xt, a.nrow = npred, a.ncol = 27, a.has_missing = flags & 1, a.pred_leaf = 0;
       a.tree_begin = 0, a.tree_end = ntree, a.out_stride = a.tree_end;
@@ -372,7 +372,7 @@ int qcoh_oh_run1(qcoh_oh_handle h, const qcoh_run1_in *in, qcoh_run1_out *out) {
   CU(cudaStreamSynchronize(g.stream));
   if ((inf_flags & 2) && !std::isinf(c.missing)) {
     o->oh_ml_valid = false;
-    throw Error("Check failed: valid: Input data contains `inf` or `nan`");
+    throw inf_error();
   }
   API_END
 }

@@ -126,7 +126,7 @@ ConstWindow hold(Booster *b, int tree0, int ntree) {
 // One prediction = one launch per range of kRangeTrees trees (kernels.hpp; the tables hold kConstTreesMax and are
 // re-filled, stream-ordered, when a range leaves them) and the float32 partial sum travels through `out`, so the sum
 // order — tree 0, 1, 2, ... — and with it every bit of the result is the same as in a single launch.
-// launch(window, range args) launches one range: launch_predict on key tiles, launch_predict_dense on a dense array.
+// launch(window, range args) launches one range: launch_predict on key tiles, launch_predict_inplace on a caller's values.
 template <class Launch>
 static void predict_ranges(Booster *b, const PredictArgs &a, cudaStream_t s, Launch &&launch) {
   const int t_end = a.tree_end;
@@ -153,17 +153,39 @@ void launch_predict_chunked(Booster *b, PredictArgs a, cudaStream_t s) {
   predict_ranges(b, a, s, [&](const ConstWindow &w, const PredictArgs &c) { return launch_predict(b->dev, w, c, s); });
 }
 
-static void seal(DMatrix *d) {
+// buf.need(n), taking XGDMatrixFree's spare buffer first when buf has none and the spare is large enough
+template <class Buf>
+static auto need_pooled(Buf &buf, Buf &spare, size_t n) {
+  if (!buf.p && spare.p && spare.cap >= n) buf.swap(spare);
+  return buf.need(n);
+}
+
+// The key tiles of d from its X (seal_tiles) or, given a device column table (element (r, c) at col[c][r * stride[c]]),
+// from the table, which seal_columns also writes to X.
+static void seal(DMatrix *d, const float *const *col = nullptr, const int64_t *stride = nullptr) {
   ensure_device();
   int *fl = d->flags.need(1);
   CU(cudaMemsetAsync(fl, 0, sizeof(int), g.stream));
-  if (g_spare_Xt.cap >= tile_words(d->nrow, d->ncol) && g_spare_Xt.p && !d->Xt.p) d->Xt.swap(g_spare_Xt);
-  CU(launch_seal_tiles(d->X.p, d->nrow, (int)d->ncol, d->missing, d->Xt.need(tile_words(d->nrow, d->ncol)), fl, g.stream));
+  uint32_t *Xt = need_pooled(d->Xt, g_spare_Xt, tile_words(d->nrow, d->ncol));
+  if (col)
+    CU(launch_seal_columns(col, stride, d->nrow, (int)d->ncol, d->missing, d->X.p, Xt, fl, g.stream));
+  else
+    CU(launch_seal_tiles(d->X.p, d->nrow, (int)d->ncol, d->missing, Xt, fl, g.stream));
   CU(cudaMemcpyAsync(&d->hflags, fl, sizeof(int), cudaMemcpyDeviceToHost, g.stream));
   CU(cudaStreamSynchronize(g.stream));
   d->sealed = true;
-  // xgboost src/data/data.cc SparsePage::Push: a finite `missing` with inf data is an error
-  if (d->hflags & 2) throw Error("Check failed: valid: Input data contains `inf` or `nan`");
+  if (d->hflags & 2) throw inf_error();
+}
+
+static void check_columns(const Booster *b, uint64_t ncol) {
+  if (ncol > b->host.num_feature)
+    throw Error("Check failed: Number of columns does not match number of features in booster. Columns: " + std::to_string(ncol) +
+                " Features: " + std::to_string(b->host.num_feature));
+}
+
+static void check_tile_cap(const std::string &pre, uint64_t ncol) {
+  if (ncol > kMaxMatrixCols)
+    throw Error(pre + std::to_string(ncol) + " columns; libqcoh's tile form holds at most " + std::to_string(kMaxMatrixCols));
 }
 
 static unsigned trees_used(const Booster *b, unsigned ntree_limit) {
@@ -175,9 +197,7 @@ static void predict_into(Booster *b, DMatrix *d, int option_mask, unsigned ntree
   upload(b);
   if (!d->sealed) seal(d);
   if (option_mask & ~3) throw Error("option_mask " + std::to_string(option_mask) + ": only 0 (value), 1 (margin) and 2 (leaf index) are supported");
-  if (d->ncol > b->host.num_feature)
-    throw Error("Check failed: Number of columns does not match number of features in booster. Columns: " +
-                std::to_string(d->ncol) + " Features: " + std::to_string(b->host.num_feature));
+  check_columns(b, d->ncol);
   PredictArgs a;
   a.Xt = d->Xt.p, a.nrow = d->nrow, a.ncol = (int32_t)d->ncol;
   a.has_missing = ((d->hflags & 1) || d->ncol < b->host.num_feature) ? 1 : 0;
@@ -201,10 +221,7 @@ static const ShapForest &shap_on_device(Booster *b, DMatrix *d) {
   const ShapForest &s = shap_tables(b);
   upload(b);
   if (!d->sealed) seal(d);
-  const uint32_t nf = b->host.num_feature;
-  if (d->ncol > nf)
-    throw Error("Check failed: Number of columns does not match number of features in booster. Columns: " +
-                std::to_string(d->ncol) + " Features: " + std::to_string(nf));
+  check_columns(b, d->ncol);
   if (!b->shap_uploaded) {
     const size_t nb = (size_t)s.num_bins(), nn = s.mean.size();
     CU(cudaMemcpy(b->d_shap_bins.need(nb * 32), s.bins.data(), nb * 32 * sizeof(uint4), cudaMemcpyHostToDevice));
@@ -498,16 +515,13 @@ static void create_pipelined(DMatrix *d, const float *data, Booster *b) {
   const uint64_t cr = chunk_rows(pinned);
   const size_t nchunk = (size_t)((nrow + cr - 1) / cr);
   float *X = d->X.p;
-  if (g_spare_Xt.cap >= tile_words(nrow, ncol) && g_spare_Xt.p && !d->Xt.p) d->Xt.swap(g_spare_Xt);
-  uint32_t *Xt = d->Xt.need(tile_words(nrow, ncol));
+  uint32_t *Xt = need_pooled(d->Xt, g_spare_Xt, tile_words(nrow, ncol));
   const bool spec = b != nullptr;
   float *sdev = nullptr, *shost = nullptr;
   if (spec) {
     upload(b);
-    if (g_spare_spec.cap >= nrow && g_spare_spec.p) d->spec_dev.swap(g_spare_spec);
-    sdev = d->spec_dev.need(nrow);
-    if (g_spare_pin.cap >= nrow && g_spare_pin.p) d->spec_host.swap(g_spare_pin);
-    shost = d->spec_host.need(nrow);
+    sdev = need_pooled(d->spec_dev, g_spare_spec, nrow);
+    shost = need_pooled(d->spec_host, g_spare_pin, nrow);
   }
   int *fl = g_chunk_flags.need(nchunk);
   int *hfl = g_h_chunk_flags.need(nchunk);
@@ -526,7 +540,7 @@ static void create_pipelined(DMatrix *d, const float *data, Booster *b) {
     flags |= hfl[c];
     if (hfl[c] & 2) {
       drain();
-      throw Error("Check failed: valid: Input data contains `inf` or `nan`");
+      throw inf_error();
     }
     if (!spec) return;
     PredictArgs a;
@@ -566,67 +580,92 @@ static void bind_for_pointer_query() {
   else (void)cudaGetLastError();
 }
 
-// The column table of a columnar interface whose columns are all in device memory: col[c] and stride[c] in floats.
-static void device_columns(const std::string &pre, const ColumnarInterface &ci, std::vector<const float *> &col, std::vector<int64_t> &stride) {
+// A caller's values, described once for the inplace predicts and the DMatrix constructors: C-contiguous host rows at
+// `host`, or device memory, either one C-contiguous [nrow][ncol] array at col[0] (`rows`) or a column table, element
+// (r, c) at col[c][r * stride[c]] (strides in floats).
+struct MatrixSource {
+  uint64_t nrow = 0, ncol = 0;
+  const float *host = nullptr;
+  bool rows = false;
+  std::vector<const float *> col;
+  std::vector<int64_t> stride;
+  std::vector<uint64_t> streams;  // CUDA Array Interface streams the device input was written on
+};
+
+// The source of a 2-D array interface: host rows, device rows, or for any other device layout the column table, column
+// c at base + c * col_stride with the row stride.  host_call: NULL when host memory is taken, else the counterpart call
+// that takes it (named in the refusal).  Refusals come before any device work.
+static MatrixSource array_source(const char *caller, const ArrayInterface &ai, const char *host_call) {
+  const std::string pre = std::string(caller) + ": ";
+  check_tile_cap(pre, ai.ncol);
+  MatrixSource src;
+  src.nrow = ai.nrow, src.ncol = ai.ncol;
+  src.rows = ai.col_bytes == 4 && ai.row_bytes == (int64_t)(4 * ai.ncol);
+  const bool empty = ai.nrow * ai.ncol == 0;
+  const float *data = reinterpret_cast<const float *>((uintptr_t)ai.addr);
   bind_for_pointer_query();
-  col.clear(), stride.clear();
-  for (size_t c = 0; c < ci.addr.size(); ++c) {
-    const float *p = reinterpret_cast<const float *>((uintptr_t)ci.addr[c]);
-    if (ci.nrow && !is_device_ptr(p)) throw Error(pre + "column " + std::to_string(c) + " is in host memory (the Cuda calls take device columns)");
-    col.push_back(p), stride.push_back(ci.stride_bytes[c] / 4);
+  const bool on_device = !empty && is_device_ptr(data);
+  if (host_call && !empty && !on_device) throw Error(pre + "the array is in host memory (" + host_call + " takes host arrays)");
+  if (!empty && !on_device) {
+    if (!src.rows)
+      throw Error(pre + "a host array must be C-contiguous: strides [" + std::to_string(4 * ai.ncol) + ", 4] or null, got [" +
+                  std::to_string(ai.row_bytes) + ", " + std::to_string(ai.col_bytes) + "]");
+    src.host = data;
+    return src;
   }
+  if (src.rows) src.col.push_back(data);
+  else
+    for (uint64_t c = 0; c < ai.ncol; ++c) src.col.push_back(data + c * (uint64_t)(ai.col_bytes / 4)), src.stride.push_back(ai.row_bytes / 4);
+  if (ai.has_stream) src.streams.push_back(ai.stream);
+  return src;
 }
 
-// XGBoosterPredictFromDense / XGBoosterPredictFromCudaArray / XGBoosterPredictFromCudaColumnar (libxgboost 1.6.0
-// Learner::InplacePredict, value and margin): predict_dense_kernel (predict_columns_kernel for a list of columns) builds
-// the key tiles from the caller's array in shared memory.  A device array is read where it is, with its strides; a host
-// array is copied chunk by chunk (copy_chunks) and each chunk predicted as it lands.  Returns the float32 margins, in
-// the booster's device buffer (on_device) or its pinned host buffer; both stay valid until the next predict or free on
-// that booster.  Every refusal comes before any device work.
-enum class Inplace { kDense, kCudaArray, kCudaColumnar };
-static const float *predict_inplace(const char *caller, Inplace kind, BoosterHandle handle, const char *values,
-                                    const char *config, DMatrixHandle m, const bst_ulong **out_shape, bst_ulong *out_dim) {
+// The source of a columnar interface: its column table, every column in device memory.
+static MatrixSource columnar_source(const char *caller, const ColumnarInterface &ci) {
+  bind_for_pointer_query();
+  MatrixSource src;
+  src.nrow = ci.nrow, src.ncol = ci.addr.size(), src.streams = ci.streams;
+  for (size_t c = 0; c < ci.addr.size(); ++c) {
+    const float *p = reinterpret_cast<const float *>((uintptr_t)ci.addr[c]);
+    if (ci.nrow && !is_device_ptr(p))
+      throw Error(std::string(caller) + ": column " + std::to_string(c) + " is in host memory (the Cuda calls take device columns)");
+    src.col.push_back(p), src.stride.push_back(ci.stride_bytes[c] / 4);
+  }
+  return src;
+}
+
+// The checks of XGBoosterPredictFromDense / FromCudaArray / FromCudaColumnar (libxgboost 1.6.0 Learner::InplacePredict,
+// value and margin), in order: inplace_booster before the values are parsed, inplace_config after; the source builder
+// then checks where the values are.  Every refusal comes before any device work.
+static Booster *inplace_booster(const char *caller, BoosterHandle handle, const bst_ulong **out_shape, bst_ulong *out_dim,
+                                const float **out_result) {
   const std::string pre = std::string(caller) + ": ";
-  const bool cuda_array = kind != Inplace::kDense, columnar = kind == Inplace::kCudaColumnar;
+  if (!out_result) throw Error(pre + "NULL output argument");
   Booster *b = B(handle);
   if (!out_shape || !out_dim) throw Error(pre + "NULL output argument");
   if (!b->loaded) throw Error("Booster has no model: call XGBoosterLoadModel first");
-  ArrayInterface ai;
-  ColumnarInterface cl;
-  if (columnar) {
-    cl = parse_columnar_interface(values, caller);
-    ai.nrow = cl.nrow, ai.ncol = cl.addr.size();
-  } else {
-    ai = parse_array_interface(values, caller);
-  }
+  return b;
+}
+
+static PredictConfig inplace_config(const char *caller, const Booster *b, const char *config, DMatrixHandle m, uint64_t ncol) {
+  const std::string pre = std::string(caller) + ": ";
   const PredictConfig c = parse_predict_config(config, caller, true);
   if (m) throw Error(pre + "the proxy DMatrix must be NULL (inplace prediction takes no base margin)");
   if (c.type != 0 && c.type != 1)
     throw Error(pre + "prediction type " + std::to_string(c.type) + " is not supported inplace (0 value, 1 margin)");
   if (c.iteration_begin < 0 || c.iteration_end < 0) throw Error(pre + "negative iteration range");
   if (c.iteration_begin != 0) throw Error(pre + "iteration_begin = " + std::to_string(c.iteration_begin) + " is not supported (only 0)");
-  if (ai.ncol > b->host.num_feature)
-    throw Error("Check failed: Number of columns does not match number of features in booster. Columns: " +
-                std::to_string(ai.ncol) + " Features: " + std::to_string(b->host.num_feature));
-  if (ai.ncol > kMaxMatrixCols)
-    throw Error(pre + std::to_string(ai.ncol) + " columns; libqcoh's tile form holds at most " + std::to_string(kMaxMatrixCols));
-  const uint64_t nrow = ai.nrow, ncol = ai.ncol;
-  const bool empty = nrow * ncol == 0;
-  std::vector<const float *> cols;
-  std::vector<int64_t> strides;
-  bool on_device = false;
-  const float *data = reinterpret_cast<const float *>((uintptr_t)ai.addr);
-  if (columnar) {
-    device_columns(pre, cl, cols, strides);
-    on_device = true;
-  } else {
-    bind_for_pointer_query();
-    on_device = !empty && is_device_ptr(data);
-    if (cuda_array && !empty && !on_device) throw Error(pre + "the array is in host memory (XGBoosterPredictFromDense takes host arrays)");
-    if (!empty && !on_device && (ai.col_bytes != 4 || ai.row_bytes != (int64_t)(4 * ncol)))
-      throw Error(pre + "a host array must be C-contiguous: strides [" + std::to_string(4 * ncol) + ", 4] or null, got [" +
-                  std::to_string(ai.row_bytes) + ", " + std::to_string(ai.col_bytes) + "]");
-  }
+  check_columns(b, ncol);
+  return c;
+}
+
+// Inplace prediction of the values in src: predict_inplace_kernel builds the key tiles in shared memory, from rows (host
+// rows are copied chunk by chunk by copy_chunks and each chunk predicted as it lands) or from the column table.  Returns
+// the float32 margins, in the booster's device buffer (device_result) or its pinned host buffer; both stay valid until
+// the next predict or free on that booster.
+static const float *predict_inplace(Booster *b, const MatrixSource &src, const PredictConfig &c, bool device_result,
+                                    const bst_ulong **out_shape, bst_ulong *out_dim) {
+  const uint64_t nrow = src.nrow, ncol = src.ncol;
   ensure_device();
   upload(b);
   const unsigned limit = (unsigned)std::min<int64_t>(c.iteration_end, (int64_t)UINT32_MAX);
@@ -638,47 +677,38 @@ static const float *predict_inplace(const char *caller, Inplace kind, BoosterHan
   a.nrow = nrow, a.ncol = (int32_t)ncol;
   a.tree_begin = 0, a.tree_end = (int32_t)trees_used(b, limit);
   a.out = dv;
-  DenseArgs da;
-  da.missing = c.missing, da.flags = fl;
-  auto predict = [&](const PredictArgs &pa, const DenseArgs &d) {
-    predict_ranges(b, pa, g.stream, [&](const ConstWindow &w, const PredictArgs &r) { return launch_predict_dense(b->dev, w, r, d, g.stream); });
-  };
-  if (columnar) {
-    wait_for_streams(cl.streams);
-    predict_ranges(b, a, g.stream, [&](const ConstWindow &w, const PredictArgs &r) {
-      return launch_predict_columns(b->dev, w, r, cols.data(), strides.data(), c.missing, fl, g.stream);
+  auto predict = [&](const PredictArgs &pa, bool rows, const float *const *col, const int64_t *stride) {
+    predict_ranges(b, pa, g.stream, [&](const ConstWindow &w, const PredictArgs &r) {
+      return launch_predict_inplace(b->dev, w, r, rows, col, stride, c.missing, fl, g.stream);
     });
-  } else if (on_device || empty) {
-    if (ai.has_stream) wait_for_streams({ai.stream});
-    da.X = data, da.row_stride = ai.row_bytes / 4, da.col_stride = ai.col_bytes / 4;
-    predict(a, da);
-  } else {
+  };
+  if (src.host) {
     // the chunks land in the spare matrix buffer of XGDMatrixFree, which is given back afterwards
     DevBuf<float> X;
-    if (g_spare_X.cap >= nrow * ncol) X.swap(g_spare_X);
-    X.need(nrow * ncol);
-    const bool pinned = is_pinned_host(data);
-    copy_chunks(data, nrow, ncol, pinned, chunk_rows(pinned), X.p, [&](size_t ci, uint64_t r0, uint64_t nr) {
+    need_pooled(X, g_spare_X, nrow * ncol);
+    const bool pinned = is_pinned_host(src.host);
+    copy_chunks(src.host, nrow, ncol, pinned, chunk_rows(pinned), X.p, [&](size_t ci, uint64_t r0, uint64_t nr) {
       CU(cudaEventRecord(chunk_event(ci), g.copy_stream));
       CU(cudaStreamWaitEvent(g.stream, chunk_event(ci), 0));
       PredictArgs pa = a;
       pa.nrow = nr, pa.out = dv + r0;
-      DenseArgs d = da;
-      d.X = X.p + r0 * ncol, d.row_stride = (int64_t)ncol, d.col_stride = 1;
-      predict(pa, d);
+      const float *chunk = X.p + r0 * ncol;
+      predict(pa, true, &chunk, nullptr);
     }, [](size_t) {});
     CU(cudaStreamSynchronize(g.stream));  // the chunk buffer is read before it goes back to the pool
     if (X.cap > g_spare_X.cap) X.swap(g_spare_X);
+  } else {
+    wait_for_streams(src.streams);
+    predict(a, src.rows, src.col.data(), src.stride.data());
   }
   CU(cudaMemcpyAsync(hfl, fl, sizeof(int), cudaMemcpyDeviceToHost, g.stream));
   float *out = dv;
-  if (!cuda_array) {
+  if (!device_result) {
     out = b->h_result.need(nrow);
     CU(cudaMemcpyAsync(out, dv, nrow * sizeof(float), cudaMemcpyDeviceToHost, g.stream));
   }
   CU(cudaStreamSynchronize(g.stream));
-  // xgboost src/data/data.cc SparsePage::Push: a finite `missing` with inf data is an error (the kernel's flag)
-  if (*hfl & 2) throw Error("Check failed: valid: Input data contains `inf` or `nan`");
+  if (*hfl & 2) throw inf_error();
   b->h_shape = c.strict_shape ? std::vector<bst_ulong>{nrow, 1} : std::vector<bst_ulong>{nrow};
   *out_shape = b->h_shape.data();
   *out_dim = (bst_ulong)b->h_shape.size();
@@ -693,36 +723,23 @@ static void pool_buffers(DMatrix *d) {
   if (d->spec_dev.cap > g_spare_spec.cap) d->spec_dev.swap(g_spare_spec);
 }
 
-// Where the values of a new DMatrix are: C-contiguous host rows, or a column table in device memory, element (r, c) at
-// col[c][r * stride[c]] (strides in floats).  `row_major`: the table is one C-contiguous [nrow][ncol] device array at
-// col[0].
-struct MatrixSource {
-  uint64_t nrow = 0, ncol = 0;
-  const float *host = nullptr;
-  std::vector<const float *> col;
-  std::vector<int64_t> stride;
-  bool row_major = false;
-  std::vector<uint64_t> streams;  // CUDA Array Interface streams the device input was written on
-};
-
-// The DMatrix of XGDMatrixCreateFromDense / FromCudaArrayInterface / FromCudaColumnar, sealed when this returns (the
-// caller may then free or overwrite its arrays).  It is the DMatrix XGDMatrixCreateFromMat makes from the same values in
-// row-major order, bit for bit: host rows take create_pipelined, as there (with the `speculate` setting); a C-contiguous
-// device array is copied and sealed by seal_tiles, as there; any other layout is sealed by seal_columns, which also
-// writes the row-major X.  On failure no handle is created and the buffers go back to the pools.
-static void create_from_columns(const MatrixSource &src, float missing, DMatrixHandle *out) {
+// The DMatrix of the values in src, sealed when this returns (the caller may then free or overwrite its arrays): the
+// DMatrix XGDMatrixCreateFromMat makes from the same values in row-major order, bit for bit.  Host rows take
+// create_pipelined (with the `speculate` setting); device rows are copied and sealed by seal_tiles; a column table is
+// sealed by seal_columns, which also writes the row-major X.  On failure no handle is created and the buffers go back to
+// the pools.
+static void create_matrix(const MatrixSource &src, float missing, DMatrixHandle *out) {
   ensure_device();
   std::unique_ptr<DMatrix> d(new DMatrix());
   d->nrow = src.nrow, d->ncol = src.ncol, d->missing = missing;
   const size_t n = (size_t)src.nrow * src.ncol;
-  if (g_spare_X.cap >= n && g_spare_X.p) d->X.swap(g_spare_X);
   try {
-    d->X.need(n);
+    need_pooled(d->X, g_spare_X, n);
     if (n && src.host) {
       Booster *b = g.speculate ? g_last_booster : nullptr;
       if (b && !(b->loaded && src.ncol <= b->host.num_feature)) b = nullptr;
       create_pipelined(d.get(), src.host, b);
-    } else if (n == 0 || src.row_major) {
+    } else if (n == 0 || src.rows) {
       if (n) {
         wait_for_streams(src.streams);
         CU(cudaMemcpyAsync(d->X.p, src.col[0], n * sizeof(float), cudaMemcpyDeviceToDevice, g.stream));
@@ -731,16 +748,7 @@ static void create_from_columns(const MatrixSource &src, float missing, DMatrixH
       seal(d.get());
     } else {
       wait_for_streams(src.streams);
-      if (g_spare_Xt.cap >= tile_words(d->nrow, d->ncol) && g_spare_Xt.p) d->Xt.swap(g_spare_Xt);
-      int *fl = d->flags.need(1);
-      CU(cudaMemsetAsync(fl, 0, sizeof(int), g.stream));
-      CU(launch_seal_columns(src.col.data(), src.stride.data(), d->nrow, (int)d->ncol, missing, d->X.p,
-                             d->Xt.need(tile_words(d->nrow, d->ncol)), fl, g.stream));
-      CU(cudaMemcpyAsync(&d->hflags, fl, sizeof(int), cudaMemcpyDeviceToHost, g.stream));
-      CU(cudaStreamSynchronize(g.stream));
-      d->sealed = true;
-      // xgboost src/data/data.cc SparsePage::Push: a finite `missing` with inf data is an error
-      if (d->hflags & 2) throw Error("Check failed: valid: Input data contains `inf` or `nan`");
+      seal(d.get(), src.col.data(), src.stride.data());
     }
   } catch (...) {
     drain();
@@ -749,31 +757,6 @@ static void create_from_columns(const MatrixSource &src, float missing, DMatrixH
   }
   g_live_handles.insert(d.get());
   *out = d.release();
-}
-
-// The source of XGDMatrixCreateFromDense (cuda = false) / FromCudaArrayInterface (cuda = true): a 2-D array interface,
-// column c at base + c * col_stride with the row stride.  Refusals come before any device work.
-static MatrixSource array_source(const std::string &pre, const ArrayInterface &ai, bool cuda) {
-  if (ai.ncol > kMaxMatrixCols)
-    throw Error(pre + std::to_string(ai.ncol) + " columns; libqcoh's tile form holds at most " + std::to_string(kMaxMatrixCols));
-  MatrixSource src;
-  src.nrow = ai.nrow, src.ncol = ai.ncol;
-  const bool empty = ai.nrow * ai.ncol == 0;
-  const float *data = reinterpret_cast<const float *>((uintptr_t)ai.addr);
-  bind_for_pointer_query();
-  const bool on_device = !empty && is_device_ptr(data);
-  if (cuda && !empty && !on_device) throw Error(pre + "the array is in host memory (XGDMatrixCreateFromDense takes host arrays)");
-  if (!empty && !on_device && (ai.col_bytes != 4 || ai.row_bytes != (int64_t)(4 * ai.ncol)))
-    throw Error(pre + "a host array must be C-contiguous: strides [" + std::to_string(4 * ai.ncol) + ", 4] or null, got [" +
-                std::to_string(ai.row_bytes) + ", " + std::to_string(ai.col_bytes) + "]");
-  if (!empty && !on_device) {
-    src.host = data;
-    return src;
-  }
-  src.row_major = ai.col_bytes == 4 && ai.row_bytes == (int64_t)(4 * ai.ncol);
-  for (uint64_t c = 0; c < ai.ncol; ++c) src.col.push_back(data + c * (uint64_t)(ai.col_bytes / 4)), src.stride.push_back(ai.row_bytes / 4);
-  if (ai.has_stream) src.streams.push_back(ai.stream);
-  return src;
 }
 
 }  // namespace qcoh
@@ -849,28 +832,15 @@ int XGDMatrixCreateFromMat(const float *data, bst_ulong nrow, bst_ulong ncol, fl
   API_BEGIN
   if (!out) throw Error("XGDMatrixCreateFromMat: out is NULL");
   if (!data && nrow && ncol) throw Error("XGDMatrixCreateFromMat: data is NULL");
-  if (ncol > kMaxMatrixCols) throw Error("XGDMatrixCreateFromMat: " + std::to_string(ncol) + " columns; libqcoh's tile form holds at most " + std::to_string(kMaxMatrixCols));
+  check_tile_cap("XGDMatrixCreateFromMat: ", ncol);
   ensure_device();
-  std::unique_ptr<DMatrix> d(new DMatrix());
-  d->nrow = nrow, d->ncol = ncol, d->missing = missing;
-  const size_t n = (size_t)nrow * ncol;
-  if (g_spare_X.cap >= n && g_spare_X.p) d->X.swap(g_spare_X);
-  d->X.need(n);
   // borrowed for this call only (the reference deallocates xx_carr right after predict,
   // OH_GridCompMod.F90:383): the data is in HBM when this returns.
-  if (n && !is_device_ptr(data)) {
-    Booster *b = g.speculate ? g_last_booster : nullptr;
-    if (b && !(b->loaded && ncol <= b->host.num_feature)) b = nullptr;
-    create_pipelined(d.get(), data, b);
-  } else {
-    if (n) {
-      CU(cudaMemcpyAsync(d->X.p, data, n * sizeof(float), cudaMemcpyDeviceToDevice, g.stream));
-      CU(cudaStreamSynchronize(g.stream));
-    }
-    seal(d.get());
-  }
-  g_live_handles.insert(d.get());
-  *out = d.release();
+  MatrixSource src;
+  src.nrow = nrow, src.ncol = ncol, src.rows = true;
+  if (nrow && ncol && !is_device_ptr(data)) src.host = data;
+  else src.col.push_back(data);
+  create_matrix(src, missing, out);
   API_END
 }
 
@@ -989,37 +959,46 @@ int XGBoosterPredictFromDMatrix(BoosterHandle handle, DMatrixHandle dmat, const 
 int XGBoosterPredictFromDense(BoosterHandle handle, const char *values, const char *config, DMatrixHandle m,
                               const bst_ulong **out_shape, bst_ulong *out_dim, const float **out_result) {
   API_BEGIN
-  if (!out_result) throw Error("XGBoosterPredictFromDense: NULL output argument");
-  *out_result = predict_inplace("XGBoosterPredictFromDense", Inplace::kDense, handle, values, config, m, out_shape, out_dim);
+  const char *caller = "XGBoosterPredictFromDense";
+  Booster *b = inplace_booster(caller, handle, out_shape, out_dim, out_result);
+  const ArrayInterface ai = parse_array_interface(values, caller);
+  const PredictConfig c = inplace_config(caller, b, config, m, ai.ncol);
+  *out_result = predict_inplace(b, array_source(caller, ai, nullptr), c, false, out_shape, out_dim);
   API_END
 }
 
 int XGBoosterPredictFromCudaArray(BoosterHandle handle, const char *values, const char *config, DMatrixHandle m,
                                   const bst_ulong **out_shape, bst_ulong *out_dim, const float **out_result) {
   API_BEGIN
-  if (!out_result) throw Error("XGBoosterPredictFromCudaArray: NULL output argument");
-  *out_result = predict_inplace("XGBoosterPredictFromCudaArray", Inplace::kCudaArray, handle, values, config, m, out_shape, out_dim);
+  const char *caller = "XGBoosterPredictFromCudaArray";
+  Booster *b = inplace_booster(caller, handle, out_shape, out_dim, out_result);
+  const ArrayInterface ai = parse_array_interface(values, caller);
+  const PredictConfig c = inplace_config(caller, b, config, m, ai.ncol);
+  *out_result = predict_inplace(b, array_source(caller, ai, "XGBoosterPredictFromDense"), c, true, out_shape, out_dim);
   API_END
 }
 
 int XGBoosterPredictFromCudaColumnar(BoosterHandle handle, const char *values, const char *config, DMatrixHandle m,
                                      const bst_ulong **out_shape, bst_ulong *out_dim, const float **out_result) {
   API_BEGIN
-  if (!out_result) throw Error("XGBoosterPredictFromCudaColumnar: NULL output argument");
-  *out_result = predict_inplace("XGBoosterPredictFromCudaColumnar", Inplace::kCudaColumnar, handle, values, config, m, out_shape, out_dim);
+  const char *caller = "XGBoosterPredictFromCudaColumnar";
+  Booster *b = inplace_booster(caller, handle, out_shape, out_dim, out_result);
+  const ColumnarInterface ci = parse_columnar_interface(values, caller);
+  const PredictConfig c = inplace_config(caller, b, config, m, ci.addr.size());
+  *out_result = predict_inplace(b, columnar_source(caller, ci), c, true, out_shape, out_dim);
   API_END
 }
 
 // libxgboost 1.6.0's array-interface DMatrix constructors (src/c_api/c_api.cc), what xgboost's Python DMatrix(cupy /
 // torch / cuDF) calls: `config` is {"missing": number, "nthread": int}.  The result is an ordinary DMatrix
-// (create_from_columns).
+// (create_matrix).
 int XGDMatrixCreateFromDense(const char *data, const char *config, DMatrixHandle *out) {
   API_BEGIN
   const char *caller = "XGDMatrixCreateFromDense";
   if (!out) throw Error(std::string(caller) + ": out is NULL");
   const ArrayInterface ai = parse_array_interface(data, caller);
   const float missing = parse_dmatrix_config(config, caller);
-  create_from_columns(array_source(std::string(caller) + ": ", ai, false), missing, out);
+  create_matrix(array_source(caller, ai, nullptr), missing, out);
   API_END
 }
 
@@ -1029,7 +1008,7 @@ int XGDMatrixCreateFromCudaArrayInterface(const char *data, const char *config, 
   if (!out) throw Error(std::string(caller) + ": out is NULL");
   const ArrayInterface ai = parse_array_interface(data, caller);
   const float missing = parse_dmatrix_config(config, caller);
-  create_from_columns(array_source(std::string(caller) + ": ", ai, true), missing, out);
+  create_matrix(array_source(caller, ai, "XGDMatrixCreateFromDense"), missing, out);
   API_END
 }
 
@@ -1039,10 +1018,7 @@ int XGDMatrixCreateFromCudaColumnar(const char *data, const char *config, DMatri
   if (!out) throw Error(std::string(caller) + ": out is NULL");
   const ColumnarInterface ci = parse_columnar_interface(data, caller);
   const float missing = parse_dmatrix_config(config, caller);
-  MatrixSource src;
-  src.nrow = ci.nrow, src.ncol = ci.addr.size(), src.streams = ci.streams;
-  device_columns(std::string(caller) + ": ", ci, src.col, src.stride);
-  create_from_columns(src, missing, out);
+  create_matrix(columnar_source(caller, ci), missing, out);
   API_END
 }
 
@@ -1335,7 +1311,7 @@ int qcoh_booster_get_duo_info(BoosterHandle handle, int *blk_shift, int *has_def
 
 int qcoh_dmatrix_create_device(bst_ulong nrow, bst_ulong ncol, float missing, DMatrixHandle *out) {
   API_BEGIN
-  if (ncol > kMaxMatrixCols) throw Error("qcoh_dmatrix_create_device: " + std::to_string(ncol) + " columns; libqcoh's tile form holds at most " + std::to_string(kMaxMatrixCols));
+  check_tile_cap("qcoh_dmatrix_create_device: ", ncol);
   ensure_device();
   std::unique_ptr<DMatrix> d(new DMatrix());
   d->nrow = nrow, d->ncol = ncol, d->missing = missing;

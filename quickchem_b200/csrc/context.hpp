@@ -30,6 +30,10 @@ struct Error : std::runtime_error {
   using std::runtime_error::runtime_error;
 };
 
+// xgboost src/data/data.cc SparsePage::Push: a finite `missing` with inf data is an error (flag bit 2 of the seal and
+// of the predicts that read a caller's values)
+inline Error inf_error() { return Error("Check failed: valid: Input data contains `inf` or `nan`"); }
+
 #define CU(call)                                                                                      \
   do {                                                                                                \
     cudaError_t e__ = (call);                                                                         \

@@ -1039,6 +1039,40 @@ JV parse_json_value(const char *json, const std::string &what) {
   }
   return JV();
 }
+
+// The fields a 2-D array interface and a 1-D column share, read in the order of their refusals, each message starting
+// with `pre`: typestr and mask; then layout(need) reads the shape and strides (need(key) refuses a missing key) and
+// returns what a NULL data address is refused for, empty when the array has no elements; then the data and stream.
+struct InterfaceFields {
+  uint64_t addr = 0;
+  bool has_stream = false;
+  uint64_t stream = 0;
+};
+template <class Layout>
+InterfaceFields read_interface(const JV &obj, const std::string &pre, Layout &&layout) {
+  auto need = [&](const char *key) -> const JV & {
+    const JV *v = obj.find(key);
+    if (!v) fail(pre + "array interface is missing the key '" + key + "'");
+    return *v;
+  };
+  const JV &ty = need("typestr");
+  if (ty.kind != JV::Str || ty.str != "<f4")
+    fail(pre + "typestr '" + (ty.kind == JV::Str ? ty.str : std::string("?")) + "': only little-endian float32 ('<f4') is accepted");
+  if (obj.find("mask")) fail(pre + "masked arrays are not supported (the array interface has a 'mask' entry)");
+  const std::string null_for = layout(need);
+  const JV &data = need("data");
+  if (data.kind != JV::Arr || data.arr.empty()) fail(pre + "'data' must be [address, readonly]");
+  InterfaceFields f;
+  f.addr = (uint64_t)data.arr[0].as_int();
+  if (f.addr == 0 && !null_for.empty()) fail(pre + "the data address is NULL for " + null_for);
+  const JV *s = obj.find("stream");
+  if (s && s->kind != JV::Null) {
+    f.stream = (uint64_t)s->as_int();
+    if (f.stream == 0) fail(pre + "stream 0 is not valid in the CUDA Array Interface (1: legacy default stream, 2: per-thread default stream)");
+    f.has_stream = true;
+  }
+  return f;
+}
 }  // namespace
 
 PredictConfig parse_predict_config(const char *json, const char *caller, bool inplace) {
@@ -1067,41 +1101,26 @@ PredictConfig parse_predict_config(const char *json, const char *caller, bool in
 ArrayInterface parse_array_interface(const char *json, const char *caller) {
   const std::string pre = std::string(caller) + ": ";
   const JV root = parse_json_object(json, pre + "array interface");
-  auto need = [&](const char *key) -> const JV & {
-    const JV *v = root.find(key);
-    if (!v) fail(pre + "array interface is missing the key '" + key + "'");
-    return *v;
-  };
-  const JV &ty = need("typestr");
-  if (ty.kind != JV::Str || ty.str != "<f4")
-    fail(pre + "typestr '" + (ty.kind == JV::Str ? ty.str : std::string("?")) + "': only little-endian float32 ('<f4') is accepted");
-  if (root.find("mask")) fail(pre + "masked arrays are not supported (the array interface has a 'mask' entry)");
-  const JV &shape = need("shape");
-  if (shape.kind != JV::Arr || shape.arr.size() != 2)
-    fail(pre + "the array must be 2-D [nrow, ncol]; its shape has " + std::to_string(shape.kind == JV::Arr ? shape.arr.size() : 0) + " dimensions");
   ArrayInterface a;
-  const int64_t nr = shape.arr[0].as_int(), nc = shape.arr[1].as_int();
-  if (nr < 0 || nc < 0) fail(pre + "negative shape [" + std::to_string(nr) + ", " + std::to_string(nc) + "]");
-  a.nrow = (uint64_t)nr, a.ncol = (uint64_t)nc;
-  a.row_bytes = 4 * nc;
-  const JV *st = root.find("strides");
-  if (st && st->kind != JV::Null) {
-    if (st->kind != JV::Arr || st->arr.size() != 2) fail(pre + "strides must be null or [row_bytes, col_bytes]");
-    const int64_t rb = st->arr[0].as_int(), cb = st->arr[1].as_int();
-    if (rb < 0 || cb < 0 || rb % 4 || cb % 4)
-      fail(pre + "strides [" + std::to_string(rb) + ", " + std::to_string(cb) + "]: they must be non-negative multiples of 4 bytes");
-    a.row_bytes = rb, a.col_bytes = cb;
-  }
-  const JV &data = need("data");
-  if (data.kind != JV::Arr || data.arr.empty()) fail(pre + "'data' must be [address, readonly]");
-  a.addr = (uint64_t)data.arr[0].as_int();
-  if (a.addr == 0 && a.nrow * a.ncol > 0) fail(pre + "the data address is NULL for a " + std::to_string(nr) + " x " + std::to_string(nc) + " array");
-  const JV *s = root.find("stream");
-  if (s && s->kind != JV::Null) {
-    a.stream = (uint64_t)s->as_int();
-    if (a.stream == 0) fail(pre + "stream 0 is not valid in the CUDA Array Interface (1: legacy default stream, 2: per-thread default stream)");
-    a.has_stream = true;
-  }
+  const InterfaceFields f = read_interface(root, pre, [&](auto &&need) {
+    const JV &shape = need("shape");
+    if (shape.kind != JV::Arr || shape.arr.size() != 2)
+      fail(pre + "the array must be 2-D [nrow, ncol]; its shape has " + std::to_string(shape.kind == JV::Arr ? shape.arr.size() : 0) + " dimensions");
+    const int64_t nr = shape.arr[0].as_int(), nc = shape.arr[1].as_int();
+    if (nr < 0 || nc < 0) fail(pre + "negative shape [" + std::to_string(nr) + ", " + std::to_string(nc) + "]");
+    a.nrow = (uint64_t)nr, a.ncol = (uint64_t)nc;
+    a.row_bytes = 4 * nc;
+    const JV *st = root.find("strides");
+    if (st && st->kind != JV::Null) {
+      if (st->kind != JV::Arr || st->arr.size() != 2) fail(pre + "strides must be null or [row_bytes, col_bytes]");
+      const int64_t rb = st->arr[0].as_int(), cb = st->arr[1].as_int();
+      if (rb < 0 || cb < 0 || rb % 4 || cb % 4)
+        fail(pre + "strides [" + std::to_string(rb) + ", " + std::to_string(cb) + "]: they must be non-negative multiples of 4 bytes");
+      a.row_bytes = rb, a.col_bytes = cb;
+    }
+    return a.nrow * a.ncol > 0 ? "a " + std::to_string(nr) + " x " + std::to_string(nc) + " array" : std::string();
+  });
+  a.addr = f.addr, a.has_stream = f.has_stream, a.stream = f.stream;
   return a;
 }
 
@@ -1126,42 +1145,27 @@ ColumnarInterface parse_columnar_interface(const char *json, const char *caller)
     const JV &col = root.arr[c];
     const std::string at = pre + "column " + std::to_string(c) + ": ";
     if (col.kind != JV::Obj) fail(at + "must be an array interface (a JSON object)");
-    auto need = [&](const char *key) -> const JV & {
-      const JV *v = col.find(key);
-      if (!v) fail(at + "array interface is missing the key '" + key + "'");
-      return *v;
-    };
-    const JV &ty = need("typestr");
-    if (ty.kind != JV::Str || ty.str != "<f4")
-      fail(at + "typestr '" + (ty.kind == JV::Str ? ty.str : std::string("?")) + "': only little-endian float32 ('<f4') is accepted");
-    if (col.find("mask")) fail(at + "masked arrays are not supported (the array interface has a 'mask' entry)");
-    const JV &shape = need("shape");
-    if (shape.kind != JV::Arr || shape.arr.size() != 1)
-      fail(at + "a column must be 1-D [nrow]; its shape has " + std::to_string(shape.kind == JV::Arr ? shape.arr.size() : 0) + " dimensions");
-    const int64_t nr = shape.arr[0].as_int();
-    if (nr < 0) fail(at + "negative shape [" + std::to_string(nr) + "]");
-    if (c == 0) ci.nrow = (uint64_t)nr;
-    else if ((uint64_t)nr != ci.nrow)
-      fail(at + "the columns differ in length: column " + std::to_string(c) + " has " + std::to_string(nr) + " rows, column 0 has " +
-           std::to_string(ci.nrow));
     int64_t sb = 4;
-    const JV *st = col.find("strides");
-    if (st && st->kind != JV::Null) {
-      if (st->kind != JV::Arr || st->arr.size() != 1) fail(at + "strides must be null or [bytes]");
-      sb = st->arr[0].as_int();
-      if (sb <= 0 || sb % 4) fail(at + "strides [" + std::to_string(sb) + "]: the stride must be a positive multiple of 4 bytes");
-    }
-    const JV &data = need("data");
-    if (data.kind != JV::Arr || data.arr.empty()) fail(at + "'data' must be [address, readonly]");
-    const uint64_t addr = (uint64_t)data.arr[0].as_int();
-    if (addr == 0 && nr > 0) fail(at + "the data address is NULL for a column of " + std::to_string(nr) + " rows");
-    const JV *s = col.find("stream");
-    if (s && s->kind != JV::Null) {
-      const uint64_t v = (uint64_t)s->as_int();
-      if (v == 0) fail(at + "stream 0 is not valid in the CUDA Array Interface (1: legacy default stream, 2: per-thread default stream)");
-      if (std::find(ci.streams.begin(), ci.streams.end(), v) == ci.streams.end()) ci.streams.push_back(v);
-    }
-    ci.addr.push_back(addr);
+    const InterfaceFields f = read_interface(col, at, [&](auto &&need) {
+      const JV &shape = need("shape");
+      if (shape.kind != JV::Arr || shape.arr.size() != 1)
+        fail(at + "a column must be 1-D [nrow]; its shape has " + std::to_string(shape.kind == JV::Arr ? shape.arr.size() : 0) + " dimensions");
+      const int64_t nr = shape.arr[0].as_int();
+      if (nr < 0) fail(at + "negative shape [" + std::to_string(nr) + "]");
+      if (c == 0) ci.nrow = (uint64_t)nr;
+      else if ((uint64_t)nr != ci.nrow)
+        fail(at + "the columns differ in length: column " + std::to_string(c) + " has " + std::to_string(nr) + " rows, column 0 has " +
+             std::to_string(ci.nrow));
+      const JV *st = col.find("strides");
+      if (st && st->kind != JV::Null) {
+        if (st->kind != JV::Arr || st->arr.size() != 1) fail(at + "strides must be null or [bytes]");
+        sb = st->arr[0].as_int();
+        if (sb <= 0 || sb % 4) fail(at + "strides [" + std::to_string(sb) + "]: the stride must be a positive multiple of 4 bytes");
+      }
+      return nr > 0 ? "a column of " + std::to_string(nr) + " rows" : std::string();
+    });
+    if (f.has_stream && std::find(ci.streams.begin(), ci.streams.end(), f.stream) == ci.streams.end()) ci.streams.push_back(f.stream);
+    ci.addr.push_back(f.addr);
     ci.stride_bytes.push_back(sb);
   }
   return ci;

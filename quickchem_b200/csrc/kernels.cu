@@ -13,8 +13,7 @@
 //                             nodes (boosters the records do not hold)
 //       predict_soa_kernel    K2 with the tile assembled straight from the Run1 SoA fields (run1_feature, which
 //                             oh_pack reads the features with too)
-//       predict_dense_kernel  K2 with the tile assembled from a caller's strided float array (inplace prediction)
-//       predict_columns_kernel  the same from a column table (columnar inplace prediction)
+//       predict_inplace_kernel  K2 with the tile assembled from a caller's rows or column table (inplace prediction)
 //   K6  shap_paths / shap_reduce / shap_approx   per-feature contributions (exact TreeSHAP, approximate Saabas)
 //       shap_inter / shap_inter_reduce / shap_inter_expand   SHAP interaction values (conditioned TreeSHAP)
 //   K1  oh_state / oh_sums / oh_pack    Run1 feature assembly (:1240-1257, :1441-1488, :303-345)
@@ -802,9 +801,9 @@ __global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_soa_kernel(D
   a.out[m] = export_transform(acc, a.exp10, a.scale);
 }
 
-// ---- inplace variant: the tile is assembled straight from a caller's dense float array ------------------------
-// (XGBoosterPredictFromDense / XGBoosterPredictFromCudaArray).  The same tile as predict_tiles_kernel walks — feature
-// slots of 1 KB, absent columns missing, the key-0 slot last — built in shared memory from the strided array, so no
+// ---- inplace variant: the tile is assembled straight from a caller's float array ----------------------------------
+// (XGBoosterPredictFromDense / FromCudaArray / FromCudaColumnar).  The same tile as predict_tiles_kernel walks — feature
+// slots of 1 KB, absent columns missing, the key-0 slot last — built in shared memory from the caller's values, so no
 // copy of the array and no key tiles go to HBM.  Rows keep their order: a warp takes the default-direction walk when
 // one of its 32 rows holds a missing entry, and MissingWalk serves it when Walk cannot walk missing entries.  Ranges
 // of trees are separate launches (the partial sum travels through `out` as in predict_tiles_kernel); each one
@@ -820,34 +819,18 @@ __device__ __forceinline__ uint32_t inplace_key(float x, float missing, bool chk
   return float_key(x);
 }
 
-// The rest of an inplace launch once the loader has put a tile's keys in slots 0..ncol-1, shared by predict_dense_kernel
-// and predict_columns_kernel: absent columns are missing, the key-0 slot goes last, the inf flag is voted, and each live
-// thread walks its row (the default-direction walk when one of the warp's rows holds a missing entry).
-template <class Walk, class MissingWalk>
-__device__ __forceinline__ void walk_inplace_tile(const DeviceForest &f, const PredictArgs &a, uint32_t *skey, int tid, uint64_t r0,
-                                                  bool live, int flags, int *flag_out) {
-  const int ncol = a.ncol;
-  for (int c = ncol; c < f.nfeat; ++c) skey[c * kStride + tid] = kKeyMissing;
-  skey[f.nfeat * kStride + tid] = 0u;
-  // __syncthreads_or returns a truth value, not the bitwise OR: one vote for the inf flag
-  if (__syncthreads_or(flags & 2) != 0) {
-    if (tid == 0) atomicOr(flag_out, 2);
-  }
-  const bool hm = __any_sync(0xffffffffu, flags & 1) || ncol < f.nfeat;
-  if (!live) return;
-  const uint32_t my = (uint32_t)__cvta_generic_to_shared(skey + tid);
-  row_result<false>(f, a, r0 + (uint64_t)tid, true, [&](auto &&emit) {
-    if (!hm)
-      Walk::template run<false, false>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
-    else if (Walk::walks_missing(f))
-      Walk::template run<true, false>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
-    else
-      MissingWalk::template run<true, false>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
-  });
-}
+// The inplace input of one launch: one C-contiguous [nrow][ncol] array at t.col[0] (`rows`), or a column table, element
+// (r, c) at t.col[c][r * t.stride[c]].  The table (31 x 16 B) travels in the kernel parameters.
+struct InplaceArgs {
+  int rows;
+  ColumnParams<kMaxFeatures> t;
+  float missing;
+  int *flags;  // |= 2 on +-inf input when `missing` is finite
+};
 
 template <class Walk, class MissingWalk>
-__global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_dense_kernel(DeviceForest f, PredictArgs a, DenseArgs d) {
+__global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_inplace_kernel(DeviceForest f, PredictArgs a,
+                                                                                    const __grid_constant__ InplaceArgs d) {
   extern __shared__ __align__(128) uint32_t skey[];
   const int tid = threadIdx.x, ncol = a.ncol;
   const uint64_t r0 = (uint64_t)blockIdx.x * kBlock;
@@ -857,12 +840,12 @@ __global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_dense_kernel
   const bool chk_inf = !isinf(d.missing);
   int flags = 0;
   auto key = [&](float x) { return inplace_key(x, d.missing, chk_inf, flags); };
-  if (d.col_stride == 1 && d.row_stride == ncol) {
-    // contiguous rows: one flat coalesced copy into a row-major staging area of odd stride (conflict-free per-thread
-    // row reads, as in seal_tiles_kernel) that aliases the key slots; each thread lifts its row through registers
+  if (d.rows) {
+    // one flat coalesced copy into a row-major staging area of odd stride (conflict-free per-thread row reads, as in
+    // seal_tiles_kernel) that aliases the key slots; each thread lifts its row through registers
     float *stage = reinterpret_cast<float *>(skey);
     const int ld = ncol | 1, n = nr * ncol;
-    const float *__restrict__ src = d.X + r0 * (uint64_t)ncol;
+    const float *__restrict__ src = d.t.col[0] + r0 * (uint64_t)ncol;
     if (ld == ncol && (((uintptr_t)src) & 15u) == 0u) {
       const float4 *s4 = reinterpret_cast<const float4 *>(src);
       float4 *d4 = reinterpret_cast<float4 *>(stage);
@@ -883,37 +866,28 @@ __global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_dense_kernel
     for (int c = 0; c < (int)kMaxFeatures; ++c)
       if (c < ncol) skey[c * kStride + tid] = k[c];
   } else {
-    // any other strides: element by element; a feature-major array is coalesced per feature
-    const float *__restrict__ src = d.X + (r0 + (uint64_t)tid) * d.row_stride;
-    for (int c = 0; c < ncol; ++c) skey[c * kStride + tid] = live ? key(__ldg(src + (int64_t)c * d.col_stride)) : 0u;
+    // element by element; a column of unit stride is coalesced
+    const int64_t r = (int64_t)(r0 + (uint64_t)tid);
+    for (int c = 0; c < ncol; ++c) skey[c * kStride + tid] = live ? key(__ldg(d.t.col[c] + r * d.t.stride[c])) : 0u;
   }
-  walk_inplace_tile<Walk, MissingWalk>(f, a, skey, tid, r0, live, flags, d.flags);
-}
-
-// ---- columnar inplace variant (XGBoosterPredictFromCudaColumnar): predict_dense_kernel's element-wise loader fed from a
-// column table, element (r, c) at col[c][r * stride[c]]; a column of unit stride is coalesced.  The table (31 x 16 B)
-// travels in the kernel parameters.
-struct ColumnsArgs {
-  ColumnParams<kMaxFeatures> t;
-  float missing;
-  int *flags;  // |= 2 on +-inf input when `missing` is finite
-};
-
-template <class Walk, class MissingWalk>
-__global__ void __launch_bounds__(kBlock, Walk::kMinBlocks) predict_columns_kernel(DeviceForest f, PredictArgs a,
-                                                                                    const __grid_constant__ ColumnsArgs d) {
-  extern __shared__ __align__(128) uint32_t skey[];
-  const int tid = threadIdx.x, ncol = a.ncol;
-  const uint64_t r0 = (uint64_t)blockIdx.x * kBlock;
-  const uint64_t left = a.nrow - r0;
-  const int nr = left < (uint64_t)kBlock ? (int)left : kBlock;
-  const bool live = tid < nr;
-  const bool chk_inf = !isinf(d.missing);
-  int flags = 0;
-  const int64_t r = (int64_t)(r0 + (uint64_t)tid);
-  for (int c = 0; c < ncol; ++c)
-    skey[c * kStride + tid] = live ? inplace_key(__ldg(d.t.col[c] + r * d.t.stride[c]), d.missing, chk_inf, flags) : 0u;
-  walk_inplace_tile<Walk, MissingWalk>(f, a, skey, tid, r0, live, flags, d.flags);
+  // absent columns are missing and the key-0 slot goes last
+  for (int c = ncol; c < f.nfeat; ++c) skey[c * kStride + tid] = kKeyMissing;
+  skey[f.nfeat * kStride + tid] = 0u;
+  // __syncthreads_or returns a truth value, not the bitwise OR: one vote for the inf flag
+  if (__syncthreads_or(flags & 2) != 0) {
+    if (tid == 0) atomicOr(d.flags, 2);
+  }
+  const bool hm = __any_sync(0xffffffffu, flags & 1) || ncol < f.nfeat;
+  if (!live) return;
+  const uint32_t my = (uint32_t)__cvta_generic_to_shared(skey + tid);
+  row_result<false>(f, a, r0 + (uint64_t)tid, true, [&](auto &&emit) {
+    if (!hm)
+      Walk::template run<false, false>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
+    else if (Walk::walks_missing(f))
+      Walk::template run<true, false>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
+    else
+      MissingWalk::template run<true, false>(f, my, a.ctree0, a.tree_begin, a.tree_end, emit);
+  });
 }
 
 // The layout rule of the predict launches: the two-level records when the window holds the record tops of trees
@@ -948,54 +922,36 @@ cudaError_t launch_predict_soa(const DeviceForest &f, const ConstWindow &w, cons
   return QC_LAUNCHED();
 }
 
-cudaError_t launch_predict_dense(const DeviceForest &f, const ConstWindow &w, const PredictArgs &args, const DenseArgs &d, cudaStream_t s) {
-  if (args.nrow == 0 || args.tree_end <= args.tree_begin) return cudaSuccess;
-  if (args.ncol > f.nfeat || f.nfeat > (int)kMaxFeatures || args.pred_leaf) return cudaErrorInvalidValue;
-  // the key slots 0..nfeat; the row-major staging area of the contiguous loader ((ncol | 1) KB) fits in them
-  const size_t smem = (size_t)kStride * (size_t)(f.nfeat + 1) * sizeof(uint32_t);
-  const uint64_t grid = tile_count(args.nrow);
-  if (grid > 0x7fffffffull) return cudaErrorInvalidConfiguration;
-  PredictArgs a = args;
-  a.ctree0 = w.tree0;
-  // as in launch_predict_soa: the layout of clean rows; the kernel sends a warp with missing entries the records cannot
-  // walk to the 8-byte nodes without the table
-  const Layout l = layout(f, w, a.tree_begin, a.tree_end, false);
-  auto k = predict_dense_kernel<RecordsWalk, NodesTexWalk>;
-  if (f.duo_shallow) k = predict_dense_kernel<RecordsShallowWalk, NodesTexWalk>;
-  if (l == Layout::kNodesTable) k = predict_dense_kernel<NodesTableWalk, NodesTableWalk>;
-  if (l == Layout::kNodesTex) k = predict_dense_kernel<NodesTexWalk, NodesTexWalk>;
-  if (l == Layout::kNodesLsu) k = predict_dense_kernel<NodesLsuWalk, NodesLsuWalk>;
-  cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return e;
-  k<<<dim3((unsigned)grid), kBlock, smem, s>>>(f, a, d);
-  count_predict(l == Layout::kRecords ? kDenseDuo : kDenseNodes8);
-  return QC_LAUNCHED();
-}
-
-cudaError_t launch_predict_columns(const DeviceForest &f, const ConstWindow &w, const PredictArgs &args, const float *const *col,
+cudaError_t launch_predict_inplace(const DeviceForest &f, const ConstWindow &w, const PredictArgs &args, bool rows, const float *const *col,
                                   const int64_t *stride, float missing, int *flags, cudaStream_t s) {
   if (args.nrow == 0 || args.tree_end <= args.tree_begin) return cudaSuccess;
   if (args.ncol > f.nfeat || f.nfeat > (int)kMaxFeatures || args.pred_leaf) return cudaErrorInvalidValue;
+  // the key slots 0..nfeat; the row-major staging area of the rows loader ((ncol | 1) KB) fits in them
   const size_t smem = (size_t)kStride * (size_t)(f.nfeat + 1) * sizeof(uint32_t);
   const uint64_t grid = tile_count(args.nrow);
   if (grid > 0x7fffffffull) return cudaErrorInvalidConfiguration;
   PredictArgs a = args;
   a.ctree0 = w.tree0;
-  ColumnsArgs d;
+  InplaceArgs d;
   memset(&d, 0, sizeof d);
-  for (int c = 0; c < a.ncol; ++c) d.t.col[c] = col[c], d.t.stride[c] = stride[c];
+  d.rows = rows ? 1 : 0;
+  if (rows) d.t.col[0] = col[0];
+  else
+    for (int c = 0; c < a.ncol; ++c) d.t.col[c] = col[c], d.t.stride[c] = stride[c];
   d.missing = missing, d.flags = flags;
-  // the layout rule and the instantiations of launch_predict_dense
+  // as in launch_predict_soa: the layout of clean rows; the kernel sends a warp with missing entries the records cannot
+  // walk to the 8-byte nodes without the table
   const Layout l = layout(f, w, a.tree_begin, a.tree_end, false);
-  auto k = predict_columns_kernel<RecordsWalk, NodesTexWalk>;
-  if (f.duo_shallow) k = predict_columns_kernel<RecordsShallowWalk, NodesTexWalk>;
-  if (l == Layout::kNodesTable) k = predict_columns_kernel<NodesTableWalk, NodesTableWalk>;
-  if (l == Layout::kNodesTex) k = predict_columns_kernel<NodesTexWalk, NodesTexWalk>;
-  if (l == Layout::kNodesLsu) k = predict_columns_kernel<NodesLsuWalk, NodesLsuWalk>;
+  auto k = predict_inplace_kernel<RecordsWalk, NodesTexWalk>;
+  if (f.duo_shallow) k = predict_inplace_kernel<RecordsShallowWalk, NodesTexWalk>;
+  if (l == Layout::kNodesTable) k = predict_inplace_kernel<NodesTableWalk, NodesTableWalk>;
+  if (l == Layout::kNodesTex) k = predict_inplace_kernel<NodesTexWalk, NodesTexWalk>;
+  if (l == Layout::kNodesLsu) k = predict_inplace_kernel<NodesLsuWalk, NodesLsuWalk>;
   cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   k<<<dim3((unsigned)grid), kBlock, smem, s>>>(f, a, d);
-  count_predict(l == Layout::kRecords ? kColumnsDuo : kColumnsNodes8);
+  if (l == Layout::kRecords) count_predict(rows ? kDenseDuo : kColumnsDuo);
+  else count_predict(rows ? kDenseNodes8 : kColumnsNodes8);
   return QC_LAUNCHED();
 }
 

@@ -100,20 +100,12 @@ cudaError_t launch_seal_columns(const float *const *col, const int64_t *stride, 
 
 cudaError_t launch_predict(const DeviceForest &f, const ConstWindow &w, const PredictArgs &a, cudaStream_t s);
 
-// Inplace prediction from a dense float array (XGBoosterPredictFromDense / FromCudaArray): row r, column c of the
-// array is X[r * row_stride + c * col_stride].  The predict kernel builds its key tiles from it in shared memory
-// (value / margin sums only); PredictArgs::Xt and has_missing are not read.
-struct DenseArgs {
-  const float *X = nullptr;  // device
-  int64_t row_stride = 0;    // in floats
-  int64_t col_stride = 1;
-  float missing = -999.f;    // entries that are NaN or == missing are missing
-  int *flags = nullptr;      // |= 2 on +-inf input when `missing` is finite
-};
-cudaError_t launch_predict_dense(const DeviceForest &f, const ConstWindow &w, const PredictArgs &a, const DenseArgs &d, cudaStream_t s);
-// The same from a column table (XGBoosterPredictFromCudaColumnar): element (r, c) is col[c][r * stride[c]], as for
-// launch_seal_columns; at most kMaxFeatures columns.
-cudaError_t launch_predict_columns(const DeviceForest &f, const ConstWindow &w, const PredictArgs &a, const float *const *col,
+// Inplace prediction from a caller's device values (XGBoosterPredictFromDense / FromCudaArray / FromCudaColumnar):
+// `rows`, one C-contiguous [nrow][ncol] array at col[0] (stride is not read), else a column table, element (r, c) at
+// col[c][r * stride[c]] as for launch_seal_columns, at most kMaxFeatures columns.  The predict kernel builds its key
+// tiles from it in shared memory (value / margin sums only); PredictArgs::Xt and has_missing are not read.  Entries
+// that are NaN or == missing are missing; flags[0] |= 2 on +-inf input when `missing` is finite.
+cudaError_t launch_predict_inplace(const DeviceForest &f, const ConstWindow &w, const PredictArgs &a, bool rows, const float *const *col,
                                    const int64_t *stride, float missing, int *flags, cudaStream_t s);
 
 // Per-feature contributions (forest.hpp ShapForest).  out: [nrow][nfeat + 1] floats, column nfeat = `bias`.

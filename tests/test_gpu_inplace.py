@@ -1,7 +1,8 @@
-"""Inplace prediction on the GPU (XGBoosterPredictFromDense / XGBoosterPredictFromCudaArray, predict_dense_kernel): the
+"""Inplace prediction on the GPU (XGBoosterPredictFromDense / XGBoosterPredictFromCudaArray, predict_inplace_kernel): the
 margins are bit-equal to the C oracle's and to XGDMatrixCreateFromMat + XGBoosterPredictFromDMatrix on the same array
 and `missing`, for every layout of the array, both node layouts (duo_mode), forests that need several tree ranges and
-the host path's chunked copy; the dense families serve, and no key tiles are sealed."""
+the host path's chunked copy; the dense families serve C-contiguous arrays and the columns families any other layout,
+and no key tiles are sealed."""
 import ctypes as C
 
 import numpy as np
@@ -111,6 +112,11 @@ def test_layouts_of_the_array_give_the_same_bits(gpu, oracle, small_model_path, 
         for name, (dev, strides, offset) in layouts.items():
             got = b.inplace_predict(dev, shape=(n, nc), strides=strides, offset=offset)
             assert np.array_equal(_u32(got), ref), (name, nc)
+            if n:
+                # C-contiguous (row-major, and offset by one float: a base that is not 16-byte aligned) takes the rows
+                # loader; any other strides the column table
+                loader = "dense" if name in ("row-major", "offset by one float") else "columns"
+                assert gpu.last_predict_kernel() == loader + ("_duo" if duo_mode else "_nodes8"), (name, nc)
             dev.free()
 
 
