@@ -897,9 +897,23 @@ struct PathElem {
 
 uint32_t threshold_key(float thr) { return 0u - neg_threshold_key(thr); }
 
-void collect_paths(const HostTree &t, int32_t n, std::vector<PathElem> &path,
+// The kernels keep an element's one fraction in the sign of its float32 zero fraction, so every stored zero fraction
+// must be a positive, finite float32; covers that are each finite and positive can still multiply past that range.
+void collect_paths(size_t ti, const HostTree &t, int32_t n, std::vector<PathElem> &path,
                    std::vector<std::pair<std::vector<PathElem>, float>> &out) {
   if (t.cleft[n] == -1) {
+    for (const PathElem &e : path) {
+      const float z = (float)e.zero;
+      if (!(z > 0.f) || !std::isfinite(z)) {
+        char msg[320];
+        snprintf(msg, sizeof msg,
+                 "contributions need every path's product of cover(child) / cover(parent) over the splits on one "
+                 "feature to be a positive, finite float32, but tree %zu leaf %d has %g on feature %u: this booster "
+                 "cannot be explained",
+                 ti, n, e.zero, e.feat);
+        fail(msg);
+      }
+    }
     out.emplace_back(path, t.info[n]);
     return;
   }
@@ -916,7 +930,7 @@ void collect_paths(const HostTree &t, int32_t n, std::vector<PathElem> &path,
     else p[i].hi = std::min(p[i].hi, k);
     p[i].miss &= (dl == (side == 0)) ? 1u : 0u;
     p[i].zero *= (double)t.sum_hess[c] / (double)t.sum_hess[n];
-    collect_paths(t, c, p, out);
+    collect_paths(ti, t, c, p, out);
   }
 }
 }  // namespace
@@ -938,7 +952,7 @@ ShapForest build_shap(const HostForest &h, const FlatForest &f) {
     for (uint32_t i = n0; i < f.tree_offset[ti + 1]; ++i) s.mean[i] = m[(size_t)f.orig_id[i]];
     std::vector<std::pair<std::vector<PathElem>, float>> paths;
     std::vector<PathElem> root;
-    collect_paths(t, 0, root, paths);
+    collect_paths(ti, t, 0, root, paths);
     // first-fit decreasing into 32-lane bins; lengths include the bias element (<= kMaxFeatures + 1 = 32)
     std::vector<size_t> order(paths.size());
     for (size_t i = 0; i < order.size(); ++i) order[i] = i;

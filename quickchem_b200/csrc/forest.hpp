@@ -117,7 +117,8 @@ struct ShapForest {
   std::vector<uint32_t> feat_bins;
   int64_t num_bins() const { return (int64_t)(bins.size() / 128); }
 };
-// Throws unless every node of every tree has a finite, positive cover (sum_hess).
+// Throws unless every node of every tree has a finite, positive cover (sum_hess) and every merged zero fraction is a
+// positive, finite float32.
 ShapForest build_shap(const struct HostForest &h, const struct FlatForest &f);
 // Fills s.feat_off / s.feat_bins for features [0, nfeat).
 void build_shap_by_feature(ShapForest &s, uint32_t nfeat);
